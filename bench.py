@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- filtered observation-steps/s (N x K per second) of the batched CD-EKF hot path on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -22,6 +22,13 @@ communicator).  Trajectories are independent and shard with no data-path collect
 `--impl reference`: the CPU restatement of the reference algorithm (oracle/, C + OpenMP, all host cores) on a bounded
             sample of the same workload.  The reference's own JAX path cannot run here (jax/diffrax are not
             installable in this image; BASELINE.md section 2) -- this is a "CPU restatement (not JAX)".
+`--dump-outputs DIR`: after the timed steps, write what the last timed step returned as DIR/<name>.npy (float64): the
+            per-trajectory outputs of the posterior (marginal_loglik, filtered/predicted means and covariances) for a
+            fixed, seeded sample of rank 0's trajectories, at most 60 MB in all, and ll_sum, the summed log-likelihood
+            of the whole batch.  The inputs depend on the arguments only, so two builds run with the same arguments can
+            be compared output for output.
+
+The benchmark writes nothing into the source tree, which may be read-only.
 """
 import argparse
 import ctypes
@@ -36,6 +43,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # no __pycache__ in the source tree
 
 METRIC = "filtered observation-steps/sec (N x K per second)"
 UNIT = "obs-steps/s"
@@ -68,7 +76,12 @@ def parse():
     ap.add_argument("--simple-data", action="store_true",
                     help="emissions = 8*randn instead of a simulated Lorenz-63 truth (profiling runs: skips the "
                          "~100k setup launches that would otherwise sit in front of the profiled kernel)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step to DIR/<name>.npy (see the module docstring)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 def l63(x, s=10.0, r=28.0, b=8.0 / 3.0):
@@ -312,7 +325,8 @@ def make_times_rows(first, count, K, seed, block=8192):
 
 def time_resident(job, args, steps, ctx):
     """W warm-up passes, then `steps` passes through the public API with resident inputs, bracketed by barrier + sync;
-    CUDA events on the launching stream, max over ranks.  Returns (ms total, launches, ll_total, non-finite count, clocks)."""
+    CUDA events on the launching stream, max over ranks.  Returns (ms total, launches, ll_total, non-finite count, clocks,
+    (posterior, summed log-likelihood) of the last timed pass)."""
     import torch
     import cd_dynamax_b200 as cd
     from cd_dynamax_b200 import _engine as E
@@ -342,8 +356,8 @@ def time_resident(job, args, steps, ctx):
     ctx["barrier"]()
     e0.record()
     for _ in range(steps):
+        post = None  # the previous pass's outputs are freed before this pass allocates its own
         post, s = step()
-        del post
     e1.record()
     ctx["barrier"]()
     launches = lib.cdk_launch_count() - launches0
@@ -351,7 +365,27 @@ def time_resident(job, args, steps, ctx):
     if world > 1:
         dist.all_reduce(tmax, op=dist.ReduceOp.MAX)
     clocks = sampler.stop() if rank == 0 else None
-    return float(tmax.item()), int(launches), ll_total, n_bad, clocks
+    return float(tmax.item()), int(launches), ll_total, n_bad, clocks, (post, s)
+
+
+DUMP_BYTES = 60_000_000
+
+
+def dump_outputs(out_dir, post, ll_sum, seed=CFG["seed"]):
+    """Write the outputs of one timed pass as out_dir/<name>.npy: ll_sum, and every per-trajectory field of the posterior
+    for the same sample of trajectories (all of them when they fit in DUMP_BYTES, else a sorted sample drawn with a fixed
+    seed, so that it depends on the batch size only)."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    fields = {k: v for k, v in post._asdict().items() if v is not None}
+    n = fields["marginal_loglik"].shape[0]
+    row_bytes = sum(v[:1].numel() * v.element_size() for v in fields.values())
+    rows = min(n, DUMP_BYTES // row_bytes)
+    idx = np.sort(np.random.default_rng(seed).choice(n, size=rows, replace=False)) if rows < n else np.arange(n)
+    sel = torch.as_tensor(idx, device=fields["marginal_loglik"].device)
+    for name, v in fields.items():
+        np.save(os.path.join(out_dir, name + ".npy"), v.index_select(0, sel).cpu().numpy())
+    np.save(os.path.join(out_dir, "ll_sum.npy"), ll_sum.cpu().numpy())
 
 
 def time_kernel(job, ctx, reps=7):
@@ -509,7 +543,10 @@ def run_ours(args):
 
     # ---- headline mode ----
     job, n_total = make_job(args.scaling)
-    total_ms, launches, ll_total, n_bad, clocks = time_resident(job, args, args.steps, ctx)
+    total_ms, launches, ll_total, n_bad, clocks, (post, s) = time_resident(job, args, args.steps, ctx)
+    if args.dump_outputs and rank == 0 and post is not None:
+        dump_outputs(args.dump_outputs, post, s)
+    del post, s
     kernel_ms = time_kernel(job, ctx)
     e2e_ms, e2e_steps, h2d, d2h, _, ll_host = time_e2e(job, args, ctx)
     e2e_ok = None
@@ -533,7 +570,7 @@ def run_ours(args):
         del job.y_dev, job.t_dev
         torch.cuda.empty_cache()
         job2, n_total2 = make_job(other_mode)
-        o_ms, o_launches, o_ll, o_bad, _ = time_resident(job2, args, args.steps, ctx)
+        o_ms, o_launches, o_ll, o_bad = time_resident(job2, args, args.steps, ctx)[:4]
         o_kernel_ms = time_kernel(job2, ctx)
         other = {"scaling": other_mode, "n_traj_total": n_total2, "n_traj_per_gpu": job2.N,
                  "value": n_total2 * K * args.steps / (o_ms * 1e-3), "unit": UNIT, "ms_per_step": o_ms / args.steps,

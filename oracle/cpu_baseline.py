@@ -2,41 +2,52 @@
 import ctypes
 import os
 import subprocess
+import tempfile
 import time
 
 import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
+SRC = os.path.join(HERE, "cd_oracle_c.c")
 SO = os.path.join(HERE, "_build", "libcdoracle.so")
 SOLVER_IDS = {"euler": 0, "heun": 1, "midpoint": 2, "ralston": 3, "bosh3": 4, "rk4": 5, "dopri5": 6}
 _lib = None
+_so = None  # the library load() opened
 
 
-def build(force=False):
-    """gcc -O3 -march=native -fopenmp. -march=native binds the .so to the build host's ISA, so the GPU box rebuilds it
-    on first use if the CPU differs (see load())."""
-    src = os.path.join(HERE, "cd_oracle_c.c")
-    if force or not os.path.exists(SO) or os.path.getmtime(SO) < os.path.getmtime(src):
-        # the image exports CC=/opt/gcc/bin/gcc, which lacks libgomp; prefer the distro gcc, fall back to serial
+def _fresh(so):
+    """The library at `so` is newer than the source and was built on a CPU of this model (see build())."""
+    try:
+        return os.path.getmtime(so) >= os.path.getmtime(SRC) and open(so + ".host").read() == _host_tag()
+    except OSError:
+        return False
+
+
+def build(force=False, out_dir=os.path.dirname(SO)):
+    """gcc -O3 -march=native -fopenmp into out_dir/libcdoracle.so.  -march=native binds the .so to the build host's ISA,
+    so a marker next to it records the CPU model it was built on, and load() rebuilds it if the CPU differs."""
+    so = os.path.join(out_dir, "libcdoracle.so")
+    if force or not _fresh(so):
+        # an exported CC may name a compiler without libgomp: prefer the system gcc, fall back to a serial build
         cc = "/usr/bin/gcc" if os.path.exists("/usr/bin/gcc") else "gcc"
-        r = subprocess.run(["make", "-C", HERE, "-B", "_build/libcdoracle.so", f"CC={cc}"], capture_output=True, text=True)
+        make = ["make", "-C", HERE, "-B", f"BUILD={out_dir}", so, f"CC={cc}"]
+        r = subprocess.run(make, capture_output=True, text=True)
         if r.returncode != 0:
-            r = subprocess.run(["make", "-C", HERE, "-B", "_build/libcdoracle.so", f"CC={cc}",
-                                "CFLAGS=-O3 -fPIC -std=gnu11"], capture_output=True, text=True)
+            r = subprocess.run(make + ["CFLAGS=-O3 -fPIC -std=gnu11"], capture_output=True, text=True)
         if r.returncode != 0:
             raise RuntimeError("building oracle/cd_oracle_c.c failed:\n" + r.stdout + r.stderr)
-    return SO
+        with open(so + ".host", "w") as f:
+            f.write(_host_tag())
+    return so
 
 
 def load():
-    global _lib
+    """Open the library build() left in the tree; if it is missing or was built for another CPU, build a private copy in
+    the temporary directory instead, so that a read-only checkout works too."""
+    global _lib, _so
     if _lib is None:
-        marker = SO + ".host"
-        host = _host_tag()
-        stale = not os.path.exists(marker) or open(marker).read() != host
-        build(force=stale)
-        open(marker, "w").write(host)
-        L = ctypes.CDLL(SO)
+        _so = SO if _fresh(SO) else build(out_dir=os.path.join(tempfile.gettempdir(), f"cd_oracle_{os.getuid()}"))
+        L = ctypes.CDLL(_so)
         dp, i, ll, d = ctypes.c_void_p, ctypes.c_int, ctypes.c_longlong, ctypes.c_double
         L.cdo_filter.argtypes = [i, ll, i, i, i, i, i, d, d, i, i] + [dp] * 11 + [dp] * 5 + [i]
         L.cdo_filter.restype = ll
@@ -47,7 +58,7 @@ def load():
 
 def _has_openmp():
     try:
-        return b"GOMP" in open(SO, "rb").read()
+        return b"GOMP" in open(_so, "rb").read()
     except OSError:
         return False
 
