@@ -16,6 +16,7 @@ _NP_DT = {"f64": np.float64, "f32": np.float32}
 # core (per-trajectory) rank of every input slot
 _CORE_NDIM = {L.IN_Y: 2, L.IN_T: 1, L.IN_U: 2, L.IN_M0: 1, L.IN_P0: 2, L.IN_F: None, L.IN_B: 1, L.IN_BU: 2,
               L.IN_L: 2, L.IN_QC: 2, L.IN_H: 2, L.IN_D: 1, L.IN_DU: 2, L.IN_R: 2, L.IN_FM: 2, L.IN_FP: 3}
+_SLOT_NAMES = {L.IN_Y: "IN_Y", L.IN_T: "IN_T", L.IN_U: "IN_U"}
 
 
 def device():
@@ -114,9 +115,11 @@ def run(entry: str, dt: str, N: int, K: int, n: int, m: int, inputs: Dict[int, o
         desc_fields: dict, theta_core_ndim: int = 1, scross_rows: Optional[int] = None,
         status: Optional[torch.Tensor] = None, host_out: bool = False,
         dev_inputs: Optional[dict] = None, scratch: Optional[torch.Tensor] = None,
-        core_ndim_override: Optional[dict] = None, t_cols: Optional[int] = None,
+        core_ndim_override: Optional[dict] = None,
         out_shapes: Optional[dict] = None) -> Dict[int, torch.Tensor]:
     """Call one C-ABI entry point. `inputs` maps slot -> array-like (None = absent); a leading N marks it batched.
+    The time stamps, emissions and inputs must have the per-trajectory shapes [K] ([K + 1] for a forecast or a sampler
+    from a fixed initial state), [K, m] and [K, d_u]; anything else raises ValueError before any device work.
     Returns slot -> tensor for every slot in `want` (+ OUT_STATUS): device tensors, or -- with `host_out`, which the
     API shims set when the caller handed in host arrays -- pinned host tensors whose copies have completed.
     `dev_inputs`, when given, receives slot -> staged device tensor (a smoother reuses the filter's staged inputs).
@@ -124,21 +127,14 @@ def run(entry: str, dt: str, N: int, K: int, n: int, m: int, inputs: Dict[int, o
     (cdk_scratch_bytes, sized per trajectory) it is allocated here -- or taken from `scratch`, which is how the type-1
     smoother gets the pushforward cache its filter wrote -- and returned as out[OUT_SCRATCH]."""
     desc_fields = dict(desc_fields)
-    lib = L.lib(desc_fields.pop("lib_path", None))  # a variant library for a user-defined drift, else the stock one
-    dev = device()
-    d = L.new_desc()
-    d.N, d.K, d.n, d.m = N, K, n, m
-    for k, v in desc_fields.items():
-        if k == "flags":
-            d.reserved[2] = int(v)
-        elif k == "grad_groups":
-            d.reserved[3] = int(v)
-        else:
-            setattr(d, k, v)
     tdt = _TORCH_DT[dt]
     esz = 8 if dt == "f64" else 4
-    cur = torch.cuda.current_stream(dev)
-    # ---- classify inputs; decide whether to stream host-resident batched inputs in chunks ----
+    # ---- classify inputs (before any device work: a mis-shaped batch is rejected here, not read out of bounds) ----
+    # per-trajectory shapes of the slots whose extent depends on K: a forecast and a sampler started from a fixed state
+    # read K + 1 time stamps (t_init first), every other entry point K (slot_elems, cdk_api.cu)
+    flags = int(desc_fields.get("flags", 0))
+    t_cols = K + 1 if flags & (L.FLAG_PREDICT_ONLY | L.FLAG_FIXED_INIT) else K
+    core_shape = {L.IN_T: (t_cols,), L.IN_Y: (K, m), L.IN_U: (K, int(desc_fields.get("d_u", 0)))}
     metas = {}
     stream_bytes = 0
     mask = 0
@@ -146,7 +142,7 @@ def run(entry: str, dt: str, N: int, K: int, n: int, m: int, inputs: Dict[int, o
         x = inputs.get(slot)
         if x is None:
             continue
-        shape = tuple(x.shape) if hasattr(x, "shape") else tuple(np.shape(x))
+        shape = full_shape = tuple(x.shape) if hasattr(x, "shape") else tuple(np.shape(x))
         core = _CORE_NDIM[slot] if _CORE_NDIM[slot] is not None else theta_core_ndim
         if core_ndim_override and slot in core_ndim_override:
             core = core_ndim_override[slot]  # e.g. IN_R as the [m] diagonal (CDK_FLAG_DIAG_R)
@@ -161,11 +157,26 @@ def run(entry: str, dt: str, N: int, K: int, n: int, m: int, inputs: Dict[int, o
             mask |= 1 << slot
         elif len(shape) != core:
             raise ValueError(f"input slot {slot}: expected rank {core} or {core + 1}, got shape {shape}")
+        if slot in core_shape and tuple(shape[1:] if batched else shape) != core_shape[slot]:
+            raise ValueError(f"input slot {_SLOT_NAMES[slot]}: per-trajectory shape {tuple(shape[1:] if batched else shape)} "
+                             f"!= {core_shape[slot]} (full shape {full_shape}, N={N}, K={K})")
         row = int(np.prod(shape[1:], dtype=np.int64)) if batched else 0
         host = _is_host(x)
         metas[slot] = (x, batched, row, host)
         if batched and host:
             stream_bytes += N * row * esz
+    lib = L.lib(desc_fields.pop("lib_path", None))  # a variant library for a user-defined drift, else the stock one
+    dev = device()
+    d = L.new_desc()
+    d.N, d.K, d.n, d.m = N, K, n, m
+    for k, v in desc_fields.items():
+        if k == "flags":
+            d.reserved[2] = int(v)
+        elif k == "grad_groups":
+            d.reserved[3] = int(v)
+        else:
+            setattr(d, k, v)
+    cur = torch.cuda.current_stream(dev)
     d.batched_mask = mask
     nchunks = STREAM_CHUNKS if (stream_bytes >= STREAM_MIN_BYTES and N >= 2 * STREAM_CHUNKS) else 1
     if host_out and N >= 2 * STREAM_CHUNKS:

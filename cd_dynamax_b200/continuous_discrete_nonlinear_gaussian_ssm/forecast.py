@@ -105,7 +105,7 @@ def cdnlgssm_forecast(params, init_forecast, t_init, t_forecast=None, hyperparam
         want.append(L.OUT_PM)
     if output_fields is None or "forecasted_state_covariances" in output_fields:
         want.append(L.OUT_PP)
-    out = E.run(entry, dt, N, K, n, m, ins, want, fields, host_out=(kind != "cuda"), t_cols=K + 1)
+    out = E.run(entry, dt, N, K, n, m, ins, want, fields, host_out=(kind != "cuda"))
     g = lambda s: E.from_dev(_sq(out[s], batched), kind) if s in out else None
     return GSSMForecast(forecasted_state_means=g(L.OUT_PM), forecasted_state_covariances=g(L.OUT_PP))
 
@@ -125,7 +125,7 @@ def _sample(params, m0, P0, T, N, K, fixed, key, diffeqsolve_settings, kind, dt,
                   rng_offset=int(rng_offset), flags=L.FLAG_FIXED_INIT if fixed else 0)
     want = ([L.OUT_FM] if want_states else []) + ([L.OUT_PM] if want_emissions else [])
     out = E.run("cdk_sample_path", dt, N, K, n, m, ins, want, fields, host_out=(kind != "cuda"),
-                t_cols=K + 1 if fixed else K, out_shapes={L.OUT_PM: (N, K, m)})
+                out_shapes={L.OUT_PM: (N, K, m)})
     g = lambda s: E.from_dev(_sq(out[s], batched), kind) if s in out else None
     return g(L.OUT_FM), g(L.OUT_PM)
 

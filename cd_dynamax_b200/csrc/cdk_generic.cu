@@ -1242,7 +1242,8 @@ __global__ void generic_smooth_kernel(const GArgs<T> g) {
     int* st = static_cast<int*>(a.out[CDK_OUT_STATUS]);
     bool bad = false;
     for (int i = 0; i < n; ++i) bad |= !isfinite(ms[i]);
-    if (status == 0 && bad) status = 1;
+    // NaN smoothed moments after a filter that hit max_steps are that failure, not a new one: keep the filter's status
+    if (status == 0 && bad && st[traj] == 0) status = 1;
     if (status != 0) st[traj] = status;  // keep the filter's status unless the backward pass adds a failure
   }
 }

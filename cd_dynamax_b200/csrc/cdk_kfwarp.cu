@@ -197,6 +197,20 @@ __device__ __forceinline__ bool pushforward(const KwTab& tab, const double dt0, 
       __syncwarp();
       mm<false, false, 16, 2, 2>(accA.v, sRk, sYA);
       __syncwarp();
+      // the substep is tnext - tprev = fl(tprev + dt0) - tprev, which differs from dt0 by up to half an ulp of t: 1.8e-12
+      // at t = 1e4, i.e. 7e-10 of dt0 = 0.0025, and the reference steps with that length.  Rk(dt) = Rk(dt0) + (dt - dt0) F
+      // Rk(dt0) + O(dt0^S (dt - dt0)): one more product restores it.  Below 2^-40 dt0 the term is under 2^-40 dt0 |F| of A
+      // per step and the product is skipped, so grids at moderate t keep the one-product step.
+      const double ddt = dt - dt0;
+      if (fabs(ddt) > 0x1p-40 * dt0) {
+        F16 fa;
+        store_c<2, 2>(accA.v, sYA);
+        __syncwarp();
+        mm<false, false, 16, 2, 2>(fa.v, sF, sYA);
+        __syncwarp();
+#pragma unroll
+        for (int i = 0; i < 8; ++i) (&accA.v[0][0][0])[i] = fma(ddt, (&fa.v[0][0][0])[i], (&accA.v[0][0][0])[i]);
+      }
     }
     if constexpr (POLY) {
       // Horner evaluation of the step polynomial (see KwTab): v = L y + g, w = c_S v, w = c_j v + dt L w (j = S-1 .. 1),
@@ -846,7 +860,8 @@ __global__ void __launch_bounds__(32 * KS_WPC, 2) kf_warp_smooth(const KArgs<dou
   if (lane == 0 && a.out[CDK_OUT_STATUS]) {
     bool bad = false;
     for (int i = 0; i < n; ++i) bad |= !isfinite(sms[i]);
-    if (status == 0 && bad) status = 1;
+    // NaN smoothed moments after a filter that hit max_steps are that failure, not a new one: keep the filter's status
+    if (status == 0 && bad && static_cast<int*>(a.out[CDK_OUT_STATUS])[traj] == 0) status = 1;
     if (status != 0) static_cast<int*>(a.out[CDK_OUT_STATUS])[traj] = status;  // keep the filter's status otherwise
   }
 }

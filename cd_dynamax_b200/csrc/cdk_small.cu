@@ -1153,7 +1153,8 @@ __global__ void __launch_bounds__(32 * 14, 1) eks_small_lw(const KArgs<T> a, con
     bool bad = false;
 #pragma unroll
     for (int i = 0; i < NX; ++i) bad |= !isfinite(s.m[i]);
-    if (status == 0 && bad) status = 1;
+    // NaN smoothed moments after a filter that hit max_steps are that failure, not a new one: keep the filter's status
+    if (status == 0 && bad && static_cast<int*>(a.out[CDK_OUT_STATUS])[traj] == 0) status = 1;
     if (status != 0) static_cast<int*>(a.out[CDK_OUT_STATUS])[traj] = status;  // keep the filter's status otherwise
   }
 }

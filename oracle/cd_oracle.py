@@ -67,6 +67,16 @@ class SolverSettings:
     solver: str = "dopri5"  # reference default for ODEs (diffrax_utils.py:121-124)
     dt0: float = 0.01  # diffrax_utils.py:50
     max_steps: int = 100000  # diffrax_utils.py:52
+    # dtype of the stepping (times, dt0, clip tolerance); None = the dtype of the state.  np.float32 with an fp64 state
+    # takes exactly the substeps an fp32 run takes (fp32 times, tol 1e-6) with fp64 arithmetic, so that a comparison
+    # with the fp32 kernels measures arithmetic precision alone.
+    time_dtype: Optional[type] = None
+
+
+def _stepping(settings: SolverSettings, dtype):
+    """(time dtype, dt0, tol) of the diffrax stepping rule for a state of `dtype`."""
+    tdt = np.dtype(settings.time_dtype if settings.time_dtype is not None else dtype)
+    return tdt, tdt.type(settings.dt0), tdt.type(_tol_for(tdt))
 
 
 def _tol_for(dtype) -> float:
@@ -101,10 +111,9 @@ def rk_solve(rhs: Callable, t0, t1, y0: Sequence[np.ndarray], settings: SolverSe
     tab = TABLEAUX[settings.solver]
     a, b = tab["a"], tab["b"]
     dtype = y0[0].dtype
-    t0 = np.asarray(t0, dtype)
-    t1 = np.asarray(t1, dtype)
-    dt0 = dtype.type(settings.dt0)
-    tol = dtype.type(_tol_for(dtype))
+    tdt, dt0, tol = _stepping(settings, dtype)
+    t0 = np.asarray(t0, tdt)
+    t1 = np.asarray(t1, tdt)
     y = tuple(np.array(c, dtype, copy=True) for c in y0)
     tprev = t0.copy()
     tnext = np.minimum(t0 + dt0, t1)
@@ -123,7 +132,8 @@ def rk_solve(rhs: Callable, t0, t1, y0: Sequence[np.ndarray], settings: SolverSe
             tprev = np.where(over, t1, tprev)  # abandon those lanes
         if not active.any():
             break
-        dt = np.where(active, tnext - tprev, dtype.type(0))
+        dt = np.where(active, tnext - tprev, tdt.type(0)).astype(dtype)
+        tp = tprev.astype(dtype)
         ks = []
         for i in range(len(b)):
             yi = y
@@ -133,7 +143,7 @@ def rk_solve(rhs: Callable, t0, t1, y0: Sequence[np.ndarray], settings: SolverSe
                     for ci, c in enumerate(y)
                 )
             ci_t = dtype.type(sum(a[i])) if i > 0 else dtype.type(0)
-            fi = rhs(tprev + ci_t * dt, yi)
+            fi = rhs(tp + ci_t * dt, yi)
             ks.append(tuple(bc(dt, f) * f for f in fi))
         ynew = tuple(
             c + sum(dtype.type(b[j]) * ks[j][ci] for j in range(len(b)) if b[j] != 0.0) for ci, c in enumerate(y)
@@ -493,7 +503,7 @@ def cdlgssm_smoother(
                 return (-dm, -dP)  # reverse_rhs, diffrax_utils.py:13-25
 
             # :688 passes NO diffeqsolve settings -> always the defaults; integrate s in [0, t1-t0] (:131-135)
-            (ms, Ps), _, _ = rk_solve(rhs, np.zeros_like(t0), t1 - t0, (ms, Ps), SolverSettings())
+            (ms, Ps), _, _ = rk_solve(rhs, np.zeros_like(t0), t1 - t0, (ms, Ps), SolverSettings(time_dtype=settings.time_dtype))
             cross[:, k] = np.nan  # :792
         else:
             raise ValueError(smoother_type)
@@ -841,8 +851,7 @@ def ensemble_kalman_filter(
     )
     ll = np.zeros(N, dtype)
     status = np.zeros(N, np.int32)
-    dt0 = np.dtype(dtype).type(settings.dt0)
-    tol = np.dtype(dtype).type(_tol_for(dtype))
+    tdt, dt0, tol = _stepping(settings, dtype)
     Em1 = np.dtype(dtype).type(E - 1)
 
     def moments(Z):
@@ -876,8 +885,8 @@ def ensemble_kalman_filter(
         else:
             X, ll, mf, Pf = update(X, k, ll)
         # _predict :47-89 -- per-member SDE solve over the gap
-        tprev = t0s[:, k].copy()
-        t1 = t1s[:, k]
+        tprev = t0s[:, k].astype(tdt)
+        t1 = t1s[:, k].astype(tdt)
         tnext = np.minimum(tprev + dt0, t1)
         sub = 0
         nst = np.zeros(N, np.int64)
@@ -939,8 +948,7 @@ def sample_paths(p: NonlinearParams, t, seed=0, rng_offset=0, settings=SolverSet
     cholR = cholesky(R)
     traj = np.arange(N)
     m0 = c(p.m0, 1)
-    dt0 = np.dtype(dtype).type(settings.dt0)
-    tol = np.dtype(dtype).type(_tol_for(dtype))
+    tdt, dt0, tol = _stepping(settings, dtype)
     xs, ys = np.zeros((N, K, n), dtype), np.zeros((N, K, mdim), dtype)
 
     def emit(x, row, step):
@@ -955,8 +963,8 @@ def sample_paths(p: NonlinearParams, t, seed=0, rng_offset=0, settings=SolverSet
         x = m0 + _mv(cholesky(c(p.P0, 2)), z)
         emit(x, 0, 0)
     for k in range(0 if fixed_init else 1, K):
-        tprev = (t[:, k] if fixed_init else t[:, k - 1]).copy()
-        t1 = t[:, k + 1] if fixed_init else t[:, k]
+        tprev = (t[:, k] if fixed_init else t[:, k - 1]).astype(tdt)
+        t1 = (t[:, k + 1] if fixed_init else t[:, k]).astype(tdt)
         tnext = np.minimum(tprev + dt0, t1)
         sub = 0
         nst = np.zeros(N, np.int64)

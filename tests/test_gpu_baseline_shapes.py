@@ -386,8 +386,8 @@ def test_c2_full_size_sharding_invariance_and_oracle_sample():
     assert e < TOL
 
 
-# ---- fp32 entry points: one stated bound each (oracle in fp64 on the fp32-rounded inputs, so the comparison isolates the
-# ---- arithmetic precision).  The reference's own fp32 "match" ladder is 1e-5 .. 1e-4 on well-conditioned linear models
+# ---- fp32 entry points: one stated bound each (oracle in fp64 on the fp32-rounded inputs, stepping on fp32 times with the
+# ---- fp32 tolerance -- the substeps the fp32 kernels take -- so the comparison isolates the arithmetic precision).  The reference's own fp32 "match" ladder is 1e-5 .. 1e-4 on well-conditioned linear models
 # ---- (test_utils.py:160-180); chaotic drifts amplify rounding by e^{lambda t}.
 def _f32(*arrs):
     return [np.asarray(a, np.float32) for a in arrs]
@@ -407,7 +407,7 @@ def test_fp32_kf_filter_and_smoothers_bound():
     hp = cd.KFHyperParams(dt_final=0.01, diffeqsolve_settings={"solver": "rk4", "dt0": 0.01})
     g32 = {k: (v if v is None else np.asarray(v, np.float32)) for k, v in g.items()}
     r = o.cdlgssm_smoother(po, _as64(y32), _as64(t32), dt_final=float(np.float32(0.01)),
-                           settings=o.SolverSettings("rk4", float(np.float32(0.01))))
+                           settings=o.SolverSettings("rk4", float(np.float32(0.01)), time_dtype=np.float32))
     for stype in ("cd_smoother_1", "cd_smoother_2"):
         s = cd.cdlgssm_smoother(linear_params_api(g32), y32, t32[..., None], hp, smoother_type=stype)
         assert s.smoothed_means.dtype == np.float32
@@ -416,7 +416,7 @@ def test_fp32_kf_filter_and_smoothers_bound():
         assert e < 2e-4
         r2 = r if stype == "cd_smoother_1" else o.cdlgssm_smoother(
             po, _as64(y32), _as64(t32), dt_final=float(np.float32(0.01)),
-            settings=o.SolverSettings("rk4", float(np.float32(0.01))), smoother_type=2)
+            settings=o.SolverSettings("rk4", float(np.float32(0.01)), time_dtype=np.float32), smoother_type=2)
         for fld in ("filtered_means", "filtered_covariances", "smoothed_means", "smoothed_covariances"):
             e = scaled_err(getattr(s, fld), r2[fld])
             record(f"fp32_kf_{stype}:{fld}", e)
@@ -435,7 +435,7 @@ def test_fp32_ukf_bound():
     assert f.filtered_means.dtype == np.float32
     po = o.NonlinearParams(m0=g["m0"], P0=g["P0"], drift=o.Lorenz63Drift(*g["theta"]), L=g["L"], Qc=g["Qc"], H=g["H"],
                            R=g["R"], d=g["d"])
-    r = o.unscented_kalman_filter(po, _as64(y32), _as64(t32), settings=o.SolverSettings("rk4", float(np.float32(0.0025))))
+    r = o.unscented_kalman_filter(po, _as64(y32), _as64(t32), settings=o.SolverSettings("rk4", float(np.float32(0.0025)), time_dtype=np.float32))
     e = max_rel_err(f.marginal_loglik, r["marginal_loglik"])
     record("fp32_ukf:marginal_loglik", e)
     assert e < 5e-4
@@ -454,7 +454,7 @@ def test_fp32_l96_register_ode_bound(algo, solver, dt0):
     g, po, t, y = _l96_case(N=3, K=8, seed=71)
     y32, t32 = _f32(y, t)
     st = {"solver": solver, "dt0": dt0}
-    so = o.SolverSettings(solver, float(np.float32(dt0)))
+    so = o.SolverSettings(solver, float(np.float32(dt0)), time_dtype=np.float32)
     if algo == "ekf":
         f = cd.cdnlgssm_filter(nonlinear_params_api(g), y32, t32[..., None], cd.EKFHyperParams(diffeqsolve_settings=st))
         r = o.extended_kalman_filter(po, _as64(y32), _as64(t32), settings=so)
@@ -480,7 +480,7 @@ def test_fp32_enkf_bound():
     po = o.NonlinearParams(m0=g["m0"], P0=g["P0"], drift=o.LinearDrift(g["theta"][:16].reshape(4, 4), g["theta"][16:]),
                            L=g["L"], Qc=g["Qc"], H=g["H"], R=g["R"], d=g["d"])
     r = o.ensemble_kalman_filter(po, _as64(y32), _as64(t32), E=256, seed=77,
-                                 settings=o.SolverSettings("euler", float(np.float32(dt0))))
+                                 settings=o.SolverSettings("euler", float(np.float32(dt0)), time_dtype=np.float32))
     e = max_rel_err(f.marginal_loglik, r["marginal_loglik"])
     record("fp32_enkf:marginal_loglik", e)
     assert e < 1e-3
@@ -506,7 +506,7 @@ def test_fp32_enkf_l96_light_mapping(monkeypatch):
     assert f1.filtered_means.dtype == np.float32
     for fld in FIELDS:
         assert scaled_err(getattr(f1, fld), np.asarray(getattr(f0, fld), np.float64)) < 2e-4, fld
-    r = o.ensemble_kalman_filter(po, _as64(y32), _as64(t32), E=512, seed=5, settings=o.SolverSettings("euler", float(np.float32(0.005))))
+    r = o.ensemble_kalman_filter(po, _as64(y32), _as64(t32), E=512, seed=5, settings=o.SolverSettings("euler", float(np.float32(0.005)), time_dtype=np.float32))
     assert max_rel_err(f1.marginal_loglik, r["marginal_loglik"]) < 5e-3
     for fld in FIELDS:
         assert scaled_err(getattr(f1, fld), r[fld]) < 5e-3, fld
@@ -523,7 +523,7 @@ def test_fp32_eks_bound():
     assert s.smoothed_means.dtype == np.float32
     po = o.NonlinearParams(m0=L63["m0"], P0=L63["P0"], drift=o.Lorenz63Drift(*L63["theta"]), L=L63["L"], Qc=L63["Qc"],
                            H=L63["H"], R=L63["R"], d=L63["d"])
-    r = o.extended_kalman_smoother(po, _as64(y32), _as64(t32), settings=o.SolverSettings("rk4", float(np.float32(0.0025))))
+    r = o.extended_kalman_smoother(po, _as64(y32), _as64(t32), settings=o.SolverSettings("rk4", float(np.float32(0.0025)), time_dtype=np.float32))
     for fld in ("smoothed_means", "smoothed_covariances"):
         e = scaled_err(getattr(s, fld), r[fld])
         record(f"fp32_eks:{fld}", e)

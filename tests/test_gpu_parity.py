@@ -254,9 +254,10 @@ def test_ekf_l63_fp32_variant_bound():
     assert f32.filtered_means.dtype == np.float32
     po = o.NonlinearParams(m0=g["m0"], P0=g["P0"], drift=make_drift("lorenz63", g["theta"], 3), L=g["L"], Qc=g["Qc"],
                            H=g["H"], R=g["R"], d=g["d"])
-    # oracle in fp64 on the SAME (fp32-rounded) times, so the comparison isolates arithmetic precision
+    # oracle in fp64 on the SAME (fp32-rounded) times, stepping in fp32 (fp32 times and tolerance: the kernel's substeps),
+    # so the comparison isolates arithmetic precision
     r = o.extended_kalman_filter(po, y.astype(np.float32), t.astype(np.float32).astype(np.float64),
-                                 settings=o.SolverSettings("rk4", float(np.float32(0.0025))))
+                                 settings=o.SolverSettings("rk4", float(np.float32(0.0025)), time_dtype=np.float32))
     assert max_rel_err(f32.marginal_loglik, r["marginal_loglik"]) < 2e-4
     for fld in FIELDS:
         assert scaled_err(getattr(f32, fld), r[fld]) < 2e-3, fld
