@@ -113,7 +113,7 @@ __global__ void __launch_bounds__(SP_TPB) sample_path_kernel(const KArgs<T> a) {
   const T* m0 = a.in[CDK_IN_M0] + traj * a.in_stride[CDK_IN_M0];
   T* XS = static_cast<T*>(a.out[CDK_OUT_FM]);
   T* YS = static_cast<T*>(a.out[CDK_OUT_PM]);
-  const T dt0 = T(d.dt0), tol = clip_tol<T>();
+  const T dt0 = T(d.dt0);
   T x[NXA], xe[NXA], z[NXA];
   int status = 0;
 
@@ -167,16 +167,15 @@ __global__ void __launch_bounds__(SP_TPB) sample_path_kernel(const KArgs<T> a) {
   for (int k = first; k < K; ++k) {
     // transition over [t_{k-1}, t_k] (fixed: [T[k], T[k+1]])
     const T t0 = fixed ? Tm[k] : Tm[k - 1], t1 = fixed ? Tm[k + 1] : Tm[k];
-    T tprev = t0, tnext = fmin(t0 + dt0, t1);
-    int nsteps = 0;
-    while (tprev < t1) {
-      if (nsteps >= d.max_steps) {
+    StepClock<T> clk(t0, t1, dt0);
+    while (clk.running()) {
+      if (clk.n >= d.max_steps) {
         status = 2;
         for (int i = 0; i < n; ++i) x[i] = T(NAN);
         break;
       }
-      const T dt = tnext - tprev, sqdt = sqrt(dt);
-      normals(RNG_DYN, k, nsteps, n, z);
+      const T dt = clk.dt(), sqdt = sqrt(dt);
+      normals(RNG_DYN, k, clk.n, n, z);
       if (diagG) {
 #pragma unroll(NX > 0 ? NX : 1)
         for (int i = 0; i < NXA; ++i)
@@ -212,17 +211,14 @@ __global__ void __launch_bounds__(SP_TPB) sample_path_kernel(const KArgs<T> a) {
         for (int i = 0; i < NXA; ++i)
           if (i < n) x[i] = xe[i];
       }
-      ++nsteps;
-      tprev = tnext;
-      const T cand = tprev + dt0;
-      tnext = cand > t1 - tol ? t1 : cand;
+      clk.advance();
     }
     emit(k, fixed ? k + 1 : k);
   }
   if (a.out[CDK_OUT_STATUS]) {
     bool bad = false;
     for (int i = 0; i < n; ++i) bad |= !isfinite(x[i]);
-    static_cast<int*>(a.out[CDK_OUT_STATUS])[traj] = status ? status : (bad ? 1 : 0);
+    static_cast<int*>(a.out[CDK_OUT_STATUS])[traj] = final_status(status, !bad);
   }
 }
 

@@ -23,6 +23,51 @@ __host__ __device__ inline T clip_tol() {
   return sizeof(T) == 8 ? T(1e-10) : T(1e-6);
 }
 
+// The substeps of one gap [t0, t1] under diffrax ConstantStepSize, in the element type T of the times (fp32 kernels step
+// fp32 times with tol = 1e-6).  Every kernel steps its gaps with this rule:
+//
+//   StepClock<T> c(t0, t1, dt0);
+//   while (c.running() && c.n < max_steps) { step(c.dt()); c.advance(); }
+//   if (c.running()) ... max_steps exceeded (status 2) ...
+//
+// The first substep ends at min(t0 + dt0, t1); every later one at cand = tprev + dt0, or at t1 if cand > t1 - tol.  A gap
+// that is already complete keeps tprev == tnext == t1 (a substep of length 0).  The members are the loop's registers.
+template <typename T>
+struct StepClock {
+  T tprev, tnext, t1, dt0;
+  int n;         // substeps taken
+  bool clipped;  // the current substep ends at t1: the first if t0 + dt0 >= t1, a later one if tprev + dt0 > t1 - tol
+
+  __host__ __device__ __forceinline__ StepClock(T t0, T t1_, T dt0_)
+      : tprev(t0), tnext(fmin(t0 + dt0_, t1_)), t1(t1_), dt0(dt0_), n(0), clipped(!(t0 + dt0_ < t1_)) {}
+  __host__ __device__ __forceinline__ bool running() const { return tprev < t1; }
+  __host__ __device__ __forceinline__ T dt() const { return tnext - tprev; }
+  // the current substep has the nominal length dt0 (up to the rounding of tprev + dt0)
+  __host__ __device__ __forceinline__ bool full() const { return !clipped; }
+  __host__ __device__ __forceinline__ void advance() {
+    ++n;
+    tprev = tnext;
+    const T cand = tprev + dt0;
+    clipped = cand > t1 - clip_tol<T>();
+    tnext = clipped ? t1 : cand;
+  }
+};
+
+// Per-trajectory status (CDK_OUT_STATUS): 0 ok, 1 non-finite result, 2 max_steps exceeded.  A max_steps failure outranks
+// the NaN it causes.
+//
+// A filter's or sampler's final status, from the status of its steps and whether its result is finite.
+__host__ __device__ __forceinline__ int final_status(int status, bool finite) {
+  return status != 0 ? status : finite ? 0 : 1;
+}
+// A smoother's status, merged into st[i], which its filter wrote: non-finite smoothed moments after a filter that failed
+// are that failure, not a new one, so the filter's status stays unless the filter was clean or the backward pass itself
+// exceeded max_steps.
+__host__ __device__ __forceinline__ void merge_smoother_status(int* st, long long i, int status, bool finite) {
+  if (status == 0 && !finite && st[i] == 0) status = 1;
+  if (status != 0) st[i] = status;
+}
+
 template <typename T>
 __device__ __forceinline__ T half_log_2pi() {
   return T(0.91893853320467274178);

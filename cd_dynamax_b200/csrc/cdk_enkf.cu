@@ -355,7 +355,6 @@ __global__ void __launch_bounds__(LIGHT ? 2 * ENKF_TPB : ENKF_TPB, 1) enkf_kerne
   T* LLC = static_cast<T*>(a.out[CDK_OUT_LLCUM]);
   const long long row0 = traj * (long long)K;
   const T dt0 = T(d.dt0);
-  const T tol = clip_tol<T>();
   T ll = T(0);
   int status = 0;
 
@@ -494,17 +493,15 @@ __global__ void __launch_bounds__(LIGHT ? 2 * ENKF_TPB : ENKF_TPB, 1) enkf_kerne
     // ================= predict (inference_enkf.py:47-89): per-member SDE solve over the gap =================
     const T t0 = Tm[k];
     const T t1 = (ponly || k + 1 < K) ? Tm[k + 1] : t0 + T(d.dt_final);
-    T tprev = t0;
-    T tnext = fmin(t0 + dt0, t1);
-    int nsteps = 0;
-    while (tprev < t1) {
-      if (nsteps >= d.max_steps) {  // diffrax max_steps exceeded: poison the ensemble, abandon the gap
+    StepClock<T> clk(t0, t1, dt0);
+    while (clk.running()) {
+      if (clk.n >= d.max_steps) {  // diffrax max_steps exceeded: poison the ensemble, abandon the gap
         status = 2;
         for (int el = threadIdx.x; el < nmem; el += blockDim.x)
           for (int i = 0; i < n; ++i) X[(size_t)i * ldE + el] = T(NAN);
         break;
       }
-      const T dt = tnext - tprev;
+      const T dt = clk.dt();
       const T sqdt = sqrt(dt);
       bool light_done = false;
       if constexpr (LIGHT && NX == 40) {
@@ -530,11 +527,11 @@ __global__ void __launch_bounds__(LIGHT ? 2 * ENKF_TPB : ENKF_TPB, 1) enkf_kerne
             for (int q0 = 0; q0 < HN; q0 += 8) {
               double z8[8];
               if (q0 + 4 < HN) {
-                normal_oct((uint32_t)(e_base + el), ctr_traj, (uint32_t)k, rng_c3(RNG_DYN, nsteps, (i0 + q0) >> 2),
-                           rng_c3(RNG_DYN, nsteps, ((i0 + q0) >> 2) + 1), seed, z8);
+                normal_oct((uint32_t)(e_base + el), ctr_traj, (uint32_t)k, rng_c3(RNG_DYN, clk.n, (i0 + q0) >> 2),
+                           rng_c3(RNG_DYN, clk.n, ((i0 + q0) >> 2) + 1), seed, z8);
               } else {
                 double z4[4];
-                normal_quad((uint32_t)(e_base + el), ctr_traj, (uint32_t)k, rng_c3(RNG_DYN, nsteps, (i0 + q0) >> 2), seed, z4);
+                normal_quad((uint32_t)(e_base + el), ctr_traj, (uint32_t)k, rng_c3(RNG_DYN, clk.n, (i0 + q0) >> 2), seed, z4);
 #pragma unroll
                 for (int u = 0; u < 4; ++u) z8[u] = z4[u];
               }
@@ -566,14 +563,14 @@ __global__ void __launch_bounds__(LIGHT ? 2 * ENKF_TPB : ENKF_TPB, 1) enkf_kerne
           for (int j = 0; j < NXA; j += 8) {
             if (j + 4 < n) {  // two quads at once (normal_oct: same values, interleaved chains)
               double z8[8];
-              normal_oct((uint32_t)(e_base + el), ctr_traj, (uint32_t)k, rng_c3(RNG_DYN, nsteps, j >> 2),
-                         rng_c3(RNG_DYN, nsteps, (j >> 2) + 1), seed, z8);
+              normal_oct((uint32_t)(e_base + el), ctr_traj, (uint32_t)k, rng_c3(RNG_DYN, clk.n, j >> 2),
+                         rng_c3(RNG_DYN, clk.n, (j >> 2) + 1), seed, z8);
 #pragma unroll
               for (int u = 0; u < 8; ++u)
                 if (j + u < NXA && j + u < n) xe[j + u] = G[(j + u) * ldn + j + u] * (sqdt * (T)z8[u]);
             } else if (j < n) {
               double z4[4];
-              normal_quad((uint32_t)(e_base + el), ctr_traj, (uint32_t)k, rng_c3(RNG_DYN, nsteps, j >> 2), seed, z4);
+              normal_quad((uint32_t)(e_base + el), ctr_traj, (uint32_t)k, rng_c3(RNG_DYN, clk.n, j >> 2), seed, z4);
 #pragma unroll
               for (int u = 0; u < 4; ++u)
                 if (j + u < NXA && j + u < n) xe[j + u] = G[(j + u) * ldn + j + u] * (sqdt * (T)z4[u]);
@@ -584,7 +581,7 @@ __global__ void __launch_bounds__(LIGHT ? 2 * ENKF_TPB : ENKF_TPB, 1) enkf_kerne
           for (int i = 0; i < NXA; ++i) xe[i] = T(0);
           for (int j = 0; j < n; j += 4) {  // quads stay a runtime loop: the rank-4 update below is the unrolled part
             double z4[4];
-            normal_quad((uint32_t)(e_base + el), ctr_traj, (uint32_t)k, rng_c3(RNG_DYN, nsteps, j >> 2), seed, z4);
+            normal_quad((uint32_t)(e_base + el), ctr_traj, (uint32_t)k, rng_c3(RNG_DYN, clk.n, j >> 2), seed, z4);
             for (int u = 0; u < 4 && j + u < n; ++u) {
               const T dw = sqdt * (T)z4[u];
 #pragma unroll UF
@@ -610,19 +607,15 @@ __global__ void __launch_bounds__(LIGHT ? 2 * ENKF_TPB : ENKF_TPB, 1) enkf_kerne
             if (i < n) X[(size_t)i * ldE + el] = xe[i];
         }
       }
-      ++nsteps;
-      tprev = tnext;
-      const T cand = tprev + dt0;
-      tnext = cand > t1 - tol ? t1 : cand;
+      clk.advance();
     }
     __syncthreads();
     moments<T>(cluster, L, sh, nmem, E, C);  // predicted moments (:234-238); they also feed the next update
     write_moments(PM, PP, row0 + k);
   }
   if (rank == 0 && threadIdx.x == 0) {
-    if (status == 0 && !isfinite(ll)) status = 1;
     if (a.out[CDK_OUT_LL]) static_cast<T*>(a.out[CDK_OUT_LL])[traj] = ll;
-    if (a.out[CDK_OUT_STATUS]) static_cast<int*>(a.out[CDK_OUT_STATUS])[traj] = status;
+    if (a.out[CDK_OUT_STATUS]) static_cast<int*>(a.out[CDK_OUT_STATUS])[traj] = final_status(status, isfinite(ll));
   }
   (void)misc;
 }

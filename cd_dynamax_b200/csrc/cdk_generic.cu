@@ -313,17 +313,14 @@ __device__ bool ode_solve(const Ctx<T>& c, int kind, T* y, int S, T t0, T t1, T 
   T* ys = c.p(c.L.YS);
   T* acc = c.p(c.L.ACC);
   T* ks = c.p(c.L.KS);
-  const T tol = clip_tol<T>();
-  T tprev = t0;
-  T tnext = fmin(t0 + dt0, t1);
-  int nsteps = 0;
-  while (tprev < t1) {
-    if (nsteps >= max_steps) {
+  StepClock<T> clk(t0, t1, dt0);
+  while (clk.running()) {
+    if (clk.n >= max_steps) {
       FOR_T(e, S) y[e] = T(NAN);
       __syncthreads();
       return true;
     }
-    const T dt = tnext - tprev;
+    const T dt = clk.dt();
     for (int i = 0; i < tab.S; ++i) {
       const int nz = tab.nnz[i];
       FOR_T(e, S) {
@@ -344,10 +341,7 @@ __device__ bool ode_solve(const Ctx<T>& c, int kind, T* y, int S, T t0, T t1, T 
     }
     FOR_T(e, S) y[e] = acc[e];
     __syncthreads();
-    ++nsteps;
-    tprev = tnext;
-    const T cand = tprev + dt0;
-    tnext = cand > t1 - tol ? t1 : cand;
+    clk.advance();
   }
   return false;
 }
@@ -451,21 +445,19 @@ __device__ bool ode_solve_stencil(const Ctx<T>& c, const StencilRegs<T>& R, T* y
     kP[j] = T(0);
   }
   if (own_m) am = y[R.o_xr];
-  const T tol = clip_tol<T>();
-  T tprev = t0, tnext = fmin(t0 + dt0, t1);
-  int nsteps = 0;
+  StepClock<T> clk(t0, t1, dt0);
   bool hit = false;
   const int boff0 = L.YS, boff1 = L.KS;
   int flip = 0;
-  while (tprev < t1) {
-    if (nsteps >= max_steps) {
+  while (clk.running()) {
+    if (clk.n >= max_steps) {
       hit = true;
 #pragma unroll
       for (int j = 0; j < SEG; ++j) aP[j] = T(NAN);
       am = T(NAN);
       break;
     }
-    const T dt = tnext - tprev;
+    const T dt = clk.dt();
 #pragma unroll
     for (int j = 0; j < SEG; ++j) yP[j] = aP[j];
     ym = am;
@@ -526,10 +518,7 @@ __device__ bool ode_solve_stencil(const Ctx<T>& c, const StencilRegs<T>& R, T* y
         }
       }
     }
-    ++nsteps;
-    tprev = tnext;
-    const T cand = tprev + dt0;
-    tnext = cand > t1 - tol ? t1 : cand;
+    clk.advance();
   }
   T a0[SEG];
 #pragma unroll
@@ -568,20 +557,18 @@ __device__ bool ode_solve_stencil_dopri5(const Ctx<T>& c, const StencilRegs<T>& 
 #pragma unroll
     for (int j = 0; j < SEG; ++j) kk[q][j] = T(0);
   }
-  const T tol = clip_tol<T>();
-  T tprev = t0, tnext = fmin(t0 + dt0, t1);
-  int nsteps = 0;
+  StepClock<T> clk(t0, t1, dt0);
   bool hit = false;
   const int boff0 = L.YS, boff1 = L.KS;
-  while (tprev < t1) {
-    if (nsteps >= max_steps) {
+  while (clk.running()) {
+    if (clk.n >= max_steps) {
       hit = true;
 #pragma unroll
       for (int j = 0; j < SEG; ++j) yP[j] = T(NAN);
       ym = T(NAN);
       break;
     }
-    const T dt = tnext - tprev;
+    const T dt = clk.dt();
     T aP[SEG], am = ym;
 #pragma unroll
     for (int j = 0; j < SEG; ++j) aP[j] = yP[j];
@@ -646,10 +633,7 @@ __device__ bool ode_solve_stencil_dopri5(const Ctx<T>& c, const StencilRegs<T>& 
 #pragma unroll
     for (int j = 0; j < SEG; ++j) yP[j] = aP[j];
     ym = am;
-    ++nsteps;
-    tprev = tnext;
-    const T cand = tprev + dt0;
-    tnext = cand > t1 - tol ? t1 : cand;
+    clk.advance();
   }
   T a0[SEG];
 #pragma unroll
@@ -1095,9 +1079,8 @@ __global__ void __launch_bounds__(256, REGODE == 2 ? 1 : 2) generic_filter_kerne
     __syncthreads();
   }
   if (threadIdx.x == 0) {
-    if (status == 0 && !isfinite(ll)) status = 1;
     if (a.out[CDK_OUT_LL]) static_cast<T*>(a.out[CDK_OUT_LL])[traj] = ll;
-    if (a.out[CDK_OUT_STATUS]) static_cast<int*>(a.out[CDK_OUT_STATUS])[traj] = status;
+    if (a.out[CDK_OUT_STATUS]) static_cast<int*>(a.out[CDK_OUT_STATUS])[traj] = final_status(status, isfinite(ll));
   }
 }
 
@@ -1239,12 +1222,9 @@ __global__ void generic_smooth_kernel(const GArgs<T> g) {
     __syncthreads();
   }
   if (threadIdx.x == 0 && a.out[CDK_OUT_STATUS]) {
-    int* st = static_cast<int*>(a.out[CDK_OUT_STATUS]);
     bool bad = false;
     for (int i = 0; i < n; ++i) bad |= !isfinite(ms[i]);
-    // NaN smoothed moments after a filter that hit max_steps are that failure, not a new one: keep the filter's status
-    if (status == 0 && bad && st[traj] == 0) status = 1;
-    if (status != 0) st[traj] = status;  // keep the filter's status unless the backward pass adds a failure
+    merge_smoother_status(static_cast<int*>(a.out[CDK_OUT_STATUS]), traj, status, !bad);
   }
 }
 

@@ -159,7 +159,7 @@ __device__ __forceinline__ void store_global(const double (&d)[2][2][2], double*
 // ConstantStepSize stepping rule.  Results stay in registers (C-fragment layout); sYA / sYQ / sT are the warp's stage
 // buffers.  Returns true when max_steps was exceeded (results are NaN then, as in the reference).
 template <bool POLY>
-__device__ __forceinline__ bool pushforward(const KwTab& tab, const double dt0, const double tol, const int max_steps,
+__device__ __forceinline__ bool pushforward(const KwTab& tab, const double dt0, const int max_steps,
                                             const double t0, const double t1, const double* sF, const double* sLQL,
                                             const double* sRk, double* sYA, double* sYQ, double* sT, F16& yA, F16& yQ,
                                             const bool direct_t = false) {
@@ -174,30 +174,27 @@ __device__ __forceinline__ bool pushforward(const KwTab& tab, const double dt0, 
         yA.v[rb][cb][r] = (8 * rb + gid == 8 * cb + 2 * tig + r) ? 1.0 : 0.0;
         yQ.v[rb][cb][r] = 0.0;
       }
-  double tprev = t0;
-  double tnext = fmin(t0 + dt0, t1);
-  bool full = t0 + dt0 < t1;  // this substep has the nominal length dt0 (not clipped to the end of the gap)
-  int nsteps = 0;
-  while (tprev < t1) {
-    if (nsteps >= max_steps) {
+  StepClock<double> clk(t0, t1, dt0);
+  while (clk.running()) {
+    if (clk.n >= max_steps) {
       hit = true;
 #pragma unroll
       for (int i = 0; i < 8; ++i) (&yA.v[0][0][0])[i] = (&yQ.v[0][0][0])[i] = NAN;
       break;
     }
-    const double dt = tnext - tprev;
+    const double dt = clk.dt();
     // dA = F A is linear with constant coefficients, so one explicit RK step of length dt0 maps A to Rk A with the SAME
     // matrix Rk for every full-length substep of every gap (Rk = the RK step applied to the identity, computed once per
     // model by rk_map): one product instead of one per stage.  Clipped substeps (and Q, whose step map is not a
     // similarity transform of the truncated polynomial) take the stages.  Same result as stepping A up to rounding.
-    const bool fastA = full && sRk != nullptr;
+    const bool fastA = clk.full() && sRk != nullptr;
     F16 accA = yA, accQ = yQ, kA, kQ;
     if (fastA) {
       store_c<2, 2>(yA.v, sYA);
       __syncwarp();
       mm<false, false, 16, 2, 2>(accA.v, sRk, sYA);
       __syncwarp();
-      // the substep is tnext - tprev = fl(tprev + dt0) - tprev, which differs from dt0 by up to half an ulp of t: 1.8e-12
+      // a full substep ends at t + dt0 rounded, so its length differs from dt0 by up to half an ulp of t: 1.8e-12
       // at t = 1e4, i.e. 7e-10 of dt0 = 0.0025, and the reference steps with that length.  Rk(dt) = Rk(dt0) + (dt - dt0) F
       // Rk(dt0) + O(dt0^S (dt - dt0)): one more product restores it.  Below 2^-40 dt0 the term is under 2^-40 dt0 |F| of A
       // per step and the product is skipped, so grids at moderate t keep the one-product step.
@@ -305,11 +302,7 @@ __device__ __forceinline__ bool pushforward(const KwTab& tab, const double dt0, 
     }
     yA = accA;
     yQ = accQ;
-    ++nsteps;
-    tprev = tnext;
-    const double cand = tprev + dt0;
-    full = !(cand > t1 - tol);
-    tnext = full ? cand : t1;
+    clk.advance();
   }
   return hit;
 }
@@ -519,7 +512,7 @@ __global__ void __launch_bounds__(32 * KW_WPC, 3) kf_warp_filter(const KArgs<dou
   double* LLC = static_cast<double*>(a.out[CDK_OUT_LLCUM]);
   double* AQ = (d.reserved[2] & CDK_FLAG_KEEP_PUSHFORWARD) ? static_cast<double*>(a.out[CDK_OUT_SCRATCH]) : nullptr;
   const long long row0 = traj * (long long)K;
-  const double dt0 = d.dt0, tol = clip_tol<double>();
+  const double dt0 = d.dt0;
   double ll = 0.0;
   int status = 0;
   double y_next = lane < m ? Y[lane] : 0.0;
@@ -633,7 +626,7 @@ __global__ void __launch_bounds__(32 * KW_WPC, 3) kf_warp_filter(const KArgs<dou
     }
     // ================= pushforward (A, Q) over [t0, t1] from (I, 0)  (:105-144; diffrax ConstantStepSize) =================
     F16 yA, yQ;
-    if (pushforward<POLY>(tab, dt0, tol, d.max_steps, t0, t1, sF, sLQL, sRk, sYA, sYQ, sT, yA, yQ, (use_rk & 2) != 0)) status = 2;
+    if (pushforward<POLY>(tab, dt0, d.max_steps, t0, t1, sF, sLQL, sRk, sYA, sYQ, sT, yA, yQ, (use_rk & 2) != 0)) status = 2;
     if (AQ && k + 1 < K) {  // CDK_FLAG_KEEP_PUSHFORWARD: the type-1 smoother will read (A_k, Q_k) back
       double* dst = AQ + ((traj * (long long)(K - 1) + k) * 2) * n * n;
       store_global(yA.v, dst, n);
@@ -664,9 +657,8 @@ __global__ void __launch_bounds__(32 * KW_WPC, 3) kf_warp_filter(const KArgs<dou
     }
   }
   if (lane == 0) {
-    if (status == 0 && !isfinite(ll)) status = 1;
     if (a.out[CDK_OUT_LL]) static_cast<double*>(a.out[CDK_OUT_LL])[traj] = ll;
-    if (a.out[CDK_OUT_STATUS]) static_cast<int*>(a.out[CDK_OUT_STATUS])[traj] = status;
+    if (a.out[CDK_OUT_STATUS]) static_cast<int*>(a.out[CDK_OUT_STATUS])[traj] = final_status(status, isfinite(ll));
   }
 }
 
@@ -727,7 +719,7 @@ __global__ void __launch_bounds__(32 * KS_WPC, 2) kf_warp_smooth(const KArgs<dou
   double* __restrict__ SPg = static_cast<double*>(a.out[CDK_OUT_SP]) + traj * (long long)K * n * n;
   double* __restrict__ SCg =
       a.out[CDK_OUT_SCROSS] ? static_cast<double*>(a.out[CDK_OUT_SCROSS]) + traj * (long long)(K - 1) * n * n : nullptr;
-  const double dt0 = d.dt0, tol = clip_tol<double>();
+  const double dt0 = d.dt0;
   int status = 0;
   const double* AQ =
       (d.reserved[2] & CDK_FLAG_KEEP_PUSHFORWARD) ? static_cast<const double*>(a.out[CDK_OUT_SCRATCH]) : nullptr;
@@ -754,7 +746,7 @@ __global__ void __launch_bounds__(32 * KS_WPC, 2) kf_warp_smooth(const KArgs<dou
       const double* src = AQ + ((traj * (long long)(K - 1) + k) * 2) * n * n;
       load_global(yA.v, src, n);
       load_global(yQ.v, src + n * n, n);  // (zero padding: the padded rows of P_f are zero, so A's identity pad is moot)
-    } else if (pushforward<POLY>(tab, dt0, tol, d.max_steps, t0, t1, sF, sLQL, sRk, sYA, sYQ, sT, yA, yQ, (use_rk & 2) != 0)) {
+    } else if (pushforward<POLY>(tab, dt0, d.max_steps, t0, t1, sF, sLQL, sRk, sYA, sYQ, sT, yA, yQ, (use_rk & 2) != 0)) {
       status = 2;
     }
     store_c<2, 2>(yA.v, sYA);
@@ -860,9 +852,7 @@ __global__ void __launch_bounds__(32 * KS_WPC, 2) kf_warp_smooth(const KArgs<dou
   if (lane == 0 && a.out[CDK_OUT_STATUS]) {
     bool bad = false;
     for (int i = 0; i < n; ++i) bad |= !isfinite(sms[i]);
-    // NaN smoothed moments after a filter that hit max_steps are that failure, not a new one: keep the filter's status
-    if (status == 0 && bad && static_cast<int*>(a.out[CDK_OUT_STATUS])[traj] == 0) status = 1;
-    if (status != 0) static_cast<int*>(a.out[CDK_OUT_STATUS])[traj] = status;  // keep the filter's status otherwise
+    merge_smoother_status(static_cast<int*>(a.out[CDK_OUT_STATUS]), traj, status, !bad);
   }
 }
 

@@ -565,7 +565,6 @@ __global__ void __launch_bounds__(SLICED ? 32 * 12 : 32 * WPC, WPC == 7 ? 2 : 1)
   }
   const T dt0 = T(a.d.dt0);
   const T dtf = T(a.d.dt_final);
-  const T tol = clip_tol<T>();
   const int max_steps = a.d.max_steps;
   const int num_iter = a.d.num_iter;
   T* __restrict__ LLC = static_cast<T*>(a.out[CDK_OUT_LLCUM]);
@@ -588,15 +587,6 @@ __global__ void __launch_bounds__(SLICED ? 32 * 12 : 32 * WPC, WPC == 7 ? 2 : 1)
       if (a.out[CDK_OUT_PP]) tma_store_2d(&maps.m[3], &sm.pp[0][0][0], k0 * NX * NX, c1);
     }
     asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-  };
-  // one RK step with the diffrax stepping rule (tnext = tprev + dt0, clipped to t1 within tol).  A lane whose gap is
-  // already complete has tnext == tprev == t1: it takes a step of length 0, which leaves its state bit-identical
-  // (y + 0 * ksum), so the substep loop needs no per-lane predication -- its trip count is warp-uniform (vote).
-  auto substep = [&](T& tprev, T& tnext, const T t1) {
-    rk_step<T, Drift, SOLVER>(th, lql, s, tnext - tprev);
-    tprev = tnext;
-    const T cand = tprev + dt0;
-    tnext = cand > t1 - tol ? t1 : cand;
   };
   auto poison = [&]() {
     status = 2;
@@ -624,8 +614,8 @@ __global__ void __launch_bounds__(SLICED ? 32 * 12 : 32 * WPC, WPC == 7 ? 2 : 1)
     T y[NY];
 #pragma unroll
     for (int c = 0; c < NY; ++c) y[c] = sm.inY[k & (LW_RING - 1)][c][lane];
-    T tprev = sm.inT[k & (LW_RING - 1)][lane];
-    const T t1 = k + 1 < KT ? sm.inT[(k + 1) & (LW_RING - 1)][lane] : tprev + dtf;
+    const T t0 = sm.inT[k & (LW_RING - 1)][lane];
+    const T t1 = k + 1 < KT ? sm.inT[(k + 1) & (LW_RING - 1)][lane] : t0 + dtf;
     if (ponly) {
       // forecast: the state is propagated, never updated
     } else if constexpr (NY == 1) {
@@ -701,13 +691,14 @@ __global__ void __launch_bounds__(SLICED ? 32 * 12 : 32 * WPC, WPC == 7 ? 2 : 1)
       }
     }
     {
-      T tnext = fmin(tprev + dt0, t1);
-      int nsteps = 0;
-      while (__any_sync(0xffffffffu, tprev < t1) && nsteps < max_steps) {
-        substep(tprev, tnext, t1);
-        ++nsteps;
+      // A lane whose gap is already complete takes substeps of length 0, which leave its state bit-identical
+      // (y + 0 * ksum), so the substep loop needs no per-lane predication -- its trip count is warp-uniform (vote).
+      StepClock<T> clk(t0, t1, dt0);
+      while (__any_sync(0xffffffffu, clk.running()) && clk.n < max_steps) {
+        rk_step<T, Drift, SOLVER>(th, lql, s, clk.dt());
+        clk.advance();
       }
-      if (tprev < t1) poison();  // diffrax max_steps exceeded: the reference result is NaN
+      if (clk.running()) poison();  // diffrax max_steps exceeded: the reference result is NaN
     }
     if (use_token) {
       __syncwarp();
@@ -807,7 +798,6 @@ __global__ void __launch_bounds__(SLICED ? 32 * 12 : 32 * WPC, WPC == 7 ? 2 : 1)
         gs.flags[lane] = (sbad ? 1 : 0) | (status << 8);
       } else if (live) {
         T llf = ll;
-        int st = status;
         if (lean) {
           // sum_k log S_k = esum log 2 + log(sprod); the -log(2 pi)/2 of every step
           // (explicit fma / single operations: the sliced and the plain instantiation must round identically)
@@ -815,9 +805,8 @@ __global__ void __launch_bounds__(SLICED ? 32 * 12 : 32 * WPC, WPC == 7 ? 2 : 1)
           llf = llf - fma(T(0.5), lsum, T(K) * half_log_2pi<T>());
           if (sbad) llf = T(NAN);
         }
-        if (st == 0 && !isfinite(llf)) st = 1;
         if (a.out[CDK_OUT_LL]) static_cast<T*>(a.out[CDK_OUT_LL])[traj] = llf;
-        if (a.out[CDK_OUT_STATUS]) static_cast<int*>(a.out[CDK_OUT_STATUS])[traj] = st;
+        if (a.out[CDK_OUT_STATUS]) static_cast<int*>(a.out[CDK_OUT_STATUS])[traj] = final_status(status, isfinite(llf));
       }
     }
     if (SLICED) __syncthreads();
@@ -962,7 +951,7 @@ __global__ void __launch_bounds__(32 * 14, 1) eks_small_lw(const KArgs<T> a, con
   prefetch(K - 1);
   prefetch(K - 2);
   prefetch(K - 3);
-  const T dt0 = T(a.d.dt0), tol = clip_tol<T>();
+  const T dt0 = T(a.d.dt0);
   const int max_steps = a.d.max_steps;
   int status = 0;
 
@@ -1116,16 +1105,12 @@ __global__ void __launch_bounds__(32 * 14, 1) eks_small_lw(const KArgs<T> a, con
           for (int j = i; j < NX; ++j) kk.P[pidx<NX>(i, j)] = lql[pidx<NX>(i, j)] - (GP[i][j] + GP[j][i]);
       };
       const T span = t1 - t0;  // integrate s from 0 to t_{k+1} - t_k
-      T tprev = T(0), tnext = fmin(dt0, span);
-      int nsteps = 0;
-      while (tprev < span && nsteps < max_steps) {
-        rk_step_fn<T, NX, SOLVER>(s, tnext - tprev, rhs);
-        ++nsteps;
-        tprev = tnext;
-        const T cand = tprev + dt0;
-        tnext = cand > span - tol ? span : cand;
+      StepClock<T> clk(T(0), span, dt0);
+      while (clk.running() && clk.n < max_steps) {
+        rk_step_fn<T, NX, SOLVER>(s, clk.dt(), rhs);
+        clk.advance();
       }
-      if (tprev < span) {  // diffrax max_steps exceeded: NaN, as in the reference
+      if (clk.running()) {  // diffrax max_steps exceeded: NaN, as in the reference
         status = 2;
 #pragma unroll
         for (int i = 0; i < NX; ++i) s.m[i] = T(NAN);
@@ -1153,9 +1138,7 @@ __global__ void __launch_bounds__(32 * 14, 1) eks_small_lw(const KArgs<T> a, con
     bool bad = false;
 #pragma unroll
     for (int i = 0; i < NX; ++i) bad |= !isfinite(s.m[i]);
-    // NaN smoothed moments after a filter that hit max_steps are that failure, not a new one: keep the filter's status
-    if (status == 0 && bad && static_cast<int*>(a.out[CDK_OUT_STATUS])[traj] == 0) status = 1;
-    if (status != 0) static_cast<int*>(a.out[CDK_OUT_STATUS])[traj] = status;  // keep the filter's status otherwise
+    merge_smoother_status(static_cast<int*>(a.out[CDK_OUT_STATUS]), traj, status, !bad);
   }
 }
 
@@ -1310,10 +1293,10 @@ __global__ void __launch_bounds__(128) ekf_l63_grad_kernel(const KArgs<double> a
         k[NX + NP + NX + pidx<NX>(i, j)] = (G2[i][j] + G2[j][i]) + dlql[pidx<NX>(i, j)];
       }
   };
-  const T dt0 = T(a.d.dt0), dtf = T(a.d.dt_final), tol = clip_tol<T>();
+  const T dt0 = T(a.d.dt0), dtf = T(a.d.dt_final);
   const int max_steps = a.d.max_steps;
   T ll = T(0), llt = T(0);
-  T tprev = Tm[0];
+  T t0 = Tm[0];
   for (int k = 0; k < K; ++k) {
     // ---- measurement update and its tangent (H' = dH, R' = dR, d' = dd are the parameter seeds) ----
     T HP[NX], HPt[NX];
@@ -1358,21 +1341,17 @@ __global__ void __launch_bounds__(128) ekf_l63_grad_kernel(const KArgs<double> a
       y[i] += Kg[i] * r;
     }
     // ---- predict across the gap (diffrax stepping rule) ----
-    const T t1 = k + 1 < K ? Tm[k + 1] : tprev + dtf;
-    T tnext = fmin(tprev + dt0, t1);
-    int nsteps = 0;
-    while (tprev < t1 && nsteps < max_steps) {
-      rk_step_flat<T, NE, SOLVER>(y, tnext - tprev, rhs);
-      ++nsteps;
-      tprev = tnext;
-      const T cand = tprev + dt0;
-      tnext = cand > t1 - tol ? t1 : cand;
+    const T t1 = k + 1 < K ? Tm[k + 1] : t0 + dtf;
+    StepClock<T> clk(t0, t1, dt0);
+    while (clk.running() && clk.n < max_steps) {
+      rk_step_flat<T, NE, SOLVER>(y, clk.dt(), rhs);
+      clk.advance();
     }
-    if (tprev < t1) {
+    if (clk.running()) {
 #pragma unroll
       for (int e = 0; e < NE; ++e) y[e] = T(NAN);
     }
-    tprev = t1;
+    t0 = t1;
   }
   if (a.out[CDK_OUT_LL]) static_cast<T*>(a.out[CDK_OUT_LL])[traj] = ll;
   grad[traj * grad_stride + col] = llt;
@@ -1522,7 +1501,7 @@ __global__ void __launch_bounds__(128) ekf_l63_grad_rev_kernel(const KArgs<doubl
   const double* fp = FPg + traj * (long long)K * 9;
   const double* pm = PMg + traj * (long long)K * 3;
   const double* pp = PPg + traj * (long long)K * 9;
-  const double dt0 = a.d.dt0, tol = clip_tol<double>();
+  const double dt0 = a.d.dt0;
   const int max_steps = a.d.max_steps;
   GradAcc g;
   for (int i = 0; i < 3; ++i) g.th[i] = g.H[i] = 0.0;
@@ -1542,48 +1521,33 @@ __global__ void __launch_bounds__(128) ekf_l63_grad_rev_kernel(const KArgs<doubl
       St<double, 3> y0;
       load_state(fm + (long long)k * 3, fp + (long long)k * 9, y0);
       const double t0 = Tm[k], t1 = Tm[k + 1];
-      // number of substeps (diffrax stepping rule); the time grid does not depend on the state
-      int q = 0;
-      {
-        double tp = t0, tn = fmin(t0 + dt0, t1);
-        while (tp < t1 && q < max_steps) {
-          ++q;
-          tp = tn;
-          const double c = tp + dt0;
-          tn = c > t1 - tol ? t1 : c;
-        }
-      }
+      // number of substeps; the time grid does not depend on the state
+      StepClock<double> count(t0, t1, dt0);
+      while (count.running() && count.n < max_steps) count.advance();
+      const int q = count.n;
       // start state of substep i for i % stride == 0 (i / stride < GR_CKPT) is kept; the others are re-integrated
       const int stride = (q + GR_CKPT - 1) / GR_CKPT > 0 ? (q + GR_CKPT - 1) / GR_CKPT : 1;
       St<double, 3> ck[GR_CKPT];
       {
         St<double, 3> s = y0;
-        double tp = t0, tn = fmin(t0 + dt0, t1);
+        StepClock<double> clk(t0, t1, dt0);
         for (int i = 0; i < q; ++i) {
           if (i % stride == 0) ck[i / stride] = s;
-          rk_step<double, DriftL63, SOLVER>(th, lql, s, tn - tp);
-          tp = tn;
-          const double c = tp + dt0;
-          tn = c > t1 - tol ? t1 : c;
+          rk_step<double, DriftL63, SOLVER>(th, lql, s, clk.dt());
+          clk.advance();
         }
       }
       for (int i = q - 1; i >= 0; --i) {
         // (tprev, tnext) and the start state of substep i
         const int base = (i / stride) * stride;
-        double tp = t0, tn = fmin(t0 + dt0, t1);
-        for (int u = 0; u < base; ++u) {
-          tp = tn;
-          const double c = tp + dt0;
-          tn = c > t1 - tol ? t1 : c;
-        }
+        StepClock<double> clk(t0, t1, dt0);
+        for (int u = 0; u < base; ++u) clk.advance();
         St<double, 3> s = ck[i / stride];
         for (int u = base; u < i; ++u) {
-          rk_step<double, DriftL63, SOLVER>(th, lql, s, tn - tp);
-          tp = tn;
-          const double c = tp + dt0;
-          tn = c > t1 - tol ? t1 : c;
+          rk_step<double, DriftL63, SOLVER>(th, lql, s, clk.dt());
+          clk.advance();
         }
-        l63_rk_step_vjp<SOLVER>(th, lql, s, tn - tp, lam, g);
+        l63_rk_step_vjp<SOLVER>(th, lql, s, clk.dt(), lam, g);
       }
     }
     // ---- update k, backwards.  Forward (ekf_update, scalar emission):  HP = H P, S = HP.H + R, r = y - H.m - d,

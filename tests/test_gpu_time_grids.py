@@ -1,4 +1,8 @@
-"""Every kernel's copy of the diffrax ConstantStepSize rule on time grids that reach its last-bit branches.
+"""Every kernel's substep loop under the diffrax ConstantStepSize rule, on time grids that reach its last-bit branches.
+
+The kernels call one rule, StepClock (csrc/cdk_common.cuh; its host build is tested against the oracle in
+test_step_rule_host), from many loops; each loop still owns its bounds, its max_steps check and what it does per substep,
+so each call site below is probed on its own.
 
 The rule: the first substep of a gap is tnext = min(t0 + dt0, t1); every later one is cand = tprev + dt0, tnext = t1 if
 cand > t1 - tol else cand (tol = 1e-10 for fp64 times, 1e-6 for fp32).  A grid of random gaps almost never lands within
@@ -14,7 +18,7 @@ Three checks per kernel:
 Entry point -> kernel -> what runs here (a reviewer can hold this against the dispatch in cdk_api.cu, kf_warp_eligible and
 the ekf_small_lw launch conditions):
 
-  entry point                     kernel (copy of the rule)                  grids            probe  values
+  entry point                     kernel (call site of the rule)             grids            probe  values
   cdk_ekf_filter  L63 m=1 f64     ekf_small_lw (cdk_small.cu)                all              yes    yes
   cdk_ekf_filter  L63 sliced      ekf_small_lw, time-sliced launch           probe, K = 200   yes    (= unsliced, test_gpu_parity)
   cdk_ekf_filter  L63 m=1 f32     ekf_small_lw<float>                        probe, fp32      yes    yes (fp32 step oracle)
