@@ -3,7 +3,8 @@ hd-UQ/cd_dynamax.  The reference's entry points keep their names and signatures;
 sm_100a CUDA kernels behind a C ABI (include/cdk.h, cd_dynamax_b200/lib/libcdk.so).  There is no CPU fallback."""
 from . import solvers
 from .continuous_discrete_linear_gaussian_ssm import (ContDiscreteLinearGaussianSSM, KFHyperParams, ParamsCDLGSSM,
-                                                      ParamsCDLGSSMDynamics, cdlgssm_filter, cdlgssm_smoother,
+                                                      ParamsCDLGSSMDynamics, cdlgssm_filter,
+                                                      cdlgssm_marginal_log_prob_and_grad, cdlgssm_smoother,
                                                       make_cdlgssm_params)
 from .continuous_discrete_nonlinear_gaussian_ssm import (ContDiscreteNonlinearGaussianSSM, EKFHyperParams,
                                                          EnKFHyperParams, LearnableLinear, LearnableLorenz63,

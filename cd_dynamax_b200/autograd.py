@@ -6,8 +6,12 @@ stack (INTEGRATION.md section 2) -- forward = the CUDA filter, backward = the ha
     ll.sum().backward()                                                       # torch leaves of `params`
 
 What `fit_sgd` minimises upstream is `-vmap(marginal_log_prob)(...).sum()` (src/ssm_temissions.py:550-568,
-src/utils/optimize_utils.py:102).  Lorenz-63 drift, scalar linear emission, fp64 (the coverage of cdk_ekf_grad_f64)."""
+src/utils/optimize_utils.py:102).  Lorenz-63 drift, scalar linear emission, fp64 (the coverage of cdk_ekf_grad_f64).
+
+The linear CD Kalman filter has the same shape, cdlgssm_marginal_log_prob (backward = cdk_kf_grad_f64)."""
 import torch
+
+from .continuous_discrete_linear_gaussian_ssm.inference import cdlgssm_marginal_log_prob_and_grad
 
 from .continuous_discrete_nonlinear_gaussian_ssm.inference_ekf import EKFHyperParams, ekf_marginal_log_prob_and_grad
 
@@ -59,3 +63,43 @@ def ekf_marginal_log_prob(params, emissions, t_emissions=None, hyperparams: EKFH
     leaves = _leaves(params)
     tensors = [leaves[n] if isinstance(leaves[n], torch.Tensor) else torch.as_tensor(leaves[n]) for n in _LEAVES]
     return _EKFLogLik.apply(params, emissions, t_emissions, hyperparams, *tensors)
+
+
+_KF_LEAVES = (("dynamics", "weights"), ("dynamics", "bias"), ("dynamics", "diffusion_coefficient"),
+              ("dynamics", "diffusion_cov"), ("emissions", "weights"), ("emissions", "bias"), ("emissions", "cov"),
+              ("initial", "mean"), ("initial", "cov"))
+
+
+class _KFLogLik(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, params, emissions, t_emissions, filter_hyperparams, names, *leaf_tensors):
+        ll, grads = cdlgssm_marginal_log_prob_and_grad(params, emissions, t_emissions, filter_hyperparams)
+        ll = torch.as_tensor(ll)
+        ctx.grads = [torch.as_tensor(getattr(getattr(grads, grp), fld)) for grp, fld in names]
+        ctx.leaves = [(tuple(t.shape), t.device, t.dtype) for t in leaf_tensors]
+        ctx.batched = ll.dim() == 1
+        return ll
+
+    @staticmethod
+    def backward(ctx, grad_ll):
+        out = []
+        for g, (shape, device, dtype) in zip(ctx.grads, ctx.leaves):
+            g = g.to(grad_ll.device)
+            if ctx.batched:
+                g = g * grad_ll.reshape((-1,) + (1,) * (g.dim() - 1))
+                if len(shape) < g.dim():  # a parameter shared by the batch: sum over trajectories
+                    g = g.sum(0)
+            else:
+                g = g * grad_ll
+            out.append(g.reshape(shape).to(device=device, dtype=dtype))
+        return (None, None, None, None, None) + tuple(out)
+
+
+def cdlgssm_marginal_log_prob(params, emissions, t_emissions=None, filter_hyperparams=None):
+    """Per-trajectory marginal log-likelihood of the linear CD Kalman filter as a differentiable torch tensor (fp64,
+    n <= 16, m <= 8, full R, no inputs: the coverage of cdk_kf_grad_f64).  Every torch leaf among F, b, L, Qc, H, d, R,
+    m0, P0 of `params` with requires_grad receives its gradient on `.backward()`; a leaf shared by a batch of
+    trajectories receives the sum over them."""
+    names = tuple(nm for nm in _KF_LEAVES if getattr(getattr(params, nm[0]), nm[1]) is not None)
+    tensors = [torch.as_tensor(getattr(getattr(params, grp), fld)) for grp, fld in names]
+    return _KFLogLik.apply(params, emissions, t_emissions, filter_hyperparams, names, *tensors)

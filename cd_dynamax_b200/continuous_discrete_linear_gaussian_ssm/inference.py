@@ -4,6 +4,7 @@ same names, argument order and result tuples; the arithmetic runs in libcdk.so o
 Batched form (what `jax.vmap` produces in the reference, src/ssm_temissions.py:555-567): emissions [N,K,m],
 t_emissions [N,K,1]; any parameter may carry a leading N as well.
 """
+import ctypes
 from typing import Any, NamedTuple, Optional
 
 import numpy as np
@@ -182,3 +183,96 @@ def cdlgssm_smoother(params: ParamsCDLGSSM, emissions, t_emissions=None,
                                  filtered_covariances=g(out[L.OUT_FP]), smoothed_means=g(sm[L.OUT_SM]),
                                  smoothed_covariances=g(sm[L.OUT_SP]),
                                  smoothed_cross_covariances=g(sm[L.OUT_SCROSS]))
+
+
+def _grad_chunk(N: int, row_bytes: int) -> int:
+    """Trajectories per launch of cdk_kf_grad whose device scratch fits half of the free device memory."""
+    free, _ = torch.cuda.mem_get_info()
+    return max(1, min(N, (free // 2) // max(row_bytes, 1)))
+
+
+def _rows(ins, lo, hi, N):
+    """The [lo, hi) trajectories of every input that carries a leading N (see _engine.run's classification)."""
+    out = {}
+    for slot, x in ins.items():
+        core = E._CORE_NDIM[slot] if E._CORE_NDIM[slot] is not None else 2
+        shp = _shape(x)
+        out[slot] = x[lo:hi] if (len(shp) == core + 1 and shp[0] == N and N > 1) else x
+    return out
+
+
+def _mm(A, B):
+    """A @ B for the small [.., n, n] blocks of the gradient, one elementwise pass per inner index: every row of a batch
+    gets the same bits whatever the batch size (a batched GEMM may pick a different kernel per batch size)."""
+    acc = A[..., :, :1] * B[..., :1, :]
+    for k in range(1, A.shape[-1]):
+        acc = acc + A[..., :, k:k + 1] * B[..., k:k + 1, :]
+    return acc
+
+
+def cdlgssm_marginal_log_prob_and_grad(params: ParamsCDLGSSM, emissions, t_emissions=None,
+                                       filter_hyperparams: Optional[KFHyperParams] = None, inputs=None):
+    """Marginal log-likelihood of `cdlgssm_filter` and its gradient with respect to the model parameters.
+
+    -> (marginal_loglik, grads): `grads` is a ParamsCDLGSSM shaped like `params` -- what
+    `jax.value_and_grad(lambda p: cdlgssm_filter(p, ...).marginal_loglik)` gives the reference's fit_sgd
+    (src/utils/optimize_utils.py:102, src/ssm_temissions.py:550-568) -- with a leading N for batched emissions (one
+    gradient per trajectory).  Leaves absent from `params` (a None bias, the input weights) are None.  It is the
+    derivative of exactly the discrete filter cdlgssm_filter runs, from cdk_kf_grad_f64 (one forward filter pass and one
+    reverse-mode launch).  The symmetric parameters (emissions.cov, initial.cov) get the symmetric part (G + G^T)/2 of
+    the entry-wise gradient G, which is what a PSD parameterisation consumes; diffusion_coefficient L and diffusion_cov
+    Qc get the chain rule through Sigma = L Qc L^T: L_bar = Sigma_bar L (Qc + Qc^T), Qc_bar = L^T Sigma_bar L.
+
+    Coverage: fp64, n <= 16, m <= 8, full R, no inputs, every solver; anything else raises NotImplementedError.  A
+    batch whose scratch does not fit half of the free device memory runs in several launches (same result, bit for bit).
+    """
+    hp = filter_hyperparams if filter_hyperparams is not None else KFHyperParams()
+    if inputs is not None and _shape(inputs)[-1] > 0:
+        raise NotImplementedError("cdlgssm_marginal_log_prob_and_grad: inputs (B, D) are not supported")
+    if _diag_r(params):
+        raise NotImplementedError("cdlgssm_marginal_log_prob_and_grad: a diagonal (1-D) emissions.cov is not supported")
+    if E.pick_dtype(emissions) != "f64":
+        raise NotImplementedError("cdlgssm_marginal_log_prob_and_grad: gradients are fp64 only")
+    kind = E.kind_of(emissions)
+    Y, T, _, batched = prepare_data(emissions, t_emissions, None)
+    N, K, m = _shape(Y)
+    n = _shape(params.emissions.weights)[-1]
+    if n > 16 or m > 8:
+        raise NotImplementedError(f"cdlgssm_marginal_log_prob_and_grad: needs n <= 16 and m <= 8 (n = {n}, m = {m})")
+    ins = _linear_inputs(params, Y, T, None, n, m, 0)
+    fields = dict(E.parse_settings(hp.diffeqsolve_settings), dt_final=float(hp.dt_final), d_u=0)
+    cols = L.grad_cols_kf(n, m)
+    d = L.new_desc()
+    d.N, d.K, d.n, d.m = 1, K, n, m
+    chunk = _grad_chunk(N, int(L.lib().cdk_scratch_bytes(ctypes.byref(d), b"cdk_kf_grad")))
+    parts = []
+    for lo in range(0, N, chunk):
+        hi = min(N, lo + chunk)
+        dev_ins = {}
+        try:
+            out = E.run("cdk_kf_grad", "f64", hi - lo, K, n, m, _rows(ins, lo, hi, N), (L.OUT_LL, L.OUT_GRAD), fields,
+                        theta_core_ndim=2, host_out=(kind != "cuda"), dev_inputs=dev_ins,
+                        out_shapes={L.OUT_GRAD: (hi - lo, cols)})
+        except L.CdkError as e:
+            raise NotImplementedError(str(e)) from e
+        G = out[L.OUT_GRAD]
+        Sb = G[:, n * n + n:2 * n * n + n].reshape(hi - lo, n, n)
+        Lm, Qc = dev_ins[L.IN_L].detach().to(G.device), dev_ins[L.IN_QC].detach().to(G.device)
+        parts.append((out[L.OUT_LL], G, _mm(_mm(Sb, Lm), Qc + Qc.transpose(-1, -2)), _mm(_mm(Lm.transpose(-1, -2), Sb), Lm)))
+    ll, G, gL, gQc = (torch.cat(p) for p in zip(*parts))
+    o = 0
+    blocks = {}
+    for name, shp in (("F", (n, n)), ("b", (n,)), ("Sigma", (n, n)), ("H", (m, n)), ("d", (m,)), ("R", (m, m)),
+                      ("m0", (n,)), ("P0", (n, n))):
+        size = int(np.prod(shp))
+        blocks[name] = G[:, o:o + size].reshape((N,) + shp)
+        o += size
+    g = lambda t: E.from_dev(_sq(t, batched), kind)
+    dyn, em = params.dynamics, params.emissions
+    grads = ParamsCDLGSSM(
+        initial=ParamsLGSSMInitial(mean=g(blocks["m0"]), cov=g(blocks["P0"])),
+        dynamics=ParamsCDLGSSMDynamics(weights=g(blocks["F"]), bias=g(blocks["b"]) if dyn.bias is not None else None,
+                                       input_weights=None, diffusion_coefficient=g(gL), diffusion_cov=g(gQc)),
+        emissions=ParamsLGSSMEmissions(weights=g(blocks["H"]), bias=g(blocks["d"]) if em.bias is not None else None,
+                                       input_weights=None, cov=g(blocks["R"])))
+    return g(ll), grads

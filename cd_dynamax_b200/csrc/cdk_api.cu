@@ -352,6 +352,24 @@ int cdk_ekf_grad_f64(const cdk_desc* d, const void* const* in, void* const* out,
   return rc;
 }
 
+int cdk_kf_grad_f64(const cdk_desc* d, const void* const* in, void* const* out, cdk_stream_t stream) {
+  if (d && (d->reserved[2] & CDK_FLAG_PREDICT_ONLY))
+    return fail(CDK_E_UNSUPPORTED, "cdk_kf_grad_f64: CDK_FLAG_PREDICT_ONLY has no log-likelihood to differentiate");
+  int rc = validate(d, in, out, ALGO_KF_FILTER);
+  if (rc != CDK_OK) return rc;
+  if (d->d_u > 0) return fail(CDK_E_UNSUPPORTED, "cdk_kf_grad_f64: inputs (d_u > 0) are not supported");
+  if (d->reserved[2] & CDK_FLAG_DIAG_R) return fail(CDK_E_UNSUPPORTED, "cdk_kf_grad_f64: CDK_FLAG_DIAG_R is not supported");
+  if (d->n > 16 || d->m > 8) return fail(CDK_E_UNSUPPORTED, "cdk_kf_grad_f64: needs n <= 16 and m <= 8");
+  if (d->reserved[3] != 0) return fail(CDK_E_UNSUPPORTED, "cdk_kf_grad_f64: desc.reserved[3] must be 0");
+  if (d->N == 0) return CDK_OK;
+  if (!out[CDK_OUT_GRAD]) return fail(CDK_E_NULL, "cdk_kf_grad_f64 needs out[CDK_OUT_GRAD]");
+  if (!out[CDK_OUT_SCRATCH]) return fail(CDK_E_NULL, "cdk_kf_grad_f64 needs out[CDK_OUT_SCRATCH] (cdk_scratch_bytes)");
+  KArgs<double> a = make_args<double>(d, in, out, ALGO_KF_FILTER);
+  rc = launch_kf_grad(a, static_cast<double*>(out[CDK_OUT_GRAD]), reinterpret_cast<cudaStream_t>(stream));
+  if (rc == CDK_E_UNSUPPORTED) return fail(rc, "cdk_kf_grad_f64: the forward pass needs the warp filter (CDK_KF_WARP=0 disables it)");
+  return rc;
+}
+
 size_t cdk_scratch_bytes(const cdk_desc* d, const char* entry_point) {
   if (!d || !entry_point) return 0;
   // the EnKF keeps its ensemble in (distributed) shared memory; the only device scratch is the optional pushforward
@@ -359,6 +377,8 @@ size_t cdk_scratch_bytes(const cdk_desc* d, const char* entry_point) {
   const bool kf = strstr(entry_point, "kf_filter") != nullptr && strstr(entry_point, "ekf") == nullptr &&
                   strstr(entry_point, "ukf") == nullptr && strstr(entry_point, "enkf") == nullptr;
   const bool ks = strstr(entry_point, "kf_smooth") != nullptr && strstr(entry_point, "ekf") == nullptr;
+  if (strstr(entry_point, "kf_grad") != nullptr && strstr(entry_point, "ekf_grad") == nullptr)
+    return (size_t)cdk::kf_grad_scratch_doubles(*d) * sizeof(double);
   if (strstr(entry_point, "ekf_grad") != nullptr)
     return (d->reserved[3] & CDK_GRAD_REVERSE) ? (size_t)d->N * (size_t)d->K * 24u * sizeof(double) : 0;
   if ((kf || ks) && (d->reserved[2] & CDK_FLAG_KEEP_PUSHFORWARD) && cdk::kf_warp_eligible(*d, ks) && d->K > 1)
@@ -408,7 +428,7 @@ static int xla_dispatch(cdk_stream_t stream, void** buffers, const char* opaque,
       {"cdk_ekf_smooth_f64", cdk_ekf_smooth_f64}, {"cdk_ekf_smooth_f32", cdk_ekf_smooth_f32},
       {"cdk_ukf_filter_f64", cdk_ukf_filter_f64}, {"cdk_ukf_filter_f32", cdk_ukf_filter_f32},
       {"cdk_enkf_filter_f64", cdk_enkf_filter_f64}, {"cdk_enkf_filter_f32", cdk_enkf_filter_f32},
-      {"cdk_ekf_grad_f64", cdk_ekf_grad_f64},
+      {"cdk_ekf_grad_f64", cdk_ekf_grad_f64},     {"cdk_kf_grad_f64", cdk_kf_grad_f64},
       {"cdk_sample_path_f64", cdk_sample_path_f64}, {"cdk_sample_path_f32", cdk_sample_path_f32},
       {"cdk_emission_moments_f64", cdk_emission_moments_f64}, {"cdk_emission_moments_f32", cdk_emission_moments_f32}};
   for (auto& e : table)

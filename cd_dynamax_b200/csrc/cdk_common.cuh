@@ -218,6 +218,8 @@ int launch_ekf_small(const KArgs<T>& a, cudaStream_t s);
 template <typename T>
 int launch_eks_small(const KArgs<T>& a, cudaStream_t s);
 int launch_ekf_l63_grad(const KArgs<double>& a, double* grad, cudaStream_t s);
+int launch_kf_grad(const KArgs<double>& a, double* grad, cudaStream_t s);  // cdk_kfwarp.cu
+long long kf_grad_scratch_doubles(const cdk_desc& d);                      // its out[CDK_OUT_SCRATCH], in doubles
 bool kf_warp_eligible(const cdk_desc& d, bool smooth);  // fp64 requests served by kf_warp_filter / kf_warp_smooth
 int set_lw_trace(void* devbuf);
 template <typename T>

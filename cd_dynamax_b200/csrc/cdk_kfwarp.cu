@@ -856,6 +856,586 @@ __global__ void __launch_bounds__(32 * KS_WPC, 2) kf_warp_smooth(const KArgs<dou
   }
 }
 
+// ======================================================================================================================
+// Reverse-mode gradient of the filter's log-likelihood (cdk_kf_grad_f64).  kf_warp_filter runs first and writes the
+// filtered and predicted moments to scratch; kf_warp_grad then walks k = K-1 .. 0 with the adjoint (mu_bar, P_bar) of the
+// predicted moments that enter update k+1, one warp per trajectory, every n x n product on the FP64 tensor cores:
+//   update VJP      (m <= 8, warp-cooperative in shared memory like the forward update),
+//   predict VJP     mu' = A mu_f + b, P' = A P_f A^T + Q,
+//   pushforward VJP the gap is re-integrated from (I, 0) stage by stage (any tableau, Dopri5 included) with the substep
+//                   start states kept at two checkpoint levels of KG_CK slots in the trajectory's scratch, then stepped
+//                   back substep by substep: the stage inputs of the substep are rebuilt in shared memory and the stage
+//                   cotangents (Ca, Cq) give A_i_bar = F^T Ca, Q_i_bar = F^T Cq + Cq F, F_bar += Ca A_i^T + 2 Cq Q_i,
+//                   Sigma_bar += Cq (Cq stays symmetric).
+// Adjoints of symmetric matrices (P, Q, S) are kept symmetric: every perturbation of the parameters that keeps Sigma, R and
+// P0 symmetric keeps them symmetric, so this gives the exact derivative along those directions.
+// ======================================================================================================================
+constexpr int KG_CK = 32;           // checkpoint slots per level; a gap of up to KG_CK^2 substeps is re-integrated once
+constexpr int KG_STATE = 16 * 32;   // one (A, Q) state in fragment layout: 16 doubles per lane
+constexpr int KG_WPC_MAX = 8;
+
+struct KgTab {
+  int S;
+  double a[6][6];  // dense Butcher matrix (a[i][j], j < i)
+  double b[6];
+};
+
+// fragment-layout state <-> global scratch (coalesced: element i of every lane is contiguous)
+__device__ __forceinline__ void kg_save(double* __restrict__ dst, const F16& A, const F16& Q) {
+  const int lane = threadIdx.x & 31;
+#pragma unroll
+  for (int i = 0; i < 8; ++i) {
+    dst[i * 32 + lane] = (&A.v[0][0][0])[i];
+    dst[(8 + i) * 32 + lane] = (&Q.v[0][0][0])[i];
+  }
+}
+__device__ __forceinline__ void kg_load(const double* __restrict__ src, F16& A, F16& Q) {
+  const int lane = threadIdx.x & 31;
+#pragma unroll
+  for (int i = 0; i < 8; ++i) {
+    (&A.v[0][0][0])[i] = src[i * 32 + lane];
+    (&Q.v[0][0][0])[i] = src[(8 + i) * 32 + lane];
+  }
+}
+
+// One explicit RK substep of (A, Q) through the stages of any tableau.  The stage inputs are accumulated in place in
+// sStg[2 st] (A) / sStg[2 st + 1] (Q), which hold them afterwards for kg_step_vjp; y is advanced in place.
+__device__ __forceinline__ void kg_step(const KgTab& tab, const double dt, const double* sF, const double* sLQL, double* sStg,
+                                        double* sT, F16& yA, F16& yQ) {
+  F16 accA = yA, accQ = yQ;
+#pragma unroll 1
+  for (int st = 0; st < tab.S; ++st) {
+    store_c<2, 2>(yA.v, sStg + (2 * st) * KW_MAT);
+    store_c<2, 2>(yQ.v, sStg + (2 * st + 1) * KW_MAT);
+  }
+  __syncwarp();
+#pragma unroll 1
+  for (int st = 0; st < tab.S; ++st) {
+    F16 kA, fq, fqt, lq;
+    mm2_shared_a(kA.v, fq.v, sF, sStg + (2 * st) * KW_MAT, sStg + (2 * st + 1) * KW_MAT);  // F A_i, F Q_i
+    store_c<2, 2>(fq.v, sT);
+    __syncwarp();
+    load_ct(fqt.v, sT);
+    load_c<2, 2>(lq.v, sLQL);
+#pragma unroll
+    for (int i = 0; i < 8; ++i) (&fq.v[0][0][0])[i] = ((&fq.v[0][0][0])[i] + (&fqt.v[0][0][0])[i]) + (&lq.v[0][0][0])[i];
+    const double w = tab.b[st] * dt;
+    if (w != 0.0) {
+#pragma unroll
+      for (int i = 0; i < 8; ++i) {
+        (&accA.v[0][0][0])[i] = fma(w, (&kA.v[0][0][0])[i], (&accA.v[0][0][0])[i]);
+        (&accQ.v[0][0][0])[i] = fma(w, (&fq.v[0][0][0])[i], (&accQ.v[0][0][0])[i]);
+      }
+    }
+#pragma unroll 1
+    for (int s2 = st + 1; s2 < tab.S; ++s2) {  // lane-local: every lane updates its own fragment entries
+      const double c = tab.a[s2][st] * dt;
+      if (c == 0.0) continue;
+      F16 iA, iQ;
+      load_c<2, 2>(iA.v, sStg + (2 * s2) * KW_MAT);
+      load_c<2, 2>(iQ.v, sStg + (2 * s2 + 1) * KW_MAT);
+#pragma unroll
+      for (int i = 0; i < 8; ++i) {
+        (&iA.v[0][0][0])[i] = fma(c, (&kA.v[0][0][0])[i], (&iA.v[0][0][0])[i]);
+        (&iQ.v[0][0][0])[i] = fma(c, (&fq.v[0][0][0])[i], (&iQ.v[0][0][0])[i]);
+      }
+      store_c<2, 2>(iA.v, sStg + (2 * s2) * KW_MAT);
+      store_c<2, 2>(iQ.v, sStg + (2 * s2 + 1) * KW_MAT);
+    }
+    __syncwarp();
+  }
+  yA = accA;
+  yQ = accQ;
+}
+
+// VJP of the substep kg_step just took (its stage inputs in sStg): (lamA, lamQ) is the cotangent of the substep's end
+// state on entry and of its start state on exit; gF / gS accumulate F_bar / Sigma_bar.  The stage buffers are overwritten
+// with the stage-input cotangents.
+__device__ __forceinline__ void kg_step_vjp(const KgTab& tab, const double dt, const double* sFt, double* sStg, double* sCa,
+                                            double* sCq, double* sT, F16& lamA, F16& lamQ, F16& gF, F16& gS) {
+#pragma unroll 1
+  for (int st = tab.S - 1; st >= 0; --st) {
+    F16 ca, cq;
+    const double w = tab.b[st] * dt;
+#pragma unroll
+    for (int i = 0; i < 8; ++i) {
+      (&ca.v[0][0][0])[i] = w * (&lamA.v[0][0][0])[i];
+      (&cq.v[0][0][0])[i] = w * (&lamQ.v[0][0][0])[i];
+    }
+#pragma unroll 1
+    for (int s2 = st + 1; s2 < tab.S; ++s2) {
+      const double c = tab.a[s2][st] * dt;
+      if (c == 0.0) continue;
+      F16 bA, bQ;
+      load_c<2, 2>(bA.v, sStg + (2 * s2) * KW_MAT);
+      load_c<2, 2>(bQ.v, sStg + (2 * s2 + 1) * KW_MAT);
+#pragma unroll
+      for (int i = 0; i < 8; ++i) {
+        (&ca.v[0][0][0])[i] = fma(c, (&bA.v[0][0][0])[i], (&ca.v[0][0][0])[i]);
+        (&cq.v[0][0][0])[i] = fma(c, (&bQ.v[0][0][0])[i], (&cq.v[0][0][0])[i]);
+      }
+    }
+    store_c<2, 2>(ca.v, sCa);
+    store_c<2, 2>(cq.v, sCq);
+    __syncwarp();
+    F16 x, y;
+    mm<false, true, 16, 2, 2>(x.v, sCa, sStg + (2 * st) * KW_MAT);       // Ca A_i^T
+    mm<false, false, 16, 2, 2>(y.v, sCq, sStg + (2 * st + 1) * KW_MAT);  // Cq Q_i
+#pragma unroll
+    for (int i = 0; i < 8; ++i) {
+      (&gF.v[0][0][0])[i] += (&x.v[0][0][0])[i] + 2.0 * (&y.v[0][0][0])[i];
+      (&gS.v[0][0][0])[i] += (&cq.v[0][0][0])[i];
+    }
+    mm2_shared_a(x.v, y.v, sFt, sCa, sCq);  // F^T Ca, F^T Cq
+    store_c<2, 2>(y.v, sT);
+    __syncwarp();
+    F16 yt;
+    load_ct(yt.v, sT);
+#pragma unroll
+    for (int i = 0; i < 8; ++i) (&y.v[0][0][0])[i] += (&yt.v[0][0][0])[i];
+    store_c<2, 2>(x.v, sStg + (2 * st) * KW_MAT);
+    store_c<2, 2>(y.v, sStg + (2 * st + 1) * KW_MAT);
+    __syncwarp();
+  }
+#pragma unroll 1
+  for (int st = 0; st < tab.S; ++st) {  // the start state feeds every stage input with coefficient 1
+    F16 bA, bQ;
+    load_c<2, 2>(bA.v, sStg + (2 * st) * KW_MAT);
+    load_c<2, 2>(bQ.v, sStg + (2 * st + 1) * KW_MAT);
+#pragma unroll
+    for (int i = 0; i < 8; ++i) {
+      (&lamA.v[0][0][0])[i] += (&bA.v[0][0][0])[i];
+      (&lamQ.v[0][0][0])[i] += (&bQ.v[0][0][0])[i];
+    }
+  }
+  __syncwarp();
+}
+
+struct KgLayout {
+  // per-warp shared memory (doubles): P_bar, the work slots, small vectors, Cholesky factors, checkpoint clocks
+  static constexpr int VEC = 16 * 4 + 8 * 4 + 72 * 2;
+  static constexpr int CLOCK = (int)((sizeof(StepClock<double>) + 7) / 8);
+  static __host__ __device__ int slots(int S) { return 2 * S + 3 > 7 ? 2 * S + 3 : 7; }
+  static __host__ __device__ int per_warp(int S) { return (1 + slots(S)) * KW_MAT + VEC + 2 * KG_CK * CLOCK; }
+  // per-trajectory scratch (doubles): FM, FP, PM, PP of the forward pass ([N][K][...] each), the checkpoints, the status
+  static __host__ __device__ long long moments(int K, int n) { return (long long)K * (2 * n + 2 * n * n); }
+  static __host__ __device__ long long per_traj(int K, int n) { return moments(K, n) + 2 * KG_CK * KG_STATE + 1; }
+};
+
+__global__ void __launch_bounds__(32 * KG_WPC_MAX, 1) kf_warp_grad(const KArgs<double> a, const __grid_constant__ KgTab tab,
+                                                                  const int model_per_warp, const int per_warp,
+                                                                  const double* __restrict__ sc, double* __restrict__ ckpt,
+                                                                  const int* __restrict__ status, double* __restrict__ grad) {
+  extern __shared__ __align__(16) double kw_smem[];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, gid = lane >> 2, tig = lane & 3;
+  const int wpc = blockDim.x >> 5;
+  const cdk_desc& d = a.d;
+  const int n = d.n, m = d.m, K = d.K;
+  const long long N = d.N;
+  const long long traj = (long long)blockIdx.x * wpc + warp;
+  double* model = kw_smem + (model_per_warp ? warp * KwSmemCounts::PER_MODEL : 0);
+  double* wbase = kw_smem + (model_per_warp ? wpc : 1) * KwSmemCounts::PER_MODEL + warp * per_warp;
+  double* sF = model;
+  double* sLQL = sF + KW_MAT;
+  double* sH = sLQL + KW_MAT;
+  double* sR = sH + KW_MAT8;
+  double* sb = sR + KW_MAT8;
+  double* sd = sb + 16;
+  double* sFt = model + KW_RK_OFF;  // F^T in the slot of the filter's RK map
+  double* sPb = wbase;
+  double* W = sPb + KW_MAT;
+  const int nslots = KgLayout::slots(tab.S);
+  double* smu = W + nslots * KW_MAT;  // predicted mean entering the update
+  double* smub = smu + 16;            // adjoint of the mean
+  double* smf = smub + 16;            // filtered mean
+  double* sv = smf + 16;
+  double* sr = sv + 16;
+  double* sz = sr + 8;
+  double* srb = sz + 8;
+  double* sy = srb + 8;
+  double* sL0 = sy + 8;   // [8][9] Cholesky factor of S (log-likelihood)
+  double* sLb = sL0 + 72;  // [8][9] Cholesky factor of sym(S) + 1e-9 I (gain)
+  StepClock<double>* ckc1 = reinterpret_cast<StepClock<double>*>(sLb + 72);
+  StepClock<double>* ckc2 = reinterpret_cast<StepClock<double>*>(sLb + 72 + KG_CK * KgLayout::CLOCK);
+
+  const long long tj = traj < N ? traj : N - 1;
+  if (model_per_warp || warp == 0) {
+    load_model_kw(a, tj, model, W, W + KW_MAT, W + 2 * KW_MAT);
+    __syncwarp();
+    for (int e = lane; e < KW_MAT; e += 32) {
+      const int i = e / KW_LD, j = e - i * KW_LD;
+      sFt[e] = j < 16 ? sF[j * KW_LD + i] : 0.0;
+    }
+  }
+  __syncthreads();  // the only CTA-wide barrier: the shared model block is ready
+  if (traj >= N) return;
+  const int cols = 3 * n * n + m * n + m * m + 2 * n + m;
+  double* grow = grad + traj * (long long)cols;
+  if (status[traj] != 0) {
+    for (int e = lane; e < cols; e += 32) grow[e] = NAN;
+    return;
+  }
+  for (int e = lane; e < per_warp; e += 32) wbase[e] = 0.0;
+  __syncwarp();
+
+  const long long NK = N * (long long)K;
+  const double* FMg = sc + traj * (long long)K * n;
+  const double* FPg = sc + NK * n + traj * (long long)K * n * n;
+  const double* PMg = sc + NK * (n + n * n) + traj * (long long)K * n;
+  const double* PPg = sc + NK * (2 * n + n * n) + traj * (long long)K * n * n;
+  double* ck1 = ckpt + traj * (long long)(2 * KG_CK * KG_STATE);
+  double* ck2 = ck1 + KG_CK * KG_STATE;
+  const double* __restrict__ Y = a.in[CDK_IN_Y] + traj * a.in_stride[CDK_IN_Y];
+  const double* __restrict__ Tm = a.in[CDK_IN_T] + traj * a.in_stride[CDK_IN_T];
+  const double dt0 = d.dt0;
+
+  F16 gF, gS;
+#pragma unroll
+  for (int i = 0; i < 8; ++i) (&gF.v[0][0][0])[i] = (&gS.v[0][0][0])[i] = 0.0;
+  double gH[1][2][2] = {{{0.0, 0.0}, {0.0, 0.0}}}, gR[1][1][2] = {{{0.0, 0.0}}};
+  double gb = 0.0, gd = 0.0;
+
+  for (int k = K - 1; k >= 0; --k) {
+    if (k < K - 1) {
+      // ================= gap [t_k, t_{k+1}]: forward from (I, 0), substep starts at checkpoint level 1 =================
+      const double t0 = Tm[k], t1 = Tm[k + 1];
+      StepClock<double> cnt(t0, t1, dt0);
+      while (cnt.running()) cnt.advance();  // status 0: the filter took these cnt.n <= max_steps substeps
+      const int q = cnt.n;
+      const int s1 = q > KG_CK ? (q + KG_CK - 1) / KG_CK : 1;
+      F16 yA, yQ;
+#pragma unroll
+      for (int rb = 0; rb < 2; ++rb)
+#pragma unroll
+        for (int cb = 0; cb < 2; ++cb)
+#pragma unroll
+          for (int r = 0; r < 2; ++r) {
+            yA.v[rb][cb][r] = (8 * rb + gid == 8 * cb + 2 * tig + r) ? 1.0 : 0.0;
+            yQ.v[rb][cb][r] = 0.0;
+          }
+      {
+        StepClock<double> clk(t0, t1, dt0);
+        for (int i = 0; i < q; ++i) {
+          if (i % s1 == 0) {
+            kg_save(ck1 + (i / s1) * KG_STATE, yA, yQ);
+            if (lane == 0) ckc1[i / s1] = clk;
+          }
+          kg_step(tab, clk.dt(), sF, sLQL, W + 3 * KW_MAT, W + 2 * KW_MAT, yA, yQ);
+          clk.advance();
+        }
+      }
+      // ================= predict VJP: mu' = A mu_f + b, P' = A P_f A^T + Q  (cotangents smub, sPb) =================
+      double* sA = W + 3 * KW_MAT;
+      double* sPf = W + 4 * KW_MAT;
+      double* sT1 = W + 5 * KW_MAT;
+      F16 lamA, lamQ;
+      {
+        __syncwarp();
+        store_c<2, 2>(yA.v, sA);
+        F16 pf;
+        load_global(pf.v, FPg + (long long)k * n * n, n);
+        store_c<2, 2>(pf.v, sPf);
+        if (lane < 16) smf[lane] = lane < n ? FMg[(long long)k * n + lane] : 0.0;
+        if (lane < n) gb += smub[lane];
+        __syncwarp();
+        F16 t1m, t2m;
+        mm<false, false, 16, 2, 2>(t1m.v, sPb, sA);  // P'_bar A
+        store_c<2, 2>(t1m.v, sT1);
+        __syncwarp();
+        mm<false, false, 16, 2, 2>(t2m.v, sT1, sPf);  // P'_bar A P_f
+        load_c<2, 2>(lamQ.v, sPb);
+#pragma unroll
+        for (int rb = 0; rb < 2; ++rb)
+#pragma unroll
+          for (int cb = 0; cb < 2; ++cb)
+#pragma unroll
+            for (int r = 0; r < 2; ++r) {
+              const int i = 8 * rb + gid, j = 8 * cb + 2 * tig + r;
+              lamA.v[rb][cb][r] = 2.0 * t2m.v[rb][cb][r] + smub[i] * smf[j];
+            }
+        if (lane < 16) {
+          double s = 0.0;
+          for (int qq = 0; qq < n; ++qq) s += sA[qq * KW_LD + lane] * smub[qq];
+          sv[lane] = lane < n ? s : 0.0;
+        }
+        F16 pb, pbt;
+        mm<true, false, 16, 2, 2>(pb.v, sA, sT1);  // A^T P'_bar A
+        __syncwarp();
+        if (lane < 16) smub[lane] = sv[lane];
+        store_c<2, 2>(pb.v, sT1);
+        __syncwarp();
+        load_ct(pbt.v, sT1);
+#pragma unroll
+        for (int i = 0; i < 8; ++i) (&pb.v[0][0][0])[i] = 0.5 * ((&pb.v[0][0][0])[i] + (&pbt.v[0][0][0])[i]);
+        store_c<2, 2>(pb.v, sPb);
+        __syncwarp();
+      }
+      // ================= pushforward VJP, substep by substep from the last =================
+      double* sCa = W;
+      double* sCq = W + KW_MAT;
+      double* sT = W + 2 * KW_MAT;
+      double* sStg = W + 3 * KW_MAT;
+      const int nseg = q > 0 ? (q + s1 - 1) / s1 : 0;
+      for (int seg = nseg - 1; seg >= 0; --seg) {
+        const int i0 = seg * s1, len = (q - i0 < s1 ? q - i0 : s1);
+        const int s2 = len > KG_CK ? (len + KG_CK - 1) / KG_CK : 1;
+        if (len > 1) {  // level 2: the substep starts of this segment
+          StepClock<double> clk = ckc1[seg];
+          kg_load(ck1 + seg * KG_STATE, yA, yQ);
+          for (int u = 0; u < len - 1; ++u) {
+            if (u % s2 == 0) {
+              kg_save(ck2 + (u / s2) * KG_STATE, yA, yQ);
+              if (lane == 0) ckc2[u / s2] = clk;
+            }
+            kg_step(tab, clk.dt(), sF, sLQL, sStg, sT, yA, yQ);
+            clk.advance();
+          }
+          if ((len - 1) % s2 == 0) {
+            kg_save(ck2 + ((len - 1) / s2) * KG_STATE, yA, yQ);
+            if (lane == 0) ckc2[(len - 1) / s2] = clk;
+          }
+          __syncwarp();
+        }
+        for (int u = len - 1; u >= 0; --u) {
+          StepClock<double> clk = len > 1 ? ckc2[u / s2] : ckc1[seg];
+          kg_load(len > 1 ? ck2 + (u / s2) * KG_STATE : ck1 + seg * KG_STATE, yA, yQ);
+          for (int v = (len > 1 ? (u / s2) * s2 : u); v < u; ++v) {
+            kg_step(tab, clk.dt(), sF, sLQL, sStg, sT, yA, yQ);
+            clk.advance();
+          }
+          kg_step(tab, clk.dt(), sF, sLQL, sStg, sT, yA, yQ);  // rebuilds the stage inputs of substep i0 + u
+          kg_step_vjp(tab, clk.dt(), sFt, sStg, sCa, sCq, sT, lamA, lamQ, gF, gS);
+        }
+      }
+    }
+    // ================= update VJP at k (cotangents of the filtered moments in smub / sPb) =================
+    {
+      double* sP = W;
+      double* sT = W + KW_MAT;
+      double* sG = W + 2 * KW_MAT;
+      double* sS = sG + KW_MAT8;
+      double* sKt = W + 3 * KW_MAT;
+      double* sKtPb = sKt + KW_MAT8;
+      double* sGb = W + 4 * KW_MAT;
+      double* sSb = sGb + KW_MAT8;
+      double* sWm = W + 5 * KW_MAT;
+      double* sX8 = sWm + KW_MAT8;
+      double* sSi = W + 6 * KW_MAT;
+      {
+        F16 p;
+        if (k == 0) {
+          load_global(p.v, a.in[CDK_IN_P0] + traj * a.in_stride[CDK_IN_P0], n);
+          if (lane < 16) smu[lane] = lane < n ? (a.in[CDK_IN_M0] + traj * a.in_stride[CDK_IN_M0])[lane] : 0.0;
+        } else {
+          load_global(p.v, PPg + (long long)(k - 1) * n * n, n);
+          if (lane < 16) smu[lane] = lane < n ? PMg[(long long)(k - 1) * n + lane] : 0.0;
+        }
+        store_c<2, 2>(p.v, sP);
+        if (lane < 8) sy[lane] = lane < m ? Y[(long long)k * m + lane] : 0.0;
+      }
+      __syncwarp();
+      double hp[1][2][2];
+      mm<false, false, 16, 1, 2>(hp, sH, sP);  // G = H P
+      store_c<1, 2>(hp, sG);
+      store_c<1, 2>(hp, sKt);
+      if (lane < 8) {
+        double s = 0.0;
+        if (lane < m) {
+          s = sy[lane] - sd[lane];
+          for (int qq = 0; qq < n; ++qq) s -= sH[lane * KW_LD + qq] * smu[qq];
+        }
+        sr[lane] = s;
+      }
+      __syncwarp();
+      {
+        double sf[1][1][2];
+        mm<false, true, 16, 1, 1>(sf, sG, sH);  // S = H P H^T + R
+        sS[gid * KW_LD + 2 * tig] = sf[0][0][0] + sR[gid * KW_LD + 2 * tig];
+        sS[gid * KW_LD + 2 * tig + 1] = sf[0][0][1] + sR[gid * KW_LD + 2 * tig + 1];
+      }
+      __syncwarp();
+      for (int pass = 0; pass < 2; ++pass) {  // chol(S) and chol(sym(S) + 1e-9 I), as the filter
+        double* Lf = pass ? sLb : sL0;
+        for (int j = 0; j < m; ++j) {
+          if (lane >= j && lane < m) {
+            double sjj = sS[j * KW_LD + j] + (pass ? 1e-9 : 0.0);
+            for (int qq = 0; qq < j; ++qq) sjj -= Lf[j * 9 + qq] * Lf[j * 9 + qq];
+            const double dj = sqrt(sjj);
+            if (lane == j) {
+              Lf[j * 9 + j] = dj;
+            } else {
+              double v = pass ? 0.5 * (sS[lane * KW_LD + j] + sS[j * KW_LD + lane]) : sS[lane * KW_LD + j];
+              for (int qq = 0; qq < j; ++qq) v -= Lf[lane * 9 + qq] * Lf[j * 9 + qq];
+              Lf[lane * 9 + j] = v / dj;
+            }
+          }
+          __syncwarp();
+        }
+      }
+      if (lane < m) {  // column `lane` of S^-1 (un-boosted factor), in place in sSi
+        for (int i = 0; i < m; ++i) {
+          double v = i == lane ? 1.0 : 0.0;
+          for (int qq = 0; qq < i; ++qq) v -= sL0[i * 9 + qq] * sSi[qq * KW_LD + lane];
+          sSi[i * KW_LD + lane] = v / sL0[i * 9 + i];
+        }
+        for (int i = m - 1; i >= 0; --i) {
+          double v = sSi[i * KW_LD + lane];
+          for (int qq = i + 1; qq < m; ++qq) v -= sL0[qq * 9 + i] * sSi[qq * KW_LD + lane];
+          sSi[i * KW_LD + lane] = v / sL0[i * 9 + i];
+        }
+      } else if (lane >= 16 && lane < 16 + n) {  // K^T = (sym(S) + 1e-9 I)^-1 G, column lane - 16, in place in sKt
+        const int c = lane - 16;
+        for (int i = 0; i < m; ++i) {
+          double v = sKt[i * KW_LD + c];
+          for (int qq = 0; qq < i; ++qq) v -= sLb[i * 9 + qq] * sKt[qq * KW_LD + c];
+          sKt[i * KW_LD + c] = v / sLb[i * 9 + i];
+        }
+        for (int i = m - 1; i >= 0; --i) {
+          double v = sKt[i * KW_LD + c];
+          for (int qq = i + 1; qq < m; ++qq) v -= sLb[qq * 9 + i] * sKt[qq * KW_LD + c];
+          sKt[i * KW_LD + c] = v / sLb[i * 9 + i];
+        }
+      }
+      __syncwarp();
+      if (lane < 8) {  // z = S^-1 r;  r_bar = K^T mu_f_bar - z
+        double z = 0.0, kb = 0.0;
+        if (lane < m) {
+          for (int qq = 0; qq < m; ++qq) z += sSi[lane * KW_LD + qq] * sr[qq];
+          for (int qq = 0; qq < n; ++qq) kb += sKt[lane * KW_LD + qq] * smub[qq];
+        }
+        sz[lane] = z;
+        srb[lane] = lane < m ? kb - z : 0.0;
+      }
+      {
+        double x[1][2][2];
+        mm<false, false, 16, 1, 2>(x, sKt, sPb);  // K^T P_f_bar
+        store_c<1, 2>(x, sKtPb);
+      }
+      __syncwarp();
+      double sbar[1][1][2];
+      {
+        double kpk[1][1][2], u[1][2][2];
+        mm<false, true, 16, 1, 1>(kpk, sKtPb, sKt);  // K^T P_f_bar K
+        mm<false, false, 8, 1, 2>(u, sS, sKtPb);     // S K^T P_f_bar
+#pragma unroll
+        for (int r = 0; r < 2; ++r) {
+          const int i = gid, j = 2 * tig + r;
+          sbar[0][0][r] = (i < m && j < m) ? 0.5 * sz[i] * sz[j] - 0.5 * sSi[i * KW_LD + j] - kpk[0][0][r] : 0.0;
+        }
+#pragma unroll
+        for (int cb = 0; cb < 2; ++cb)
+#pragma unroll
+          for (int r = 0; r < 2; ++r) {  // K_bar^T = r mu_f_bar^T - 2 S K^T P_f_bar
+            const int i = gid, j = 8 * cb + 2 * tig + r;
+            u[0][cb][r] = i < m ? sr[i] * smub[j] - 2.0 * u[0][cb][r] : 0.0;
+          }
+        store_c<1, 2>(u, sGb);
+      }
+      __syncwarp();
+      if (lane < n) {  // G_bar = (sym(S) + 1e-9 I)^-1 K_bar^T, column `lane`, in place in sGb
+        for (int i = 0; i < m; ++i) {
+          double v = sGb[i * KW_LD + lane];
+          for (int qq = 0; qq < i; ++qq) v -= sLb[i * 9 + qq] * sGb[qq * KW_LD + lane];
+          sGb[i * KW_LD + lane] = v / sLb[i * 9 + i];
+        }
+        for (int i = m - 1; i >= 0; --i) {
+          double v = sGb[i * KW_LD + lane];
+          for (int qq = i + 1; qq < m; ++qq) v -= sLb[qq * 9 + i] * sGb[qq * KW_LD + lane];
+          sGb[i * KW_LD + lane] = v / sLb[i * 9 + i];
+        }
+      }
+      __syncwarp();
+      {
+        double gk[1][1][2];
+        mm<false, true, 16, 1, 1>(gk, sGb, sKt);  // G_bar K
+        store_c<1, 1>(gk, sX8);
+        __syncwarp();
+#pragma unroll
+        for (int r = 0; r < 2; ++r) {  // S_bar -= sym(G_bar K)
+          const int i = gid, j = 2 * tig + r;
+          sbar[0][0][r] -= 0.5 * (gk[0][0][r] + sX8[j * KW_LD + i]);
+          gR[0][0][r] += sbar[0][0][r];
+        }
+        store_c<1, 1>(sbar, sSb);
+      }
+      __syncwarp();
+      {
+        double p1[1][2][2], p2[1][2][2], p3[1][2][2], gbv[1][2][2];
+        mm<false, false, 8, 1, 2>(p1, sSb, sG);   // S_bar G
+        mm<false, false, 16, 1, 2>(p2, sGb, sP);  // G_bar P
+        mm<false, false, 8, 1, 2>(p3, sSb, sH);   // S_bar H
+        load_c<1, 2>(gbv, sGb);
+#pragma unroll
+        for (int cb = 0; cb < 2; ++cb)
+#pragma unroll
+          for (int r = 0; r < 2; ++r) {
+            const int i = gid, j = 8 * cb + 2 * tig + r;
+            gH[0][cb][r] += 2.0 * p1[0][cb][r] + p2[0][cb][r] - srb[i] * smu[j];
+            p3[0][cb][r] += gbv[0][cb][r];  // W = S_bar H + G_bar
+          }
+        store_c<1, 2>(p3, sWm);
+      }
+      if (lane < m) gd -= srb[lane];
+      if (lane < n) {  // mu_bar = mu_f_bar - H^T r_bar
+        double s = 0.0;
+        for (int i = 0; i < m; ++i) s += sH[i * KW_LD + lane] * srb[i];
+        smub[lane] -= s;
+      }
+      __syncwarp();
+      {
+        F16 X, Xt, pb;
+        mm<true, false, 8, 2, 2>(X.v, sH, sWm);  // H^T W
+        store_c<2, 2>(X.v, sT);
+        __syncwarp();
+        load_ct(Xt.v, sT);
+        load_c<2, 2>(pb.v, sPb);
+#pragma unroll
+        for (int i = 0; i < 8; ++i)
+          (&pb.v[0][0][0])[i] += 0.5 * ((&X.v[0][0][0])[i] + (&Xt.v[0][0][0])[i]);  // P_bar = P_f_bar + H^T S_bar H + sym(H^T G_bar)
+        __syncwarp();
+        store_c<2, 2>(pb.v, sPb);
+        __syncwarp();
+      }
+    }
+  }
+  // ================= gradient row: F | b | Sigma (sym) | H | d | R (sym) | m0 | P0 (sym) =================
+  double* sT = W;
+  store_global(gF.v, grow, n);
+  if (lane < n) grow[n * n + lane] = gb;
+  store_c<2, 2>(gS.v, sT);
+  __syncwarp();
+  {
+    F16 t;
+    load_ct(t.v, sT);
+#pragma unroll
+    for (int i = 0; i < 8; ++i) (&gS.v[0][0][0])[i] = 0.5 * ((&gS.v[0][0][0])[i] + (&t.v[0][0][0])[i]);
+  }
+  store_global(gS.v, grow + n * n + n, n);
+  double* gHrow = grow + 2 * n * n + n;
+#pragma unroll
+  for (int cb = 0; cb < 2; ++cb)
+#pragma unroll
+    for (int r = 0; r < 2; ++r) {
+      const int i = gid, j = 8 * cb + 2 * tig + r;
+      if (i < m && j < n) gHrow[i * n + j] = gH[0][cb][r];
+    }
+  if (lane < m) gHrow[m * n + lane] = gd;
+  double* sX8 = W + KW_MAT;
+  __syncwarp();
+  store_c<1, 1>(gR, sX8);
+  __syncwarp();
+  double* gRrow = gHrow + m * n + m;
+#pragma unroll
+  for (int r = 0; r < 2; ++r) {
+    const int i = gid, j = 2 * tig + r;
+    if (i < m && j < m) gRrow[i * m + j] = 0.5 * (gR[0][0][r] + sX8[j * KW_LD + i]);
+  }
+  if (lane < n) gRrow[m * m + lane] = smub[lane];
+  F16 p0;
+  load_c<2, 2>(p0.v, sPb);
+  store_global(p0.v, gRrow + m * m + n, n);
+}
+
 }  // namespace
 
 // Fast path coverage: KF filter and type-1 smoother, fp64, n <= 16, m <= 8, no inputs, every solver of the registry (chain
@@ -938,6 +1518,56 @@ int launch_kf_warp<double>(int algo, const KArgs<double>& a, cudaStream_t s) {
   kf<<<(unsigned)blocks, 32 * KW_WPC, smem, s>>>(a, tab, model_per_warp, use_rk);
   note_launch();
   return check_launch("kf_warp_filter");
+}
+
+long long kf_grad_scratch_doubles(const cdk_desc& d) { return d.N * KgLayout::per_traj(d.K, d.n); }
+
+// Gradient of the log-likelihood of kf_warp_filter (cdk_kf_grad_f64): the forward filter into scratch, then kf_warp_grad.
+int launch_kf_grad(const KArgs<double>& a, double* grad, cudaStream_t s) {
+  const cdk_desc& d = a.d;
+  double* sc = static_cast<double*>(a.out[CDK_OUT_SCRATCH]);
+  const long long NK = d.N * (long long)d.K;
+  const int n = d.n;
+  int* status = a.out[CDK_OUT_STATUS] ? static_cast<int*>(a.out[CDK_OUT_STATUS])
+                                      : reinterpret_cast<int*>(sc + d.N * KgLayout::per_traj(d.K, n) - d.N);
+  KArgs<double> f = a;
+  f.d.reserved[2] &= ~CDK_FLAG_KEEP_PUSHFORWARD;
+  f.out[CDK_OUT_FM] = sc;
+  f.out[CDK_OUT_FP] = sc + NK * n;
+  f.out[CDK_OUT_PM] = sc + NK * (n + n * n);
+  f.out[CDK_OUT_PP] = sc + NK * (2 * n + n * n);
+  f.out[CDK_OUT_LLCUM] = nullptr;
+  f.out[CDK_OUT_STATUS] = status;
+  f.out[CDK_OUT_SCRATCH] = nullptr;
+  f.out[CDK_OUT_GRAD] = nullptr;
+  int rc = launch_kf_warp<double>(ALGO_KF_FILTER, f, s);
+  if (rc != CDK_OK) return rc;
+  RtTab rt;
+  if (!fill_rt_tab(d.solver, rt)) return CDK_E_ENUM;
+  KgTab tab;
+  tab.S = rt.S;
+  for (int i = 0; i < 6; ++i) {
+    tab.b[i] = rt.b[i];
+    for (int j = 0; j < 6; ++j) tab.a[i][j] = 0.0;
+    for (int q = 0; q < rt.nnz[i]; ++q) tab.a[i][rt.col[i][q]] = rt.val[i][q];
+  }
+  const uint32_t model_mask = (1u << CDK_IN_F) | (1u << CDK_IN_L) | (1u << CDK_IN_QC) | (1u << CDK_IN_H) | (1u << CDK_IN_R) |
+                              (1u << CDK_IN_B) | (1u << CDK_IN_D);
+  const int model_per_warp = (d.batched_mask & model_mask) != 0;
+  // as many warps as the 227 KB of one CTA hold (the stage buffers of Dopri5 are the largest case)
+  const int per_warp = KgLayout::per_warp(tab.S);
+  const size_t budget = 227 * 1024 / sizeof(double) - (model_per_warp ? 0 : KwSmemCounts::PER_MODEL);
+  int wpc = (int)(budget / (per_warp + (model_per_warp ? KwSmemCounts::PER_MODEL : 0)));
+  wpc = wpc > KG_WPC_MAX ? KG_WPC_MAX : wpc;
+  const size_t smem = sizeof(double) * ((model_per_warp ? wpc : 1) * KwSmemCounts::PER_MODEL + (size_t)wpc * per_warp);
+  const long long blocks = (d.N + wpc - 1) / wpc;
+  if (blocks > 2147483647LL) return CDK_E_SIZE;
+  if (cudaFuncSetAttribute(kf_warp_grad, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
+    return check_launch("cudaFuncSetAttribute(kf_warp_grad)");
+  kf_warp_grad<<<(unsigned)blocks, 32 * wpc, smem, s>>>(a, tab, model_per_warp, per_warp, sc, sc + NK * (2 * n + 2 * n * n),
+                                                          status, grad);
+  note_launch();
+  return check_launch("kf_warp_grad");
 }
 
 template int launch_kf_warp<float>(int, const KArgs<float>&, cudaStream_t);

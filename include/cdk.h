@@ -104,7 +104,8 @@ enum {
   CDK_OUT_SCROSS, /* smoothed cross terms  [N,K-1,n,n] (type 1; NaN for type 2)                    */
   CDK_OUT_STATUS, /* int32 [N]: 0 ok, 1 non-finite result (non-PD / NaN), 2 max_steps exceeded      */
   CDK_OUT_SCRATCH,/* device scratch of cdk_scratch_bytes() bytes (CD-KF pushforward cache), else NULL */
-  CDK_OUT_GRAD,   /* cdk_ekf_grad_f64: d marginal log-likelihood / d parameters  [N, CDK_GRAD_COLS_L63]    */
+  CDK_OUT_GRAD,   /* d marginal log-likelihood / d parameters: cdk_ekf_grad_f64 [N, CDK_GRAD_COLS_L63],
+                   * cdk_kf_grad_f64 [N, CDK_GRAD_COLS_KF(n, m)]                                               */
   CDK_NUM_OUT
 };
 
@@ -132,7 +133,7 @@ typedef struct cdk_desc {
   double alpha, beta, kappa;    /* ukf (inference_ukf.py:31-33) */
   uint64_t rng_seed;      /* enkf: Philox4x32-10 key */
   uint64_t rng_offset;    /* enkf: added to the trajectory index in the counter (sharding across GPUs) */
-  int32_t reserved[4];    /* [0], [1]: absent-slot masks of the XLA adaptor; [2]: CDK_FLAG_* bits; [3]: cdk_ekf_grad groups */
+  int32_t reserved[4];    /* [0], [1]: absent-slot masks of the XLA adaptor; [2]: CDK_FLAG_* bits; [3]: cdk_ekf_grad groups (0 for cdk_kf_grad) */
 } cdk_desc;
 
 /* reserved[2] bit 0: keep the pushforward.  cdk_kf_filter_f64 then also writes (A_k, Q_k) of every gap k < K-1 into
@@ -198,6 +199,19 @@ CDK_DECL(cdk_enkf_filter_f32);
  * of ~2.2 per column.  Without the bit (or without scratch) the forward-mode kernels run, one launch per requested column. */
 #define CDK_GRAD_REVERSE 128
 CDK_DECL(cdk_ekf_grad_f64);
+/* Log-likelihood (out[CDK_OUT_LL]), status (out[CDK_OUT_STATUS]) and reverse-mode gradient (out[CDK_OUT_GRAD],
+ * [N, CDK_GRAD_COLS_KF(n, m)]) of the linear CD Kalman filter, for the same descriptor and inputs as cdk_kf_filter_f64:
+ * what jax.value_and_grad(marginal_log_prob) hands the reference's fit_sgd for ContDiscreteLinearGaussianSSM.  The forward
+ * pass IS cdk_kf_filter_f64 (the log-likelihood is bit-identical), its moments go to out[CDK_OUT_SCRATCH] (required,
+ * cdk_scratch_bytes(desc, "cdk_kf_grad") bytes, linear in N), then one backward launch re-integrates every gap and steps
+ * back through it.  Columns, row-major blocks in this order: F (n*n, entry-wise) | b (n) | Sigma = L Qc L^T (n*n) |
+ * H (m*n) | d (m) | R (m*m) | m0 (n) | P0 (n*n).  Symmetric parameters (Sigma, R, P0) get the symmetric part (G + G^T)/2
+ * of the entry-wise gradient G, i.e. the derivative along symmetric directions.  A trajectory whose status is not 0 gets
+ * a NaN row.  Coverage: fp64, n <= 16, m <= 8, every solver, shared or batched parameters; d_u > 0, CDK_FLAG_DIAG_R,
+ * CDK_FLAG_PREDICT_ONLY, n > 16 or m > 8 return CDK_E_UNSUPPORTED, a NULL out[CDK_OUT_GRAD] or out[CDK_OUT_SCRATCH]
+ * CDK_E_NULL (host-side checks, before any CUDA call).  desc.reserved[3] must be 0. */
+#define CDK_GRAD_COLS_KF(n, m) (3 * (n) * (n) + (m) * (n) + (m) * (m) + 2 * (n) + (m))
+CDK_DECL(cdk_kf_grad_f64);
 
 /* Forward sample paths of the model (cdnlgssm_path_sample, cd_nonlinear/models.py:525-656; what
  * SSM.sample_batch(..., transition_type="path") vmaps, src/ssm_temissions.py:187-225): x_0 ~ N(m0, P0), x_k = SDE solve of
