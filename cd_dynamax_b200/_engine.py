@@ -16,7 +16,23 @@ _NP_DT = {"f64": np.float64, "f32": np.float32}
 # core (per-trajectory) rank of every input slot
 _CORE_NDIM = {L.IN_Y: 2, L.IN_T: 1, L.IN_U: 2, L.IN_M0: 1, L.IN_P0: 2, L.IN_F: None, L.IN_B: 1, L.IN_BU: 2,
               L.IN_L: 2, L.IN_QC: 2, L.IN_H: 2, L.IN_D: 1, L.IN_DU: 2, L.IN_R: 2, L.IN_FM: 2, L.IN_FP: 3}
-_SLOT_NAMES = {L.IN_Y: "IN_Y", L.IN_T: "IN_T", L.IN_U: "IN_U"}
+_SLOT_NAMES = {L.IN_Y: "IN_Y", L.IN_T: "IN_T", L.IN_U: "IN_U", L.IN_M0: "IN_M0", L.IN_P0: "IN_P0", L.IN_F: "IN_F",
+               L.IN_B: "IN_B", L.IN_BU: "IN_BU", L.IN_L: "IN_L", L.IN_QC: "IN_QC", L.IN_H: "IN_H", L.IN_D: "IN_D",
+               L.IN_DU: "IN_DU", L.IN_R: "IN_R", L.IN_FM: "IN_FM", L.IN_FP: "IN_FP"}
+
+
+def _core_shapes(K: int, n: int, m: int, desc_fields: dict, theta_core_ndim: int) -> dict:
+    """Per-trajectory shape of every input slot: exactly the slot_elems (cdk_api.cu) entries a kernel reads from it."""
+    flags = int(desc_fields.get("flags", 0))
+    d_u = int(desc_fields.get("d_u", 0))
+    # a forecast and a sampler started from a fixed state read K + 1 time stamps (t_init first), every other entry point K
+    t_cols = K + 1 if flags & (L.FLAG_PREDICT_ONLY | L.FLAG_FIXED_INIT) else K
+    return {
+        L.IN_Y: (K, m), L.IN_T: (t_cols,), L.IN_U: (K, d_u), L.IN_M0: (n,), L.IN_P0: (n, n),
+        L.IN_F: (n, n) if theta_core_ndim == 2 else (int(desc_fields.get("n_theta", 0)),),
+        L.IN_B: (n,), L.IN_BU: (n, d_u), L.IN_L: (n, n), L.IN_QC: (n, n), L.IN_H: (m, n), L.IN_D: (m,),
+        L.IN_DU: (m, d_u), L.IN_R: (m,) if flags & L.FLAG_DIAG_R else (m, m), L.IN_FM: (K, n), L.IN_FP: (K, n, n),
+    }
 
 
 def device():
@@ -111,32 +127,13 @@ def _host_tensor(x, dt: str) -> torch.Tensor:
     return torch.from_numpy(np.ascontiguousarray(np.asarray(x), dtype=_NP_DT[dt]))
 
 
-def run(entry: str, dt: str, N: int, K: int, n: int, m: int, inputs: Dict[int, object], want: Sequence[int],
-        desc_fields: dict, theta_core_ndim: int = 1, scross_rows: Optional[int] = None,
-        status: Optional[torch.Tensor] = None, host_out: bool = False,
-        dev_inputs: Optional[dict] = None, scratch: Optional[torch.Tensor] = None,
-        core_ndim_override: Optional[dict] = None,
-        out_shapes: Optional[dict] = None) -> Dict[int, torch.Tensor]:
-    """Call one C-ABI entry point. `inputs` maps slot -> array-like (None = absent); a leading N marks it batched.
-    The time stamps, emissions and inputs must have the per-trajectory shapes [K] ([K + 1] for a forecast or a sampler
-    from a fixed initial state), [K, m] and [K, d_u]; anything else raises ValueError before any device work.
-    Returns slot -> tensor for every slot in `want` (+ OUT_STATUS): device tensors, or -- with `host_out`, which the
-    API shims set when the caller handed in host arrays -- pinned host tensors whose copies have completed.
-    `dev_inputs`, when given, receives slot -> staged device tensor (a smoother reuses the filter's staged inputs).
-    `desc_fields["flags"]` sets the CDK_FLAG_* bits (desc.reserved[2]); when the entry point then asks for device scratch
-    (cdk_scratch_bytes, sized per trajectory) it is allocated here -- or taken from `scratch`, which is how the type-1
-    smoother gets the pushforward cache its filter wrote -- and returned as out[OUT_SCRATCH]."""
-    desc_fields = dict(desc_fields)
-    tdt = _TORCH_DT[dt]
-    esz = 8 if dt == "f64" else 4
-    # ---- classify inputs (before any device work: a mis-shaped batch is rejected here, not read out of bounds) ----
-    # per-trajectory shapes of the slots whose extent depends on K: a forecast and a sampler started from a fixed state
-    # read K + 1 time stamps (t_init first), every other entry point K (slot_elems, cdk_api.cu)
-    flags = int(desc_fields.get("flags", 0))
-    t_cols = K + 1 if flags & (L.FLAG_PREDICT_ONLY | L.FLAG_FIXED_INIT) else K
-    core_shape = {L.IN_T: (t_cols,), L.IN_Y: (K, m), L.IN_U: (K, int(desc_fields.get("d_u", 0)))}
+def classify(N: int, K: int, n: int, m: int, inputs: Dict[int, object], desc_fields: dict, theta_core_ndim: int = 1,
+             core_ndim_override: Optional[dict] = None):
+    """The host-side half of `run`, which touches no device: check every input slot against the per-trajectory shape
+    its kernels read and tell shared from batched (leading N) inputs.  -> ({slot: (array, batched, row elements, host?)},
+    batched_mask).  Raises ValueError, naming the slot, on any other shape."""
+    core_shape = _core_shapes(K, n, m, desc_fields, theta_core_ndim)
     metas = {}
-    stream_bytes = 0
     mask = 0
     for slot in range(L.NUM_IN):
         x = inputs.get(slot)
@@ -153,18 +150,41 @@ def run(entry: str, dt: str, N: int, K: int, n: int, m: int, inputs: Dict[int, o
             x, shape, batched = x[0], shape[1:], False
         if batched:
             if shape[0] != N:
-                raise ValueError(f"input slot {slot}: leading axis {shape[0]} != N={N}")
+                raise ValueError(f"input slot {_SLOT_NAMES[slot]}: leading axis {shape[0]} != N={N} "
+                                 f"(full shape {full_shape})")
             mask |= 1 << slot
         elif len(shape) != core:
-            raise ValueError(f"input slot {slot}: expected rank {core} or {core + 1}, got shape {shape}")
-        if slot in core_shape and tuple(shape[1:] if batched else shape) != core_shape[slot]:
+            raise ValueError(f"input slot {_SLOT_NAMES[slot]}: expected rank {core} or {core + 1}, got shape {shape}")
+        if tuple(shape[1:] if batched else shape) != core_shape[slot]:
             raise ValueError(f"input slot {_SLOT_NAMES[slot]}: per-trajectory shape {tuple(shape[1:] if batched else shape)} "
                              f"!= {core_shape[slot]} (full shape {full_shape}, N={N}, K={K})")
         row = int(np.prod(shape[1:], dtype=np.int64)) if batched else 0
-        host = _is_host(x)
-        metas[slot] = (x, batched, row, host)
-        if batched and host:
-            stream_bytes += N * row * esz
+        metas[slot] = (x, batched, row, _is_host(x))
+    return metas, mask
+
+
+def run(entry: str, dt: str, N: int, K: int, n: int, m: int, inputs: Dict[int, object], want: Sequence[int],
+        desc_fields: dict, theta_core_ndim: int = 1, scross_rows: Optional[int] = None,
+        status: Optional[torch.Tensor] = None, host_out: bool = False,
+        dev_inputs: Optional[dict] = None, scratch: Optional[torch.Tensor] = None,
+        core_ndim_override: Optional[dict] = None,
+        out_shapes: Optional[dict] = None) -> Dict[int, torch.Tensor]:
+    """Call one C-ABI entry point. `inputs` maps slot -> array-like (None = absent); a leading N marks it batched.
+    Every slot must have the per-trajectory shape the kernels read (`_core_shapes`: [K] time stamps, [K + 1] for a
+    forecast or a sampler from a fixed initial state, [K, m] emissions, [n, n] covariances, [n_theta] drift parameters,
+    ...); anything else raises ValueError before any device work.
+    Returns slot -> tensor for every slot in `want` (+ OUT_STATUS): device tensors, or -- with `host_out`, which the
+    API shims set when the caller handed in host arrays -- pinned host tensors whose copies have completed.
+    `dev_inputs`, when given, receives slot -> staged device tensor (a smoother reuses the filter's staged inputs).
+    `desc_fields["flags"]` sets the CDK_FLAG_* bits (desc.reserved[2]); when the entry point then asks for device scratch
+    (cdk_scratch_bytes, sized per trajectory) it is allocated here -- or taken from `scratch`, which is how the type-1
+    smoother gets the pushforward cache its filter wrote -- and returned as out[OUT_SCRATCH]."""
+    desc_fields = dict(desc_fields)
+    tdt = _TORCH_DT[dt]
+    esz = 8 if dt == "f64" else 4
+    # ---- classify inputs (before any device work: a mis-shaped batch is rejected here, not read out of bounds) ----
+    metas, mask = classify(N, K, n, m, inputs, desc_fields, theta_core_ndim, core_ndim_override)
+    stream_bytes = sum(N * row * esz for _, batched, row, host in metas.values() if batched and host)
     lib = L.lib(desc_fields.pop("lib_path", None))  # a variant library for a user-defined drift, else the stock one
     dev = device()
     d = L.new_desc()

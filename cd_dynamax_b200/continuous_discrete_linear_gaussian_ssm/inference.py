@@ -90,10 +90,12 @@ def prepare_data(emissions, t_emissions, inputs):
 
 
 def _diag_r(params) -> bool:
-    """A 1-D `emissions.cov` [m] (or [N, m] when batched over parameter samples together with 3-D weights) is the diagonal
-    of R: the reference's Woodbury update (cd_linear/inference.py:240-254)."""
-    rs, hs = _shape(params.emissions.cov), _shape(params.emissions.weights)
-    return len(rs) == 1 or (len(rs) == 2 and len(hs) == 3 and rs[-1] != rs[-2])
+    """A 1-D `emissions.cov` [m] is the diagonal of R: the reference's Woodbury update (cd_linear/inference.py:240-254).
+    Batched over parameter samples it is [N, m], i.e. any 2-D covariance that is not square.  A square 2-D one is a full,
+    shared R [m, m] whatever the weights look like (so diagonals batched over N = m samples must be passed as full
+    matrices)."""
+    rs = _shape(params.emissions.cov)
+    return len(rs) == 1 or (len(rs) == 2 and rs[-1] != rs[-2])
 
 
 def _linear_inputs(params: ParamsCDLGSSM, Y, T, U, n, m, d_u):
@@ -242,6 +244,7 @@ def cdlgssm_marginal_log_prob_and_grad(params: ParamsCDLGSSM, emissions, t_emiss
     ins = _linear_inputs(params, Y, T, None, n, m, 0)
     fields = dict(E.parse_settings(hp.diffeqsolve_settings), dt_final=float(hp.dt_final), d_u=0)
     cols = L.grad_cols_kf(n, m)
+    E.classify(N, K, n, m, ins, fields, theta_core_ndim=2)  # reject mis-shaped parameters before the library is loaded
     d = L.new_desc()
     d.N, d.K, d.n, d.m = 1, K, n, m
     chunk = _grad_chunk(N, int(L.lib().cdk_scratch_bytes(ctypes.byref(d), b"cdk_kf_grad")))

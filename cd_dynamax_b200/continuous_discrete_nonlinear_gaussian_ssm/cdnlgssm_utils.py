@@ -133,15 +133,23 @@ def drift_to_theta(drift, n: int):
         cuda = [p for p in parts if p.is_cuda]
         return [p.to(cuda[0].device) for p in parts] if cuda else parts
 
+    def flat_theta(leaves):
+        """(leaf, core rank) pairs -> theta: [sum of sizes] when no leaf carries a leading N, else [N, sum of sizes] with
+        the shared leaves repeated on every row (vmap over parameter samples batches any subset of the leaves)."""
+        lead = {int(x.shape[0]) for x, core in leaves if x.dim() == core + 1}
+        if len(lead) > 1:
+            raise ValueError(f"{name}: batched leaves disagree on the leading axis: "
+                             f"{[tuple(x.shape) for x, _ in leaves]}")
+        if not lead:
+            return torch.cat([x.reshape(-1) for x, _ in leaves])
+        N = lead.pop()
+        return torch.cat([x.reshape(N, -1) if x.dim() == core + 1 else x.reshape(1, -1).expand(N, -1)
+                          for x, core in leaves], dim=-1)
+
     name = type(drift).__name__
     if name == "LearnableLinear":
         W, b = same_device([T(drift.weights), T(drift.bias)])
-        if W.dim() == 3 or b.dim() == 2:  # vmapped over parameter samples
-            N = W.shape[0] if W.dim() == 3 else b.shape[0]
-            theta = torch.cat([W.expand(N, n, n).reshape(N, n * n), b.expand(N, n)], dim=-1)
-        else:
-            theta = torch.cat([W.reshape(n * n), b.reshape(n)])
-        return L.DRIFT_LINEAR, theta, n * n + n
+        return L.DRIFT_LINEAR, flat_theta([(W, 2), (b, 1)]), n * n + n
     if name == "LearnableLorenz63":
         parts = same_device([T(drift.sigma), T(drift.rho), T(drift.beta)])
         N = max(p.numel() for p in parts)
@@ -156,10 +164,7 @@ def drift_to_theta(drift, n: int):
         return L.DRIFT_LORENZ96, theta, 1
     if name == "LearnableQuadratic":
         a, B, C = same_device([T(drift.a), T(drift.B), T(drift.C)])
-        if a.dim() != 1:
-            raise NotImplementedError("batched LearnableQuadratic parameters are not supported")
-        theta = torch.cat([a.reshape(-1), B.reshape(-1), C.reshape(-1)])
-        return L.DRIFT_QUADRATIC, theta, n + n * n + n * n * n
+        return L.DRIFT_QUADRATIC, flat_theta([(a, 1), (B, 2), (C, 3)]), n + n * n + n * n * n
     if name == "LearnableUserDrift":
         th = T(drift.theta)
         return L.DRIFT_USER, th, int(th.shape[-1]) if th.dim() else 1

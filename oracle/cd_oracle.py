@@ -232,8 +232,18 @@ def _mv(A, x):
 # f, jac: batched.  grad_div(x)[k] = sum_i d2 f_i / dx_i dx_k, the only part of the Hessian the reference's
 # "second order" term uses: 0.5*jnp.trace(H_t @ P) == 0.5 * einsum('iik,kl->l', H_t, P)  (inference_ekf.py:111-114).
 # --------------------------------------------------------------------------------------------------------------------
+def lead(v, x, core):
+    """A drift parameter `v` with core rank `core`, shaped to broadcast against states x [N, ..., n]: a per-trajectory
+    parameter [N, *core] becomes [N, 1, ..., 1, *core] (one 1 per axis between N and n: sigma points, ensemble members),
+    a shared one is returned as is."""
+    v = np.asarray(v)
+    if v.ndim == core:
+        return v
+    return v.reshape(v.shape[:1] + (1,) * (x.ndim - 2) + v.shape[1:])
+
+
 class LinearDrift:
-    """LearnableLinear: f(x) = W x + bias (cdnlgssm_utils.py:50-61). W [n,n] or [N,n,n]."""
+    """LearnableLinear: f(x) = W x + bias (cdnlgssm_utils.py:50-61). W [n,n] or [N,n,n], bias [n] or [N,n]."""
 
     drift_id = 0
 
@@ -242,16 +252,20 @@ class LinearDrift:
         self.bias = np.asarray(bias)
 
     def f(self, x):
-        return _mv(self.W, x) + self.bias
+        return _mv(lead(self.W, x, 2), x) + lead(self.bias, x, 1)
 
     def jac(self, x):
-        return np.broadcast_to(self.W, x.shape[:-1] + self.W.shape[-2:])
+        W = lead(self.W, x, 2)
+        return np.broadcast_to(W, x.shape[:-1] + W.shape[-2:])
 
     def grad_div(self, x):
         return np.zeros_like(x)
 
     def theta(self):
-        return np.concatenate([self.W.reshape(self.W.shape[:-2] + (-1,)), self.bias], axis=-1)
+        W = self.W.reshape(self.W.shape[:-2] + (-1,))
+        lead_shape = np.broadcast_shapes(W.shape[:-1], self.bias.shape[:-1])
+        return np.concatenate([np.broadcast_to(W, lead_shape + W.shape[-1:]),
+                               np.broadcast_to(self.bias, lead_shape + self.bias.shape[-1:])], axis=-1)
 
 
 class Lorenz63Drift:
@@ -263,14 +277,14 @@ class Lorenz63Drift:
         self.sigma, self.rho, self.beta = (np.asarray(v) for v in (sigma, rho, beta))
 
     def f(self, x):
-        s, r, b = (v.astype(x.dtype) for v in (self.sigma, self.rho, self.beta))
+        s, r, b = (lead(v, x, 0).astype(x.dtype) for v in (self.sigma, self.rho, self.beta))
         return np.stack(
             [s * (x[..., 1] - x[..., 0]), x[..., 0] * (r - x[..., 2]) - x[..., 1], x[..., 0] * x[..., 1] - b * x[..., 2]],
             axis=-1,
         )
 
     def jac(self, x):
-        s, r, b = (v.astype(x.dtype) for v in (self.sigma, self.rho, self.beta))
+        s, r, b = (lead(v, x, 0).astype(x.dtype) for v in (self.sigma, self.rho, self.beta))
         J = np.zeros(x.shape + (3,), x.dtype)
         J[..., 0, 0] = -s
         J[..., 0, 1] = s
@@ -299,7 +313,7 @@ class Lorenz96Drift:
 
     def f(self, x):
         xp1, xm1, xm2 = np.roll(x, -1, -1), np.roll(x, 1, -1), np.roll(x, 2, -1)
-        F = self.F.astype(x.dtype)
+        F = lead(self.F, x, 0).astype(x.dtype)  # a scalar, or [N] forcings
         return (xp1 - xm2) * xm1 - x + (F[..., None] if F.ndim else F)
 
     def jac(self, x):
@@ -417,7 +431,9 @@ def cdlgssm_filter(p: LinearParams, y, t, dt_final=1e-10, settings=SolverSetting
     # a 1-D emissions.cov (diagonal R) takes the reference's Woodbury update; its log-likelihood adds the vector to
     # H P H^T by BROADCASTING (cd_linear/inference.py:613: entry (i, j) gets R[j]) and TFP's Cholesky then factors the
     # symmetrised matrix, i.e. H P H^T + (R_i + R_j) / 2 -- restated as is (it equals diag(R) only for a constant vector)
-    diag_R = np.asarray(p.R).ndim == 1
+    # the diagonal is [m], or [N, m] batched over parameter samples (a 2-D emissions.cov that is not square)
+    Rs = np.shape(p.R)
+    diag_R = len(Rs) == 1 or (len(Rs) == 2 and Rs[0] != Rs[1])
     R = c(p.R, 1) if diag_R else c(p.R, 2)
     n = F.shape[-1]
     b = c(p.b if p.b is not None else np.zeros(n), 1)

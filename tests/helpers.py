@@ -10,26 +10,31 @@ GOLDEN_DIR = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 
 class QuadraticDrift:
-    """f_i = a_i + B_ij x_j + C_ijk x_j x_k (test-only drift with a non-zero reference 'second order' term)."""
+    """f_i = a_i + B_ij x_j + C_ijk x_j x_k (test-only drift with a non-zero reference 'second order' term).  Each of a, B,
+    C may carry a leading N (one parameter sample per trajectory); states are [N, ..., n]."""
 
     drift_id = 3
 
     def __init__(self, a, B, C):
-        self.a, self.B, self.C = a, B, C
+        self.a, self.B, self.C = np.asarray(a), np.asarray(B), np.asarray(C)
 
     def f(self, x):
-        return self.a + np.einsum("ij,...j->...i", self.B, x) + np.einsum("ijk,...j,...k->...i", self.C, x, x)
+        a, B, C = o.lead(self.a, x, 1), o.lead(self.B, x, 2), o.lead(self.C, x, 3)
+        return a + np.einsum("...ij,...j->...i", B, x) + np.einsum("...ijk,...j,...k->...i", C, x, x)
 
     def jac(self, x):
-        return self.B + np.einsum("ijk,...k->...ij", self.C, x) + np.einsum("ikj,...k->...ij", self.C, x)
+        B, C = o.lead(self.B, x, 2), o.lead(self.C, x, 3)
+        return B + np.einsum("...ijk,...k->...ij", C, x) + np.einsum("...ikj,...k->...ij", C, x)
 
     def grad_div(self, x):
         # sum_i d2 f_i / dx_i dx_k = sum_i (C_iik + C_iki)
-        g = np.einsum("iik->k", self.C) + np.einsum("iki->k", self.C)
-        return np.broadcast_to(g, x.shape)
+        g = np.einsum("...iik->...k", self.C) + np.einsum("...iki->...k", self.C)
+        return np.broadcast_to(o.lead(g, x, 1), x.shape)
 
     def theta(self):
-        return np.concatenate([self.a, self.B.ravel(), self.C.ravel()])
+        lead_shape = np.broadcast_shapes(self.a.shape[:-1], self.B.shape[:-2], self.C.shape[:-3])
+        flat = [self.a, self.B.reshape(self.B.shape[:-2] + (-1,)), self.C.reshape(self.C.shape[:-3] + (-1,))]
+        return np.concatenate([np.broadcast_to(v, lead_shape + v.shape[-1:]) for v in flat], axis=-1)
 
 
 def golden_cases(prefix):
@@ -42,15 +47,19 @@ def load_golden(name):
 
 
 def make_drift(kind, theta, n):
+    """Oracle drift from its parameter vector theta [n_theta], or [N, n_theta] for one parameter sample per trajectory."""
     kind = str(kind)
+    theta = np.asarray(theta)
     if kind == "lorenz63":
-        return o.Lorenz63Drift(*theta)
+        return o.Lorenz63Drift(theta[..., 0], theta[..., 1], theta[..., 2])
     if kind == "lorenz96":
-        return o.Lorenz96Drift(theta[0])
+        return o.Lorenz96Drift(theta[..., 0])
+    lead = theta.shape[:-1]
     if kind == "linear":
-        return o.LinearDrift(theta[: n * n].reshape(n, n), theta[n * n:])
+        return o.LinearDrift(theta[..., : n * n].reshape(lead + (n, n)), theta[..., n * n:])
     if kind == "quadratic":
-        return QuadraticDrift(theta[:n], theta[n:n + n * n].reshape(n, n), theta[n + n * n:].reshape(n, n, n))
+        return QuadraticDrift(theta[..., :n], theta[..., n:n + n * n].reshape(lead + (n, n)),
+                              theta[..., n + n * n:].reshape(lead + (n, n, n)))
     raise ValueError(kind)
 
 
