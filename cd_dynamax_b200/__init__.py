@@ -11,7 +11,8 @@ from .continuous_discrete_nonlinear_gaussian_ssm import (ContDiscreteNonlinearGa
                                                          LearnableLorenz96, LearnableMatrix, LearnableQuadratic, LearnableUserDrift,
                                                          LearnableVector, ParamsCDNLGSSM, ParamsCDNLGSSMDynamics,
                                                          ParamsCDNLGSSMEmissions, UKFHyperParams, cdnlgssm_filter,
-                                                         cdnlgssm_smoother, ekf_marginal_log_prob_and_grad, GSSMForecast,
+                                                         cdnlgssm_smoother, ekf_marginal_log_prob_and_grad,
+                                                         ekf_dense_marginal_log_prob_and_grad, GSSMForecast,
                                                          MultivariateNormalFullCovariance, cdnlgssm_emissions,
                                                          cdnlgssm_forecast, cdnlgssm_path_sample)
 from .types import (ParameterProperties, ParamsLGSSMEmissions, ParamsLGSSMInitial, PosteriorGSSMFiltered,

@@ -6,37 +6,43 @@ stack (INTEGRATION.md section 2) -- forward = the CUDA filter, backward = the ha
     ll.sum().backward()                                                       # torch leaves of `params`
 
 What `fit_sgd` minimises upstream is `-vmap(marginal_log_prob)(...).sum()` (src/ssm_temissions.py:550-568,
-src/utils/optimize_utils.py:102).  Lorenz-63 drift, scalar linear emission, fp64 (the coverage of cdk_ekf_grad_f64).
+src/utils/optimize_utils.py:102).  Every registry drift, linear emission of any size, fp64 (cdk_ekf_grad_f64 for
+Lorenz-63 with a scalar emission, cdk_ekf_grad_dense_f64 otherwise).
 
 The linear CD Kalman filter has the same shape, cdlgssm_marginal_log_prob (backward = cdk_kf_grad_f64)."""
+import numpy as np
 import torch
 
 from .continuous_discrete_linear_gaussian_ssm.inference import cdlgssm_marginal_log_prob_and_grad
 
-from .continuous_discrete_nonlinear_gaussian_ssm.inference_ekf import EKFHyperParams, ekf_marginal_log_prob_and_grad
-
-_LEAVES = ("sigma", "rho", "beta", "diffusion_coefficient", "diffusion_cov", "emission_cov", "emission_bias",
-           "emission_weights", "initial_mean", "initial_cov")
-
+from .continuous_discrete_nonlinear_gaussian_ssm.inference_ekf import (EKFHyperParams, drift_leaves,
+                                                                       ekf_dense_marginal_log_prob_and_grad,
+                                                                       ekf_marginal_log_prob_and_grad)
 
 def _val(x):
     return x.params if hasattr(x, "params") and hasattr(x, "f") else x
 
 
 def _leaves(params):
+    """Leaf name -> value: the drift's own fields (sigma / rho / beta, weights / bias, forcing, a / B / C), then the rest."""
     d, e = params.dynamics, params.emissions
-    return dict(sigma=d.drift.sigma, rho=d.drift.rho, beta=d.drift.beta, diffusion_coefficient=_val(d.diffusion_coefficient),
-                diffusion_cov=_val(d.diffusion_cov), emission_cov=_val(e.emission_cov), emission_bias=e.emission_function.bias,
-                emission_weights=e.emission_function.weights, initial_mean=_val(params.initial.mean),
-                initial_cov=_val(params.initial.cov))
+    out = {name: getattr(d.drift, name) for name, _ in drift_leaves(d.drift, 0)}
+    out.update(diffusion_coefficient=_val(d.diffusion_coefficient), diffusion_cov=_val(d.diffusion_cov),
+               emission_cov=_val(e.emission_cov), emission_bias=e.emission_function.bias,
+               emission_weights=e.emission_function.weights, initial_mean=_val(params.initial.mean),
+               initial_cov=_val(params.initial.cov))
+    return out
 
 
 class _EKFLogLik(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, params, emissions, t_emissions, hyperparams, *leaf_tensors):
-        ll, grads = ekf_marginal_log_prob_and_grad(params, emissions, t_emissions, hyperparams, wrt="all")
+    def forward(ctx, params, emissions, t_emissions, hyperparams, names, *leaf_tensors):
+        H = params.emissions.emission_function.weights
+        scalar_l63 = type(params.dynamics.drift).__name__ == "LearnableLorenz63" and tuple(np.shape(H))[-2] == 1
+        fn = ekf_marginal_log_prob_and_grad if scalar_l63 else ekf_dense_marginal_log_prob_and_grad
+        ll, grads = fn(params, emissions, t_emissions, hyperparams, wrt="all")
         ll = torch.as_tensor(ll)
-        ctx.grads = [torch.as_tensor(grads[name]) for name in _LEAVES]
+        ctx.grads = [torch.as_tensor(grads[name]) for name in names]
         ctx.shapes = [tuple(t.shape) for t in leaf_tensors]
         ctx.batched = ll.dim() == 1
         return ll
@@ -54,15 +60,17 @@ class _EKFLogLik(torch.autograd.Function):
             else:
                 g = g * grad_ll
             out.append(g.reshape(shape))
-        return (None, None, None, None) + tuple(out)
+        return (None, None, None, None, None) + tuple(out)
 
 
 def ekf_marginal_log_prob(params, emissions, t_emissions=None, hyperparams: EKFHyperParams = EKFHyperParams()):
     """Per-trajectory marginal log-likelihood of the CD-EKF as a differentiable torch tensor.  Every leaf of `params`
-    that is a torch tensor with requires_grad receives its gradient on `.backward()`."""
+    that is a torch tensor with requires_grad receives its gradient on `.backward()`: the drift's fields (named as in its
+    registry class) and the diffusion, emission and initial parameters."""
     leaves = _leaves(params)
-    tensors = [leaves[n] if isinstance(leaves[n], torch.Tensor) else torch.as_tensor(leaves[n]) for n in _LEAVES]
-    return _EKFLogLik.apply(params, emissions, t_emissions, hyperparams, *tensors)
+    names = tuple(leaves)
+    tensors = [leaves[n] if isinstance(leaves[n], torch.Tensor) else torch.as_tensor(leaves[n]) for n in names]
+    return _EKFLogLik.apply(params, emissions, t_emissions, hyperparams, names, *tensors)
 
 
 _KF_LEAVES = (("dynamics", "weights"), ("dynamics", "bias"), ("dynamics", "diffusion_coefficient"),

@@ -193,11 +193,11 @@ def _grad_chunk(N: int, row_bytes: int) -> int:
     return max(1, min(N, (free // 2) // max(row_bytes, 1)))
 
 
-def _rows(ins, lo, hi, N):
+def _rows(ins, lo, hi, N, theta_core_ndim=2):
     """The [lo, hi) trajectories of every input that carries a leading N (see _engine.run's classification)."""
     out = {}
     for slot, x in ins.items():
-        core = E._CORE_NDIM[slot] if E._CORE_NDIM[slot] is not None else 2
+        core = E._CORE_NDIM[slot] if E._CORE_NDIM[slot] is not None else theta_core_ndim
         shp = _shape(x)
         out[slot] = x[lo:hi] if (len(shp) == core + 1 and shp[0] == N and N > 1) else x
     return out

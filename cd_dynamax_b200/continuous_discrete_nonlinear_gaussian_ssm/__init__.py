@@ -2,7 +2,8 @@
 from .cdnlgssm_utils import (GSSMForecast, LearnableLinear, LearnableLorenz63, LearnableLorenz96, LearnableMatrix,
                              LearnableQuadratic, LearnableUserDrift, LearnableVector, ParamsCDNLGSSM, ParamsCDNLGSSMDynamics,
                              ParamsCDNLGSSMEmissions)
-from .inference_ekf import (EKFHyperParams, ekf_marginal_log_prob_and_grad, extended_kalman_filter,
+from .inference_ekf import (EKFHyperParams, ekf_marginal_log_prob_and_grad,
+                            ekf_dense_marginal_log_prob_and_grad, extended_kalman_filter,
                             extended_kalman_smoother, iterated_extended_kalman_filter,
                             iterated_extended_kalman_smoother)
 from .inference_enkf import EnKFHyperParams, ensemble_kalman_filter

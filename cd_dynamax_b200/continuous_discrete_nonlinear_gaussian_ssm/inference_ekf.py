@@ -3,6 +3,8 @@ extended_kalman_filter :202-326, iterated_extended_kalman_filter :328-361, exten
 iterated_extended_kalman_smoother :541-593."""
 from typing import List, NamedTuple, Optional
 
+import numpy as np
+
 from .. import _engine as E
 from .. import _lib as L
 from ..continuous_discrete_linear_gaussian_ssm.inference import _sq
@@ -79,27 +81,32 @@ def ekf_marginal_log_prob_and_grad(params, emissions, t_emissions=None, hyperpar
                                    inputs=None, wrt=("drift",)):
     """Marginal log-likelihood of the CD-EKF and its gradient with respect to the model parameters.
 
-    -> (marginal_loglik, grads): `grads` maps "sigma", "rho", "beta" (wrt "drift"), "diffusion_coefficient" [3,3],
-    "diffusion_cov" [3,3], "emission_cov" [1,1], "emission_bias" [1], "emission_weights" [1,3], "initial_mean" [3],
-    "initial_cov" [3,3] to arrays, with a leading N for batched emissions.  `wrt` = any of those group names, or "all".
+    -> (marginal_loglik, grads): `grads` maps the drift's own field names (wrt "drift": "sigma", "rho", "beta" for
+    LearnableLorenz63, "weights" [n,n] / "bias" [n] for LearnableLinear, "forcing" for LearnableLorenz96, "a" / "B" / "C"
+    for LearnableQuadratic), "diffusion_coefficient" [n,n], "diffusion_cov" [n,n], "emission_cov" [m,m],
+    "emission_bias" [m], "emission_weights" [m,n], "initial_mean" [n], "initial_cov" [n,n] to arrays, with a leading N
+    for batched emissions.  `wrt` = any of the group names of _GRAD_GROUPS, or "all".
+
+    LearnableLinear, LearnableLorenz96 and LearnableQuadratic drifts, with any emission size, run through
+    `ekf_dense_marginal_log_prob_and_grad` (cdk_ekf_grad_dense_f64).  A LearnableLorenz63 drift keeps the contract of
+    its own kernels (cdk_ekf_grad_f64, below): a scalar emission only, anything else raises NotImplementedError; call
+    `ekf_dense_marginal_log_prob_and_grad` for Lorenz-63 with a multi-component emission.  LearnableUserDrift raises
+    NotImplementedError: it would need user-supplied VJP code.
 
     This is what `jax.value_and_grad(lambda p: model.marginal_log_prob(p, ...))` yields upstream
     (src/utils/optimize_utils.py:102, src/ssm_temissions.py:550-568) -- here as the derivative of exactly the discrete
-    filter `cdnlgssm_filter` runs (cdk_ekf_grad_f64): REVERSE mode for more than the drift group (a forward filter pass
+    filter `cdnlgssm_filter` runs.  For Lorenz-63 with a scalar emission (cdk_ekf_grad_f64): REVERSE mode for more than
+    the drift group (a forward filter pass
     + one backward launch for all 23 columns, ~4 filter passes), forward mode otherwise (one launch per column), so that
     a `jax.custom_vjp` around the filter can be fed (INTEGRATION.md).  Symmetric matrices (diffusion_cov, initial_cov) are differentiated
     along symmetric directions: the result is the symmetric part (G + G^T)/2 of the entry-wise gradient G, which is what
-    any PSD parameterisation consumes; diffusion_coefficient's gradient is exact.  First step of SURVEY section 8f rank 1:
-    LearnableLorenz63 drift, scalar emission, num_iter = 1, fp64; anything else raises NotImplementedError."""
+    any PSD parameterisation consumes; diffusion_coefficient's gradient is exact.  Both paths: num_iter = 1, fp64."""
     import torch
     from ._common import nonlinear_inputs, _val
     from ..continuous_discrete_linear_gaussian_ssm.inference import _shape, prepare_data
     if type(params.dynamics.drift).__name__ != "LearnableLorenz63":
-        raise NotImplementedError("gradients are implemented for the LearnableLorenz63 drift only (SURVEY 8f rank 1)")
-    wrt = tuple(_GRAD_GROUPS) if wrt == "all" else ((wrt,) if isinstance(wrt, str) else tuple(wrt))
-    unknown = [w for w in wrt if w not in _GRAD_GROUPS]
-    if unknown:
-        raise ValueError(f"unknown gradient groups {unknown}; choose from {sorted(_GRAD_GROUPS)}")
+        return ekf_dense_marginal_log_prob_and_grad(params, emissions, t_emissions, hyperparams, inputs, wrt)
+    wrt = _parse_wrt(wrt)
     groups = 0
     for w in wrt:
         groups |= _GRAD_GROUPS[w]
@@ -107,7 +114,8 @@ def ekf_marginal_log_prob_and_grad(params, emissions, t_emissions=None, hyperpar
     Y, T, U, batched = prepare_data(emissions, t_emissions, None)
     N, K, m = _shape(Y)
     if m != 1:
-        raise NotImplementedError("gradients are implemented for scalar emissions only")
+        raise NotImplementedError("the Lorenz-63 gradient kernels take a scalar emission; "
+                                  "ekf_dense_marginal_log_prob_and_grad serves any emission size")
     n = 3
     dt = E.pick_dtype(emissions)
     if dt != "f64":
@@ -162,3 +170,107 @@ def ekf_marginal_log_prob_and_grad(params, emissions, t_emissions=None, hyperpar
     if groups & 64:
         grads["initial_cov"] = g(sym(G[:, 17:23]))
     return g(out[L.OUT_LL]), grads
+
+
+# drift leaves in the order of their theta layout (include/cdk.h drift registry), with their per-trajectory shapes
+_DRIFT_LEAVES = {
+    "LearnableLinear": lambda n: (("weights", (n, n)), ("bias", (n,))),
+    "LearnableLorenz63": lambda n: (("sigma", ()), ("rho", ()), ("beta", ())),
+    "LearnableLorenz96": lambda n: (("forcing", ()),),
+    "LearnableQuadratic": lambda n: (("a", (n,)), ("B", (n, n)), ("C", (n, n, n))),
+}
+
+
+def drift_leaves(drift, n):
+    """(name, per-trajectory shape) of the drift's parameters, in the order of its theta layout."""
+    name = type(drift).__name__
+    if name not in _DRIFT_LEAVES:
+        raise NotImplementedError(f"drift {name!r} has no gradient: it is not in the kernel registry")
+    return _DRIFT_LEAVES[name](n)
+
+
+def unflatten_theta(G_theta, drift, n):
+    """theta_bar [N, n_theta] -> {drift field name: [N, *shape]}."""
+    out, o = {}, 0
+    for name, shp in drift_leaves(drift, n):
+        size = int(np.prod(shp, dtype=np.int64))
+        out[name] = G_theta[:, o:o + size].reshape((G_theta.shape[0],) + shp)
+        o += size
+    return out
+
+
+def _parse_wrt(wrt):
+    wrt = tuple(_GRAD_GROUPS) if wrt == "all" else ((wrt,) if isinstance(wrt, str) else tuple(wrt))
+    unknown = [w for w in wrt if w not in _GRAD_GROUPS]
+    if unknown:
+        raise ValueError(f"unknown gradient groups {unknown}; choose from {sorted(_GRAD_GROUPS)}")
+    return wrt
+
+
+def ekf_dense_marginal_log_prob_and_grad(params, emissions, t_emissions=None,
+                                         hyperparams: EKFHyperParams = EKFHyperParams(), inputs=None, wrt=("drift",)):
+    """Marginal log-likelihood of the CD-EKF and its gradient for every registry drift (LearnableLinear,
+    LearnableLorenz63, LearnableLorenz96, LearnableQuadratic) and any emission size: cdk_ekf_grad_dense_f64, one forward
+    filter pass (the log-likelihood is the filter's, bit for bit) and one reverse-mode launch for all columns.
+
+    -> (marginal_loglik, grads) keyed as in `ekf_marginal_log_prob_and_grad`: the drift's own field names (wrt "drift"),
+    then "diffusion_coefficient", "diffusion_cov", "emission_cov", "emission_bias", "emission_weights", "initial_mean",
+    "initial_cov", with a leading N for batched emissions.  A batch whose scratch does not fit half of the free device
+    memory runs in several launches, with the same result bit for bit.  fp64, state_order first / second, num_iter = 1;
+    LearnableUserDrift, the zeroth order and fp32 raise NotImplementedError, mis-shaped parameters ValueError (before
+    any device work)."""
+    import ctypes
+    from ._common import nonlinear_inputs, _val
+    from ..continuous_discrete_linear_gaussian_ssm.inference import _grad_chunk, _mm, _rows, _shape, prepare_data
+    if type(params.dynamics.drift).__name__ == "LearnableUserDrift":
+        raise NotImplementedError("gradients of a user-defined drift would need user-supplied VJP device code")
+    wrt = _parse_wrt(wrt)
+    if E.pick_dtype(emissions) != "f64":
+        raise NotImplementedError("gradients are fp64 only")
+    if hyperparams.state_order == "zeroth":
+        raise NotImplementedError("gradients need state_order 'first' or 'second'")
+    kind = E.kind_of(emissions)
+    Y, T, _, batched = prepare_data(emissions, t_emissions, None)
+    N, K, m = _shape(Y)
+    n = _shape(_val(params.dynamics.diffusion_cov))[-1]
+    drift_leaves(params.dynamics.drift, n)
+    ins, drift_fields = nonlinear_inputs(params, Y, T, n, m)
+    fields = dict(E.parse_settings(hyperparams.diffeqsolve_settings), **drift_fields, **_ekf_fields(hyperparams, 1))
+    n_theta = int(fields["n_theta"])
+    E.classify(N, K, n, m, ins, fields)  # reject mis-shaped parameters before the library is loaded
+    cols = L.grad_cols_ekf(n, m, n_theta)
+    d = L.new_desc()
+    d.N, d.K, d.n, d.m, d.solver = 1, K, n, m, int(fields["solver"])
+    chunk = _grad_chunk(N, int(L.lib().cdk_scratch_bytes(ctypes.byref(d), b"cdk_ekf_grad_dense")))
+    parts = []
+    for lo in range(0, N, chunk):
+        hi = min(N, lo + chunk)
+        dev_ins = {}
+        try:
+            out = E.run("cdk_ekf_grad_dense", "f64", hi - lo, K, n, m, _rows(ins, lo, hi, N, theta_core_ndim=1),
+                        (L.OUT_LL, L.OUT_GRAD), fields, host_out=(kind != "cuda"), dev_inputs=dev_ins,
+                        out_shapes={L.OUT_GRAD: (hi - lo, cols)})
+        except L.CdkError as e:
+            raise NotImplementedError(str(e)) from e
+        G = out[L.OUT_GRAD]
+        Sb = G[:, n_theta:n_theta + n * n].reshape(hi - lo, n, n)
+        Lm, Qc = dev_ins[L.IN_L].detach().to(G.device), dev_ins[L.IN_QC].detach().to(G.device)
+        parts.append((out[L.OUT_LL], G, _mm(_mm(Sb, Lm), Qc + Qc.transpose(-1, -2)), _mm(_mm(Lm.transpose(-1, -2), Sb), Lm)))
+    import torch
+    ll, G, gL, gQc = (torch.cat(p) for p in zip(*parts))
+    g = lambda t: E.from_dev(_sq(t, batched), kind)
+    o = n_theta
+    blocks = {}
+    for name, shp in (("Sigma", (n, n)), ("H", (m, n)), ("d", (m,)), ("R", (m, m)), ("m0", (n,)), ("P0", (n, n))):
+        size = int(np.prod(shp))
+        blocks[name] = G[:, o:o + size].reshape((N,) + shp)
+        o += size
+    grads = {}
+    if "drift" in wrt:
+        grads.update({k: g(v) for k, v in unflatten_theta(G[:, :n_theta], params.dynamics.drift, n).items()})
+    for key, val in (("diffusion_coefficient", gL), ("diffusion_cov", gQc), ("emission_cov", blocks["R"]),
+                     ("emission_bias", blocks["d"]), ("emission_weights", blocks["H"]), ("initial_mean", blocks["m0"]),
+                     ("initial_cov", blocks["P0"])):
+        if key in wrt:
+            grads[key] = g(val)
+    return g(ll), grads

@@ -98,6 +98,78 @@ __device__ __forceinline__ T drift_graddiv(int id, const T* th, int n, int k) {
   return s;
 }
 
+// ---- reverse-mode contractions of the registry (cdk_ekf_grad_dense_f64) --------------------------------------------
+// Every registry drift is a polynomial of degree <= 2, so dJ_ik/dx_l is constant.  For the cotangent ab of the mean
+// right-hand side and Jb of the Jacobian J(x) (Jb = (Pb + Pb^T) P^T for the cotangent Pb of J P + (J P)^T):
+//   x-contraction      sum_ik Jb_ik dJ_ik/dx_l                 (the caller adds J^T ab)
+//   theta-contraction  sum_i ab_i df_i/dtheta_e + sum_ik Jb_ik dJ_ik/dtheta_e
+//                      + for 'second' order: sum_l ab_l 0.5 sum_k P_kl dg_k/dtheta_e, g = drift_graddiv (quadratic only)
+template <typename T>
+__device__ __forceinline__ T drift_jac_vjp_x(int id, const T* th, int n, int l, const T* Jb, int ld) {
+  switch (id) {
+    case CDK_DRIFT_LORENZ63:  // J10 = rho - z, J12 = -x, J20 = y, J21 = x
+      if (l == 0) return Jb[2 * ld + 1] - Jb[ld + 2];
+      if (l == 1) return Jb[2 * ld];
+      return -Jb[ld];
+    case CDK_DRIFT_LORENZ96: {
+      // x_l is x_{i-1} of row i = l+1 (J_{i,i+1} = x_{i-1}, J_{i,i-2} = -x_{i-1}), x_{i+1} of row l-1 and x_{i-2} of row
+      // l+2 (J_{i,i-1} = x_{i+1} - x_{i-2})
+      auto w = [&](int q) { return q < 0 ? q + n : (q >= n ? q - n : q); };
+      const int a = w(l + 1), b = w(l - 1), c = w(l + 2);
+      return Jb[a * ld + c] - Jb[a * ld + b] + Jb[b * ld + w(l - 2)] - Jb[c * ld + a];
+    }
+    case CDK_DRIFT_QUADRATIC: {  // dJ_ij/dx_l = C_ijl + C_ilj
+      const T* C = th + n + n * n;
+      T s = T(0);
+      for (int i = 0; i < n; ++i)
+        for (int j = 0; j < n; ++j) s += Jb[i * ld + j] * (C[(i * n + j) * n + l] + C[(i * n + l) * n + j]);
+      return s;
+    }
+    default: return T(0);  // linear: J = W
+  }
+}
+
+template <typename T>
+__device__ __forceinline__ T drift_theta_vjp(int id, const T* th, int n, int e, const T* x, const T* ab, const T* Jb, int ld,
+                                             const T* P, bool second) {
+  switch (id) {
+    case CDK_DRIFT_LINEAR:
+      if (e < n * n) return ab[e / n] * x[e % n] + Jb[(e / n) * ld + e % n];
+      return ab[e - n * n];
+    case CDK_DRIFT_LORENZ63:  // J00 = -sigma, J01 = sigma, J10 = rho - z, J22 = -beta
+      if (e == 0) return ab[0] * (x[1] - x[0]) - Jb[0] + Jb[1];
+      if (e == 1) return ab[1] * x[0] + Jb[ld];
+      return -ab[2] * x[2] - Jb[2 * ld + 2];
+    case CDK_DRIFT_LORENZ96: {
+      T s = T(0);
+      for (int i = 0; i < n; ++i) s += ab[i];
+      return s;
+    }
+    default: {  // quadratic: a | B | C
+      if (e < n) return ab[e];
+      if (e < n + n * n) {
+        const int q = e - n, i = q / n, j = q % n;
+        return ab[i] * x[j] + Jb[i * ld + j];
+      }
+      const int q = e - n - n * n, i = q / (n * n), j = (q / n) % n, k = q % n;
+      T s = ab[i] * x[j] * x[k] + Jb[i * ld + j] * x[k] + Jb[i * ld + k] * x[j];
+      if (second) {  // g_k = sum_i (C_iik + C_iki)
+        if (i == j) {
+          T v = T(0);
+          for (int l = 0; l < n; ++l) v += ab[l] * P[k * ld + l];
+          s += T(0.5) * v;
+        }
+        if (i == k) {
+          T v = T(0);
+          for (int l = 0; l < n; ++l) v += ab[l] * P[j * ld + l];
+          s += T(0.5) * v;
+        }
+      }
+      return s;
+    }
+  }
+}
+
 // ---- block-cooperative dense helpers (all end WITHOUT a barrier unless noted) ---------------------------------------
 // L = chol(A + boost I) (lower; reads the lower triangle of A; A != L). Upper triangle of L zeroed. Ends with a barrier.
 // BLOCKED right-looking, panels of 8 columns, in place in L.  The critical path of a Cholesky is the dependent chain

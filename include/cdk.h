@@ -105,7 +105,8 @@ enum {
   CDK_OUT_STATUS, /* int32 [N]: 0 ok, 1 non-finite result (non-PD / NaN), 2 max_steps exceeded      */
   CDK_OUT_SCRATCH,/* device scratch of cdk_scratch_bytes() bytes (CD-KF pushforward cache), else NULL */
   CDK_OUT_GRAD,   /* d marginal log-likelihood / d parameters: cdk_ekf_grad_f64 [N, CDK_GRAD_COLS_L63],
-                   * cdk_kf_grad_f64 [N, CDK_GRAD_COLS_KF(n, m)]                                               */
+                   * cdk_kf_grad_f64 [N, CDK_GRAD_COLS_KF(n, m)],
+                   * cdk_ekf_grad_dense_f64 [N, CDK_GRAD_COLS_EKF(n, m, n_theta)]                              */
   CDK_NUM_OUT
 };
 
@@ -212,6 +213,25 @@ CDK_DECL(cdk_ekf_grad_f64);
  * CDK_E_NULL (host-side checks, before any CUDA call).  desc.reserved[3] must be 0. */
 #define CDK_GRAD_COLS_KF(n, m) (3 * (n) * (n) + (m) * (n) + (m) * (m) + 2 * (n) + (m))
 CDK_DECL(cdk_kf_grad_f64);
+/* Log-likelihood (out[CDK_OUT_LL]), status (out[CDK_OUT_STATUS]) and reverse-mode gradient (out[CDK_OUT_GRAD],
+ * [N, CDK_GRAD_COLS_EKF(n, m, n_theta)]) of the CD-EKF for every registry drift (LINEAR, LORENZ63, LORENZ96, QUADRATIC)
+ * and emission size, for the same descriptor and inputs as cdk_ekf_filter_f64.  The forward pass IS the launch
+ * cdk_ekf_filter_f64 makes (the log-likelihood is bit-identical), its moments go to out[CDK_OUT_SCRATCH] (required), then
+ * one backward launch (one CTA per trajectory) re-integrates every gap and steps back through it.  Columns, row-major
+ * blocks in this order: theta (n_theta) | Sigma = L Qc L^T (n*n) | H (m*n) | d (m) | R (m*m) | m0 (n) | P0 (n*n); for a
+ * LINEAR drift theta = W | bias is the F | b of CDK_GRAD_COLS_KF.  Sigma, R and P0 get the symmetric part (G + G^T)/2.
+ * A trajectory whose status is not 0 gets a NaN row.  The gap after the last observation does not enter the
+ * log-likelihood and is not differentiated.
+ * Scratch, cdk_scratch_bytes(desc, "cdk_ekf_grad_dense") = 8 N (K (2 n + 2 n^2) + (64 + 2 S) st + 1) bytes with
+ * st = 2 ceil(n / 2) + n (n | 1) (one moment state) and S the solver's stage count: the forward moments, two levels of
+ * 32 checkpoints and the stage inputs and cotangents of one substep.
+ * Coverage: fp64, state_order first / second, num_iter = 1, full R, every solver, shared or batched parameters.
+ * state_order zeroth, num_iter > 1, CDK_DRIFT_USER, CDK_FLAG_DIAG_R, CDK_FLAG_PREDICT_ONLY, d_u > 0 and a non-zero
+ * desc.reserved[3] return CDK_E_UNSUPPORTED, a NULL out[CDK_OUT_GRAD] or out[CDK_OUT_SCRATCH] CDK_E_NULL, a shape whose
+ * backward working set exceeds the 227 KB of one CTA CDK_E_SIZE (with m = n, n <= 36 for RK4; n = 40, m = 20
+ * fits with every solver) -- all host-side checks, before any CUDA call. */
+#define CDK_GRAD_COLS_EKF(n, m, n_theta) ((n_theta) + 2 * (n) * (n) + (m) * (n) + (m) * (m) + (n) + (m))
+CDK_DECL(cdk_ekf_grad_dense_f64);
 
 /* Forward sample paths of the model (cdnlgssm_path_sample, cd_nonlinear/models.py:525-656; what
  * SSM.sample_batch(..., transition_type="path") vmaps, src/ssm_temissions.py:187-225): x_0 ~ N(m0, P0), x_k = SDE solve of
