@@ -14,7 +14,8 @@ from .continuous_discrete_nonlinear_gaussian_ssm import (ContDiscreteNonlinearGa
                                                          cdnlgssm_smoother, ekf_marginal_log_prob_and_grad,
                                                          ekf_dense_marginal_log_prob_and_grad, GSSMForecast,
                                                          MultivariateNormalFullCovariance, cdnlgssm_emissions,
-                                                         cdnlgssm_forecast, cdnlgssm_path_sample)
+                                                         cdnlgssm_forecast, cdnlgssm_path_sample,
+                                                         ukf_marginal_log_prob_and_grad)
 from .types import (ParameterProperties, ParamsLGSSMEmissions, ParamsLGSSMInitial, PosteriorGSSMFiltered,
                     PosteriorGSSMSmoothed)
 

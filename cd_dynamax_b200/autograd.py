@@ -7,7 +7,8 @@ stack (INTEGRATION.md section 2) -- forward = the CUDA filter, backward = the ha
 
 What `fit_sgd` minimises upstream is `-vmap(marginal_log_prob)(...).sum()` (src/ssm_temissions.py:550-568,
 src/utils/optimize_utils.py:102).  Every registry drift, linear emission of any size, fp64 (cdk_ekf_grad_f64 for
-Lorenz-63 with a scalar emission, cdk_ekf_grad_dense_f64 otherwise).
+Lorenz-63 with a scalar emission, cdk_ekf_grad_dense_f64 otherwise).  ukf_marginal_log_prob is the same for the
+closed-form CD-UKF (backward = cdk_ukf_grad_dense_f64).
 
 The linear CD Kalman filter has the same shape, cdlgssm_marginal_log_prob (backward = cdk_kf_grad_f64)."""
 import numpy as np
@@ -18,6 +19,7 @@ from .continuous_discrete_linear_gaussian_ssm.inference import cdlgssm_marginal_
 from .continuous_discrete_nonlinear_gaussian_ssm.inference_ekf import (EKFHyperParams, drift_leaves,
                                                                        ekf_dense_marginal_log_prob_and_grad,
                                                                        ekf_marginal_log_prob_and_grad)
+from .continuous_discrete_nonlinear_gaussian_ssm.inference_ukf import UKFHyperParams, ukf_marginal_log_prob_and_grad
 
 def _val(x):
     return x.params if hasattr(x, "params") and hasattr(x, "f") else x
@@ -34,13 +36,11 @@ def _leaves(params):
     return out
 
 
-class _EKFLogLik(torch.autograd.Function):
+class _NonlinearLogLik(torch.autograd.Function):
+    """`grad_fn(params, emissions, t_emissions, hyperparams, wrt="all")` -> (ll, grads keyed by leaf name)."""
     @staticmethod
-    def forward(ctx, params, emissions, t_emissions, hyperparams, names, *leaf_tensors):
-        H = params.emissions.emission_function.weights
-        scalar_l63 = type(params.dynamics.drift).__name__ == "LearnableLorenz63" and tuple(np.shape(H))[-2] == 1
-        fn = ekf_marginal_log_prob_and_grad if scalar_l63 else ekf_dense_marginal_log_prob_and_grad
-        ll, grads = fn(params, emissions, t_emissions, hyperparams, wrt="all")
+    def forward(ctx, grad_fn, params, emissions, t_emissions, hyperparams, names, *leaf_tensors):
+        ll, grads = grad_fn(params, emissions, t_emissions, hyperparams, wrt="all")
         ll = torch.as_tensor(ll)
         ctx.grads = [torch.as_tensor(grads[name]) for name in names]
         ctx.shapes = [tuple(t.shape) for t in leaf_tensors]
@@ -60,17 +60,31 @@ class _EKFLogLik(torch.autograd.Function):
             else:
                 g = g * grad_ll
             out.append(g.reshape(shape))
-        return (None, None, None, None, None) + tuple(out)
+        return (None, None, None, None, None, None) + tuple(out)
+
+
+def _nonlinear_log_prob(grad_fn, params, emissions, t_emissions, hyperparams):
+    leaves = _leaves(params)
+    names = tuple(leaves)
+    tensors = [leaves[n] if isinstance(leaves[n], torch.Tensor) else torch.as_tensor(leaves[n]) for n in names]
+    return _NonlinearLogLik.apply(grad_fn, params, emissions, t_emissions, hyperparams, names, *tensors)
 
 
 def ekf_marginal_log_prob(params, emissions, t_emissions=None, hyperparams: EKFHyperParams = EKFHyperParams()):
     """Per-trajectory marginal log-likelihood of the CD-EKF as a differentiable torch tensor.  Every leaf of `params`
     that is a torch tensor with requires_grad receives its gradient on `.backward()`: the drift's fields (named as in its
     registry class) and the diffusion, emission and initial parameters."""
-    leaves = _leaves(params)
-    names = tuple(leaves)
-    tensors = [leaves[n] if isinstance(leaves[n], torch.Tensor) else torch.as_tensor(leaves[n]) for n in names]
-    return _EKFLogLik.apply(params, emissions, t_emissions, hyperparams, names, *tensors)
+    H = params.emissions.emission_function.weights
+    scalar_l63 = type(params.dynamics.drift).__name__ == "LearnableLorenz63" and tuple(np.shape(H))[-2] == 1
+    fn = ekf_marginal_log_prob_and_grad if scalar_l63 else ekf_dense_marginal_log_prob_and_grad
+    return _nonlinear_log_prob(fn, params, emissions, t_emissions, hyperparams)
+
+
+def ukf_marginal_log_prob(params, emissions, t_emissions=None, hyperparams: UKFHyperParams = UKFHyperParams()):
+    """Per-trajectory marginal log-likelihood of the closed-form CD-UKF as a differentiable torch tensor
+    (ukf_marginal_log_prob_and_grad).  Every leaf of `params` that is a torch tensor with requires_grad receives its
+    gradient on `.backward()`, as in `ekf_marginal_log_prob`."""
+    return _nonlinear_log_prob(ukf_marginal_log_prob_and_grad, params, emissions, t_emissions, hyperparams)
 
 
 _KF_LEAVES = (("dynamics", "weights"), ("dynamics", "bias"), ("dynamics", "diffusion_coefficient"),

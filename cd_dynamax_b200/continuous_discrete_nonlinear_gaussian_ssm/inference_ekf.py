@@ -219,9 +219,6 @@ def ekf_dense_marginal_log_prob_and_grad(params, emissions, t_emissions=None,
     memory runs in several launches, with the same result bit for bit.  fp64, state_order first / second, num_iter = 1;
     LearnableUserDrift, the zeroth order and fp32 raise NotImplementedError, mis-shaped parameters ValueError (before
     any device work)."""
-    import ctypes
-    from ._common import nonlinear_inputs, _val
-    from ..continuous_discrete_linear_gaussian_ssm.inference import _grad_chunk, _mm, _rows, _shape, prepare_data
     if type(params.dynamics.drift).__name__ == "LearnableUserDrift":
         raise NotImplementedError("gradients of a user-defined drift would need user-supplied VJP device code")
     wrt = _parse_wrt(wrt)
@@ -229,25 +226,36 @@ def ekf_dense_marginal_log_prob_and_grad(params, emissions, t_emissions=None,
         raise NotImplementedError("gradients are fp64 only")
     if hyperparams.state_order == "zeroth":
         raise NotImplementedError("gradients need state_order 'first' or 'second'")
+    return dense_marginal_log_prob_and_grad("cdk_ekf_grad_dense", params, emissions, t_emissions,
+                                            hyperparams.diffeqsolve_settings, _ekf_fields(hyperparams, 1), wrt)
+
+
+def dense_marginal_log_prob_and_grad(entry, params, emissions, t_emissions, diffeqsolve_settings, filter_fields, wrt):
+    """The body shared by the dense EKF and UKF gradients, after their own checks: `entry` is "cdk_ekf_grad_dense" or
+    "cdk_ukf_grad_dense", `filter_fields` the descriptor fields of the filter it differentiates, `wrt` parsed by
+    _parse_wrt.  -> (marginal_loglik, grads) as documented in `ekf_dense_marginal_log_prob_and_grad`."""
+    import ctypes
+    from ._common import nonlinear_inputs, _val
+    from ..continuous_discrete_linear_gaussian_ssm.inference import _grad_chunk, _mm, _rows, _shape, prepare_data
     kind = E.kind_of(emissions)
     Y, T, _, batched = prepare_data(emissions, t_emissions, None)
     N, K, m = _shape(Y)
     n = _shape(_val(params.dynamics.diffusion_cov))[-1]
     drift_leaves(params.dynamics.drift, n)
     ins, drift_fields = nonlinear_inputs(params, Y, T, n, m)
-    fields = dict(E.parse_settings(hyperparams.diffeqsolve_settings), **drift_fields, **_ekf_fields(hyperparams, 1))
+    fields = dict(E.parse_settings(diffeqsolve_settings), **drift_fields, **filter_fields)
     n_theta = int(fields["n_theta"])
     E.classify(N, K, n, m, ins, fields)  # reject mis-shaped parameters before the library is loaded
     cols = L.grad_cols_ekf(n, m, n_theta)
     d = L.new_desc()
     d.N, d.K, d.n, d.m, d.solver = 1, K, n, m, int(fields["solver"])
-    chunk = _grad_chunk(N, int(L.lib().cdk_scratch_bytes(ctypes.byref(d), b"cdk_ekf_grad_dense")))
+    chunk = _grad_chunk(N, int(L.lib().cdk_scratch_bytes(ctypes.byref(d), entry.encode())))
     parts = []
     for lo in range(0, N, chunk):
         hi = min(N, lo + chunk)
         dev_ins = {}
         try:
-            out = E.run("cdk_ekf_grad_dense", "f64", hi - lo, K, n, m, _rows(ins, lo, hi, N, theta_core_ndim=1),
+            out = E.run(entry, "f64", hi - lo, K, n, m, _rows(ins, lo, hi, N, theta_core_ndim=1),
                         (L.OUT_LL, L.OUT_GRAD), fields, host_out=(kind != "cuda"), dev_inputs=dev_ins,
                         out_shapes={L.OUT_GRAD: (hi - lo, cols)})
         except L.CdkError as e:

@@ -4,7 +4,9 @@ unscented_kalman_filter :206-308 (the smoother does not exist upstream: raise No
 The unscented predict runs in CLOSED FORM by default: every drift of the registry is a polynomial of degree <= 2 and the
 emission is linear, and for those the 2n + 1 sigma-point sums of inference_ukf.py:130-152 are exactly
 f(m) + tr(Hess f P) / 2 and J P (csrc/cdk_generic.cu, ODE_UKFC) -- same moments up to rounding, no Cholesky factor of P at
-every RK stage.  `CDK_UKF_SIGMA_POINTS=1` in the environment (read per call) selects the literal sigma-point kernel."""
+every RK stage.  `CDK_UKF_SIGMA_POINTS=1` in the environment (read per call) selects the literal sigma-point kernel.
+
+`ukf_marginal_log_prob_and_grad` differentiates the closed-form filter (cdk_ukf_grad_dense_f64)."""
 import math
 import os
 from typing import List, NamedTuple, Optional
@@ -21,16 +23,49 @@ class UKFHyperParams(NamedTuple):
     diffeqsolve_settings: dict = {}
 
 
+def _ukf_fields(hp: UKFHyperParams):
+    return dict(dt_final=float(hp.dt_final), alpha=float(hp.alpha), beta=float(hp.beta), kappa=float(hp.kappa))
+
+
 def unscented_kalman_filter(params, emissions, t_emissions=None, hyperparams: UKFHyperParams = UKFHyperParams(),
                             inputs=None, output_fields: Optional[List[str]] = DEFAULT_FIELDS) -> PosteriorGSSMFiltered:
     from .. import _lib as L
-    fields = dict(dt_final=float(hyperparams.dt_final), alpha=float(hyperparams.alpha), beta=float(hyperparams.beta),
-                  kappa=float(hyperparams.kappa))
+    fields = _ukf_fields(hyperparams)
     if os.environ.get("CDK_UKF_SIGMA_POINTS", "0") == "1":
         fields["flags"] = L.FLAG_UKF_SIGMA_POINTS
     post, _, _ = run_filter("cdk_ukf_filter", params, emissions, t_emissions, inputs, output_fields, fields,
                             diffeqsolve_settings=hyperparams.diffeqsolve_settings)
     return post
+
+
+def ukf_marginal_log_prob_and_grad(params, emissions, t_emissions=None, hyperparams: UKFHyperParams = UKFHyperParams(),
+                                   inputs=None, wrt=("drift",)):
+    """Marginal log-likelihood of the CD-UKF and its gradient with respect to the model parameters, for every registry
+    drift (LearnableLinear, LearnableLorenz63, LearnableLorenz96, LearnableQuadratic) and any emission size:
+    cdk_ukf_grad_dense_f64, one forward pass of the closed-form filter `unscented_kalman_filter` runs (the
+    log-likelihood is the filter's, bit for bit) and one reverse-mode launch for all columns.
+
+    -> (marginal_loglik, grads) keyed as in `ekf_dense_marginal_log_prob_and_grad`: the drift's own field names (wrt
+    "drift"), then "diffusion_coefficient", "diffusion_cov", "emission_cov", "emission_bias", "emission_weights",
+    "initial_mean", "initial_cov", with a leading N for batched emissions; `wrt` = any of those groups, or "all".  A batch
+    whose scratch does not fit half of the free device memory runs in several launches, with the same result bit for
+    bit.  alpha, beta and kappa reach the filter as `unscented_kalman_filter` passes them; they do not enter the closed
+    form and get no gradient.  fp64 only.  LearnableUserDrift, fp32, non-zero inputs and CDK_UKF_SIGMA_POINTS=1 (literal
+    sigma points) raise NotImplementedError, mis-shaped parameters ValueError (before any device work)."""
+    import torch
+    from .. import _engine as E
+    from .inference_ekf import _parse_wrt, dense_marginal_log_prob_and_grad
+    if type(params.dynamics.drift).__name__ == "LearnableUserDrift":
+        raise NotImplementedError("a user-defined drift runs literal sigma points, whose gradient is not implemented")
+    wrt = _parse_wrt(wrt)
+    if E.pick_dtype(emissions) != "f64":
+        raise NotImplementedError("gradients are fp64 only")
+    if inputs is not None and bool(torch.as_tensor(inputs).ne(0).any()):
+        raise NotImplementedError("gradients with inputs are not supported")
+    if os.environ.get("CDK_UKF_SIGMA_POINTS", "0") == "1":
+        raise NotImplementedError("CDK_UKF_SIGMA_POINTS=1: only the closed-form unscented filter is differentiated")
+    return dense_marginal_log_prob_and_grad("cdk_ukf_grad_dense", params, emissions, t_emissions,
+                                            hyperparams.diffeqsolve_settings, _ukf_fields(hyperparams), wrt)
 
 
 def unscented_kalman_smoother(*args, **kwargs):

@@ -370,6 +370,46 @@ int cdk_kf_grad_f64(const cdk_desc* d, const void* const* in, void* const* out, 
   return rc;
 }
 
+// The part of cdk_ekf_grad_dense_f64 / cdk_ukf_grad_dense_f64 after their own checks: the shared-memory budget, the output
+// buffers, then the forward filter launch of `algo` with its moments in the scratch and the dense backward launch.
+static int dense_grad(int algo, const cdk_desc* d, const void* const* in, void* const* out, cdk_stream_t stream, const char* me) {
+  char msg[192];
+  auto reject = [&](int code, const char* why) {
+    snprintf(msg, sizeof(msg), "%s: %s", me, why);
+    return fail(code, msg);
+  };
+  if (!cdk::ekf_grad_dense_fits(*d)) {
+    snprintf(msg, sizeof(msg), "%s: n = %d, m = %d: the backward working set exceeds the 227 KB of one CTA (see cdk.h)", me,
+             d->n, d->m);
+    return fail(CDK_E_SIZE, msg);
+  }
+  if (d->N == 0) return CDK_OK;
+  if (!out[CDK_OUT_GRAD]) return reject(CDK_E_NULL, "needs out[CDK_OUT_GRAD]");
+  if (!out[CDK_OUT_SCRATCH]) return reject(CDK_E_NULL, "needs out[CDK_OUT_SCRATCH] (cdk_scratch_bytes)");
+  KArgs<double> a = make_args<double>(d, in, out, algo);
+  cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
+  double* sc = static_cast<double*>(out[CDK_OUT_SCRATCH]);
+  const long long NK = d->N * (long long)d->K;
+  const int n = d->n;
+  int* status = out[CDK_OUT_STATUS] ? static_cast<int*>(out[CDK_OUT_STATUS])
+                                    : reinterpret_cast<int*>(sc + cdk::ekf_grad_dense_scratch_doubles(*d) - d->N);
+  // the forward pass: the launch cdk_ekf_filter_f64 / cdk_ukf_filter_f64 makes (run()), its moments into the scratch
+  KArgs<double> f = a;
+  f.out[CDK_OUT_FM] = sc;
+  f.out[CDK_OUT_FP] = sc + NK * n;
+  f.out[CDK_OUT_PM] = sc + NK * (n + n * n);
+  f.out[CDK_OUT_PP] = sc + NK * (2 * n + n * n);
+  f.out[CDK_OUT_LLCUM] = nullptr;
+  f.out[CDK_OUT_STATUS] = status;
+  f.out[CDK_OUT_SCRATCH] = nullptr;
+  f.out[CDK_OUT_GRAD] = nullptr;
+  int rc = algo == ALGO_EKF_FILTER ? launch_ekf_small<double>(f, s) : CDK_E_UNSUPPORTED;
+  if (rc == CDK_E_UNSUPPORTED) rc = launch_generic<double>(algo, f, s);
+  if (rc == CDK_E_SIZE) return reject(rc, "the forward filter's working set exceeds the 227 KB of one CTA");
+  if (rc != CDK_OK) return rc;
+  return launch_ekf_grad_dense(a, status, static_cast<double*>(out[CDK_OUT_GRAD]), algo == ALGO_UKF_FILTER, s);
+}
+
 int cdk_ekf_grad_dense_f64(const cdk_desc* d, const void* const* in, void* const* out, cdk_stream_t stream) {
   static const char* me = "cdk_ekf_grad_dense_f64";
   char msg[192];
@@ -386,36 +426,27 @@ int cdk_ekf_grad_dense_f64(const cdk_desc* d, const void* const* in, void* const
   if (d->num_iter != 1) return reject(CDK_E_UNSUPPORTED, "num_iter must be 1 (the iterated EKF is not supported)");
   if (d->d_u > 0) return reject(CDK_E_UNSUPPORTED, "inputs (d_u > 0) are not supported");
   if (d->reserved[3] != 0) return reject(CDK_E_UNSUPPORTED, "desc.reserved[3] must be 0");
-  if (!cdk::ekf_grad_dense_fits(*d)) {
-    snprintf(msg, sizeof(msg), "%s: n = %d, m = %d: the backward working set exceeds the 227 KB of one CTA (see cdk.h)", me,
-             d->n, d->m);
-    return fail(CDK_E_SIZE, msg);
-  }
-  if (d->N == 0) return CDK_OK;
-  if (!out[CDK_OUT_GRAD]) return reject(CDK_E_NULL, "needs out[CDK_OUT_GRAD]");
-  if (!out[CDK_OUT_SCRATCH]) return reject(CDK_E_NULL, "needs out[CDK_OUT_SCRATCH] (cdk_scratch_bytes)");
-  KArgs<double> a = make_args<double>(d, in, out, ALGO_EKF_FILTER);
-  cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
-  double* sc = static_cast<double*>(out[CDK_OUT_SCRATCH]);
-  const long long NK = d->N * (long long)d->K;
-  const int n = d->n;
-  int* status = out[CDK_OUT_STATUS] ? static_cast<int*>(out[CDK_OUT_STATUS])
-                                    : reinterpret_cast<int*>(sc + cdk::ekf_grad_dense_scratch_doubles(*d) - d->N);
-  // the forward pass: the launch cdk_ekf_filter_f64 makes (run(), ALGO_EKF_FILTER), its moments into the scratch
-  KArgs<double> f = a;
-  f.out[CDK_OUT_FM] = sc;
-  f.out[CDK_OUT_FP] = sc + NK * n;
-  f.out[CDK_OUT_PM] = sc + NK * (n + n * n);
-  f.out[CDK_OUT_PP] = sc + NK * (2 * n + n * n);
-  f.out[CDK_OUT_LLCUM] = nullptr;
-  f.out[CDK_OUT_STATUS] = status;
-  f.out[CDK_OUT_SCRATCH] = nullptr;
-  f.out[CDK_OUT_GRAD] = nullptr;
-  rc = launch_ekf_small<double>(f, s);
-  if (rc == CDK_E_UNSUPPORTED) rc = launch_generic<double>(ALGO_EKF_FILTER, f, s);
-  if (rc == CDK_E_SIZE) return reject(rc, "the forward filter's working set exceeds the 227 KB of one CTA");
+  return dense_grad(ALGO_EKF_FILTER, d, in, out, stream, me);
+}
+
+int cdk_ukf_grad_dense_f64(const cdk_desc* d, const void* const* in, void* const* out, cdk_stream_t stream) {
+  static const char* me = "cdk_ukf_grad_dense_f64";
+  char msg[192];
+  auto reject = [&](int code, const char* why) {
+    snprintf(msg, sizeof(msg), "%s: %s", me, why);
+    return fail(code, msg);
+  };
+  if (d && (d->reserved[2] & CDK_FLAG_PREDICT_ONLY)) return reject(CDK_E_UNSUPPORTED, "CDK_FLAG_PREDICT_ONLY has no log-likelihood to differentiate");
+  if (d && (d->reserved[2] & CDK_FLAG_DIAG_R)) return reject(CDK_E_UNSUPPORTED, "CDK_FLAG_DIAG_R is not supported");
+  if (d && (d->reserved[2] & CDK_FLAG_UKF_SIGMA_POINTS))
+    return reject(CDK_E_UNSUPPORTED, "CDK_FLAG_UKF_SIGMA_POINTS: only the closed-form unscented predict is differentiated");
+  if (d && d->drift_id == CDK_DRIFT_USER)
+    return reject(CDK_E_UNSUPPORTED, "a user-defined drift runs literal sigma points, whose VJP is not implemented");
+  int rc = validate(d, in, out, ALGO_UKF_FILTER);
   if (rc != CDK_OK) return rc;
-  return launch_ekf_grad_dense(a, status, static_cast<double*>(out[CDK_OUT_GRAD]), s);
+  if (d->d_u > 0) return reject(CDK_E_UNSUPPORTED, "inputs (d_u > 0) are not supported");
+  if (d->reserved[3] != 0) return reject(CDK_E_UNSUPPORTED, "desc.reserved[3] must be 0");
+  return dense_grad(ALGO_UKF_FILTER, d, in, out, stream, me);
 }
 
 size_t cdk_scratch_bytes(const cdk_desc* d, const char* entry_point) {
@@ -425,10 +456,11 @@ size_t cdk_scratch_bytes(const cdk_desc* d, const char* entry_point) {
   const bool kf = strstr(entry_point, "kf_filter") != nullptr && strstr(entry_point, "ekf") == nullptr &&
                   strstr(entry_point, "ukf") == nullptr && strstr(entry_point, "enkf") == nullptr;
   const bool ks = strstr(entry_point, "kf_smooth") != nullptr && strstr(entry_point, "ekf") == nullptr;
+  // the dense gradients first: "cdk_ukf_grad_dense" also contains "kf_grad" and not "ekf_grad"
+  if (strstr(entry_point, "ekf_grad_dense") != nullptr || strstr(entry_point, "ukf_grad_dense") != nullptr)
+    return (size_t)cdk::ekf_grad_dense_scratch_doubles(*d) * sizeof(double);
   if (strstr(entry_point, "kf_grad") != nullptr && strstr(entry_point, "ekf_grad") == nullptr)
     return (size_t)cdk::kf_grad_scratch_doubles(*d) * sizeof(double);
-  if (strstr(entry_point, "ekf_grad_dense") != nullptr)
-    return (size_t)cdk::ekf_grad_dense_scratch_doubles(*d) * sizeof(double);
   if (strstr(entry_point, "ekf_grad") != nullptr)
     return (d->reserved[3] & CDK_GRAD_REVERSE) ? (size_t)d->N * (size_t)d->K * 24u * sizeof(double) : 0;
   if ((kf || ks) && (d->reserved[2] & CDK_FLAG_KEEP_PUSHFORWARD) && cdk::kf_warp_eligible(*d, ks) && d->K > 1)
@@ -479,7 +511,7 @@ static int xla_dispatch(cdk_stream_t stream, void** buffers, const char* opaque,
       {"cdk_ukf_filter_f64", cdk_ukf_filter_f64}, {"cdk_ukf_filter_f32", cdk_ukf_filter_f32},
       {"cdk_enkf_filter_f64", cdk_enkf_filter_f64}, {"cdk_enkf_filter_f32", cdk_enkf_filter_f32},
       {"cdk_ekf_grad_f64", cdk_ekf_grad_f64},     {"cdk_kf_grad_f64", cdk_kf_grad_f64},
-      {"cdk_ekf_grad_dense_f64", cdk_ekf_grad_dense_f64},
+      {"cdk_ekf_grad_dense_f64", cdk_ekf_grad_dense_f64}, {"cdk_ukf_grad_dense_f64", cdk_ukf_grad_dense_f64},
       {"cdk_sample_path_f64", cdk_sample_path_f64}, {"cdk_sample_path_f32", cdk_sample_path_f32},
       {"cdk_emission_moments_f64", cdk_emission_moments_f64}, {"cdk_emission_moments_f32", cdk_emission_moments_f32}};
   for (auto& e : table)

@@ -98,6 +98,29 @@ __device__ __forceinline__ T drift_graddiv(int id, const T* th, int n, int k) {
   return s;
 }
 
+// 0.5 * trace(Hess f_r(x) P) for the registry drifts (all polynomials of degree <= 2, so the Hessian is constant):
+// the exact second-order term of the unscented mean (NOT the reference EKF's 'second' order, whose trace runs over the
+// wrong axes -- SURVEY F8 -- and which drift_graddiv restates).
+template <typename T>
+__device__ __forceinline__ T drift_half_trhp(int id, const T* th, int n, int r, const T* P, int ld) {
+  auto ps = [&](int i, int j) { return T(0.5) * (P[i * ld + j] + P[j * ld + i]); };
+  switch (id) {
+    case CDK_DRIFT_LINEAR: return T(0);
+    case CDK_DRIFT_LORENZ63: return r == 0 ? T(0) : (r == 1 ? -ps(0, 2) : ps(0, 1));  // f1 = x (rho - z) - y, f2 = x y - b z
+    case CDK_DRIFT_LORENZ96: {  // f_r = (x_{r+1} - x_{r-2}) x_{r-1} - x_r + F
+      const int ip = r + 1 == n ? 0 : r + 1, im1 = r == 0 ? n - 1 : r - 1, im2 = im1 == 0 ? n - 1 : im1 - 1;
+      return ps(ip, im1) - ps(im2, im1);
+    }
+    default: {  // f_r = a_r + B_rj x_j + C_rjk x_j x_k
+      const T* C = th + n + n * n;
+      T s = T(0);
+      for (int j = 0; j < n; ++j)
+        for (int k = 0; k < n; ++k) s += C[(r * n + j) * n + k] * ps(j, k);
+      return s;
+    }
+  }
+}
+
 // ---- reverse-mode contractions of the registry (cdk_ekf_grad_dense_f64) --------------------------------------------
 // Every registry drift is a polynomial of degree <= 2, so dJ_ik/dx_l is constant.  For the cotangent ab of the mean
 // right-hand side and Jb of the Jacobian J(x) (Jb = (Pb + Pb^T) P^T for the cotangent Pb of J P + (J P)^T):
@@ -168,6 +191,47 @@ __device__ __forceinline__ T drift_theta_vjp(int id, const T* th, int n, int e, 
       return s;
     }
   }
+}
+
+// Reverse-mode contractions of drift_half_trhp (cdk_ukf_grad_dense_f64) for the cotangent ab of the mean right-hand side.
+// The term is linear in sym(P) and the Hessians are constant, so
+//   P-contraction      P_bar_jk += 0.5 sum_r ab_r (Hess f_r)_jk    (symmetric in j, k)
+//   theta-contraction  quadratic only (Hess f_r = C_r + C_r^T): C_bar_rjk += ab_r sym(P)_jk; the other Hessians are fixed
+template <typename T>
+__device__ __forceinline__ T drift_half_trhp_vjp_p(int id, const T* th, int n, int j, int k, const T* ab) {
+  switch (id) {
+    case CDK_DRIFT_LORENZ63: {  // Hess f_1 = -(e0 e2^T + e2 e0^T), Hess f_2 = e0 e1^T + e1 e0^T
+      const int lo = j < k ? j : k, hi = j < k ? k : j;
+      if (lo == 0 && hi == 2) return T(-0.5) * ab[1];
+      if (lo == 0 && hi == 1) return T(0.5) * ab[2];
+      return T(0);
+    }
+    case CDK_DRIFT_LORENZ96: {
+      // Hess f_r: +1 at (r+1, r-1) and (r-1, r+1), -1 at (r-2, r-1) and (r-1, r-2); for row j these are the rows
+      // r = j-1, j+1 (+1, columns j-2, j+2) and r = j+2, j+1 (-1, columns j+1, j-1).  n = 4 folds j-2 onto j+2: both add.
+      auto w = [&](int q) { return q < 0 ? q + n : (q >= n ? q - n : q); };
+      T v = T(0);
+      if (k == w(j - 2)) v += ab[w(j - 1)];
+      if (k == w(j + 2)) v += ab[w(j + 1)];
+      if (k == w(j + 1)) v -= ab[w(j + 2)];
+      if (k == w(j - 1)) v -= ab[w(j + 1)];
+      return T(0.5) * v;
+    }
+    case CDK_DRIFT_QUADRATIC: {
+      const T* C = th + n + n * n;
+      T s = T(0);
+      for (int r = 0; r < n; ++r) s += ab[r] * (C[(r * n + j) * n + k] + C[(r * n + k) * n + j]);
+      return T(0.5) * s;
+    }
+    default: return T(0);  // linear: no second-order term
+  }
+}
+
+template <typename T>
+__device__ __forceinline__ T drift_half_trhp_vjp_theta(int id, int n, int e, const T* ab, const T* P, int ld) {
+  if (id != CDK_DRIFT_QUADRATIC || e < n + n * n) return T(0);
+  const int q = e - n - n * n, r = q / (n * n), j = (q / n) % n, k = q % n;
+  return ab[r] * (T(0.5) * (P[j * ld + k] + P[k * ld + j]));
 }
 
 // ---- block-cooperative dense helpers (all end WITHOUT a barrier unless noted) ---------------------------------------

@@ -1,8 +1,8 @@
-// cdk_ekfgrad.cu -- reverse-mode gradient of the CD-EKF log-likelihood for every registry drift and emission size
-// (cdk_ekf_grad_dense_f64): ONE CTA PER TRAJECTORY, like generic_filter_kernel.
+// cdk_ekfgrad.cu -- reverse-mode gradient of the CD-EKF and closed-form CD-UKF log-likelihoods for every registry drift
+// and emission size (cdk_ekf_grad_dense_f64, cdk_ukf_grad_dense_f64): ONE CTA PER TRAJECTORY, like generic_filter_kernel.
 //
-// The forward pass is the filter launch cdk_ekf_filter_f64 makes, with its filtered and predicted moments written to the
-// scratch.  ekf_grad_dense_kernel then walks k = K-1 .. 0 with the cotangent (mu_bar, P_bar) of the moments entering
+// The forward pass is the filter launch cdk_ekf_filter_f64 (cdk_ukf_filter_f64) makes, with its filtered and predicted
+// moments written to the scratch.  ekf_grad_dense_kernel then walks k = K-1 .. 0 with the cotangent (mu_bar, P_bar) of the moments entering
 // update k+1:
 //   update VJP      both Cholesky factors recomputed from the stored predicted moments (the un-boosted one of the
 //                   log-density, sym(S) + 1e-9 I of the gain); accumulates H_bar, d_bar, R_bar;
@@ -16,6 +16,16 @@
 //   theta_bar += theta-contraction(a, Jb),  Sigma_bar += A
 // with the registry contractions of cdk_dense.cuh.  The gap after the last observation does not affect the
 // log-likelihood and is not differentiated.
+//
+// UKF mode (EgArgs::ukf).  The closed-form unscented predict (cdk_generic.cu, ODE_UKFC) replaces the bracketed EKF term
+// by the exact half-trace 0.5 tr(Hess f . sym P) (drift_half_trhp, for every drift whatever state_order says), whose VJP
+// adds 0.5 sum_r a_r Hess f_r to P_bar and, for the quadratic drift, a_r sym(P) to C_bar_r.  The update VJP is the EKF's,
+// symmetrisation of P_f_bar included, although the UKF update leaves P_f unsymmetrised: the parameters only ever move the
+// covariances along symmetric directions (Sigma, R and P0 get symmetric parts), and on symmetric moments the UKF update
+// is, in exact arithmetic, the EKF update -- P - Kt^T S Kt is then symmetric -- so the two updates have the same
+// derivative along every direction the parameter gradient sees.  The forward's rounding-level antisymmetric part of P
+// is carried unchanged across a gap by the symmetric right-hand side, here as in the filter.  The torch reference
+// (oracle/cd_torch_ukf.py) differentiates the unsymmetrised update literally and pins the gradient.
 #include "cdk_dense.cuh"
 
 namespace cdk {
@@ -64,6 +74,7 @@ struct EgArgs {
   const int* status;
   double* grad;
   int cols;
+  int ukf;         // the closed-form UKF's predict (half-trace mean term) instead of the EKF's
 };
 
 struct Eg {
@@ -73,7 +84,7 @@ struct Eg {
   __device__ Eg(const EgArgs& g_, double* sh_) : g(g_), L(g_.lay), sh(sh_) {}
   __device__ double* p(int off) const { return sh + off; }
   __device__ bool second() const {
-    return g.k.d.state_order == CDK_ORDER_SECOND && g.k.d.drift_id == CDK_DRIFT_QUADRATIC;
+    return !g.ukf && g.k.d.state_order == CDK_ORDER_SECOND && g.k.d.drift_id == CDK_DRIFT_QUADRATIC;
   }
 };
 
@@ -100,6 +111,7 @@ __device__ void eg_rhs(const Eg& c, const double* y, double* k, double dt) {
       for (int q = 0; q < n; ++q) s += drift_graddiv<double>(id, th, n, q) * P[q * ld + i];
       f += 0.5 * s;
     }
+    if (c.g.ukf) f += drift_half_trhp<double>(id, th, n, i, P, ld);
     k[i] = dt * f;
   }
   __syncthreads();
@@ -147,8 +159,18 @@ __device__ void eg_rhs_vjp(const Eg& c, const double* y, const double* kb, doubl
       outP[q * ld + l] += 0.5 * drift_graddiv<double>(id, th, n, q) * ab[l];
     }
   }
+  const bool ukf = c.g.ukf;
+  if (ukf) {
+    FOR_T(e, n * n) {
+      const int q = e / n, l = e - q * n;
+      outP[q * ld + l] += drift_half_trhp_vjp_p<double>(id, th, n, q, l, ab);
+    }
+  }
   double* thb = c.p(L.THB);
-  FOR_T(e, L.nth) thb[e] += drift_theta_vjp<double>(id, th, n, e, y, ab, Jb, ld, P, second);
+  FOR_T(e, L.nth) {
+    thb[e] += drift_theta_vjp<double>(id, th, n, e, y, ab, Jb, ld, P, second);
+    if (ukf) thb[e] += drift_half_trhp_vjp_theta<double>(id, n, e, ab, P, ld);
+  }
   __syncthreads();
 }
 
@@ -485,7 +507,8 @@ __global__ void __launch_bounds__(256) ekf_grad_dense_kernel(const EgArgs g) {
 
 }  // namespace
 
-// The layout of cdk_ekf_grad_dense_f64's scratch and shared memory for `d` (false: beyond the 227 KB of one CTA)
+// The layout of the scratch and shared memory of cdk_ekf_grad_dense_f64 and cdk_ukf_grad_dense_f64 for `d` (false: beyond
+// the 227 KB of one CTA)
 static bool eg_layout(const cdk_desc& d, EgLay& lay, RtTab& rt) {
   if (!fill_rt_tab(d.solver, rt)) return false;
   lay = EgLay(d, rt.S);
@@ -505,8 +528,9 @@ long long ekf_grad_dense_scratch_doubles(const cdk_desc& d) {
   return d.N * ((long long)d.K * (2 * d.n + 2 * d.n * d.n) + lay.bwd() + 1);
 }
 
-// The backward launch behind a forward filter pass whose moments are in out[CDK_OUT_SCRATCH] and whose status is `status`.
-int launch_ekf_grad_dense(const KArgs<double>& a, const int* status, double* grad, cudaStream_t s) {
+// The backward launch behind a forward filter pass whose moments are in out[CDK_OUT_SCRATCH] and whose status is `status`;
+// `ukf`: the forward pass was the closed-form UKF filter.
+int launch_ekf_grad_dense(const KArgs<double>& a, const int* status, double* grad, bool ukf, cudaStream_t s) {
   EgArgs g;
   g.k = a;
   if (!eg_layout(a.d, g.lay, g.tab)) return CDK_E_SIZE;
@@ -518,6 +542,7 @@ int launch_ekf_grad_dense(const KArgs<double>& a, const int* status, double* gra
   g.status = status;
   g.grad = grad;
   g.cols = CDK_GRAD_COLS_EKF(a.d.n, a.d.m, a.d.n_theta);
+  g.ukf = ukf ? 1 : 0;
   const int nmax = a.d.n > a.d.m ? a.d.n : a.d.m;
   const int threads = nmax <= 4 ? 32 : (nmax <= 8 ? 64 : (nmax <= 16 ? 128 : 256));
   const size_t smem = (size_t)g.lay.total * sizeof(double);

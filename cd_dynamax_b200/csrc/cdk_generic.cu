@@ -94,29 +94,6 @@ struct Ctx {
   __device__ T* p(int off) const { return sh + off; }
 };
 
-// 0.5 * trace(Hess f_r(x) P) for the registry drifts (all polynomials of degree <= 2, so the Hessian is constant):
-// the exact second-order term of the unscented mean (NOT the reference EKF's 'second' order, whose trace runs over the
-// wrong axes -- SURVEY F8 -- and which drift_graddiv restates).
-template <typename T>
-__device__ __forceinline__ T drift_half_trhp(int id, const T* th, int n, int r, const T* P, int ld) {
-  auto ps = [&](int i, int j) { return T(0.5) * (P[i * ld + j] + P[j * ld + i]); };
-  switch (id) {
-    case CDK_DRIFT_LINEAR: return T(0);
-    case CDK_DRIFT_LORENZ63: return r == 0 ? T(0) : (r == 1 ? -ps(0, 2) : ps(0, 1));  // f1 = x (rho - z) - y, f2 = x y - b z
-    case CDK_DRIFT_LORENZ96: {  // f_r = (x_{r+1} - x_{r-2}) x_{r-1} - x_r + F
-      const int ip = r + 1 == n ? 0 : r + 1, im1 = r == 0 ? n - 1 : r - 1, im2 = im1 == 0 ? n - 1 : im1 - 1;
-      return ps(ip, im1) - ps(im2, im1);
-    }
-    default: {  // f_r = a_r + B_rj x_j + C_rjk x_j x_k
-      const T* C = th + n + n * n;
-      T s = T(0);
-      for (int j = 0; j < n; ++j)
-        for (int k = 0; k < n; ++k) s += C[(r * n + j) * n + k] * ps(j, k);
-      return s;
-    }
-  }
-}
-
 // (J(x) P)[r][c] for the stencil drifts, straight from x and P (4 / 3 terms per entry instead of a length-n dot product)
 template <typename T>
 __device__ __forceinline__ T stencil_jp(int id, const T* th, int n, int r, int c, const T* x, const T* P, int ld) {

@@ -229,9 +229,26 @@ CDK_DECL(cdk_kf_grad_f64);
  * state_order zeroth, num_iter > 1, CDK_DRIFT_USER, CDK_FLAG_DIAG_R, CDK_FLAG_PREDICT_ONLY, d_u > 0 and a non-zero
  * desc.reserved[3] return CDK_E_UNSUPPORTED, a NULL out[CDK_OUT_GRAD] or out[CDK_OUT_SCRATCH] CDK_E_NULL, a shape whose
  * backward working set exceeds the 227 KB of one CTA CDK_E_SIZE (with m = n, n <= 36 for RK4; n = 40, m = 20
- * fits with every solver) -- all host-side checks, before any CUDA call. */
+ * fits with every solver) -- all host-side checks, before any CUDA call.
+ * CDK_GRAD_COLS_EKF is shared with cdk_ukf_grad_dense_f64, whose rows have the same layout. */
 #define CDK_GRAD_COLS_EKF(n, m, n_theta) ((n_theta) + 2 * (n) * (n) + (m) * (n) + (m) * (m) + (n) + (m))
 CDK_DECL(cdk_ekf_grad_dense_f64);
+/* Log-likelihood (out[CDK_OUT_LL]), status (out[CDK_OUT_STATUS]) and reverse-mode gradient (out[CDK_OUT_GRAD],
+ * [N, CDK_GRAD_COLS_EKF(n, m, n_theta)], the row layout of cdk_ekf_grad_dense_f64) of the CD-UKF for every registry
+ * drift and emission size, for the same descriptor and inputs as cdk_ukf_filter_f64: what jax.value_and_grad of
+ * marginal_log_prob with UKFHyperParams hands the reference's fit_sgd.  The forward pass IS the launch cdk_ukf_filter_f64
+ * makes, in closed form (the log-likelihood is bit-identical on the register-resident and the shared-memory moment ODE
+ * alike), its moments go to out[CDK_OUT_SCRATCH] (required, cdk_scratch_bytes(desc, "cdk_ukf_grad_dense") bytes: the
+ * formula of cdk_ekf_grad_dense_f64), then the backward launch of cdk_ekf_grad_dense_f64 runs with the unscented mean
+ * term 0.5 tr(Hess f . P).  Sigma, R and P0 get the symmetric part (G + G^T)/2; a trajectory whose status is not 0 gets
+ * a NaN row.  alpha, beta and kappa do not enter the closed form and get no gradient; state_order and num_iter do not
+ * apply and are ignored, as by the filter.
+ * Coverage: fp64, full R, every solver, shared or batched parameters, the same shapes as cdk_ekf_grad_dense_f64.
+ * CDK_DRIFT_USER and CDK_FLAG_UKF_SIGMA_POINTS (literal sigma points, whose VJP is not implemented), CDK_FLAG_DIAG_R,
+ * CDK_FLAG_PREDICT_ONLY, d_u > 0 and a non-zero desc.reserved[3] return CDK_E_UNSUPPORTED, a NULL out[CDK_OUT_GRAD] or
+ * out[CDK_OUT_SCRATCH] CDK_E_NULL, a backward working set beyond the 227 KB of one CTA CDK_E_SIZE -- all host-side
+ * checks, before any CUDA call. */
+CDK_DECL(cdk_ukf_grad_dense_f64);
 
 /* Forward sample paths of the model (cdnlgssm_path_sample, cd_nonlinear/models.py:525-656; what
  * SSM.sample_batch(..., transition_type="path") vmaps, src/ssm_temissions.py:187-225): x_0 ~ N(m0, P0), x_k = SDE solve of
