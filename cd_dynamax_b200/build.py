@@ -68,9 +68,11 @@ def build(force=False, verbose=False):
 
 
 USER_SOURCES = ["cdk_api.cu", "cdk_generic.cu", "cdk_enkf.cu", "cdk_aux.cu"]  # the units that see the drift registry
+USER_GRAD_SOURCES = USER_SOURCES + ["cdk_ekfgrad.cu"]  # ... plus the dense EKF gradient (build_user_drift(grad=True))
+USER_KEEP = 8  # variants kept in lib/user, newest first
 
 
-def build_user_drift(device_code: str, verbose=False) -> str:
+def build_user_drift(device_code: str, grad: bool = False, verbose=False) -> str:
     """Compile a VARIANT of libcdk.so whose drift registry contains CDK_DRIFT_USER = the given CUDA device code
     (SURVEY 8f rank 4: the reference accepts any Python drift callable, cdnlgssm_utils.py:13-36; a CUDA kernel needs device
     code).  `device_code` must define, inside `namespace cdk_user { ... }`:
@@ -79,13 +81,25 @@ def build_user_drift(device_code: str, verbose=False) -> str:
         template <typename T> __device__ T jac(const T* th, int n, int i, int j, const T* x);  // d f_i / d x_j
         template <typename T> __device__ T graddiv(const T* th, int n, int k, const T* x);     // sum_i d2 f_i/dx_i dx_k
                                                                                                // (EKF 'second'; else 0)
-    Returns the path of cd_dynamax_b200/lib/user/libcdk_user_<hash>.so (cached by content hash; ~1 minute of nvcc the first
-    time).  The variant exports the same C ABI (include/cdk.h); the register kernels that do not see the registry
-    (cdk_small.cu, cdk_kfwarp.cu) are linked from the stock build."""
+    grad=True also compiles the dense EKF gradient (cdk_ekf_grad_dense_f64) for this drift.  It instantiates the three
+    templates with T = cdk_dual::Dual<W> (csrc/cdk_dual.cuh), a forward-mode dual number, and takes every derivative the
+    reverse pass needs (df/dtheta, dJ/dx, dJ/dtheta, dg/dx, dg/dtheta) from them, so the code must then stay within the
+    dual-number contract: arithmetic on T only (+ - * / and unary -, mixed with int / double constants, compound
+    assignment, comparisons, T(c)) and the UNQUALIFIED functions sqrt exp log sin cos tan tanh sinh cosh atan fabs
+    pow(T, double).  Qualified calls (::sin, std::exp) and intrinsics (__expf) do not compile with the dual type.  The
+    cost is n_theta (n^2 + 2n) / W dual drift evaluations per stage VJP: fine for up to about a hundred parameters, the
+    wrong mode for thousands.  grad=False builds exactly the filter units, and code that compiles for float / double only
+    keeps working there.
+
+    Returns the path of cd_dynamax_b200/lib/user/libcdk_user_<hash>.so (cached by content hash, `grad` included; ~1 minute
+    of nvcc the first time; the USER_KEEP newest variants are kept).  The variant exports the same C ABI (include/cdk.h);
+    the units that do not see the registry (cdk_small.cu, cdk_kfwarp.cu, and cdk_ekfgrad.cu unless grad) are linked from
+    the stock build."""
     import hashlib
     build()  # the stock objects
     key = hashlib.sha1()
     key.update(device_code.encode())
+    key.update(b"grad" if grad else b"filter")
     for f in sorted(os.listdir(CSRC)) + ["../../include/cdk.h", "../build.py"]:
         key.update(open(os.path.join(CSRC, f), "rb").read())
     tag = key.hexdigest()[:16]
@@ -100,8 +114,9 @@ def build_user_drift(device_code: str, verbose=False) -> str:
     with open(header, "w") as fh:
         fh.write("// generated by cd_dynamax_b200.build.build_user_drift\n#pragma once\n" + device_code + "\n")
     flag = f'-DCDK_USER_DRIFT_HEADER="{header}"'
+    units = USER_GRAD_SOURCES if grad else USER_SOURCES
     jobs = []
-    for s in USER_SOURCES:
+    for s in units:
         src, obj = os.path.join(CSRC, s), os.path.join(work, s.replace(".cu", ".o"))
         jobs.append((s, [_nvcc()] + NVCC_FLAGS + [flag, "-c", src, "-o", obj]))
     with concurrent.futures.ThreadPoolExecutor(max_workers=len(jobs)) as ex:
@@ -112,18 +127,17 @@ def build_user_drift(device_code: str, verbose=False) -> str:
                 sys.stderr.write(f"--- {futs[f]} ---\n{r.stdout}{r.stderr}\n")
             if r.returncode != 0:
                 raise RuntimeError(f"nvcc failed on {futs[f]} (user drift):\n{r.stderr[-4000:]}")
-    objs = [os.path.join(work, s.replace(".cu", ".o")) for s in USER_SOURCES]
-    objs += [os.path.join(OBJ, s.replace(".cu", ".o")) for s in SOURCES if s not in USER_SOURCES]
+    objs = [os.path.join(work, s.replace(".cu", ".o")) for s in units]
+    objs += [os.path.join(OBJ, s.replace(".cu", ".o")) for s in SOURCES if s not in units]
     tmp = lib + ".tmp"
     r = subprocess.run([_nvcc(), "-shared", "-o", tmp] + objs + ["-gencode", "arch=compute_100a,code=sm_100a", "-lcudart", "-ldl",
                                                                 "-Xlinker", "-Bsymbolic"], capture_output=True, text=True)
     if r.returncode != 0:
         raise RuntimeError("link failed (user drift):\n" + r.stdout + r.stderr)
     os.replace(tmp, lib)
-    # housekeeping: every change of the sources or of the device code is a new content hash; keep the four newest variants
-    import shutil
+    # housekeeping: every change of the sources or of the device code is a new content hash; keep the newest variants
     old = sorted((f for f in os.listdir(udir) if f.startswith("libcdk_user_") and f.endswith(".so")),
-                 key=lambda f: os.path.getmtime(os.path.join(udir, f)), reverse=True)[4:]
+                 key=lambda f: os.path.getmtime(os.path.join(udir, f)), reverse=True)[USER_KEEP:]
     for f in old:
         os.remove(os.path.join(udir, f))
         shutil.rmtree(os.path.join(OBJ, "user_" + f[len("libcdk_user_"):-3]), ignore_errors=True)

@@ -35,7 +35,8 @@ def nonlinear_inputs(params, Y, T, n, m):
     fields = dict(drift_id=drift_id, n_theta=n_theta, emission_id=0)
     if drift_id == L.DRIFT_USER:
         from .. import build as _build
-        fields["lib_path"] = _build.build_user_drift(params.dynamics.drift.device_code)
+        drift = params.dynamics.drift
+        fields["lib_path"] = _build.build_user_drift(drift.device_code, grad=bool(drift.differentiable))
     return ins, fields
 
 

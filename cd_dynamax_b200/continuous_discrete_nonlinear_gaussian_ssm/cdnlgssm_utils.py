@@ -79,10 +79,16 @@ class LearnableUserDrift(NamedTuple):
     needs device code, so the drift is given as CUDA C++ source (see cd_dynamax_b200.build.build_user_drift for the three
     functions it must define in `namespace cdk_user`) plus its parameter vector `theta` ([n_theta] or [N, n_theta]); the
     first use compiles a variant of libcdk.so with that code in the drift registry (cached by content hash).  `py_f` is an
-    optional NumPy callable f(x, theta) for host-side use (e.g. the reference-style `.f`)."""
+    optional NumPy callable f(x, theta) for host-side use (e.g. the reference-style `.f`).
+
+    `differentiable=True` declares that the device code stays within the dual-number contract of
+    cd_dynamax_b200.build.build_user_drift (T arithmetic and the unqualified math functions only), and selects the variant
+    that also holds the EKF gradient: ekf_marginal_log_prob_and_grad then returns d ll / d theta under "theta", and
+    autograd.ekf_marginal_log_prob takes a torch `theta`.  The drift's filter calls use that same variant."""
     device_code: str
     theta: Any
     py_f: Any = None
+    differentiable: bool = False
 
     def f(self, x, u=None, t=None):
         if self.py_f is None:

@@ -90,8 +90,9 @@ def ekf_marginal_log_prob_and_grad(params, emissions, t_emissions=None, hyperpar
     LearnableLinear, LearnableLorenz96 and LearnableQuadratic drifts, with any emission size, run through
     `ekf_dense_marginal_log_prob_and_grad` (cdk_ekf_grad_dense_f64).  A LearnableLorenz63 drift keeps the contract of
     its own kernels (cdk_ekf_grad_f64, below): a scalar emission only, anything else raises NotImplementedError; call
-    `ekf_dense_marginal_log_prob_and_grad` for Lorenz-63 with a multi-component emission.  LearnableUserDrift raises
-    NotImplementedError: it would need user-supplied VJP code.
+    `ekf_dense_marginal_log_prob_and_grad` for Lorenz-63 with a multi-component emission.  A LearnableUserDrift with
+    differentiable=True runs through the dense function too and gets its gradient under "theta" ([n_theta] or
+    [N, n_theta]); with differentiable=False it raises NotImplementedError before any build or device work.
 
     This is what `jax.value_and_grad(lambda p: model.marginal_log_prob(p, ...))` yields upstream
     (src/utils/optimize_utils.py:102, src/ssm_temissions.py:550-568) -- here as the derivative of exactly the discrete
@@ -184,6 +185,9 @@ _DRIFT_LEAVES = {
 def drift_leaves(drift, n):
     """(name, per-trajectory shape) of the drift's parameters, in the order of its theta layout."""
     name = type(drift).__name__
+    if name == "LearnableUserDrift":
+        shp = np.shape(drift.theta)
+        return (("theta", (int(shp[-1]) if len(shp) else 1,)),)
     if name not in _DRIFT_LEAVES:
         raise NotImplementedError(f"drift {name!r} has no gradient: it is not in the kernel registry")
     return _DRIFT_LEAVES[name](n)
@@ -216,11 +220,16 @@ def ekf_dense_marginal_log_prob_and_grad(params, emissions, t_emissions=None,
     -> (marginal_loglik, grads) keyed as in `ekf_marginal_log_prob_and_grad`: the drift's own field names (wrt "drift"),
     then "diffusion_coefficient", "diffusion_cov", "emission_cov", "emission_bias", "emission_weights", "initial_mean",
     "initial_cov", with a leading N for batched emissions.  A batch whose scratch does not fit half of the free device
-    memory runs in several launches, with the same result bit for bit.  fp64, state_order first / second, num_iter = 1;
-    LearnableUserDrift, the zeroth order and fp32 raise NotImplementedError, mis-shaped parameters ValueError (before
-    any device work)."""
-    if type(params.dynamics.drift).__name__ == "LearnableUserDrift":
-        raise NotImplementedError("gradients of a user-defined drift would need user-supplied VJP device code")
+    memory runs in several launches, with the same result bit for bit.  fp64, state_order first / second, num_iter = 1.
+    A LearnableUserDrift with differentiable=True gets its gradient under "theta": the variant library built with
+    build_user_drift(code, grad=True) takes the drift's derivatives from dual-number evaluations of its own device code.
+    A LearnableUserDrift with differentiable=False, the zeroth order and fp32 raise NotImplementedError, mis-shaped
+    parameters ValueError (before any device work)."""
+    drift = params.dynamics.drift
+    if type(drift).__name__ == "LearnableUserDrift" and not drift.differentiable:
+        raise NotImplementedError("the gradient of a user-defined drift needs LearnableUserDrift(..., differentiable=True), "
+                                  "which declares that its device code stays within the dual-number contract "
+                                  "(cd_dynamax_b200.build.build_user_drift)")
     wrt = _parse_wrt(wrt)
     if E.pick_dtype(emissions) != "f64":
         raise NotImplementedError("gradients are fp64 only")

@@ -373,14 +373,18 @@ int cdk_kf_grad_f64(const cdk_desc* d, const void* const* in, void* const* out, 
 // The part of cdk_ekf_grad_dense_f64 / cdk_ukf_grad_dense_f64 after their own checks: the shared-memory budget, the output
 // buffers, then the forward filter launch of `algo` with its moments in the scratch and the dense backward launch.
 static int dense_grad(int algo, const cdk_desc* d, const void* const* in, void* const* out, cdk_stream_t stream, const char* me) {
-  char msg[192];
+  char msg[256];
   auto reject = [&](int code, const char* why) {
     snprintf(msg, sizeof(msg), "%s: %s", me, why);
     return fail(code, msg);
   };
   if (!cdk::ekf_grad_dense_fits(*d)) {
-    snprintf(msg, sizeof(msg), "%s: n = %d, m = %d: the backward working set exceeds the 227 KB of one CTA (see cdk.h)", me,
-             d->n, d->m);
+    if (d->drift_id == CDK_DRIFT_USER)
+      snprintf(msg, sizeof(msg), "%s: n = %d, m = %d, n_theta = %d: the backward working set with the user drift's dual "
+               "copy of [x | theta] exceeds the 227 KB of one CTA (see cdk.h)", me, d->n, d->m, d->n_theta);
+    else
+      snprintf(msg, sizeof(msg), "%s: n = %d, m = %d: the backward working set exceeds the 227 KB of one CTA (see cdk.h)", me,
+               d->n, d->m);
     return fail(CDK_E_SIZE, msg);
   }
   if (d->N == 0) return CDK_OK;
@@ -412,14 +416,17 @@ static int dense_grad(int algo, const cdk_desc* d, const void* const* in, void* 
 
 int cdk_ekf_grad_dense_f64(const cdk_desc* d, const void* const* in, void* const* out, cdk_stream_t stream) {
   static const char* me = "cdk_ekf_grad_dense_f64";
-  char msg[192];
+  char msg[256];
   auto reject = [&](int code, const char* why) {
     snprintf(msg, sizeof(msg), "%s: %s", me, why);
     return fail(code, msg);
   };
   if (d && (d->reserved[2] & CDK_FLAG_PREDICT_ONLY)) return reject(CDK_E_UNSUPPORTED, "CDK_FLAG_PREDICT_ONLY has no log-likelihood to differentiate");
   if (d && (d->reserved[2] & CDK_FLAG_DIAG_R)) return reject(CDK_E_UNSUPPORTED, "CDK_FLAG_DIAG_R is not supported");
-  if (d && d->drift_id == CDK_DRIFT_USER) return reject(CDK_E_UNSUPPORTED, "a user-defined drift would need user VJP code");
+  if (d && d->drift_id == CDK_DRIFT_USER && !cdk::ekf_grad_has_user_drift())
+    return reject(CDK_E_UNSUPPORTED, "a user-defined drift is differentiated only by a variant library built with its "
+                                     "gradient unit: build_user_drift(code, grad=True), i.e. LearnableUserDrift(..., "
+                                     "differentiable=True)");
   int rc = validate(d, in, out, ALGO_EKF_FILTER);
   if (rc != CDK_OK) return rc;
   if (d->state_order == CDK_ORDER_ZEROTH) return reject(CDK_E_UNSUPPORTED, "state_order zeroth is not supported");

@@ -14,6 +14,9 @@ __host__ __device__ inline int ldp(int c) { return c | 1; }
 //   template <typename T, class XF> __device__ T f(const T* th, int n, int i, XF x);     // f_i; x(j) reads component j
 //   template <typename T> __device__ T jac(const T* th, int n, int i, int j, const T* x); // d f_i / d x_j
 //   template <typename T> __device__ T graddiv(const T* th, int n, int k, const T* x);    // sum_i d2 f_i / dx_i dx_k (or 0)
+// A differentiable drift (build_user_drift(code, grad=True)) is also instantiated with T = cdk_dual::Dual<W>
+// (cdk_dual.cuh) by the dense EKF gradient, so it must use only T arithmetic and the UNQUALIFIED functions sqrt exp log
+// sin cos tan tanh sinh cosh atan fabs pow(T, double); ::sin, std::exp or __expf do not compile with the dual type.
 #ifdef CDK_USER_DRIFT_HEADER
 #include CDK_USER_DRIFT_HEADER
 #define CDK_HAS_USER_DRIFT 1

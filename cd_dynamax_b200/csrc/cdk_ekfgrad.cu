@@ -15,7 +15,9 @@
 //   As = A + A^T,  P_bar = J^T As [+ 0.5 g a^T],  Jb = As P^T,  m_bar = J^T a + x-contraction(Jb),
 //   theta_bar += theta-contraction(a, Jb),  Sigma_bar += A
 // with the registry contractions of cdk_dense.cuh.  The gap after the last observation does not affect the
-// log-likelihood and is not differentiated.
+// log-likelihood and is not differentiated.  A user drift (CDK_DRIFT_USER, in a variant built with
+// build_user_drift(code, grad=True)) replaces the registry contractions by dual-number evaluations of its own code
+// (eg_user_vjp, cdk_dual.cuh, DESIGN 4.2f); all of that is compiled only under CDK_HAS_USER_DRIFT.
 //
 // UKF mode (EgArgs::ukf).  The closed-form unscented predict (cdk_generic.cu, ODE_UKFC) replaces the bracketed EKF term
 // by the exact half-trace 0.5 tr(Hess f . sym P) (drift_half_trhp, for every drift whatever state_order says), whose VJP
@@ -27,6 +29,9 @@
 // is carried unchanged across a gap by the symmetric right-hand side, here as in the filter.  The torch reference
 // (oracle/cd_torch_ukf.py) differentiates the unsymmetrised update literally and pins the gradient.
 #include "cdk_dense.cuh"
+#if CDK_HAS_USER_DRIFT
+#include "cdk_dual.cuh"
+#endif
 
 namespace cdk {
 namespace {
@@ -34,12 +39,26 @@ namespace {
 constexpr int EG_CK = 32;  // checkpoint slots per level: a gap of up to EG_CK^2 substeps is re-integrated once
 constexpr int EG_CLOCK = (int)((sizeof(StepClock<double>) + 7) / 8);
 
+__host__ __device__ inline int eg_threads(int n, int m) {
+  const int nmax = n > m ? n : m;
+  return nmax <= 4 ? 32 : (nmax <= 8 ? 64 : (nmax <= 16 ? 128 : 256));
+}
+
+#if CDK_HAS_USER_DRIFT
+// Directions seeded per dual evaluation of the user's drift (the W of cdk_dual::Dual; see DESIGN 4.2f for the choice).
+constexpr int EG_DW = 8;
+using EgDual = cdk_dual::Dual<EG_DW>;
+#endif
+
 // Shared-memory layout (doubles), computed on the host.  A moment state [mu | P] has st = mpoff + n * ldn entries, the
 // layout of generic_filter_kernel.  With m <= n the update's [m x n] buffers alias ODE buffers that are idle then.
 struct EgLay {
   int n, m, ldn, ldm, nn, mpoff, st, nth, S;
   int TH, THB, LQL, H, R, DV, SIGB, HB, RB, DB, YC, YS, KS, ACC, YB, J, W1, W2;
   int G, KT, U, GB, SM, L0, LB, SI, SB, RV, ZV, RBV, YV, CLK, total;
+#if CDK_HAS_USER_DRIFT
+  int DU, PART, WQ, GV;
+#endif
   EgLay() = default;
   __host__ __device__ EgLay(const cdk_desc& d, int stages) {
     n = d.n; m = d.m; ldn = ldp(n); ldm = ldp(m); nn = n * ldn; nth = d.n_theta; S = stages;
@@ -59,6 +78,16 @@ struct EgLay {
     SM = take(m * ldm); L0 = take(m * ldm); LB = take(m * ldm); SI = take(m * ldm); SB = take(m * ldm);
     RV = take(m); ZV = take(m); RBV = take(m); YV = take(m);
     CLK = take(2 * EG_CK * EG_CLOCK);
+#if CDK_HAS_USER_DRIFT
+    // user drift: one dual copy of [x | theta] for the CTA, one partial sum of EG_DW tangents per thread, w_q and g(x)
+    DU = PART = WQ = GV = 0;
+    if (d.drift_id == CDK_DRIFT_USER) {
+      DU = take((n + nth) * (EG_DW + 1));
+      PART = take(eg_threads(n, m) * EG_DW);
+      WQ = take(n);
+      GV = take(n);
+    }
+#endif
     total = o;
   }
   // per-trajectory backward scratch (doubles): checkpoints at two levels, stage inputs, stage cotangents
@@ -84,6 +113,9 @@ struct Eg {
   __device__ Eg(const EgArgs& g_, double* sh_) : g(g_), L(g_.lay), sh(sh_) {}
   __device__ double* p(int off) const { return sh + off; }
   __device__ bool second() const {
+#if CDK_HAS_USER_DRIFT
+    if (g.k.d.drift_id == CDK_DRIFT_USER) return !g.ukf && g.k.d.state_order == CDK_ORDER_SECOND;
+#endif
     return !g.ukf && g.k.d.state_order == CDK_ORDER_SECOND && g.k.d.drift_id == CDK_DRIFT_QUADRATIC;
   }
 };
@@ -108,6 +140,11 @@ __device__ void eg_rhs(const Eg& c, const double* y, double* k, double dt) {
     double f = drift_f<double>(id, th, n, i, [&](int j) { return y[j]; });
     if (second) {
       double s = 0.0;
+#if CDK_HAS_USER_DRIFT
+      if (id == CDK_DRIFT_USER) {  // the x-dependent g(x) of the filter (cdk_generic.cu, ODE_EKF)
+        for (int q = 0; q < n; ++q) s += cdk_user::graddiv<double>(th, n, q, y) * P[q * ld + i];
+      } else
+#endif
       for (int q = 0; q < n; ++q) s += drift_graddiv<double>(id, th, n, q) * P[q * ld + i];
       f += 0.5 * s;
     }
@@ -122,6 +159,98 @@ __device__ void eg_rhs(const Eg& c, const double* y, double* k, double dt) {
   }
   __syncthreads();
 }
+
+#if CDK_HAS_USER_DRIFT
+// The mean and parameter cotangents of eg_rhs_vjp for the user drift, from dual evaluations of its own f / jac / graddiv
+// at the stage input y (J, Jb and outP = J^T As are in place).  With w_q = 0.5 sum_i P_qi a_i ('second' order only):
+//   m_bar_l      = (J^T a)_l + sum_ik Jb_ik dJ_ik/dx_l + sum_q w_q dg_q/dx_l
+//   theta_bar_e += sum_i a_i df_i/dtheta_e + sum_ik Jb_ik dJ_ik/dtheta_e + sum_q w_q dg_q/dtheta_e
+//   P_bar       += 0.5 g(x) a^T
+// The n + n_theta directions (x, then theta) are seeded EG_DW at a time into the CTA's one dual copy of [x | theta];
+// for each chunk the threads share out the evaluations (jac (i, k), f i, graddiv q), each sums its weighted tangents in
+// registers, and one thread per direction adds the per-thread partial sums in thread order: the result is the same bits
+// from run to run.  Ends with a barrier.
+__device__ void eg_user_vjp(const Eg& c, const double* y, const double* ab, const double* Jb, double* out, double* outP,
+                            bool second) {
+  const EgLay& L = c.L;
+  const int n = L.n, ld = L.ldn, nv = n + L.nth;
+  const double* th = c.p(L.TH);
+  const double* P = y + L.mpoff;
+  const double* J = c.p(L.J);
+  double* wq = c.p(L.WQ);
+  double* gv = c.p(L.GV);
+  double* part = c.p(L.PART);
+  double* thb = c.p(L.THB);
+  EgDual* xd = reinterpret_cast<EgDual*>(c.p(L.DU));
+  EgDual* td = xd + n;
+  FOR_T(l, n) {
+    double s = 0.0;
+    for (int i = 0; i < n; ++i) s += J[i * ld + l] * ab[i];
+    out[l] = s;
+    if (second) {
+      double w = 0.0;
+      for (int i = 0; i < n; ++i) w += P[l * ld + i] * ab[i];
+      wq[l] = 0.5 * w;
+      gv[l] = cdk_user::graddiv<double>(th, n, l, y);
+    }
+  }
+  FOR_T(v, nv) xd[v] = EgDual(v < n ? y[v] : th[v - n]);
+  __syncthreads();
+  if (second) {
+    FOR_T(e, n * n) {
+      const int q = e / n, l = e - q * n;
+      outP[q * ld + l] += 0.5 * gv[q] * ab[l];
+    }
+  }
+  const int nj = n * n, E = nj + n + (second ? n : 0);
+  for (int c0 = 0; c0 < nv; c0 += EG_DW) {
+    FOR_T(e, nv * EG_DW) {
+      const int v = e / EG_DW, w = e - v * EG_DW;
+      xd[v].d[w] = c0 + w == v ? 1.0 : 0.0;
+    }
+    __syncthreads();
+    const bool fth = c0 + EG_DW > n;  // the chunk holds parameter directions: f's tangents enter (its x-tangents are J)
+    double acc[EG_DW];
+#pragma unroll
+    for (int w = 0; w < EG_DW; ++w) acc[w] = 0.0;
+    for (int e = threadIdx.x; e < E; e += blockDim.x) {
+      if (e < nj) {
+        const int i = e / n, k = e - i * n;
+        const EgDual v = cdk_user::jac<EgDual>(td, n, i, k, xd);
+        const double wt = Jb[i * ld + k];
+#pragma unroll
+        for (int w = 0; w < EG_DW; ++w) acc[w] += wt * v.d[w];
+      } else if (e < nj + n) {
+        if (!fth) continue;
+        const int i = e - nj;
+        const EgDual v = cdk_user::f<EgDual>(td, n, i, [&](int j) { return xd[j]; });
+        const double wt = ab[i];
+#pragma unroll
+        for (int w = 0; w < EG_DW; ++w)
+          if (c0 + w >= n) acc[w] += wt * v.d[w];
+      } else {
+        const int q = e - nj - n;
+        const EgDual v = cdk_user::graddiv<EgDual>(td, n, q, xd);
+        const double wt = wq[q];
+#pragma unroll
+        for (int w = 0; w < EG_DW; ++w) acc[w] += wt * v.d[w];
+      }
+    }
+#pragma unroll
+    for (int w = 0; w < EG_DW; ++w) part[threadIdx.x * EG_DW + w] = acc[w];
+    __syncthreads();
+    FOR_T(w, EG_DW) {
+      const int v = c0 + w;
+      if (v < nv) {
+        double s = 0.0;
+        for (int t = 0; t < (int)blockDim.x; ++t) s += part[t * EG_DW + w];
+        if (v < n) out[v] += s; else thb[v - n] += s;
+      }
+    }
+  }
+  __syncthreads();
+}
+#endif
 
 // VJP of the right-hand side at y (shared) for the cotangent kb (shared, already scaled by dt): writes the cotangent of y
 // to `out` (the stage's slot in the scratch) and accumulates theta_bar and Sigma_bar.  Ends with a barrier.
@@ -148,6 +277,12 @@ __device__ void eg_rhs_vjp(const Eg& c, const double* y, const double* kb, doubl
   mm_dmma<double, false, true>(As, ld, P, ld, n, n, n, [&](int i, int j, double v) { Jb[i * ld + j] = v; });    // As P^T
   __syncthreads();
   const bool second = c.second();
+#if CDK_HAS_USER_DRIFT
+  if (id == CDK_DRIFT_USER) {
+    eg_user_vjp(c, y, ab, Jb, out, outP, second);
+    return;
+  }
+#endif
   FOR_T(l, n) {
     double s = drift_jac_vjp_x<double>(id, th, n, l, Jb, ld);
     for (int i = 0; i < n; ++i) s += J[i * ld + l] * ab[i];
@@ -521,6 +656,8 @@ bool ekf_grad_dense_fits(const cdk_desc& d) {
   return eg_layout(d, lay, rt);
 }
 
+bool ekf_grad_has_user_drift() { return CDK_HAS_USER_DRIFT != 0; }
+
 long long ekf_grad_dense_scratch_doubles(const cdk_desc& d) {
   EgLay lay;
   RtTab rt;
@@ -543,8 +680,7 @@ int launch_ekf_grad_dense(const KArgs<double>& a, const int* status, double* gra
   g.grad = grad;
   g.cols = CDK_GRAD_COLS_EKF(a.d.n, a.d.m, a.d.n_theta);
   g.ukf = ukf ? 1 : 0;
-  const int nmax = a.d.n > a.d.m ? a.d.n : a.d.m;
-  const int threads = nmax <= 4 ? 32 : (nmax <= 8 ? 64 : (nmax <= 16 ? 128 : 256));
+  const int threads = eg_threads(a.d.n, a.d.m);
   const size_t smem = (size_t)g.lay.total * sizeof(double);
   if (smem > 48 * 1024 && cudaFuncSetAttribute(ekf_grad_dense_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
     return check_launch("cudaFuncSetAttribute(ekf_grad_dense_kernel)");

@@ -225,8 +225,12 @@ CDK_DECL(cdk_kf_grad_f64);
  * Scratch, cdk_scratch_bytes(desc, "cdk_ekf_grad_dense") = 8 N (K (2 n + 2 n^2) + (64 + 2 S) st + 1) bytes with
  * st = 2 ceil(n / 2) + n (n | 1) (one moment state) and S the solver's stage count: the forward moments, two levels of
  * 32 checkpoints and the stage inputs and cotangents of one substep.
- * Coverage: fp64, state_order first / second, num_iter = 1, full R, every solver, shared or batched parameters.
- * state_order zeroth, num_iter > 1, CDK_DRIFT_USER, CDK_FLAG_DIAG_R, CDK_FLAG_PREDICT_ONLY, d_u > 0 and a non-zero
+ * Coverage: fp64, state_order first / second, num_iter = 1, full R, every solver, shared or batched parameters, and
+ * CDK_DRIFT_USER in a variant built with build_user_drift(code, grad=True), whose backward pass takes the drift's
+ * derivatives from dual-number evaluations of the user's f / jac / graddiv (the
+ * scratch formula is the same; the shared memory adds a dual copy of [x | theta], and an n_theta that does not fit
+ * returns CDK_E_SIZE).  The stock library and a filter-only variant reject CDK_DRIFT_USER with CDK_E_UNSUPPORTED.
+ * state_order zeroth, num_iter > 1, CDK_FLAG_DIAG_R, CDK_FLAG_PREDICT_ONLY, d_u > 0 and a non-zero
  * desc.reserved[3] return CDK_E_UNSUPPORTED, a NULL out[CDK_OUT_GRAD] or out[CDK_OUT_SCRATCH] CDK_E_NULL, a shape whose
  * backward working set exceeds the 227 KB of one CTA CDK_E_SIZE (with m = n, n <= 36 for RK4; n = 40, m = 20
  * fits with every solver) -- all host-side checks, before any CUDA call.
