@@ -15,7 +15,8 @@ from .continuous_discrete_nonlinear_gaussian_ssm import (ContDiscreteNonlinearGa
                                                          ekf_dense_marginal_log_prob_and_grad, GSSMForecast,
                                                          MultivariateNormalFullCovariance, cdnlgssm_emissions,
                                                          cdnlgssm_forecast, cdnlgssm_path_sample,
-                                                         ukf_marginal_log_prob_and_grad)
+                                                         ukf_marginal_log_prob_and_grad,
+                                                         ukf_sigma_points_marginal_log_prob_and_grad)
 from .types import (ParameterProperties, ParamsLGSSMEmissions, ParamsLGSSMInitial, PosteriorGSSMFiltered,
                     PosteriorGSSMSmoothed)
 

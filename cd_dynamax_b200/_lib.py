@@ -27,7 +27,8 @@ def grad_cols_kf(n, m):
 
 
 def grad_cols_ekf(n, m, n_theta):
-    """CDK_GRAD_COLS_EKF(n, m, n_theta): columns of out[CDK_OUT_GRAD] of cdk_ekf_grad_dense_f64 and cdk_ukf_grad_dense_f64."""
+    """CDK_GRAD_COLS_EKF(n, m, n_theta): columns of out[CDK_OUT_GRAD] of cdk_ekf_grad_dense_f64, cdk_ukf_grad_dense_f64 and
+    cdk_ukf_grad_sigma_f64."""
     return n_theta + 2 * n * n + m * n + m * m + n + m
 
 
@@ -37,6 +38,7 @@ ENTRY_POINTS.append("cdk_ekf_grad_f64")
 ENTRY_POINTS.append("cdk_kf_grad_f64")
 ENTRY_POINTS.append("cdk_ekf_grad_dense_f64")
 ENTRY_POINTS.append("cdk_ukf_grad_dense_f64")
+ENTRY_POINTS.append("cdk_ukf_grad_sigma_f64")
 ENTRY_POINTS += ["cdk_sample_path_f64", "cdk_sample_path_f32", "cdk_emission_moments_f64", "cdk_emission_moments_f32"]
 OTHER_SYMBOLS = ["cdk_desc_init", "cdk_scratch_bytes", "cdk_ll_sum_f64", "cdk_ll_sum_f32", "cdk_ll_allreduce",
                  "cdk_xla_custom_call", "cdk_xla_custom_call_status", "cdk_xla_last_rc", "cdk_fma_probe_f64", "cdk_fma_probe_f32", "cdk_fma3_probe_f64", "cdk_dmma_probe_f64", "cdk_rng_probe_f64", "cdk_launch_count", "cdk_debug_set_trace", "cdk_has_user_drift", "cdk_version",

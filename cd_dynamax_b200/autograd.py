@@ -8,7 +8,8 @@ stack (INTEGRATION.md section 2) -- forward = the CUDA filter, backward = the ha
 What `fit_sgd` minimises upstream is `-vmap(marginal_log_prob)(...).sum()` (src/ssm_temissions.py:550-568,
 src/utils/optimize_utils.py:102).  Every registry drift, linear emission of any size, fp64 (cdk_ekf_grad_f64 for
 Lorenz-63 with a scalar emission, cdk_ekf_grad_dense_f64 otherwise).  ukf_marginal_log_prob is the same for the
-closed-form CD-UKF (backward = cdk_ukf_grad_dense_f64).
+closed-form CD-UKF (backward = cdk_ukf_grad_dense_f64), ukf_sigma_points_marginal_log_prob for the CD-UKF with literal
+sigma points (backward = cdk_ukf_grad_sigma_f64; registry drifts and differentiable user drifts).
 
 The linear CD Kalman filter has the same shape, cdlgssm_marginal_log_prob (backward = cdk_kf_grad_f64)."""
 import numpy as np
@@ -19,7 +20,8 @@ from .continuous_discrete_linear_gaussian_ssm.inference import cdlgssm_marginal_
 from .continuous_discrete_nonlinear_gaussian_ssm.inference_ekf import (EKFHyperParams, drift_leaves,
                                                                        ekf_dense_marginal_log_prob_and_grad,
                                                                        ekf_marginal_log_prob_and_grad)
-from .continuous_discrete_nonlinear_gaussian_ssm.inference_ukf import UKFHyperParams, ukf_marginal_log_prob_and_grad
+from .continuous_discrete_nonlinear_gaussian_ssm.inference_ukf import (UKFHyperParams, ukf_marginal_log_prob_and_grad,
+                                                                       ukf_sigma_points_marginal_log_prob_and_grad)
 
 def _val(x):
     return x.params if hasattr(x, "params") and hasattr(x, "f") else x
@@ -85,6 +87,15 @@ def ukf_marginal_log_prob(params, emissions, t_emissions=None, hyperparams: UKFH
     (ukf_marginal_log_prob_and_grad).  Every leaf of `params` that is a torch tensor with requires_grad receives its
     gradient on `.backward()`, as in `ekf_marginal_log_prob`."""
     return _nonlinear_log_prob(ukf_marginal_log_prob_and_grad, params, emissions, t_emissions, hyperparams)
+
+
+def ukf_sigma_points_marginal_log_prob(params, emissions, t_emissions=None,
+                                       hyperparams: UKFHyperParams = UKFHyperParams()):
+    """Per-trajectory marginal log-likelihood of the CD-UKF with literal sigma points as a differentiable torch tensor
+    (ukf_sigma_points_marginal_log_prob_and_grad).  Every leaf of `params` that is a torch tensor with requires_grad
+    receives its gradient on `.backward()`, as in `ekf_marginal_log_prob`; for a LearnableUserDrift(...,
+    differentiable=True) that includes a torch `theta`."""
+    return _nonlinear_log_prob(ukf_sigma_points_marginal_log_prob_and_grad, params, emissions, t_emissions, hyperparams)
 
 
 _KF_LEAVES = (("dynamics", "weights"), ("dynamics", "bias"), ("dynamics", "diffusion_coefficient"),

@@ -240,8 +240,8 @@ def ekf_dense_marginal_log_prob_and_grad(params, emissions, t_emissions=None,
 
 
 def dense_marginal_log_prob_and_grad(entry, params, emissions, t_emissions, diffeqsolve_settings, filter_fields, wrt):
-    """The body shared by the dense EKF and UKF gradients, after their own checks: `entry` is "cdk_ekf_grad_dense" or
-    "cdk_ukf_grad_dense", `filter_fields` the descriptor fields of the filter it differentiates, `wrt` parsed by
+    """The body shared by the dense EKF and UKF gradients, after their own checks: `entry` is "cdk_ekf_grad_dense",
+    "cdk_ukf_grad_dense" or "cdk_ukf_grad_sigma", `filter_fields` the descriptor fields of the filter it differentiates, `wrt` parsed by
     _parse_wrt.  -> (marginal_loglik, grads) as documented in `ekf_dense_marginal_log_prob_and_grad`."""
     import ctypes
     from ._common import nonlinear_inputs, _val

@@ -6,7 +6,9 @@ emission is linear, and for those the 2n + 1 sigma-point sums of inference_ukf.p
 f(m) + tr(Hess f P) / 2 and J P (csrc/cdk_generic.cu, ODE_UKFC) -- same moments up to rounding, no Cholesky factor of P at
 every RK stage.  `CDK_UKF_SIGMA_POINTS=1` in the environment (read per call) selects the literal sigma-point kernel.
 
-`ukf_marginal_log_prob_and_grad` differentiates the closed-form filter (cdk_ukf_grad_dense_f64)."""
+`ukf_marginal_log_prob_and_grad` differentiates the closed-form filter (cdk_ukf_grad_dense_f64),
+`ukf_sigma_points_marginal_log_prob_and_grad` the literal sigma-point filter (cdk_ukf_grad_sigma_f64), which is also
+the one a LearnableUserDrift runs."""
 import math
 import os
 from typing import List, NamedTuple, Optional
@@ -56,15 +58,49 @@ def ukf_marginal_log_prob_and_grad(params, emissions, t_emissions=None, hyperpar
     from .. import _engine as E
     from .inference_ekf import _parse_wrt, dense_marginal_log_prob_and_grad
     if type(params.dynamics.drift).__name__ == "LearnableUserDrift":
-        raise NotImplementedError("a user-defined drift runs literal sigma points, whose gradient is not implemented")
+        raise NotImplementedError("a user-defined drift runs literal sigma points: use "
+                                  "ukf_sigma_points_marginal_log_prob_and_grad")
     wrt = _parse_wrt(wrt)
     if E.pick_dtype(emissions) != "f64":
         raise NotImplementedError("gradients are fp64 only")
     if inputs is not None and bool(torch.as_tensor(inputs).ne(0).any()):
         raise NotImplementedError("gradients with inputs are not supported")
     if os.environ.get("CDK_UKF_SIGMA_POINTS", "0") == "1":
-        raise NotImplementedError("CDK_UKF_SIGMA_POINTS=1: only the closed-form unscented filter is differentiated")
+        raise NotImplementedError("CDK_UKF_SIGMA_POINTS=1: the literal sigma-point filter is differentiated by "
+                                  "ukf_sigma_points_marginal_log_prob_and_grad")
     return dense_marginal_log_prob_and_grad("cdk_ukf_grad_dense", params, emissions, t_emissions,
+                                            hyperparams.diffeqsolve_settings, _ukf_fields(hyperparams), wrt)
+
+
+def ukf_sigma_points_marginal_log_prob_and_grad(params, emissions, t_emissions=None,
+                                                hyperparams: UKFHyperParams = UKFHyperParams(), inputs=None,
+                                                wrt=("drift",)):
+    """Marginal log-likelihood of the CD-UKF with LITERAL sigma points (inference_ukf.py:130-152: a Cholesky factor of P
+    and 2n + 1 drift evaluations at every RK stage) and its gradient with respect to the model parameters:
+    cdk_ukf_grad_sigma_f64, one forward pass of the sigma-point filter (`unscented_kalman_filter` with
+    CDK_UKF_SIGMA_POINTS=1; the log-likelihood is that filter's, bit for bit) and one reverse-mode launch for all
+    columns.  It always differentiates the sigma-point filter, whatever CDK_UKF_SIGMA_POINTS says.
+
+    Every registry drift, and a LearnableUserDrift(..., differentiable=True), whose gradient comes under "theta" (the
+    variant library built with build_user_drift(code, grad=True) takes the theta-derivatives of its f from dual numbers
+    and its x-derivatives from its jac).  -> (marginal_loglik, grads) keyed as in `ekf_dense_marginal_log_prob_and_grad`;
+    `wrt` = any of its groups, or "all".  alpha, beta and kappa get no gradient.  fp64 only.  fp32, non-zero inputs and
+    a LearnableUserDrift with differentiable=False raise NotImplementedError, mis-shaped parameters ValueError (before any
+    device work)."""
+    import torch
+    from .. import _engine as E
+    from .inference_ekf import _parse_wrt, dense_marginal_log_prob_and_grad
+    drift = params.dynamics.drift
+    if type(drift).__name__ == "LearnableUserDrift" and not drift.differentiable:
+        raise NotImplementedError("the gradient of a user-defined drift needs LearnableUserDrift(..., differentiable=True), "
+                                  "which declares that its device code stays within the dual-number contract "
+                                  "(cd_dynamax_b200.build.build_user_drift)")
+    wrt = _parse_wrt(wrt)
+    if E.pick_dtype(emissions) != "f64":
+        raise NotImplementedError("gradients are fp64 only")
+    if inputs is not None and bool(torch.as_tensor(inputs).ne(0).any()):
+        raise NotImplementedError("gradients with inputs are not supported")
+    return dense_marginal_log_prob_and_grad("cdk_ukf_grad_sigma", params, emissions, t_emissions,
                                             hyperparams.diffeqsolve_settings, _ukf_fields(hyperparams), wrt)
 
 

@@ -370,15 +370,17 @@ int cdk_kf_grad_f64(const cdk_desc* d, const void* const* in, void* const* out, 
   return rc;
 }
 
-// The part of cdk_ekf_grad_dense_f64 / cdk_ukf_grad_dense_f64 after their own checks: the shared-memory budget, the output
-// buffers, then the forward filter launch of `algo` with its moments in the scratch and the dense backward launch.
-static int dense_grad(int algo, const cdk_desc* d, const void* const* in, void* const* out, cdk_stream_t stream, const char* me) {
+// The part of cdk_ekf_grad_dense_f64 / cdk_ukf_grad_dense_f64 / cdk_ukf_grad_sigma_f64 after their own checks: the
+// shared-memory budget, the output buffers, then the forward filter launch of `algo` with its moments in the scratch and the
+// dense backward launch (`sigma`: through the literal sigma-point predict; d has CDK_FLAG_UKF_SIGMA_POINTS set then).
+static int dense_grad(int algo, const cdk_desc* d, const void* const* in, void* const* out, cdk_stream_t stream, const char* me,
+                      bool sigma = false) {
   char msg[256];
   auto reject = [&](int code, const char* why) {
     snprintf(msg, sizeof(msg), "%s: %s", me, why);
     return fail(code, msg);
   };
-  if (!cdk::ekf_grad_dense_fits(*d)) {
+  if (!cdk::ekf_grad_dense_fits(*d, sigma)) {
     if (d->drift_id == CDK_DRIFT_USER)
       snprintf(msg, sizeof(msg), "%s: n = %d, m = %d, n_theta = %d: the backward working set with the user drift's dual "
                "copy of [x | theta] exceeds the 227 KB of one CTA (see cdk.h)", me, d->n, d->m, d->n_theta);
@@ -411,7 +413,7 @@ static int dense_grad(int algo, const cdk_desc* d, const void* const* in, void* 
   if (rc == CDK_E_UNSUPPORTED) rc = launch_generic<double>(algo, f, s);
   if (rc == CDK_E_SIZE) return reject(rc, "the forward filter's working set exceeds the 227 KB of one CTA");
   if (rc != CDK_OK) return rc;
-  return launch_ekf_grad_dense(a, status, static_cast<double*>(out[CDK_OUT_GRAD]), algo == ALGO_UKF_FILTER, s);
+  return launch_ekf_grad_dense(a, status, static_cast<double*>(out[CDK_OUT_GRAD]), algo == ALGO_UKF_FILTER && !sigma, sigma, s);
 }
 
 int cdk_ekf_grad_dense_f64(const cdk_desc* d, const void* const* in, void* const* out, cdk_stream_t stream) {
@@ -446,14 +448,37 @@ int cdk_ukf_grad_dense_f64(const cdk_desc* d, const void* const* in, void* const
   if (d && (d->reserved[2] & CDK_FLAG_PREDICT_ONLY)) return reject(CDK_E_UNSUPPORTED, "CDK_FLAG_PREDICT_ONLY has no log-likelihood to differentiate");
   if (d && (d->reserved[2] & CDK_FLAG_DIAG_R)) return reject(CDK_E_UNSUPPORTED, "CDK_FLAG_DIAG_R is not supported");
   if (d && (d->reserved[2] & CDK_FLAG_UKF_SIGMA_POINTS))
-    return reject(CDK_E_UNSUPPORTED, "CDK_FLAG_UKF_SIGMA_POINTS: only the closed-form unscented predict is differentiated");
+    return reject(CDK_E_UNSUPPORTED, "CDK_FLAG_UKF_SIGMA_POINTS: differentiated by cdk_ukf_grad_sigma_f64");
   if (d && d->drift_id == CDK_DRIFT_USER)
-    return reject(CDK_E_UNSUPPORTED, "a user-defined drift runs literal sigma points, whose VJP is not implemented");
+    return reject(CDK_E_UNSUPPORTED, "a user-defined drift runs literal sigma points: differentiated by cdk_ukf_grad_sigma_f64");
   int rc = validate(d, in, out, ALGO_UKF_FILTER);
   if (rc != CDK_OK) return rc;
   if (d->d_u > 0) return reject(CDK_E_UNSUPPORTED, "inputs (d_u > 0) are not supported");
   if (d->reserved[3] != 0) return reject(CDK_E_UNSUPPORTED, "desc.reserved[3] must be 0");
   return dense_grad(ALGO_UKF_FILTER, d, in, out, stream, me);
+}
+
+int cdk_ukf_grad_sigma_f64(const cdk_desc* d, const void* const* in, void* const* out, cdk_stream_t stream) {
+  static const char* me = "cdk_ukf_grad_sigma_f64";
+  char msg[256];
+  auto reject = [&](int code, const char* why) {
+    snprintf(msg, sizeof(msg), "%s: %s", me, why);
+    return fail(code, msg);
+  };
+  if (d && (d->reserved[2] & CDK_FLAG_PREDICT_ONLY)) return reject(CDK_E_UNSUPPORTED, "CDK_FLAG_PREDICT_ONLY has no log-likelihood to differentiate");
+  if (d && (d->reserved[2] & CDK_FLAG_DIAG_R)) return reject(CDK_E_UNSUPPORTED, "CDK_FLAG_DIAG_R is not supported");
+  if (d && d->drift_id == CDK_DRIFT_USER && !cdk::ekf_grad_has_user_drift())
+    return reject(CDK_E_UNSUPPORTED, "a user-defined drift is differentiated only by a variant library built with its "
+                                     "gradient unit: build_user_drift(code, grad=True), i.e. LearnableUserDrift(..., "
+                                     "differentiable=True)");
+  if (!d) return validate(d, in, out, ALGO_UKF_FILTER);
+  cdk_desc sd = *d;  // the forward pass is the sigma-point filter whatever the caller's flags say
+  sd.reserved[2] |= CDK_FLAG_UKF_SIGMA_POINTS;
+  int rc = validate(&sd, in, out, ALGO_UKF_FILTER);
+  if (rc != CDK_OK) return rc;
+  if (sd.d_u > 0) return reject(CDK_E_UNSUPPORTED, "inputs (d_u > 0) are not supported");
+  if (sd.reserved[3] != 0) return reject(CDK_E_UNSUPPORTED, "desc.reserved[3] must be 0");
+  return dense_grad(ALGO_UKF_FILTER, &sd, in, out, stream, me, true);
 }
 
 size_t cdk_scratch_bytes(const cdk_desc* d, const char* entry_point) {
@@ -463,8 +488,9 @@ size_t cdk_scratch_bytes(const cdk_desc* d, const char* entry_point) {
   const bool kf = strstr(entry_point, "kf_filter") != nullptr && strstr(entry_point, "ekf") == nullptr &&
                   strstr(entry_point, "ukf") == nullptr && strstr(entry_point, "enkf") == nullptr;
   const bool ks = strstr(entry_point, "kf_smooth") != nullptr && strstr(entry_point, "ekf") == nullptr;
-  // the dense gradients first: "cdk_ukf_grad_dense" also contains "kf_grad" and not "ekf_grad"
-  if (strstr(entry_point, "ekf_grad_dense") != nullptr || strstr(entry_point, "ukf_grad_dense") != nullptr)
+  // the dense gradients first: "cdk_ukf_grad_dense" and "cdk_ukf_grad_sigma" also contain "kf_grad" and not "ekf_grad"
+  if (strstr(entry_point, "ekf_grad_dense") != nullptr || strstr(entry_point, "ukf_grad_dense") != nullptr ||
+      strstr(entry_point, "ukf_grad_sigma") != nullptr)
     return (size_t)cdk::ekf_grad_dense_scratch_doubles(*d) * sizeof(double);
   if (strstr(entry_point, "kf_grad") != nullptr && strstr(entry_point, "ekf_grad") == nullptr)
     return (size_t)cdk::kf_grad_scratch_doubles(*d) * sizeof(double);
@@ -519,6 +545,7 @@ static int xla_dispatch(cdk_stream_t stream, void** buffers, const char* opaque,
       {"cdk_enkf_filter_f64", cdk_enkf_filter_f64}, {"cdk_enkf_filter_f32", cdk_enkf_filter_f32},
       {"cdk_ekf_grad_f64", cdk_ekf_grad_f64},     {"cdk_kf_grad_f64", cdk_kf_grad_f64},
       {"cdk_ekf_grad_dense_f64", cdk_ekf_grad_dense_f64}, {"cdk_ukf_grad_dense_f64", cdk_ukf_grad_dense_f64},
+      {"cdk_ukf_grad_sigma_f64", cdk_ukf_grad_sigma_f64},
       {"cdk_sample_path_f64", cdk_sample_path_f64}, {"cdk_sample_path_f32", cdk_sample_path_f32},
       {"cdk_emission_moments_f64", cdk_emission_moments_f64}, {"cdk_emission_moments_f32", cdk_emission_moments_f32}};
   for (auto& e : table)

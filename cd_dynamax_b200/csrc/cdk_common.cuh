@@ -223,11 +223,11 @@ int launch_ekf_l63_grad(const KArgs<double>& a, double* grad, cudaStream_t s);
 int launch_kf_grad(const KArgs<double>& a, double* grad, cudaStream_t s);  // cdk_kfwarp.cu
 long long kf_grad_scratch_doubles(const cdk_desc& d);                      // its out[CDK_OUT_SCRATCH], in doubles
 bool kf_warp_eligible(const cdk_desc& d, bool smooth);  // fp64 requests served by kf_warp_filter / kf_warp_smooth
-// cdk_ekfgrad.cu: the backward launch of cdk_ekf_grad_dense_f64 (ukf: of cdk_ukf_grad_dense_f64), its scratch (doubles) and
-// its shared-memory budget
-int launch_ekf_grad_dense(const KArgs<double>& a, const int* status, double* grad, bool ukf, cudaStream_t s);
+// cdk_ekfgrad.cu: the backward launch of cdk_ekf_grad_dense_f64 (ukf: of cdk_ukf_grad_dense_f64; sigma: of
+// cdk_ukf_grad_sigma_f64), its scratch (doubles) and its shared-memory budget
+int launch_ekf_grad_dense(const KArgs<double>& a, const int* status, double* grad, bool ukf, bool sigma, cudaStream_t s);
 long long ekf_grad_dense_scratch_doubles(const cdk_desc& d);
-bool ekf_grad_dense_fits(const cdk_desc& d);
+bool ekf_grad_dense_fits(const cdk_desc& d, bool sigma);
 int set_lw_trace(void* devbuf);
 template <typename T>
 int launch_generic(int algo, const KArgs<T>& a, cudaStream_t s);

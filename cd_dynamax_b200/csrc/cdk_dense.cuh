@@ -155,17 +155,19 @@ __device__ __forceinline__ T drift_jac_vjp_x(int id, const T* th, int n, int l, 
   }
 }
 
-template <typename T>
+// JB = false: the f-part sum_i ab_i df_i/dtheta_e alone (Jb, P and second unused) -- all the theta-contraction the
+// sigma-point UKF gradient needs, its sigma points entering f only (drift_theta_vjp_f).
+template <typename T, bool JB = true>
 __device__ __forceinline__ T drift_theta_vjp(int id, const T* th, int n, int e, const T* x, const T* ab, const T* Jb, int ld,
                                              const T* P, bool second) {
   switch (id) {
     case CDK_DRIFT_LINEAR:
-      if (e < n * n) return ab[e / n] * x[e % n] + Jb[(e / n) * ld + e % n];
+      if (e < n * n) return JB ? ab[e / n] * x[e % n] + Jb[(e / n) * ld + e % n] : ab[e / n] * x[e % n];
       return ab[e - n * n];
     case CDK_DRIFT_LORENZ63:  // J00 = -sigma, J01 = sigma, J10 = rho - z, J22 = -beta
-      if (e == 0) return ab[0] * (x[1] - x[0]) - Jb[0] + Jb[1];
-      if (e == 1) return ab[1] * x[0] + Jb[ld];
-      return -ab[2] * x[2] - Jb[2 * ld + 2];
+      if (e == 0) return JB ? ab[0] * (x[1] - x[0]) - Jb[0] + Jb[1] : ab[0] * (x[1] - x[0]);
+      if (e == 1) return JB ? ab[1] * x[0] + Jb[ld] : ab[1] * x[0];
+      return JB ? -ab[2] * x[2] - Jb[2 * ld + 2] : -ab[2] * x[2];
     case CDK_DRIFT_LORENZ96: {
       T s = T(0);
       for (int i = 0; i < n; ++i) s += ab[i];
@@ -175,9 +177,10 @@ __device__ __forceinline__ T drift_theta_vjp(int id, const T* th, int n, int e, 
       if (e < n) return ab[e];
       if (e < n + n * n) {
         const int q = e - n, i = q / n, j = q % n;
-        return ab[i] * x[j] + Jb[i * ld + j];
+        return JB ? ab[i] * x[j] + Jb[i * ld + j] : ab[i] * x[j];
       }
       const int q = e - n - n * n, i = q / (n * n), j = (q / n) % n, k = q % n;
+      if (!JB) return ab[i] * x[j] * x[k];
       T s = ab[i] * x[j] * x[k] + Jb[i * ld + j] * x[k] + Jb[i * ld + k] * x[j];
       if (second) {  // g_k = sum_i (C_iik + C_iki)
         if (i == j) {
@@ -194,6 +197,11 @@ __device__ __forceinline__ T drift_theta_vjp(int id, const T* th, int n, int e, 
       return s;
     }
   }
+}
+
+template <typename T>
+__device__ __forceinline__ T drift_theta_vjp_f(int id, int n, int e, const T* x, const T* ab) {
+  return drift_theta_vjp<T, false>(id, nullptr, n, e, x, ab, nullptr, 0, nullptr, false);
 }
 
 // Reverse-mode contractions of drift_half_trhp (cdk_ukf_grad_dense_f64) for the cotangent ab of the mean right-hand side.
@@ -413,8 +421,9 @@ __device__ void chol_warp(int w, T* L, int n, int ld) {
 // broadcast values -- one shared-memory load and CB FMAs per lane and step, no barrier until the end.  (History: one
 // THREAD per right-hand side with serial dot products, ~21k cycles for m = 20, n = 40 with six of eight warps parked at
 // the barrier -- 17 % of the UKF observation-step, profiles/r02_generic_ukf_rowseg*.)  Chunks are dealt from the LAST warp
-// down so that warp 0, which evaluates the log-density first (mvn_ll_warp), gets the fewest.
-template <typename T, bool TWO>
+// down so that warp 0, which evaluates the log-density first (mvn_ll_warp), gets the fewest.  FWD = false skips the forward
+// substitution: then X solves L^T X = B alone (the Cholesky VJP of the sigma-point UKF gradient).
+template <typename T, bool TWO, bool FWD = true>
 __device__ __forceinline__ void chol_solve_chunks(const T* L, int n, int ld, const T* B, T* X, int c, int ldb) {
   constexpr int CB = 5;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarp = blockDim.x >> 5;
@@ -431,7 +440,7 @@ __device__ __forceinline__ void chol_solve_chunks(const T* L, int n, int ld, con
       x0[q] = (v0 && col0 + q < c) ? B[r0 * ldb + col0 + q] : T(0);
       x1[q] = (v1 && col0 + q < c) ? B[r1 * ldb + col0 + q] : T(0);
     }
-    for (int i = 0; i < n; ++i) {  // L z = b
+    for (int i = 0; FWD && i < n; ++i) {  // L z = b
       const int src = i & 31;
       const bool hi = TWO && i >= 32;
       const T l0 = (v0 && r0 > i) ? L[r0 * ld + i] : T(0);
@@ -484,6 +493,17 @@ __device__ void chol_solve(const T* L, int n, int ld, const T* B, T* X, int c, i
 template <typename T>
 __device__ void chol_solve(const T* L, int n, int ld, T* B, int c, int ldb) {
   chol_solve<T>(L, n, ld, B, B, c, ldb);
+}
+
+// Solve L^T X = B in place (B [n x c], leading dimension ldb): the backward phase of chol_solve.  Ends with a barrier.
+template <typename T>
+__device__ void chol_solve_lt(const T* L, int n, int ld, T* B, int c, int ldb) {
+  if (n <= 32) {
+    chol_solve_chunks<T, false, false>(L, n, ld, B, B, c, ldb);
+  } else {
+    chol_solve_chunks<T, true, false>(L, n, ld, B, B, c, ldb);
+  }
+  __syncthreads();
 }
 
 // log N(r; 0, L L^T) = -0.5 |L^-1 r|^2 - sum_i log L_ii - (m / 2) log(2 pi) for m <= 64, by WARP 0 (the MVN.log_prob of every
@@ -619,6 +639,62 @@ __device__ __forceinline__ void mm_dmma_strip(const T* __restrict__ A, int lda, 
       }
     }
   }
+}
+
+// ---- the literal sigma-point unscented moment ODE (cdk_ukf_filter with CDK_FLAG_UKF_SIGMA_POINTS, cdk_ukf_grad_sigma) ----
+// lambda = alpha^2 (n + kappa) - n;  c = sqrt(n + lambda);  w = 1 / (2 (n + lambda));  w0 = lambda / (n + lambda)
+template <typename T>
+struct UkfSigmaWeights {
+  T lam, cs, w, w0;
+  __device__ explicit UkfSigmaWeights(const cdk_desc& d) {
+    lam = T(d.alpha * d.alpha * (d.n + d.kappa) - d.n);
+    cs = sqrt(T(d.n) + lam);
+    w = T(1) / (T(2) * (T(d.n) + lam));
+    w0 = lam / (T(d.n) + lam);
+  }
+};
+
+// k = dt * rhs(m, P) of Sarkka eq. 3.183 (inference_ukf.py:130-152).  With X = [m, m + c L_i, m - c L_i], Lc = chol(P):
+//   dm = w0 f(m) + w sum_i (f(X_i^+) + f(X_i^-))
+//   f_X^T W X = sum_k w_c[k] (f_k - fbar)(x_k - xbar)^T = w c sum_i (f_i^+ - f_i^-) L_i^T     (xbar = m)
+//   dP = w c (D Lc^T + Lc D^T) + Sigma,  D[:, i] = f(X_i^+) - f(X_i^-)
+// m, P, lql (Sigma), Lc, dF (D) and the outputs km, kP are n x ld blocks in shared memory; Lc and dF are left holding
+// chol(P) and D.  Ends with a barrier.
+template <typename T>
+__device__ void ukf_sigma_rhs(const cdk_desc& d, const T* th, int n, int ld, const T* mm, const T* P, const T* lql, T* Lc,
+                              T* dF, T* km, T* kP, T dt) {
+  T* sF = kP;  // sF[j*ld + i] = f_j(X_i^+) + f_j(X_i^-): parked in the output block until the row sums are taken
+  chol<T>(P, Lc, n, ld, T(0));
+  const UkfSigmaWeights<T> u(d);
+  const T cs = u.cs, w = u.w, w0 = u.w0;
+  FOR_T(e, n * n) {
+    const int j = e / n, i = e - j * n;
+    const T fp = drift_f<T>(d.drift_id, th, n, j, [&](int q) { return mm[q] + cs * Lc[q * ld + i]; });
+    const T fm = drift_f<T>(d.drift_id, th, n, j, [&](int q) { return mm[q] - cs * Lc[q * ld + i]; });
+    dF[j * ld + i] = fp - fm;
+    sF[j * ld + i] = fp + fm;
+  }
+  __syncthreads();
+  FOR_T(j, n) {
+    T s = T(0);
+    for (int i = 0; i < n; ++i) s += sF[j * ld + i];
+    const T f0 = drift_f<T>(d.drift_id, th, n, j, [&](int q) { return mm[q]; });
+    km[j] = dt * (w0 * f0 + w * s);
+  }
+  __syncthreads();  // the row sums are taken: the output block may be overwritten
+  const T wc = w * cs;
+  T* DL = kP;  // dF Lc^T, symmetrised in place below
+  mm_dmma<T, false, true>(dF, ld, Lc, ld, n, n, n, [&](int i, int j, double v) { DL[i * ld + j] = (T)v; });
+  __syncthreads();
+  FOR_T(e, n * n) {
+    const int a = e / n, b = e - a * n;
+    if (a <= b) {  // one thread owns the pair (a, b), (b, a)
+      const T dab = DL[a * ld + b], dba = DL[b * ld + a];
+      kP[a * ld + b] = dt * (wc * (dab + dba) + lql[a * ld + b]);
+      if (a != b) kP[b * ld + a] = dt * (wc * (dba + dab) + lql[b * ld + a]);
+    }
+  }
+  __syncthreads();
 }
 
 }  // namespace cdk

@@ -1,5 +1,7 @@
-// cdk_ekfgrad.cu -- reverse-mode gradient of the CD-EKF and closed-form CD-UKF log-likelihoods for every registry drift
-// and emission size (cdk_ekf_grad_dense_f64, cdk_ukf_grad_dense_f64): ONE CTA PER TRAJECTORY, like generic_filter_kernel.
+// cdk_ekfgrad.cu -- reverse-mode gradient of the CD-EKF, closed-form CD-UKF and sigma-point CD-UKF log-likelihoods for
+// every registry drift and emission size (cdk_ekf_grad_dense_f64, cdk_ukf_grad_dense_f64, cdk_ukf_grad_sigma_f64; the
+// last also for user drifts): ONE CTA PER TRAJECTORY, like generic_filter_kernel.  The sigma-point predict's right-hand
+// side and its VJP are described at eg_sigma_rhs_vjp (ukf_sigma_grad_kernel, DESIGN 4.2g).
 //
 // The forward pass is the filter launch cdk_ekf_filter_f64 (cdk_ukf_filter_f64) makes, with its filtered and predicted
 // moments written to the scratch.  ekf_grad_dense_kernel then walks k = K-1 .. 0 with the cotangent (mu_bar, P_bar) of the moments entering
@@ -120,13 +122,19 @@ struct Eg {
   }
 };
 
-// k = dt * rhs(y), y and k in shared memory.  Ends with a barrier.
+// k = dt * rhs(y), y and k in shared memory.  Ends with a barrier.  SIGMA: the literal sigma-point unscented predict of
+// the filter (ukf_sigma_rhs), with Lc and D in W1 and W2 as there.
+template <bool SIGMA>
 __device__ void eg_rhs(const Eg& c, const double* y, double* k, double dt) {
   const EgLay& L = c.L;
   const int n = L.n, ld = L.ldn, id = c.g.k.d.drift_id;
   const double* th = c.p(L.TH);
   const double* lql = c.p(L.LQL);
   const double* P = y + L.mpoff;
+  if (SIGMA) {
+    ukf_sigma_rhs<double>(c.g.k.d, th, n, ld, y, P, lql, c.p(L.W1), c.p(L.W2), k, k + L.mpoff, dt);
+    return;
+  }
   double* J = c.p(L.J);
   double* JP = c.p(L.W1);
   FOR_T(e, n * n) {
@@ -309,7 +317,180 @@ __device__ void eg_rhs_vjp(const Eg& c, const double* y, const double* kb, doubl
   __syncthreads();
 }
 
+#if CDK_HAS_USER_DRIFT
+// theta_bar_e += sum_p sum_j Fb[p][j] df_j/dtheta_e (X_p) over the np points X (rows of ldn; Fb likewise) for the user
+// drift: dual evaluations of its f with only theta seeded, EG_DW directions at a time, into the CTA's one dual copy of
+// theta; x enters as plain constants.  The per-thread partial sums are added in thread order, as in eg_user_vjp.
+// Ends with a barrier.
+__device__ void eg_user_theta(const Eg& c, const double* X, const double* Fb, int np) {
+  const EgLay& L = c.L;
+  const int n = L.n, ld = L.ldn, nth = L.nth, E = np * n;
+  const double* th = c.p(L.TH);
+  double* part = c.p(L.PART);
+  double* thb = c.p(L.THB);
+  EgDual* td = reinterpret_cast<EgDual*>(c.p(L.DU)) + n;
+  FOR_T(v, nth) td[v] = EgDual(th[v]);
+  __syncthreads();
+  for (int c0 = 0; c0 < nth; c0 += EG_DW) {
+    FOR_T(e, nth * EG_DW) {
+      const int v = e / EG_DW, w = e - v * EG_DW;
+      td[v].d[w] = c0 + w == v ? 1.0 : 0.0;
+    }
+    __syncthreads();
+    double acc[EG_DW];
+#pragma unroll
+    for (int w = 0; w < EG_DW; ++w) acc[w] = 0.0;
+    for (int e = threadIdx.x; e < E; e += blockDim.x) {
+      const int p = e / n, j = e - p * n;
+      const double* x = X + p * ld;
+      const EgDual v = cdk_user::f<EgDual>(td, n, j, [&](int q) { return EgDual(x[q]); });
+      const double wt = Fb[p * ld + j];
+#pragma unroll
+      for (int w = 0; w < EG_DW; ++w) acc[w] += wt * v.d[w];
+    }
+#pragma unroll
+    for (int w = 0; w < EG_DW; ++w) part[threadIdx.x * EG_DW + w] = acc[w];
+    __syncthreads();
+    FOR_T(w, EG_DW) {
+      const int v = c0 + w;
+      if (v < nth) {
+        double s = 0.0;
+        for (int t = 0; t < (int)blockDim.x; ++t) s += part[t * EG_DW + w];
+        thb[v] += s;
+      }
+    }
+  }
+  __syncthreads();
+}
+#endif
+
+// theta_bar += sum over the np points X (rows) of sum_j Fb[p][j] df_j/dtheta (X_p): the registry's f-contraction, one thread
+// per parameter and the points in order; the user drift's from dual numbers.  Ends with a barrier.
+__device__ void eg_sigma_theta(const Eg& c, const double* X, const double* Fb, int np) {
+  const EgLay& L = c.L;
+  const int n = L.n, ld = L.ldn, id = c.g.k.d.drift_id;
+#if CDK_HAS_USER_DRIFT
+  if (id == CDK_DRIFT_USER) {
+    eg_user_theta(c, X, Fb, np);
+    return;
+  }
+#endif
+  double* thb = c.p(L.THB);
+  FOR_T(e, L.nth) {
+    double s = 0.0;
+    for (int p = 0; p < np; ++p) s += drift_theta_vjp_f<double>(id, n, e, X + p * ld, Fb + p * ld);
+    thb[e] += s;
+  }
+  __syncthreads();
+}
+
+// VJP of the sigma-point right-hand side (ukf_sigma_rhs) at y = (m, P) for the cotangent kb = (a, A) (already scaled by dt):
+// writes the cotangent of y to `out` (the stage's slot in the scratch) and accumulates theta_bar and Sigma_bar.  With
+// Lc = chol(P), X_i^+- = m +- c Lc[:, i], D[:, i] = f(X_i^+) - f(X_i^-), wc = w c:
+//   As = A + A^T,  Sigma_bar += A,  D_bar = wc As Lc,  Lc_bar = wc As D (direct part)
+//   F_bar_i^+- = w a +- D_bar[:, i],  f0_bar = w0 a,  X_bar_i^+- = J(X_i^+-)^T F_bar_i^+-
+//   m_bar = J(m)^T f0_bar + sum_i (X_bar_i^+ + X_bar_i^-),  Lc_bar[:, i] += c (X_bar_i^+ - X_bar_i^-)
+//   theta_bar += sum over the 2n + 1 points of F_bar^T df/dtheta
+//   P_bar = sym(Lc^-T Phi(Lc^T tril(Lc_bar)) Lc^-1),  Phi: the lower triangle with the diagonal halved
+// (the symmetric Cholesky VJP, torch's linalg.cholesky backward).  The stage VJP leaves YC, ACC, J, W1 and W2 idle; they
+// hold Lc, As (then F_bar), D (then X_bar), D_bar (then the transposed solve) and Lc_bar, and the sigma points of one sign
+// (then Phi) sit behind the layout at XS = L.total.  Ends with a barrier.
+__device__ void eg_sigma_rhs_vjp(const Eg& c, const double* y, const double* kb, double* out) {
+  const EgLay& L = c.L;
+  const cdk_desc& d = c.g.k.d;
+  const int n = L.n, ld = L.ldn, id = d.drift_id;
+  const double* th = c.p(L.TH);
+  const double* mm = y;
+  const double* P = y + L.mpoff;
+  const double* ab = kb;
+  const double* Ab = kb + L.mpoff;
+  double* Lc = c.p(L.YC);
+  double* As = c.p(L.ACC);
+  double* Fb = As;
+  double* D = c.p(L.J);
+  double* Xb = D;
+  double* Db = c.p(L.W1);
+  double* Lb = c.p(L.W2);
+  double* X = c.p(L.total);
+  double* sigb = c.p(L.SIGB);
+  double* outP = out + L.mpoff;
+  FOR_T(e, n * n) {
+    const int i = e / n, j = e - i * n;
+    As[i * ld + j] = Ab[i * ld + j] + Ab[j * ld + i];
+    sigb[i * ld + j] += Ab[i * ld + j];
+  }
+  // chol's first loop copies P into Lc (YC) before its first barrier; the loop above writes only As (ACC) and SIGB, which
+  // that copy does not touch, so no barrier is needed here.  chol ends with a barrier.
+  chol<double>(P, Lc, n, ld, 0.0);
+  const UkfSigmaWeights<double> u(d);
+  const double cs = u.cs, w = u.w, wc = u.w * u.cs;
+  FOR_T(e, n * n) {
+    const int j = e / n, i = e - j * n;
+    const double fp = drift_f<double>(id, th, n, j, [&](int q) { return mm[q] + cs * Lc[q * ld + i]; });
+    const double fm = drift_f<double>(id, th, n, j, [&](int q) { return mm[q] - cs * Lc[q * ld + i]; });
+    D[j * ld + i] = fp - fm;
+  }
+  __syncthreads();
+  mm_dmma<double, false, false>(As, ld, Lc, ld, n, n, n, [&](int i, int j, double v) { Db[i * ld + j] = wc * v; });
+  mm_dmma<double, false, false>(As, ld, D, ld, n, n, n, [&](int i, int j, double v) { Lb[i * ld + j] = wc * v; });
+  __syncthreads();
+  for (int sg = 0; sg < 2; ++sg) {  // the points X_i^+ (rows of X), then X_i^-
+    FOR_T(e, n * n) {
+      const int i = e / n, q = e - i * n;
+      const double v = cs * Lc[q * ld + i];
+      X[i * ld + q] = sg == 0 ? mm[q] + v : mm[q] - v;
+      Fb[i * ld + q] = sg == 0 ? w * ab[q] + Db[q * ld + i] : w * ab[q] - Db[q * ld + i];
+    }
+    __syncthreads();
+    FOR_T(e, n * n) {
+      const int i = e / n, l = e - i * n;
+      const double* x = X + i * ld;
+      double xb = 0.0;
+      for (int j = 0; j < n; ++j) xb += drift_jac<double>(id, th, n, j, l, x) * Fb[i * ld + j];
+      if (sg == 0) {
+        Xb[i * ld + l] = xb;
+        Lb[l * ld + i] += cs * xb;
+      } else {
+        Xb[i * ld + l] += xb;
+        Lb[l * ld + i] -= cs * xb;
+      }
+    }
+    eg_sigma_theta(c, X, Fb, n);
+  }
+  FOR_T(j, n) Fb[j] = u.w0 * ab[j];  // the centre point m
+  __syncthreads();
+  FOR_T(l, n) {
+    double s = 0.0;
+    for (int j = 0; j < n; ++j) s += drift_jac<double>(id, th, n, j, l, mm) * Fb[j];
+    for (int i = 0; i < n; ++i) s += Xb[i * ld + l];
+    out[l] = s;
+  }
+  FOR_T(e, n * n) {  // only the lower triangle of Lc_bar enters
+    const int i = e / n, j = e - i * n;
+    if (j > i) Lb[i * ld + j] = 0.0;
+  }
+  eg_sigma_theta(c, mm, Fb, 1);
+  // ---- Cholesky VJP: Phi(Lc^T Lc_bar) into X, two solves with Lc^T, P_bar = sym ----
+  mm_dmma<double, true, false>(Lc, ld, Lb, ld, n, n, n, [&](int i, int j, double v) {
+    X[i * ld + j] = i > j ? v : (i == j ? 0.5 * v : 0.0);
+  });
+  __syncthreads();
+  chol_solve_lt<double>(Lc, n, ld, X, n, ld);  // Y = Lc^-T Phi
+  FOR_T(e, n * n) {
+    const int i = e / n, j = e - i * n;
+    Db[i * ld + j] = X[j * ld + i];
+  }
+  __syncthreads();
+  chol_solve_lt<double>(Lc, n, ld, Db, n, ld);  // Z^T = Lc^-T Y^T,  Z = Lc^-T Phi Lc^-1
+  FOR_T(e, n * n) {
+    const int i = e / n, j = e - i * n;
+    outP[i * ld + j] = 0.5 * (Db[i * ld + j] + Db[j * ld + i]);
+  }
+  __syncthreads();
+}
+
 // One substep of the state YC (in place) through the stages of any tableau; the stage inputs are left in stg[s * st].
+template <bool SIGMA>
 __device__ void eg_step(const Eg& c, double dt, double* __restrict__ stg) {
   const EgLay& L = c.L;
   const int st = L.st, S = L.S;
@@ -324,7 +505,7 @@ __device__ void eg_step(const Eg& c, double dt, double* __restrict__ stg) {
   for (int s = 0; s < S; ++s) {
     FOR_T(e, st) ys[e] = stg[s * st + e];
     __syncthreads();
-    eg_rhs(c, ys, k, dt);
+    eg_rhs<SIGMA>(c, ys, k, dt);
     const double b = c.g.tab.b[s];
     FOR_T(e, st) {
       const double kv = k[e];
@@ -342,6 +523,7 @@ __device__ void eg_step(const Eg& c, double dt, double* __restrict__ stg) {
 
 // VJP of the substep eg_step just took (stage inputs in stg): YB is the cotangent of its end state on entry and of its
 // start state on exit.  stb[s * st] receives the stage-input cotangents.
+template <bool SIGMA>
 __device__ void eg_step_vjp(const Eg& c, double dt, const double* __restrict__ stg, double* __restrict__ stb) {
   const EgLay& L = c.L;
   const int st = L.st, S = L.S;
@@ -360,7 +542,11 @@ __device__ void eg_step_vjp(const Eg& c, double dt, const double* __restrict__ s
       ys[e] = stg[s * st + e];
     }
     __syncthreads();
-    eg_rhs_vjp(c, ys, kb, stb + s * st);
+    if (SIGMA) {
+      eg_sigma_rhs_vjp(c, ys, kb, stb + s * st);
+    } else {
+      eg_rhs_vjp(c, ys, kb, stb + s * st);
+    }
   }
   FOR_T(e, st) {
     double v = yb[e];
@@ -483,9 +669,10 @@ __device__ void eg_save(double* __restrict__ dst, const double* src, int st) {
   FOR_T(e, st) dst[e] = src[e];
 }
 
-__global__ void __launch_bounds__(256) ekf_grad_dense_kernel(const EgArgs g) {
-  extern __shared__ __align__(16) unsigned char smem_raw[];
-  Eg c(g, reinterpret_cast<double*>(smem_raw));
+// The backward walk of one trajectory (one CTA); SIGMA: the literal sigma-point unscented predict.
+template <bool SIGMA>
+__device__ __forceinline__ void eg_body(const EgArgs& g, double* smem) {
+  Eg c(g, smem);
   const EgLay& L = c.L;
   const KArgs<double>& a = g.k;
   const cdk_desc& d = a.d;
@@ -564,7 +751,7 @@ __global__ void __launch_bounds__(256) ekf_grad_dense_kernel(const EgArgs g) {
             eg_save(ck1 + (i / s1) * st, yc, st);
             if (threadIdx.x == 0) ckc1[i / s1] = clk;
           }
-          eg_step(c, clk.dt(), stg);
+          eg_step<SIGMA>(c, clk.dt(), stg);
           clk.advance();
         }
       }
@@ -581,7 +768,7 @@ __global__ void __launch_bounds__(256) ekf_grad_dense_kernel(const EgArgs g) {
               eg_save(ck2 + (u / s2) * st, yc, st);
               if (threadIdx.x == 0) ckc2[u / s2] = clk;
             }
-            eg_step(c, clk.dt(), stg);
+            eg_step<SIGMA>(c, clk.dt(), stg);
             clk.advance();
           }
           if ((len - 1) % s2 == 0) {
@@ -595,11 +782,11 @@ __global__ void __launch_bounds__(256) ekf_grad_dense_kernel(const EgArgs g) {
           eg_load(yc, len > 1 ? ck2 + (u / s2) * st : ck1 + seg * st, st);
           __syncthreads();
           for (int v = (len > 1 ? (u / s2) * s2 : u); v < u; ++v) {
-            eg_step(c, clk.dt(), stg);
+            eg_step<SIGMA>(c, clk.dt(), stg);
             clk.advance();
           }
-          eg_step(c, clk.dt(), stg);  // the stage inputs of substep i0 + u
-          eg_step_vjp(c, clk.dt(), stg, stb);
+          eg_step<SIGMA>(c, clk.dt(), stg);  // the stage inputs of substep i0 + u
+          eg_step_vjp<SIGMA>(c, clk.dt(), stg, stb);
         }
       }
     }
@@ -640,20 +827,36 @@ __global__ void __launch_bounds__(256) ekf_grad_dense_kernel(const EgArgs g) {
   FOR_T(i, n) gm0[i] = yb[i];
 }
 
-}  // namespace
-
-// The layout of the scratch and shared memory of cdk_ekf_grad_dense_f64 and cdk_ukf_grad_dense_f64 for `d` (false: beyond
-// the 227 KB of one CTA)
-static bool eg_layout(const cdk_desc& d, EgLay& lay, RtTab& rt) {
-  if (!fill_rt_tab(d.solver, rt)) return false;
-  lay = EgLay(d, rt.S);
-  return (size_t)lay.total * sizeof(double) <= 227u * 1024u;
+__global__ void __launch_bounds__(256) ekf_grad_dense_kernel(const EgArgs g) {
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  eg_body<false>(g, reinterpret_cast<double*>(smem_raw));
 }
 
-bool ekf_grad_dense_fits(const cdk_desc& d) {
+// cdk_ukf_grad_sigma_f64: the same walk through the literal sigma-point predict (its own instantiation, so that the
+// EKF and closed-form UKF kernel above keeps its code)
+__global__ void __launch_bounds__(256) ukf_sigma_grad_kernel(const EgArgs g) {
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  eg_body<true>(g, reinterpret_cast<double*>(smem_raw));
+}
+
+}  // namespace
+
+// Shared memory of the backward kernel in doubles: the layout, and for the sigma-point predict one more n x ldn block (XS,
+// behind the layout) for the sigma points of one sign
+static long long eg_smem_doubles(const EgLay& lay, bool sigma) { return lay.total + (sigma ? (lay.nn + 1) / 2 * 2 : 0); }
+
+// The layout of the scratch and shared memory of cdk_ekf_grad_dense_f64, cdk_ukf_grad_dense_f64 and (sigma)
+// cdk_ukf_grad_sigma_f64 for `d` (false: beyond the 227 KB of one CTA)
+static bool eg_layout(const cdk_desc& d, EgLay& lay, RtTab& rt, bool sigma = false) {
+  if (!fill_rt_tab(d.solver, rt)) return false;
+  lay = EgLay(d, rt.S);
+  return (size_t)eg_smem_doubles(lay, sigma) * sizeof(double) <= 227u * 1024u;
+}
+
+bool ekf_grad_dense_fits(const cdk_desc& d, bool sigma) {
   EgLay lay;
   RtTab rt;
-  return eg_layout(d, lay, rt);
+  return eg_layout(d, lay, rt, sigma);
 }
 
 bool ekf_grad_has_user_drift() { return CDK_HAS_USER_DRIFT != 0; }
@@ -666,11 +869,11 @@ long long ekf_grad_dense_scratch_doubles(const cdk_desc& d) {
 }
 
 // The backward launch behind a forward filter pass whose moments are in out[CDK_OUT_SCRATCH] and whose status is `status`;
-// `ukf`: the forward pass was the closed-form UKF filter.
-int launch_ekf_grad_dense(const KArgs<double>& a, const int* status, double* grad, bool ukf, cudaStream_t s) {
+// `ukf`: the forward pass was the closed-form UKF filter; `sigma`: the sigma-point UKF filter (ukf_sigma_grad_kernel).
+int launch_ekf_grad_dense(const KArgs<double>& a, const int* status, double* grad, bool ukf, bool sigma, cudaStream_t s) {
   EgArgs g;
   g.k = a;
-  if (!eg_layout(a.d, g.lay, g.tab)) return CDK_E_SIZE;
+  if (!eg_layout(a.d, g.lay, g.tab, sigma)) return CDK_E_SIZE;
   for (int i = 0; i < 6; ++i)
     for (int j = 0; j < 6; ++j) g.a[i][j] = 0.0;
   for (int i = 0; i < g.tab.S; ++i)
@@ -679,12 +882,19 @@ int launch_ekf_grad_dense(const KArgs<double>& a, const int* status, double* gra
   g.status = status;
   g.grad = grad;
   g.cols = CDK_GRAD_COLS_EKF(a.d.n, a.d.m, a.d.n_theta);
-  g.ukf = ukf ? 1 : 0;
+  g.ukf = ukf || sigma ? 1 : 0;
   const int threads = eg_threads(a.d.n, a.d.m);
-  const size_t smem = (size_t)g.lay.total * sizeof(double);
+  const size_t smem = (size_t)eg_smem_doubles(g.lay, sigma) * sizeof(double);
+  if (a.d.N > 2147483647LL) return CDK_E_SIZE;
+  if (sigma) {
+    if (smem > 48 * 1024 && cudaFuncSetAttribute(ukf_sigma_grad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
+      return check_launch("cudaFuncSetAttribute(ukf_sigma_grad_kernel)");
+    ukf_sigma_grad_kernel<<<(unsigned)a.d.N, threads, smem, s>>>(g);
+    note_launch();
+    return check_launch("ukf_sigma_grad_kernel");
+  }
   if (smem > 48 * 1024 && cudaFuncSetAttribute(ekf_grad_dense_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
     return check_launch("cudaFuncSetAttribute(ekf_grad_dense_kernel)");
-  if (a.d.N > 2147483647LL) return CDK_E_SIZE;
   ekf_grad_dense_kernel<<<(unsigned)a.d.N, threads, smem, s>>>(g);
   note_launch();
   return check_launch("ekf_grad_dense_kernel");

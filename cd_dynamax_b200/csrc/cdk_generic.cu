@@ -237,48 +237,8 @@ __device__ void ode_rhs(const Ctx<T>& c, int kind, const T* ys, T* k, T dt) {
     __syncthreads();
     return;
   }
-  // ODE_UKF: Sarkka eq. 3.183 (inference_ukf.py:130-152).  With X = [m, m + c L_i, m - c L_i], Lc = chol(P):
-  //   dm = w0 f(m) + w sum_i (f(X_i^+) + f(X_i^-)),      w = 1 / (2 (n + lambda)),  c = sqrt(n + lambda)
-  //   f_X^T W X = sum_k w_c[k] (f_k - fbar)(x_k - xbar)^T = w c sum_i (f_i^+ - f_i^-) L_i^T     (xbar = m)
-  {
-    const T* th = c.p(L.TH);
-    T* Lc = c.p(L.W1);
-    T* dF = c.p(L.W2);  // dF[j*ld + i] = f_j(X_i^+) - f_j(X_i^-)
-    T* sF = kP;         // sF[j*ld + i] = f_j(X_i^+) + f_j(X_i^-): parked in the output block until the row sums are taken
-    chol<T>(P, Lc, n, ld, T(0));
-    const T lam = T(d.alpha * d.alpha * (d.n + d.kappa) - d.n);
-    const T cs = sqrt(T(d.n) + lam);
-    const T w = T(1) / (T(2) * (T(d.n) + lam));
-    const T w0 = lam / (T(d.n) + lam);
-    FOR_T(e, n * n) {
-      const int j = e / n, i = e - j * n;
-      const T fp = drift_f<T>(d.drift_id, th, n, j, [&](int q) { return mm[q] + cs * Lc[q * ld + i]; });
-      const T fm = drift_f<T>(d.drift_id, th, n, j, [&](int q) { return mm[q] - cs * Lc[q * ld + i]; });
-      dF[j * ld + i] = fp - fm;
-      sF[j * ld + i] = fp + fm;
-    }
-    __syncthreads();
-    FOR_T(j, n) {
-      T s = T(0);
-      for (int i = 0; i < n; ++i) s += sF[j * ld + i];
-      const T f0 = drift_f<T>(d.drift_id, th, n, j, [&](int q) { return mm[q]; });
-      km[j] = dt * (w0 * f0 + w * s);
-    }
-    __syncthreads();  // the row sums are taken: the output block may be overwritten
-    const T wc = w * cs;
-    T* DL = kP;  // dF Lc^T, symmetrised in place below
-    mm_dmma<T, false, true>(dF, ld, Lc, ld, n, n, n, [&](int i, int j, double v) { DL[i * ld + j] = (T)v; });
-    __syncthreads();
-    FOR_T(e, n * n) {
-      const int a = e / n, b = e - a * n;
-      if (a <= b) {  // one thread owns the pair (a, b), (b, a)
-        const T dab = DL[a * ld + b], dba = DL[b * ld + a];
-        kP[a * ld + b] = dt * (wc * (dab + dba) + lql[a * ld + b]);
-        if (a != b) kP[b * ld + a] = dt * (wc * (dba + dab) + lql[b * ld + a]);
-      }
-    }
-    __syncthreads();
-  }
+  // ODE_UKF: the literal sigma points (cdk_dense.cuh, ukf_sigma_rhs; the gradient's re-integration calls it too)
+  ukf_sigma_rhs<T>(d, c.p(L.TH), n, ld, mm, P, lql, c.p(L.W1), c.p(L.W2), km, kP, dt);
 }
 
 // Integrate y (length S, shared memory, in place) from t0 to t1 with the fixed-step explicit RK in g.tab.

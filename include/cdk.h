@@ -106,7 +106,7 @@ enum {
   CDK_OUT_SCRATCH,/* device scratch of cdk_scratch_bytes() bytes (CD-KF pushforward cache), else NULL */
   CDK_OUT_GRAD,   /* d marginal log-likelihood / d parameters: cdk_ekf_grad_f64 [N, CDK_GRAD_COLS_L63],
                    * cdk_kf_grad_f64 [N, CDK_GRAD_COLS_KF(n, m)],
-                   * cdk_ekf_grad_dense_f64 [N, CDK_GRAD_COLS_EKF(n, m, n_theta)]                              */
+                   * cdk_ekf_grad_dense_f64 / cdk_ukf_grad_dense_f64 / cdk_ukf_grad_sigma_f64 [N, CDK_GRAD_COLS_EKF] */
   CDK_NUM_OUT
 };
 
@@ -248,11 +248,29 @@ CDK_DECL(cdk_ekf_grad_dense_f64);
  * a NaN row.  alpha, beta and kappa do not enter the closed form and get no gradient; state_order and num_iter do not
  * apply and are ignored, as by the filter.
  * Coverage: fp64, full R, every solver, shared or batched parameters, the same shapes as cdk_ekf_grad_dense_f64.
- * CDK_DRIFT_USER and CDK_FLAG_UKF_SIGMA_POINTS (literal sigma points, whose VJP is not implemented), CDK_FLAG_DIAG_R,
- * CDK_FLAG_PREDICT_ONLY, d_u > 0 and a non-zero desc.reserved[3] return CDK_E_UNSUPPORTED, a NULL out[CDK_OUT_GRAD] or
- * out[CDK_OUT_SCRATCH] CDK_E_NULL, a backward working set beyond the 227 KB of one CTA CDK_E_SIZE -- all host-side
- * checks, before any CUDA call. */
+ * CDK_DRIFT_USER and CDK_FLAG_UKF_SIGMA_POINTS (literal sigma points: cdk_ukf_grad_sigma_f64 differentiates those),
+ * CDK_FLAG_DIAG_R, CDK_FLAG_PREDICT_ONLY, d_u > 0 and a non-zero desc.reserved[3] return CDK_E_UNSUPPORTED, a NULL
+ * out[CDK_OUT_GRAD] or out[CDK_OUT_SCRATCH] CDK_E_NULL, a backward working set beyond the 227 KB of one CTA CDK_E_SIZE --
+ * all host-side checks, before any CUDA call. */
 CDK_DECL(cdk_ukf_grad_dense_f64);
+/* Log-likelihood (out[CDK_OUT_LL]), status (out[CDK_OUT_STATUS]) and reverse-mode gradient (out[CDK_OUT_GRAD],
+ * [N, CDK_GRAD_COLS_EKF(n, m, n_theta)], the row layout of cdk_ekf_grad_dense_f64) of the CD-UKF with LITERAL sigma
+ * points, for the same descriptor and inputs as cdk_ukf_filter_f64.  The entry point sets CDK_FLAG_UKF_SIGMA_POINTS on
+ * its own copy of the descriptor, so the forward pass IS the launch cdk_ukf_filter_f64 makes with that flag (the
+ * log-likelihood is bit-identical to it) whatever the caller's flags say.  Its moments go to out[CDK_OUT_SCRATCH]
+ * (required, cdk_scratch_bytes(desc, "cdk_ukf_grad_sigma") bytes: the formula of cdk_ekf_grad_dense_f64 -- the sigma
+ * points of the backward pass live in shared memory), then one backward launch (ukf_sigma_grad_kernel) steps back
+ * through the sigma-point moment ODE: a Cholesky factor of P, 2n + 1 drift evaluations and their VJPs, and the Cholesky
+ * VJP at every stage.  Its shared memory is that of cdk_ekf_grad_dense_f64 plus one n x (n | 1) block (n = 40, m = 20
+ * fits with every solver).  Sigma, R and P0 get the symmetric part (G + G^T)/2; a trajectory whose status is not 0 gets a
+ * NaN row.  alpha, beta and kappa get no gradient (beta does not enter the predict; alpha and kappa are hyper-parameters).
+ * Coverage: fp64, full R, every solver, shared or batched parameters, every registry drift, and CDK_DRIFT_USER in a
+ * variant built with build_user_drift(code, grad=True) (the theta-derivatives of f from dual numbers; an n_theta that
+ * does not fit returns CDK_E_SIZE).  The stock library and a filter-only variant reject CDK_DRIFT_USER with
+ * CDK_E_UNSUPPORTED.  CDK_FLAG_DIAG_R, CDK_FLAG_PREDICT_ONLY, d_u > 0 and a non-zero desc.reserved[3] return
+ * CDK_E_UNSUPPORTED, a NULL out[CDK_OUT_GRAD] or out[CDK_OUT_SCRATCH] CDK_E_NULL, a backward working set beyond the
+ * 227 KB of one CTA CDK_E_SIZE -- all host-side checks, before any CUDA call. */
+CDK_DECL(cdk_ukf_grad_sigma_f64);
 
 /* Forward sample paths of the model (cdnlgssm_path_sample, cd_nonlinear/models.py:525-656; what
  * SSM.sample_batch(..., transition_type="path") vmaps, src/ssm_temissions.py:187-225): x_0 ~ N(m0, P0), x_k = SDE solve of
