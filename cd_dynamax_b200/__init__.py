@@ -9,6 +9,7 @@ from .continuous_discrete_linear_gaussian_ssm import (ContDiscreteLinearGaussian
 from .continuous_discrete_nonlinear_gaussian_ssm import (ContDiscreteNonlinearGaussianSSM, EKFHyperParams,
                                                          EnKFHyperParams, LearnableLinear, LearnableLorenz63,
                                                          LearnableLorenz96, LearnableMatrix, LearnableQuadratic, LearnableUserDrift,
+                                                         LearnableUserEmission,
                                                          LearnableVector, ParamsCDNLGSSM, ParamsCDNLGSSMDynamics,
                                                          ParamsCDNLGSSMEmissions, UKFHyperParams, cdnlgssm_filter,
                                                          cdnlgssm_smoother, ekf_marginal_log_prob_and_grad,

@@ -25,12 +25,14 @@ def _core_shapes(K: int, n: int, m: int, desc_fields: dict, theta_core_ndim: int
     """Per-trajectory shape of every input slot: exactly the slot_elems (cdk_api.cu) entries a kernel reads from it."""
     flags = int(desc_fields.get("flags", 0))
     d_u = int(desc_fields.get("d_u", 0))
+    # a user emission (CDK_EMISSION_USER) reads its parameter vector phi [n_phi] from the H slot
+    h_shape = (int(desc_fields["n_phi"]),) if int(desc_fields.get("emission_id", 0)) == L.EMISSION_USER else (m, n)
     # a forecast and a sampler started from a fixed state read K + 1 time stamps (t_init first), every other entry point K
     t_cols = K + 1 if flags & (L.FLAG_PREDICT_ONLY | L.FLAG_FIXED_INIT) else K
     return {
         L.IN_Y: (K, m), L.IN_T: (t_cols,), L.IN_U: (K, d_u), L.IN_M0: (n,), L.IN_P0: (n, n),
         L.IN_F: (n, n) if theta_core_ndim == 2 else (int(desc_fields.get("n_theta", 0)),),
-        L.IN_B: (n,), L.IN_BU: (n, d_u), L.IN_L: (n, n), L.IN_QC: (n, n), L.IN_H: (m, n), L.IN_D: (m,),
+        L.IN_B: (n,), L.IN_BU: (n, d_u), L.IN_L: (n, n), L.IN_QC: (n, n), L.IN_H: h_shape, L.IN_D: (m,),
         L.IN_DU: (m, d_u), L.IN_R: (m,) if flags & L.FLAG_DIAG_R else (m, m), L.IN_FM: (K, n), L.IN_FP: (K, n, n),
     }
 
@@ -133,6 +135,8 @@ def classify(N: int, K: int, n: int, m: int, inputs: Dict[int, object], desc_fie
     its kernels read and tell shared from batched (leading N) inputs.  -> ({slot: (array, batched, row elements, host?)},
     batched_mask).  Raises ValueError, naming the slot, on any other shape."""
     core_shape = _core_shapes(K, n, m, desc_fields, theta_core_ndim)
+    if int(desc_fields.get("emission_id", 0)) == L.EMISSION_USER:
+        core_ndim_override = {**(core_ndim_override or {}), L.IN_H: 1}
     metas = {}
     mask = 0
     for slot in range(L.NUM_IN):
@@ -185,7 +189,8 @@ def run(entry: str, dt: str, N: int, K: int, n: int, m: int, inputs: Dict[int, o
     # ---- classify inputs (before any device work: a mis-shaped batch is rejected here, not read out of bounds) ----
     metas, mask = classify(N, K, n, m, inputs, desc_fields, theta_core_ndim, core_ndim_override)
     stream_bytes = sum(N * row * esz for _, batched, row, host in metas.values() if batched and host)
-    lib = L.lib(desc_fields.pop("lib_path", None))  # a variant library for a user-defined drift, else the stock one
+    lib = L.lib(desc_fields.pop("lib_path", None))  # a variant library for user device code, else the stock one
+    desc_fields.pop("n_phi", None)  # the kernels take it from the library's own num_params
     dev = device()
     d = L.new_desc()
     d.N, d.K, d.n, d.m = N, K, n, m

@@ -11,6 +11,7 @@ NUM_IN, NUM_OUT = 16, 12
  OUT_GRAD) = range(12)
 SOLVERS = {"euler": 0, "heun": 1, "midpoint": 2, "ralston": 3, "bosh3": 4, "rk4": 5, "dopri5": 6}
 DRIFT_LINEAR, DRIFT_LORENZ63, DRIFT_LORENZ96, DRIFT_QUADRATIC, DRIFT_USER = 0, 1, 2, 3, 4
+EMISSION_LINEAR, EMISSION_USER = 0, 1
 ORDERS = {"zeroth": 0, "first": 1, "second": 2}
 FLAG_KEEP_PUSHFORWARD = 1  # CDK_FLAG_KEEP_PUSHFORWARD (desc.reserved[2])
 FLAG_UKF_SIGMA_POINTS = 2  # CDK_FLAG_UKF_SIGMA_POINTS
@@ -41,7 +42,7 @@ ENTRY_POINTS.append("cdk_ukf_grad_dense_f64")
 ENTRY_POINTS.append("cdk_ukf_grad_sigma_f64")
 ENTRY_POINTS += ["cdk_sample_path_f64", "cdk_sample_path_f32", "cdk_emission_moments_f64", "cdk_emission_moments_f32"]
 OTHER_SYMBOLS = ["cdk_desc_init", "cdk_scratch_bytes", "cdk_ll_sum_f64", "cdk_ll_sum_f32", "cdk_ll_allreduce",
-                 "cdk_xla_custom_call", "cdk_xla_custom_call_status", "cdk_xla_last_rc", "cdk_fma_probe_f64", "cdk_fma_probe_f32", "cdk_fma3_probe_f64", "cdk_dmma_probe_f64", "cdk_rng_probe_f64", "cdk_launch_count", "cdk_debug_set_trace", "cdk_has_user_drift", "cdk_version",
+                 "cdk_xla_custom_call", "cdk_xla_custom_call_status", "cdk_xla_last_rc", "cdk_fma_probe_f64", "cdk_fma_probe_f32", "cdk_fma3_probe_f64", "cdk_dmma_probe_f64", "cdk_rng_probe_f64", "cdk_launch_count", "cdk_debug_set_trace", "cdk_has_user_drift", "cdk_has_user_emission", "cdk_user_emission_params", "cdk_version",
                  "cdk_last_error"]
 
 
@@ -69,8 +70,8 @@ _variants = {}
 
 
 def lib(path=None):
-    """Load libcdk.so once (or, with `path`, a variant built by build.build_user_drift: same ABI, user drift compiled
-    in). Raises (never falls back) if the CUDA extension has not been built."""
+    """Load libcdk.so once (or, with `path`, a variant built by build.build_variant: same ABI, a user drift and / or
+    emission compiled in). Raises (never falls back) if the CUDA extension has not been built."""
     global _lib
     if path is None and _lib is not None:
         return _lib
@@ -118,6 +119,9 @@ def lib(path=None):
     L.cdk_last_error.restype = ctypes.c_char_p
     assert ctypes.sizeof(CdkDesc) == _c_sizeof_desc(L), "cdk_desc layout mismatch between Python and C"
     L.cdk_has_user_drift.restype = ctypes.c_int
+    L.cdk_has_user_emission.restype = ctypes.c_int
+    L.cdk_user_emission_params.argtypes = [ctypes.c_int, ctypes.c_int]
+    L.cdk_user_emission_params.restype = ctypes.c_int
     if path is None:
         _lib = L
     else:

@@ -17,6 +17,7 @@ import torch
 
 from .continuous_discrete_linear_gaussian_ssm.inference import cdlgssm_marginal_log_prob_and_grad
 
+from .continuous_discrete_nonlinear_gaussian_ssm._common import reject_user_emission
 from .continuous_discrete_nonlinear_gaussian_ssm.inference_ekf import (EKFHyperParams, drift_leaves,
                                                                        ekf_dense_marginal_log_prob_and_grad,
                                                                        ekf_marginal_log_prob_and_grad)
@@ -66,6 +67,7 @@ class _NonlinearLogLik(torch.autograd.Function):
 
 
 def _nonlinear_log_prob(grad_fn, params, emissions, t_emissions, hyperparams):
+    reject_user_emission(params, grad_fn.__name__)
     leaves = _leaves(params)
     names = tuple(leaves)
     tensors = [leaves[n] if isinstance(leaves[n], torch.Tensor) else torch.as_tensor(leaves[n]) for n in names]
@@ -76,6 +78,7 @@ def ekf_marginal_log_prob(params, emissions, t_emissions=None, hyperparams: EKFH
     """Per-trajectory marginal log-likelihood of the CD-EKF as a differentiable torch tensor.  Every leaf of `params`
     that is a torch tensor with requires_grad receives its gradient on `.backward()`: the drift's fields (named as in its
     registry class) and the diffusion, emission and initial parameters."""
+    reject_user_emission(params, "ekf_marginal_log_prob")
     H = params.emissions.emission_function.weights
     scalar_l63 = type(params.dynamics.drift).__name__ == "LearnableLorenz63" and tuple(np.shape(H))[-2] == 1
     fn = ekf_marginal_log_prob_and_grad if scalar_l63 else ekf_dense_marginal_log_prob_and_grad

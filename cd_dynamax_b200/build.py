@@ -72,6 +72,19 @@ USER_GRAD_SOURCES = USER_SOURCES + ["cdk_ekfgrad.cu"]  # ... plus the dense EKF 
 USER_KEEP = 8  # variants kept in lib/user, newest first
 
 
+def variant_key(drift_code=None, emission_code=None, grad=False) -> str:
+    """Content hash naming the variant of build_variant(drift_code, emission_code, grad): the device codes (each marked
+    present or absent), `grad`, the library sources and this file."""
+    import hashlib
+    key = hashlib.sha1()
+    for part in (drift_code, emission_code):
+        key.update(b"-" if part is None else b"%d:" % len(part.encode()) + part.encode())
+    key.update(b"grad" if grad else b"filter")
+    for f in sorted(os.listdir(CSRC)) + ["../../include/cdk.h", "../build.py"]:
+        key.update(open(os.path.join(CSRC, f), "rb").read())
+    return key.hexdigest()[:16]
+
+
 def build_user_drift(device_code: str, grad: bool = False, verbose=False) -> str:
     """Compile a VARIANT of libcdk.so whose drift registry contains CDK_DRIFT_USER = the given CUDA device code
     (SURVEY 8f rank 4: the reference accepts any Python drift callable, cdnlgssm_utils.py:13-36; a CUDA kernel needs device
@@ -91,18 +104,32 @@ def build_user_drift(device_code: str, grad: bool = False, verbose=False) -> str
     wrong mode for thousands.  grad=False builds exactly the filter units, and code that compiles for float / double only
     keeps working there.
 
-    Returns the path of cd_dynamax_b200/lib/user/libcdk_user_<hash>.so (cached by content hash, `grad` included; ~1 minute
-    of nvcc the first time; the USER_KEEP newest variants are kept).  The variant exports the same C ABI (include/cdk.h);
-    the units that do not see the registry (cdk_small.cu, cdk_kfwarp.cu, and cdk_ekfgrad.cu unless grad) are linked from
-    the stock build."""
-    import hashlib
+    The same as build_variant(device_code, None, grad): see there for the cache and the returned path."""
+    return build_variant(device_code, None, grad, verbose)
+
+
+def build_variant(drift_code=None, emission_code=None, grad: bool = False, verbose=False) -> str:
+    """Compile a VARIANT of libcdk.so with a user-defined drift (CDK_DRIFT_USER, `drift_code`: see build_user_drift), a
+    user-defined emission (CDK_EMISSION_USER, `emission_code`), or both.  `emission_code` must define, inside
+    `namespace cdk_user_emission { ... }`, for T = float and double:
+
+        __host__ __device__ int num_params(int n, int m);                                        // n_phi, length of phi
+        template <typename T, class XF> __device__ T h(const T* phi, int n, int m, int a, XF x);   // h_a(x; phi); x(j) = x_j
+        template <typename T> __device__ T jac(const T* phi, int n, int m, int a, int j, const T* x); // d h_a / d x_j
+
+    Nothing differentiates the emission: the gradient entry points reject it.  grad=True (the drift's dense EKF gradient)
+    needs a drift.
+
+    Returns the path of cd_dynamax_b200/lib/user/libcdk_user_<hash>.so, cached by content hash (variant_key: both codes
+    and `grad`; ~1 minute of nvcc the first time; the USER_KEEP newest variants are kept).  The variant exports the same C
+    ABI (include/cdk.h); the units that do not see the registries (cdk_small.cu, cdk_kfwarp.cu, and cdk_ekfgrad.cu unless
+    grad) are linked from the stock build."""
+    if drift_code is None and emission_code is None:
+        raise ValueError("build_variant needs a drift code, an emission code or both")
+    if grad and drift_code is None:
+        raise ValueError("grad=True compiles the gradient of a user drift: it needs drift_code")
     build()  # the stock objects
-    key = hashlib.sha1()
-    key.update(device_code.encode())
-    key.update(b"grad" if grad else b"filter")
-    for f in sorted(os.listdir(CSRC)) + ["../../include/cdk.h", "../build.py"]:
-        key.update(open(os.path.join(CSRC, f), "rb").read())
-    tag = key.hexdigest()[:16]
+    tag = variant_key(drift_code, emission_code, grad)
     udir = os.path.join(LIBDIR, "user")
     os.makedirs(udir, exist_ok=True)
     lib = os.path.join(udir, f"libcdk_user_{tag}.so")
@@ -110,15 +137,20 @@ def build_user_drift(device_code: str, grad: bool = False, verbose=False) -> str
         return lib
     work = os.path.join(OBJ, f"user_{tag}")
     os.makedirs(work, exist_ok=True)
-    header = os.path.join(work, "cdk_user_drift.cuh")
-    with open(header, "w") as fh:
-        fh.write("// generated by cd_dynamax_b200.build.build_user_drift\n#pragma once\n" + device_code + "\n")
-    flag = f'-DCDK_USER_DRIFT_HEADER="{header}"'
+    flags = []
+    for code, name, macro in ((drift_code, "cdk_user_drift.cuh", "CDK_USER_DRIFT_HEADER"),
+                              (emission_code, "cdk_user_emission.cuh", "CDK_USER_EMISSION_HEADER")):
+        if code is None:
+            continue
+        header = os.path.join(work, name)
+        with open(header, "w") as fh:
+            fh.write("// generated by cd_dynamax_b200.build.build_variant\n#pragma once\n" + code + "\n")
+        flags.append(f'-D{macro}="{header}"')
     units = USER_GRAD_SOURCES if grad else USER_SOURCES
     jobs = []
     for s in units:
         src, obj = os.path.join(CSRC, s), os.path.join(work, s.replace(".cu", ".o"))
-        jobs.append((s, [_nvcc()] + NVCC_FLAGS + [flag, "-c", src, "-o", obj]))
+        jobs.append((s, [_nvcc()] + NVCC_FLAGS + flags + ["-c", src, "-o", obj]))
     with concurrent.futures.ThreadPoolExecutor(max_workers=len(jobs)) as ex:
         futs = {ex.submit(subprocess.run, cmd, capture_output=True, text=True): name for name, cmd in jobs}
         for f in concurrent.futures.as_completed(futs):
@@ -126,14 +158,14 @@ def build_user_drift(device_code: str, grad: bool = False, verbose=False) -> str
             if verbose or r.returncode != 0:
                 sys.stderr.write(f"--- {futs[f]} ---\n{r.stdout}{r.stderr}\n")
             if r.returncode != 0:
-                raise RuntimeError(f"nvcc failed on {futs[f]} (user drift):\n{r.stderr[-4000:]}")
+                raise RuntimeError(f"nvcc failed on {futs[f]} (user device code):\n{r.stderr[-4000:]}")
     objs = [os.path.join(work, s.replace(".cu", ".o")) for s in units]
     objs += [os.path.join(OBJ, s.replace(".cu", ".o")) for s in SOURCES if s not in units]
     tmp = lib + ".tmp"
     r = subprocess.run([_nvcc(), "-shared", "-o", tmp] + objs + ["-gencode", "arch=compute_100a,code=sm_100a", "-lcudart", "-ldl",
                                                                 "-Xlinker", "-Bsymbolic"], capture_output=True, text=True)
     if r.returncode != 0:
-        raise RuntimeError("link failed (user drift):\n" + r.stdout + r.stderr)
+        raise RuntimeError("link failed (user device code):\n" + r.stdout + r.stderr)
     os.replace(tmp, lib)
     # housekeeping: every change of the sources or of the device code is a new content hash; keep the newest variants
     old = sorted((f for f in os.listdir(udir) if f.startswith("libcdk_user_") and f.endswith(".so")),

@@ -1,6 +1,6 @@
 # mirrors src/continuous_discrete_nonlinear_gaussian_ssm/__init__.py:1-7
 from .cdnlgssm_utils import (GSSMForecast, LearnableLinear, LearnableLorenz63, LearnableLorenz96, LearnableMatrix,
-                             LearnableQuadratic, LearnableUserDrift, LearnableVector, ParamsCDNLGSSM, ParamsCDNLGSSMDynamics,
+                             LearnableQuadratic, LearnableUserDrift, LearnableUserEmission, LearnableVector, ParamsCDNLGSSM, ParamsCDNLGSSMDynamics,
                              ParamsCDNLGSSMEmissions)
 from .inference_ekf import (EKFHyperParams, ekf_marginal_log_prob_and_grad,
                             ekf_dense_marginal_log_prob_and_grad, extended_kalman_filter,

@@ -21,22 +21,53 @@ def _val(x):
     return x.params if hasattr(x, "params") and hasattr(x, "f") else x
 
 
+def is_user_emission(params):
+    return type(params.emissions.emission_function).__name__ == "LearnableUserEmission"
+
+
+def reject_user_emission(params, what):
+    """`what` has no user-emission path: raise before any build or device work."""
+    if is_user_emission(params):
+        raise NotImplementedError(f"{what} is not available for a LearnableUserEmission (a user-defined emission has no "
+                                  "gradient and no emission-moment helper); it runs through the filters, the EKS and the "
+                                  "path sampler only")
+
+
+def emission_dim(params):
+    """m from the emission covariance ([m, m] or [N, m, m]): the emission function need not have weights."""
+    return _shape(_val(params.emissions.emission_cov))[-1]
+
+
 def nonlinear_inputs(params, Y, T, n, m):
     em = params.emissions.emission_function
-    if type(em).__name__ != "LearnableLinear":
-        raise NotImplementedError("emission_function must be LearnableLinear (h(x) = H x + d): arbitrary Python "
-                                  "emission callables cannot run inside a CUDA kernel")
+    user_em = is_user_emission(params)
+    if not user_em and type(em).__name__ != "LearnableLinear":
+        raise NotImplementedError("emission_function must be LearnableLinear (h(x) = H x + d) or a LearnableUserEmission "
+                                  "(CUDA device code): arbitrary Python emission callables cannot run inside a CUDA kernel")
     drift_id, theta, n_theta = drift_to_theta(params.dynamics.drift, n)
     ins = {
         L.IN_Y: Y, L.IN_T: T, L.IN_M0: _val(params.initial.mean), L.IN_P0: _val(params.initial.cov), L.IN_F: theta,
         L.IN_L: _val(params.dynamics.diffusion_coefficient), L.IN_QC: _val(params.dynamics.diffusion_cov),
-        L.IN_H: em.weights, L.IN_D: em.bias, L.IN_R: _val(params.emissions.emission_cov),
+        L.IN_H: em.phi if user_em else em.weights, L.IN_D: None if user_em else em.bias,
+        L.IN_R: _val(params.emissions.emission_cov),
     }
-    fields = dict(drift_id=drift_id, n_theta=n_theta, emission_id=0)
-    if drift_id == L.DRIFT_USER:
+    fields = dict(drift_id=drift_id, n_theta=n_theta, emission_id=L.EMISSION_USER if user_em else L.EMISSION_LINEAR)
+    drift = params.dynamics.drift
+    if drift_id == L.DRIFT_USER or user_em:
         from .. import build as _build
-        drift = params.dynamics.drift
-        fields["lib_path"] = _build.build_user_drift(drift.device_code, grad=bool(drift.differentiable))
+        user_drift = drift_id == L.DRIFT_USER
+        if user_em:
+            fields["lib_path"] = _build.build_variant(drift.device_code if user_drift else None, em.device_code,
+                                                      grad=user_drift and bool(drift.differentiable))
+        else:
+            fields["lib_path"] = _build.build_user_drift(drift.device_code, grad=bool(drift.differentiable))
+    if user_em:
+        n_phi = int(L.lib(fields["lib_path"]).cdk_user_emission_params(n, m))
+        shp = tuple(_shape(em.phi))
+        if len(shp) not in (1, 2) or shp[-1] != n_phi:
+            raise ValueError(f"LearnableUserEmission.phi: shape {shp}, but the emission's num_params(n={n}, m={m}) = "
+                             f"{n_phi}: expected [{n_phi}] or [N, {n_phi}]")
+        fields["n_phi"] = n_phi
     return ins, fields
 
 

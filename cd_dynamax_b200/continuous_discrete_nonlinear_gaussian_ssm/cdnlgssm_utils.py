@@ -3,7 +3,8 @@
 
 A CUDA kernel cannot take an arbitrary Python callable, so the drift must be one of the registry classes below
 (`LearnableLinear`, `LearnableLorenz63` as upstream; `LearnableLorenz96` and `LearnableQuadratic` are additions) and
-the emission function must be `LearnableLinear`.  Each class still carries `.f(x, u, t)` with the upstream signature
+the emission function must be `LearnableLinear`; `LearnableUserDrift` and `LearnableUserEmission` take CUDA device code
+instead.  Each class still carries `.f(x, u, t)` with the upstream signature
 (NumPy) so that host code written against the reference keeps working.
 """
 from typing import Any, NamedTuple, Optional
@@ -94,6 +95,23 @@ class LearnableUserDrift(NamedTuple):
         if self.py_f is None:
             raise NotImplementedError("no host-side callable was given for this user drift")
         return self.py_f(_np(x), _np(self.theta))
+
+
+class LearnableUserEmission(NamedTuple):
+    """A user-defined emission function (upstream: any `LearnableFunction.f` as emission, cdnlgssm_utils.py:13-36), given
+    as CUDA C++ source (see cd_dynamax_b200.build.build_variant for the three functions it must define in
+    `namespace cdk_user_emission`) plus its parameter vector `phi` ([n_phi] or [N, n_phi], torch or NumPy); the first use
+    compiles a variant of libcdk.so with that code -- and the drift's, when the drift is a LearnableUserDrift -- in the
+    registries (cached by content hash).  The EKF, EKS, UKF, EnKF and the path sampler run it; gradients and the emission
+    moments of cdnlgssm_emissions do not.  `py_h` is an optional NumPy callable h(x, phi) for host-side use (`.f`)."""
+    device_code: str
+    phi: Any
+    py_h: Any = None
+
+    def f(self, x, u=None, t=None):
+        if self.py_h is None:
+            raise NotImplementedError("no host-side callable was given for this user emission")
+        return self.py_h(_np(x), _np(self.phi))
 
 
 class ParamsCDNLGSSMDynamics(NamedTuple):

@@ -20,7 +20,7 @@ import numpy as np
 from .. import _engine as E
 from .. import _lib as L
 from ..continuous_discrete_linear_gaussian_ssm.inference import _shape, _sq
-from ._common import _val, nonlinear_inputs
+from ._common import _val, emission_dim, is_user_emission, nonlinear_inputs, reject_user_emission
 from .inference_ekf import EKFHyperParams, _ekf_fields
 from .inference_enkf import EnKFHyperParams, key_to_seed
 from .inference_ukf import UKFHyperParams
@@ -76,7 +76,10 @@ def cdnlgssm_forecast(params, init_forecast, t_init, t_forecast=None, hyperparam
     kind = E.kind_of(m0)
     T = _times_with_init(t_init, t_forecast, m0)
     n = _shape(_val(params.dynamics.diffusion_cov))[-1]
-    m = _shape(params.emissions.emission_function.weights)[-2]
+    m = emission_dim(params)
+    if is_user_emission(params) and output_fields is not None and \
+            {"forecasted_emission_means", "forecasted_emission_covariances"} & set(output_fields):
+        reject_user_emission(params, "the forecasted emission moments")
     batched = len(_shape(m0)) == 2 or _shape(T)[0] > 1
     N = max(_shape(m0)[0] if len(_shape(m0)) == 2 else 1, _shape(T)[0])
     K = _shape(T)[1] - 1
@@ -113,7 +116,7 @@ def cdnlgssm_forecast(params, init_forecast, t_init, t_forecast=None, hyperparam
 def _sample(params, m0, P0, T, N, K, fixed, key, diffeqsolve_settings, kind, dt, batched, want_states=True,
             want_emissions=True, rng_offset=0):
     n = _shape(_val(params.dynamics.diffusion_cov))[-1]
-    m = _shape(params.emissions.emission_function.weights)[-2]
+    m = emission_dim(params)
     ins, drift_fields = nonlinear_inputs(params, None, T, n, m)
     ins = {k: v for k, v in ins.items() if v is not None}
     ins[L.IN_M0] = m0
@@ -171,6 +174,7 @@ def cdnlgssm_emissions(params, t_states, state_means, state_covs=None, inputs=No
     if isinstance(hyperparams, EnKFHyperParams):
         raise NotImplementedError("emissions_ensemble_kalman_filter re-samples an ensemble from (m, P) with a jax.random "
                                   "key; use EKFHyperParams / UKFHyperParams for the exact Gaussian emission moments")
+    reject_user_emission(params, "cdnlgssm_emissions")
     if t_states is None:
         raise ValueError("t_states must be provided for forecasting")
     em = params.emissions.emission_function

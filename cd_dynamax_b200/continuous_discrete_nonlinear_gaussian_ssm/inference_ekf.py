@@ -9,7 +9,7 @@ from .. import _engine as E
 from .. import _lib as L
 from ..continuous_discrete_linear_gaussian_ssm.inference import _sq
 from ..types import PosteriorGSSMFiltered, PosteriorGSSMSmoothed
-from ._common import DEFAULT_FIELDS, run_filter
+from ._common import DEFAULT_FIELDS, reject_user_emission, run_filter
 
 
 class EKFHyperParams(NamedTuple):
@@ -101,7 +101,9 @@ def ekf_marginal_log_prob_and_grad(params, emissions, t_emissions=None, hyperpar
     + one backward launch for all 23 columns, ~4 filter passes), forward mode otherwise (one launch per column), so that
     a `jax.custom_vjp` around the filter can be fed (INTEGRATION.md).  Symmetric matrices (diffusion_cov, initial_cov) are differentiated
     along symmetric directions: the result is the symmetric part (G + G^T)/2 of the entry-wise gradient G, which is what
-    any PSD parameterisation consumes; diffusion_coefficient's gradient is exact.  Both paths: num_iter = 1, fp64."""
+    any PSD parameterisation consumes; diffusion_coefficient's gradient is exact.  Both paths: num_iter = 1, fp64.
+    A LearnableUserEmission raises NotImplementedError: a user-defined emission has no gradient."""
+    reject_user_emission(params, "ekf_marginal_log_prob_and_grad")
     import torch
     from ._common import nonlinear_inputs, _val
     from ..continuous_discrete_linear_gaussian_ssm.inference import _shape, prepare_data
@@ -224,7 +226,8 @@ def ekf_dense_marginal_log_prob_and_grad(params, emissions, t_emissions=None,
     A LearnableUserDrift with differentiable=True gets its gradient under "theta": the variant library built with
     build_user_drift(code, grad=True) takes the drift's derivatives from dual-number evaluations of its own device code.
     A LearnableUserDrift with differentiable=False, the zeroth order and fp32 raise NotImplementedError, mis-shaped
-    parameters ValueError (before any device work)."""
+    parameters ValueError (before any device work).  A LearnableUserEmission raises NotImplementedError."""
+    reject_user_emission(params, "ekf_dense_marginal_log_prob_and_grad")
     drift = params.dynamics.drift
     if type(drift).__name__ == "LearnableUserDrift" and not drift.differentiable:
         raise NotImplementedError("the gradient of a user-defined drift needs LearnableUserDrift(..., differentiable=True), "

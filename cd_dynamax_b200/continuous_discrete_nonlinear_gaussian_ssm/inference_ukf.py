@@ -14,7 +14,7 @@ import os
 from typing import List, NamedTuple, Optional
 
 from ..types import PosteriorGSSMFiltered
-from ._common import DEFAULT_FIELDS, run_filter
+from ._common import DEFAULT_FIELDS, reject_user_emission, run_filter
 
 
 class UKFHyperParams(NamedTuple):
@@ -53,10 +53,12 @@ def ukf_marginal_log_prob_and_grad(params, emissions, t_emissions=None, hyperpar
     whose scratch does not fit half of the free device memory runs in several launches, with the same result bit for
     bit.  alpha, beta and kappa reach the filter as `unscented_kalman_filter` passes them; they do not enter the closed
     form and get no gradient.  fp64 only.  LearnableUserDrift, fp32, non-zero inputs and CDK_UKF_SIGMA_POINTS=1 (literal
-    sigma points) raise NotImplementedError, mis-shaped parameters ValueError (before any device work)."""
+    sigma points) raise NotImplementedError, mis-shaped parameters ValueError (before any device work).  So does a
+    LearnableUserEmission: a user-defined emission has no gradient."""
     import torch
     from .. import _engine as E
     from .inference_ekf import _parse_wrt, dense_marginal_log_prob_and_grad
+    reject_user_emission(params, "ukf_marginal_log_prob_and_grad")
     if type(params.dynamics.drift).__name__ == "LearnableUserDrift":
         raise NotImplementedError("a user-defined drift runs literal sigma points: use "
                                   "ukf_sigma_points_marginal_log_prob_and_grad")
@@ -86,10 +88,11 @@ def ukf_sigma_points_marginal_log_prob_and_grad(params, emissions, t_emissions=N
     and its x-derivatives from its jac).  -> (marginal_loglik, grads) keyed as in `ekf_dense_marginal_log_prob_and_grad`;
     `wrt` = any of its groups, or "all".  alpha, beta and kappa get no gradient.  fp64 only.  fp32, non-zero inputs and
     a LearnableUserDrift with differentiable=False raise NotImplementedError, mis-shaped parameters ValueError (before any
-    device work)."""
+    device work); so does a LearnableUserEmission."""
     import torch
     from .. import _engine as E
     from .inference_ekf import _parse_wrt, dense_marginal_log_prob_and_grad
+    reject_user_emission(params, "ukf_sigma_points_marginal_log_prob_and_grad")
     drift = params.dynamics.drift
     if type(drift).__name__ == "LearnableUserDrift" and not drift.differentiable:
         raise NotImplementedError("the gradient of a user-defined drift needs LearnableUserDrift(..., differentiable=True), "

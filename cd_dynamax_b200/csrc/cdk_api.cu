@@ -44,7 +44,9 @@ static long long slot_elems(const cdk_desc& d, int slot, int algo) {
     case CDK_IN_BU: return n * du;
     case CDK_IN_L: return n * n;
     case CDK_IN_QC: return n * n;
-    case CDK_IN_H: return m * n;
+    case CDK_IN_H:  // phi of a user emission (the linear model has no emission registry)
+      return (algo != ALGO_KF_FILTER && algo != ALGO_KF_SMOOTH && d.emission_id == CDK_EMISSION_USER)
+                 ? cdk::user_emission_params(d.n, d.m) : m * n;
     case CDK_IN_D: return m;
     case CDK_IN_DU: return m * du;
     case CDK_IN_R: return ((algo == ALGO_KF_FILTER || algo == ALGO_KF_SMOOTH) && (d.reserved[2] & CDK_FLAG_DIAG_R)) ? m : m * m;
@@ -76,11 +78,14 @@ static int validate(const cdk_desc* d, const void* const* in, void* const* out, 
   if (d->max_steps < 1) return fail(CDK_E_SIZE, "max_steps must be >= 1");
   const bool linear = algo == ALGO_KF_FILTER || algo == ALGO_KF_SMOOTH;
   const bool smooth = algo == ALGO_KF_SMOOTH || algo == ALGO_EKF_SMOOTH;
+  const bool user_emission = !linear && d->emission_id == CDK_EMISSION_USER;  // in[CDK_IN_D] is not read
   if (!linear && algo != ALGO_EMISSIONS) {
     if (d->drift_id < CDK_DRIFT_LINEAR || d->drift_id > CDK_DRIFT_USER) return fail(CDK_E_ENUM, "unknown drift_id");
     if (d->drift_id == CDK_DRIFT_USER && !cdk::has_user_drift())
       return fail(CDK_E_UNSUPPORTED, "CDK_DRIFT_USER needs a variant library built with the user's device code (build_user_drift)");
-    if (d->emission_id != CDK_EMISSION_LINEAR) return fail(CDK_E_ENUM, "unknown emission_id");
+    if (d->emission_id != CDK_EMISSION_LINEAR && d->emission_id != CDK_EMISSION_USER) return fail(CDK_E_ENUM, "unknown emission_id");
+    if (d->emission_id == CDK_EMISSION_USER && !cdk::has_user_emission())
+      return fail(CDK_E_UNSUPPORTED, "CDK_EMISSION_USER needs a variant library built with the user's emission code (build_variant)");
     if (d->n_theta != expected_theta(*d)) return fail(CDK_E_SIZE, "n_theta does not match drift_id / n");
     if (d->drift_id == CDK_DRIFT_LORENZ63 && d->n != 3) return fail(CDK_E_SIZE, "lorenz63 needs n == 3");
     if (d->drift_id == CDK_DRIFT_LORENZ96 && d->n < 4) return fail(CDK_E_SIZE, "lorenz96 needs n >= 4");
@@ -97,6 +102,8 @@ static int validate(const cdk_desc* d, const void* const* in, void* const* out, 
     if (d->solver != CDK_EULER && d->solver != CDK_HEUN) return fail(CDK_E_UNSUPPORTED, "EnKF supports solver euler (Euler-Maruyama) or heun");
   }
   if (algo == ALGO_EMISSIONS) {
+    if (d->emission_id == CDK_EMISSION_USER)
+      return fail(CDK_E_UNSUPPORTED, "cdk_emission_moments: the emission moments of a user-defined emission are not implemented");
     if (d->N > 0 && (!in[CDK_IN_FM] || !in[CDK_IN_H] || !in[CDK_IN_D] || !in[CDK_IN_R]))
       return fail(CDK_E_NULL, "emission moments need the state means, H, d and R");
     return CDK_OK;
@@ -106,7 +113,7 @@ static int validate(const cdk_desc* d, const void* const* in, void* const* out, 
     static const int req_s[] = {CDK_IN_T, CDK_IN_M0, CDK_IN_F, CDK_IN_L, CDK_IN_QC, CDK_IN_H, CDK_IN_D, CDK_IN_R};
     if (d->N > 0) {
       for (int s : req_s)
-        if (!in[s]) return fail(CDK_E_NULL, "a required input of the sampler is NULL");
+        if (!in[s] && !(user_emission && s == CDK_IN_D)) return fail(CDK_E_NULL, "a required input of the sampler is NULL");
       if (!(d->reserved[2] & CDK_FLAG_FIXED_INIT) && !in[CDK_IN_P0]) return fail(CDK_E_NULL, "sampling x_0 needs P0");
     }
     return CDK_OK;
@@ -124,7 +131,8 @@ static int validate(const cdk_desc* d, const void* const* in, void* const* out, 
       if (d->d_u > 0 && (!in[CDK_IN_U] || !in[CDK_IN_BU] || !in[CDK_IN_DU])) return fail(CDK_E_NULL, "d_u > 0 needs U, BU and DU");
     } else {
       for (int s : req_nl)
-        if (!in[s] && !(ponly && s == CDK_IN_Y)) return fail(CDK_E_NULL, "a required input of the nonlinear model is NULL");
+        if (!in[s] && !(ponly && s == CDK_IN_Y) && !(user_emission && s == CDK_IN_D))
+          return fail(CDK_E_NULL, "a required input of the nonlinear model is NULL");
     }
     if (smooth && (!in[CDK_IN_FM] || !in[CDK_IN_FP])) return fail(CDK_E_NULL, "smoothing needs the filtered moments");
     if (smooth && (!out[CDK_OUT_SM] || !out[CDK_OUT_SP])) return fail(CDK_E_NULL, "smoothing needs SM and SP outputs");
@@ -165,6 +173,9 @@ static int run(int algo, const cdk_desc* d, const void* const* in, void* const* 
   }
   if (algo == ALGO_ENKF_FILTER) {
     rc = launch_enkf<T>(a, s);
+    if (rc == CDK_E_SIZE && d->emission_id == CDK_EMISSION_USER)
+      return fail(rc, "enkf: the ensemble, the members' user-emission outputs and the model do not fit the shared memory of "
+                      "an 8-CTA cluster (8 x 227 KB; roughly (n + m) * E * sizeof(T) / 8 + 12 n^2 sizeof(T) per CTA)");
     return rc == CDK_E_SIZE ? fail(rc, "enkf: the ensemble and its model do not fit the shared memory of an 8-CTA cluster "
                                        "(8 x 227 KB; roughly n * E * sizeof(T) / 8 + 12 n^2 sizeof(T) per CTA)")
                             : rc;
@@ -340,7 +351,13 @@ CDK_DEF(cdk_sample_path_f32, float, ALGO_SAMPLE)
 CDK_DEF(cdk_emission_moments_f64, double, ALGO_EMISSIONS)
 CDK_DEF(cdk_emission_moments_f32, float, ALGO_EMISSIONS)
 
+// Every gradient entry point reads in[CDK_IN_H] as the m x n matrix of a linear emission: a user emission is refused
+// before any other check or launch.
+static bool user_emission_grad(const cdk_desc* d) { return d && d->emission_id == CDK_EMISSION_USER; }
+static const char* const kUserEmissionGrad = "a user-defined emission (CDK_EMISSION_USER) has no gradient";
+
 int cdk_ekf_grad_f64(const cdk_desc* d, const void* const* in, void* const* out, cdk_stream_t stream) {
+  if (user_emission_grad(d)) return fail(CDK_E_UNSUPPORTED, "cdk_ekf_grad_f64: a user-defined emission (CDK_EMISSION_USER) has no gradient");
   int rc = validate(d, in, out, ALGO_EKF_FILTER);
   if (rc != CDK_OK) return rc;
   if (d->N == 0) return CDK_OK;
@@ -423,6 +440,7 @@ int cdk_ekf_grad_dense_f64(const cdk_desc* d, const void* const* in, void* const
     snprintf(msg, sizeof(msg), "%s: %s", me, why);
     return fail(code, msg);
   };
+  if (user_emission_grad(d)) return reject(CDK_E_UNSUPPORTED, kUserEmissionGrad);
   if (d && (d->reserved[2] & CDK_FLAG_PREDICT_ONLY)) return reject(CDK_E_UNSUPPORTED, "CDK_FLAG_PREDICT_ONLY has no log-likelihood to differentiate");
   if (d && (d->reserved[2] & CDK_FLAG_DIAG_R)) return reject(CDK_E_UNSUPPORTED, "CDK_FLAG_DIAG_R is not supported");
   if (d && d->drift_id == CDK_DRIFT_USER && !cdk::ekf_grad_has_user_drift())
@@ -445,6 +463,7 @@ int cdk_ukf_grad_dense_f64(const cdk_desc* d, const void* const* in, void* const
     snprintf(msg, sizeof(msg), "%s: %s", me, why);
     return fail(code, msg);
   };
+  if (user_emission_grad(d)) return reject(CDK_E_UNSUPPORTED, kUserEmissionGrad);
   if (d && (d->reserved[2] & CDK_FLAG_PREDICT_ONLY)) return reject(CDK_E_UNSUPPORTED, "CDK_FLAG_PREDICT_ONLY has no log-likelihood to differentiate");
   if (d && (d->reserved[2] & CDK_FLAG_DIAG_R)) return reject(CDK_E_UNSUPPORTED, "CDK_FLAG_DIAG_R is not supported");
   if (d && (d->reserved[2] & CDK_FLAG_UKF_SIGMA_POINTS))
@@ -465,6 +484,7 @@ int cdk_ukf_grad_sigma_f64(const cdk_desc* d, const void* const* in, void* const
     snprintf(msg, sizeof(msg), "%s: %s", me, why);
     return fail(code, msg);
   };
+  if (user_emission_grad(d)) return reject(CDK_E_UNSUPPORTED, kUserEmissionGrad);
   if (d && (d->reserved[2] & CDK_FLAG_PREDICT_ONLY)) return reject(CDK_E_UNSUPPORTED, "CDK_FLAG_PREDICT_ONLY has no log-likelihood to differentiate");
   if (d && (d->reserved[2] & CDK_FLAG_DIAG_R)) return reject(CDK_E_UNSUPPORTED, "CDK_FLAG_DIAG_R is not supported");
   if (d && d->drift_id == CDK_DRIFT_USER && !cdk::ekf_grad_has_user_drift())
@@ -604,6 +624,8 @@ int cdk_dmma_probe_f64(int blocks, int iters, double* sink, cdk_stream_t stream)
 int cdk_debug_set_trace(void* devbuf) { return cdk::set_lw_trace(devbuf); }
 int64_t cdk_launch_count(void) { return (int64_t)g_launches.load(); }
 int cdk_has_user_drift(void) { return cdk::has_user_drift() ? 1 : 0; }
+int cdk_has_user_emission(void) { return cdk::has_user_emission() ? 1 : 0; }
+int cdk_user_emission_params(int n, int m) { return cdk::user_emission_params(n, m); }
 int cdk_version(void) { return CDK_VERSION; }
 const char* cdk_last_error(void) { return g_err; }
 

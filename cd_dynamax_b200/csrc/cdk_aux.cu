@@ -26,12 +26,13 @@ constexpr int SP_TPB = 128;
 struct SLay {
   int n, m, ldn, ldm;
   size_t TH, G, CR, CP, H, DV, W1, W2, total;  // element offsets
-  __host__ __device__ SLay(int n_, int m_, int nth) {
+  // nphi >= 0: a user emission (cdk.h CDK_EMISSION_USER) whose phi [nphi] takes the place of H (and d is not read)
+  __host__ __device__ SLay(int n_, int m_, int nth, int nphi = -1) {
     n = n_; m = m_; ldn = ldp(n); ldm = ldp(m);
     size_t o = 0;
     auto take = [&](size_t c) { size_t r = o; o += (c + 1) & ~size_t(1); return r; };
     TH = take(nth > 0 ? nth : 1); G = take((size_t)n * ldn); CR = take((size_t)m * ldm); CP = take((size_t)n * ldn);
-    H = take((size_t)m * ldn); DV = take(m); W1 = take((size_t)(n > m ? n : m) * ldp(n > m ? n : m));
+    H = take(nphi >= 0 ? (size_t)(nphi > 0 ? nphi : 1) : (size_t)m * ldn); DV = take(m); W1 = take((size_t)(n > m ? n : m) * ldp(n > m ? n : m));
     W2 = take((size_t)(n > m ? n : m) * ldp(n > m ? n : m));
     total = o;
   }
@@ -56,7 +57,8 @@ __global__ void __launch_bounds__(SP_TPB) sample_path_kernel(const KArgs<T> a) {
   T* sh = reinterpret_cast<T*>(sp_raw);
   const cdk_desc& d = a.d;
   const int n = NX > 0 ? NX : d.n, m = d.m, K = d.K;
-  const SLay L(n, m, d.n_theta);
+  const bool ue = user_emission(d);
+  const SLay L(n, m, d.n_theta, ue ? emission_params(d) : -1);
   const int ldn = L.ldn, ldm = L.ldm;
   T* th = sh + L.TH;
   T* G = sh + L.G;
@@ -75,8 +77,12 @@ __global__ void __launch_bounds__(SP_TPB) sample_path_kernel(const KArgs<T> a) {
       Lm[i * ldn + j] = a.in[CDK_IN_L][e];
       Qc[i * ldn + j] = a.in[CDK_IN_QC][e];
     }
-    FOR_T(e, m * n) H[(e / n) * ldn + (e % n)] = a.in[CDK_IN_H][e];
-    FOR_T(i, m) dv[i] = a.in[CDK_IN_D][i];
+    if (ue) {
+      FOR_T(i, emission_params(d)) H[i] = a.in[CDK_IN_H][i];  // phi
+    } else {
+      FOR_T(e, m * n) H[(e / n) * ldn + (e % n)] = a.in[CDK_IN_H][e];
+      FOR_T(i, m) dv[i] = a.in[CDK_IN_D][i];
+    }
     __syncthreads();
     chol<T>(Qc, chP, n, ldn, T(0));  // chol(Qc), parked in CP
     FOR_T(e, n * n) {                // G = L chol(Qc)  (models.py:583-588)
@@ -126,7 +132,7 @@ __global__ void __launch_bounds__(SP_TPB) sample_path_kernel(const KArgs<T> a) {
         if (j + u < dim) out[j + u] = (T)z4[u];
     }
   };
-  auto emit = [&](int row, int step) {  // y ~ N(H x + d, R) and the state itself -> row `row` of the outputs
+  auto emit = [&](int row, int step) {  // y ~ N(h(x), R), h(x) = H x + d or the user's, and the state -> row `row`
     if (XS)
       for (int i = 0; i < n; ++i) XS[(traj * (long long)K + row) * n + i] = x[i];
     if (YS) {
@@ -138,10 +144,15 @@ __global__ void __launch_bounds__(SP_TPB) sample_path_kernel(const KArgs<T> a) {
         r[p] = s;
       }
       for (int p = 0; p < m; ++p) {
-        T hx = dv[p];
+        T hx;
+        if (ue) {
+          hx = user_h<T>(H, n, m, p, [&](int j) { return x[j]; });
+        } else {
+          hx = dv[p];
 #pragma unroll(NX > 0 ? NX : 1)
-        for (int i = 0; i < NXA; ++i)
-          if (i < n) hx += H[p * ldn + i] * x[i];
+          for (int i = 0; i < NXA; ++i)
+            if (i < n) hx += H[p * ldn + i] * x[i];
+        }
         YS[(traj * (long long)K + row) * m + p] = hx + r[p];
       }
     }
@@ -290,7 +301,7 @@ int launch_sample_path(const KArgs<T>& a, cudaStream_t s) {
   const uint32_t model_mask = (1u << CDK_IN_F) | (1u << CDK_IN_L) | (1u << CDK_IN_QC) | (1u << CDK_IN_H) | (1u << CDK_IN_D) |
                               (1u << CDK_IN_R) | (1u << CDK_IN_P0);
   if (d.batched_mask & model_mask) return CDK_E_UNSUPPORTED;  // per-trajectory model parameters: not in the sampler
-  const SLay L(d.n, d.m, d.n_theta);
+  const SLay L(d.n, d.m, d.n_theta, user_emission(d) ? emission_params(d) : -1);
   const size_t smem = L.total * sizeof(T);
   const long long blocks = (d.N + SP_TPB - 1) / SP_TPB;
   if (blocks > 2147483647LL) return CDK_E_SIZE;

@@ -24,6 +24,48 @@ __host__ __device__ inline int ldp(int c) { return c | 1; }
 #define CDK_HAS_USER_DRIFT 0
 #endif
 
+// ---- user-defined emission (CDK_EMISSION_USER): only in a variant built with -DCDK_USER_EMISSION_HEADER="file" ----------
+// The header defines, in namespace cdk_user_emission:
+//   __host__ __device__ int num_params(int n, int m);                                       // length of phi
+//   template <typename T, class XF> __device__ T h(const T* phi, int n, int m, int a, XF x);   // h_a(x; phi); x(j) = x_j
+//   template <typename T> __device__ T jac(const T* phi, int n, int m, int a, int j, const T* x); // d h_a / d x_j
+// for T = float and double.  Nothing differentiates it (the gradient entry points reject the id).
+#ifdef CDK_USER_EMISSION_HEADER
+#include CDK_USER_EMISSION_HEADER
+#define CDK_HAS_USER_EMISSION 1
+#else
+#define CDK_HAS_USER_EMISSION 0
+#endif
+
+// True iff the request takes the user emission; a compile-time false in a library without one, so the callers' user-emission
+// branches vanish from those objects.
+__host__ __device__ static inline bool user_emission(const cdk_desc& d) {
+  return CDK_HAS_USER_EMISSION && d.emission_id == CDK_EMISSION_USER;
+}
+// n_phi of the user emission (0 when the request does not take it)
+__host__ __device__ static inline int emission_params(const cdk_desc& d) {
+#if CDK_HAS_USER_EMISSION
+  if (d.emission_id == CDK_EMISSION_USER) return cdk_user_emission::num_params(d.n, d.m);
+#endif
+  return 0;
+}
+template <typename T, class XF>
+__device__ __forceinline__ T user_h(const T* phi, int n, int m, int a, XF x) {
+#if CDK_HAS_USER_EMISSION
+  return cdk_user_emission::h<T>(phi, n, m, a, x);
+#else
+  return T(0);
+#endif
+}
+template <typename T>
+__device__ __forceinline__ T user_h_jac(const T* phi, int n, int m, int a, int j, const T* x) {
+#if CDK_HAS_USER_EMISSION
+  return cdk_user_emission::jac<T>(phi, n, m, a, j, x);
+#else
+  return T(0);
+#endif
+}
+
 // ---- drift registry, element-wise, on an arbitrary accessor x(j) ---------------------------------------------------
 template <typename T, class XF>
 __device__ __forceinline__ T drift_f(int id, const T* th, int n, int i, XF x) {

@@ -39,9 +39,12 @@ constexpr int ENKF_TPB = 256;
 struct ELay {
   int n, m, ldn, ldm, ldE, nth;
   // byte offsets
-  size_t X, PSUM, CPART, CXX, MEAN, H, R, CHR, DV, G, HP, S, SL, KT, SK, YV, RV, TH, MISC, DB, total;
+  size_t X, PSUM, CPART, CXX, MEAN, H, R, CHR, DV, G, HP, S, SL, KT, SK, YV, RV, TH, MISC, DB, PHI, YSUM, YPART, total;
   // dg: room for the [m x ldE] innovation block of the tensor-core gain application (EArgs::dg)
-  __host__ __device__ ELay(int n_, int m_, int nth_, int Eloc, size_t ts, int dg) {
+  // ue: a user emission (cdk.h CDK_EMISSION_USER) with nphi parameters: the [m x ldE] block then holds the members'
+  //     h(x_e); YSUM / YPART receive this CTA's partial sums of the emission moments (sum_e h(x_e); [m + n] x ldm partial
+  //     sums of dY dY^T and dX dY^T), and there is no H / d
+  __host__ __device__ ELay(int n_, int m_, int nth_, int Eloc, size_t ts, int dg, bool ue = false, int nphi = 0) {
     n = n_; m = m_; nth = nth_;
     ldn = ldp(n); ldm = ldp(m);
     ldE = ((Eloc + 31) / 32) * 32 + 4;  // = 4 (mod 32): DMMA fragment loads X[i0 + gid][e0 + tig] are conflict-free
@@ -52,7 +55,7 @@ struct ELay {
     CPART = take(8 * n * ldn);
     CXX = take(ts * n * ldn);
     MEAN = take(ts * n);
-    H = take(ts * m * ldn);
+    H = take(ue ? 0 : ts * m * ldn);
     R = take(ts * m * ldm);
     CHR = take(ts * m * ldm);
     DV = take(ts * m);
@@ -66,7 +69,10 @@ struct ELay {
     RV = take(ts * 2 * m);
     TH = take(ts * (nth > 0 ? nth : 1));
     MISC = take(64);
-    DB = take(dg ? ts * m * ldE : 0);
+    DB = take(dg || ue ? ts * m * ldE : 0);
+    PHI = take(ue ? ts * (nphi > 0 ? nphi : 1) : 0);
+    YSUM = take(ue ? 8 * m : 0);
+    YPART = take(ue ? 8 * (size_t)(m + n) * ldm : 0);
     total = o;
   }
 };
@@ -77,6 +83,7 @@ struct EArgs {
   int C;     // cluster size (CTAs per trajectory)
   int dg;    // 1: gain application X += K (Y~ - H X - d) as two tensor-core products over the CTA's members (needs ELay::DB)
   int Eloc;  // members per CTA (the last CTA may own fewer)
+  int ue;    // user emission (then dg = 0: the tensor-core gain application forms H X, which needs a linear h)
 };
 
 // ---- FP64 tensor-core partial covariance ----------------------------------------------------------------------------
@@ -174,6 +181,72 @@ __device__ void moments(cg::cluster_group& cluster, const ELay& L, unsigned char
   cluster.sync();  // nobody may overwrite psum / Cp (next moments call) or read a stale Cxx before everyone is done
 }
 
+// The emission moments of the stochastic update with a user emission (inference_enkf.py:92-148, which maps every member
+// through h): Y_e = h(x_e) per member (one thread each, into the DB block), then over the whole cluster
+//   ybar = mean_e Y_e,  C_yy = sum_e dY_e dY_e^T / (E - 1),  C_xy = sum_e dX_e dY_e^T / (E - 1)
+// with dX about the ensemble mean already in MEAN (the moments of this same ensemble).  Partial sums are combined in rank
+// order as in moments(), so every CTA holds bit-identical values.  Out (every CTA): HP = C_xy^T [m x n], S = C_yy + R,
+// rv = y - ybar.  (A linear h gives C_xy = C_xx H^T and C_yy = H C_xx H^T straight from the predicted moments; a nonlinear
+// one does not.)
+template <typename T>
+__device__ void user_emission_moments(cg::cluster_group& cluster, const ELay& L, unsigned char* sh, int nmem, int E, int C,
+                                      const T* phi, const T* yv) {
+  const int n = L.n, m = L.m, ldn = L.ldn, ldm = L.ldm, ldE = L.ldE;
+  const T* X = reinterpret_cast<const T*>(sh + L.X);
+  const T* mean = reinterpret_cast<const T*>(sh + L.MEAN);
+  const T* R = reinterpret_cast<const T*>(sh + L.R);
+  T* Yb = reinterpret_cast<T*>(sh + L.DB);
+  double* ysum = reinterpret_cast<double*>(sh + L.YSUM);
+  double* part = reinterpret_cast<double*>(sh + L.YPART);  // rows a < m: dY_a dY^T; rows m + j: dX_j dY^T
+  T* HP = reinterpret_cast<T*>(sh + L.HP);
+  T* Sm = reinterpret_cast<T*>(sh + L.S);
+  T* rv = reinterpret_cast<T*>(sh + L.RV);
+  T* ybar = rv + m;
+  for (int el = threadIdx.x; el < nmem; el += blockDim.x)
+    for (int a = 0; a < m; ++a) Yb[(size_t)a * ldE + el] = user_h<T>(phi, n, m, a, [&](int j) { return X[(size_t)j * ldE + el]; });
+  __syncthreads();
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarp = blockDim.x >> 5;
+  for (int a = warp; a < m; a += nwarp) {
+    double s = 0.0;
+    for (int e = lane; e < nmem; e += 32) s += (double)Yb[(size_t)a * ldE + e];
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+    if (lane == 0) ysum[a] = s;
+  }
+  cluster.sync();
+  FOR_T(a, m) {
+    double s = 0.0;
+    for (int r = 0; r < C; ++r) s += cluster.map_shared_rank(ysum, r)[a];
+    ybar[a] = (T)(s / (double)E);
+  }
+  __syncthreads();
+  FOR_T(e, (m + n) * m) {
+    const int r = e / m, b = e - r * m;
+    const T* u = r < m ? Yb + (size_t)r * ldE : X + (size_t)(r - m) * ldE;
+    const double uc = (double)(r < m ? ybar[r] : mean[r - m]);
+    const T* v = Yb + (size_t)b * ldE;
+    const double vc = (double)ybar[b];
+    double s = 0.0;
+    for (int el = 0; el < nmem; ++el) s += ((double)u[el] - uc) * ((double)v[el] - vc);
+    part[r * ldm + b] = s;
+  }
+  cluster.sync();
+  const double inv = 1.0 / (double)(E - 1);
+  FOR_T(e, (m + n) * m) {
+    const int r = e / m, b = e - r * m;
+    double s = 0.0;
+    for (int q = 0; q < C; ++q) s += cluster.map_shared_rank(part, q)[r * ldm + b];
+    const T v = (T)(s * inv);
+    if (r < m) {
+      Sm[r * ldm + b] = v + R[r * ldm + b];
+    } else {
+      HP[b * ldn + (r - m)] = v;
+    }
+  }
+  FOR_T(a, m) rv[a] = yv[a] - ybar[a];
+  cluster.sync();  // nobody may overwrite ysum / part (next update) before every CTA has read them
+}
+
 // Lorenz-96 drift entry and Euler-Maruyama update with the oracle's operation order and NO fused multiply-adds
 // (((x_{i+1} - x_{i-2}) x_{i-1} - x_i) + F;  (x + dt f) + noise): both member mappings and the NumPy oracle then agree bit for
 // bit given the same deviates (the compiler is otherwise free to contract differently in differently shaped code).
@@ -228,7 +301,8 @@ __global__ void __launch_bounds__(LIGHT ? 2 * ENKF_TPB : ENKF_TPB, 1) enkf_kerne
   const int n = NX > 0 ? NX : d.n, m = d.m, K = d.K, E = d.E, C = g.C;
   const int rank = (int)cluster.block_rank();
   const long long traj = blockIdx.x / C;
-  const ELay L(n, m, d.n_theta, g.Eloc, sizeof(T), g.dg);
+  const ELay L(n, m, d.n_theta, g.Eloc, sizeof(T), g.dg, g.ue, emission_params(d));
+  const bool ue = user_emission(d) && g.ue;
   const int ldn = L.ldn, ldm = L.ldm, ldE = L.ldE;
   const int e_base = rank * g.Eloc;
   const int nmem = max(0, min(g.Eloc, E - e_base));
@@ -249,6 +323,7 @@ __global__ void __launch_bounds__(LIGHT ? 2 * ENKF_TPB : ENKF_TPB, 1) enkf_kerne
   T* rv = reinterpret_cast<T*>(sh + L.RV);
   T* zv = rv + m;
   T* th = reinterpret_cast<T*>(sh + L.TH);
+  T* phi = reinterpret_cast<T*>(sh + L.PHI);
   int* misc = reinterpret_cast<int*>(sh + L.MISC);
   T* llsh = reinterpret_cast<T*>(sh + L.MISC + 16);
 
@@ -269,15 +344,19 @@ __global__ void __launch_bounds__(LIGHT ? 2 * ENKF_TPB : ENKF_TPB, 1) enkf_kerne
       Lm[i * ldn + j] = src(CDK_IN_L)[e];
       Qc[i * ldn + j] = src(CDK_IN_QC)[e];
     }
-    FOR_T(e, m * n) {
-      const int i = e / n, j = e - i * n;
-      H[i * ldn + j] = src(CDK_IN_H)[e];
+    if (ue) {
+      FOR_T(i, emission_params(d)) phi[i] = src(CDK_IN_H)[i];
+    } else {
+      FOR_T(e, m * n) {
+        const int i = e / n, j = e - i * n;
+        H[i * ldn + j] = src(CDK_IN_H)[e];
+      }
+      FOR_T(i, m) dv[i] = src(CDK_IN_D)[i];
     }
     FOR_T(e, m * m) {
       const int i = e / m, j = e - i * m;
       R[i * ldm + j] = src(CDK_IN_R)[e];
     }
-    FOR_T(i, m) dv[i] = src(CDK_IN_D)[i];
     __syncthreads();
     chol<T>(Qc, Lq, n, ldn, T(0));  // Lq = chol(Qc) in G
     FOR_T(e, n * n) {
@@ -373,6 +452,9 @@ __global__ void __launch_bounds__(LIGHT ? 2 * ENKF_TPB : ENKF_TPB, 1) enkf_kerne
     if (!ponly) {
     // ================= update (inference_enkf.py:92-148), every CTA of the cluster redundantly =================
     FOR_T(i, m) yv[i] = Y[(long long)k * m + i];
+    if (ue) {
+      user_emission_moments<T>(cluster, L, sh, nmem, E, C, phi, yv);  // HP = C_xy^T, S = C_yy + R, rv = y - ybar
+    } else {
     // HP = H Cxx (= C_xy^T because h is linear), S = H Cxx H^T + R: FP64 tensor cores
     mm_dmma<T, false, false>(H, ldn, Cxx, ldn, m, n, n, [&](int p, int j, double v) { HP[p * ldn + j] = (T)v; });
     __syncthreads();
@@ -381,6 +463,7 @@ __global__ void __launch_bounds__(LIGHT ? 2 * ENKF_TPB : ENKF_TPB, 1) enkf_kerne
       T s = dv[p];
       for (int q = 0; q < n; ++q) s += H[p * ldn + q] * mean[q];
       rv[p] = yv[p] - s;
+    }
     }
     __syncthreads();
     // MVN(ybar, S).log_prob(y) factors S un-boosted (:129); K^T = psd_solve(S, C_xy^T) factors sym(S) + 1e-9 I (:141-143):
@@ -465,11 +548,17 @@ __global__ void __launch_bounds__(LIGHT ? 2 * ENKF_TPB : ENKF_TPB, 1) enkf_kerne
       } else {
         for (int p = 0; p < m; ++p) r[p] = T(0);
       }
+      const T* Ye = reinterpret_cast<const T*>(sh + L.DB) + el;  // user emission: h(x_e), column el
       for (int p = 0; p < m; ++p) {
-        T hx = dv[p];
+        T hx;
+        if (ue) {
+          hx = Ye[(size_t)p * ldE];
+        } else {
+          hx = dv[p];
 #pragma unroll UF
-        for (int i = 0; i < NXA; ++i)
-          if (i < n) hx += H[p * ldn + i] * x[i];
+          for (int i = 0; i < NXA; ++i)
+            if (i < n) hx += H[p * ldn + i] * x[i];
+        }
         r[p] = (yv[p] + r[p]) - hx;
       }
       for (int p = 0; p < m; ++p) {
@@ -662,13 +751,14 @@ int launch_enkf(const KArgs<T>& a, cudaStream_t s) {
   g.k = a;
   g.C = 0;
   g.dg = 0;
+  g.ue = user_emission(d) ? 1 : 0;
   size_t smem = 0;
   for (int C = 1; C <= 8; C *= 2) {
     if (forced && C != forced) continue;
     const int Eloc = (((d.E + C - 1) / C) + 3) & ~3;
     if (!(forced || Eloc <= 2 * ENKF_TPB || C == 8)) continue;
-    for (int dg = dmma_gain_env; dg >= 0 && g.C == 0; --dg) {  // prefer the tensor-core gain application if its block fits
-      const ELay L(d.n, d.m, d.n_theta, Eloc, sizeof(T), dg);
+    for (int dg = g.ue ? 0 : dmma_gain_env; dg >= 0 && g.C == 0; --dg) {  // prefer the tensor-core gain application if its block fits
+      const ELay L(d.n, d.m, d.n_theta, Eloc, sizeof(T), dg, g.ue, emission_params(d));
       if (L.total <= (size_t)max_optin) {
         g.C = C;
         g.Eloc = Eloc;

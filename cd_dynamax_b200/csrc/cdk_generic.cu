@@ -31,7 +31,7 @@ __host__ __device__ inline bool ukf_closed(const cdk_desc& d) {
 // shared-memory layout, computed identically on host (size) and device (offsets); units = elements of T
 struct Lay {
   int n, m, du, ldn, ldm, nn, S, nth, mpoff;
-  int TH, LQL, H, R, DV, BV, BU, DU, YV, UV, MU, P, ODEY, YS, ACC, KS, J, W1, W2, W3, SM, SL, RV, MF, PF, C0, total;
+  int TH, LQL, H, R, DV, BV, BU, DU, YV, UV, MU, P, ODEY, YS, ACC, KS, J, W1, W2, W3, SM, SL, RV, MF, PF, C0, PHI, YP, total;
   Lay() = default;
   // reg_ode: the launcher has chosen the register-resident stencil ODE (ode_solve_stencil), so the shared-memory RHS and its
   // Jacobian buffer are never used by this launch
@@ -70,6 +70,8 @@ struct Lay {
     }
     SM = take(m * ldm); SL = take(m * ldm); RV = take(2 * m);
     MF = take(smooth ? n : 0); PF = take(smooth ? nn : 0); C0 = take(n);
+    // user emission: its parameters phi, and (UKF) the 2n + 1 sigma points pushed through h, [2n + 1] x ldm
+    PHI = take(emission_params(d)); YP = take(ukf && user_emission(d) ? (2 * n + 1) * ldm : 0);
     total = o;
   }
 };
@@ -617,13 +619,17 @@ __device__ void load_model(const Ctx<T>& c, long long traj, bool linear) {
   } else {
     FOR_T(i, a.d.n_theta) c.p(L.TH)[i] = src(CDK_IN_F)[i];
   }
-  load_mat<T>(c.p(L.H), src(CDK_IN_H), m, n, L.ldn);
+  if (!linear && user_emission(a.d)) {
+    FOR_T(i, emission_params(a.d)) c.p(L.PHI)[i] = src(CDK_IN_H)[i];  // phi; L.H then holds J = d h / dx at the mean
+  } else {
+    load_mat<T>(c.p(L.H), src(CDK_IN_H), m, n, L.ldn);
+    FOR_T(i, m) c.p(L.DV)[i] = src(CDK_IN_D)[i];
+  }
   if (a.d.reserved[2] & CDK_FLAG_DIAG_R) {
     FOR_T(i, m) c.p(L.R)[i] = src(CDK_IN_R)[i];  // 1-D emissions.cov: the diagonal (linear model only, validated)
   } else {
     load_mat<T>(c.p(L.R), src(CDK_IN_R), m, m, L.ldm);
   }
-  FOR_T(i, m) c.p(L.DV)[i] = src(CDK_IN_D)[i];
   // L Qc L^T via W1 = L, W2 = Qc, W3 = L Qc
   T* Lm = c.p(L.W1);
   T* Qc = c.p(L.W2);
@@ -792,6 +798,64 @@ __device__ T condition_on_diag_r(const Ctx<T>& c) {
   return ll_sh;
 }
 
+// The moments of the UKF update with a user emission, restating inference_ukf.py:162-203 literally (as tests/user_emission_oracle.py does):
+// sigma points X_p = m, m +- c L_i (L L^T = P, c^2 = n + lambda), Y_p = h(X_p), yhat = sum_p w_m[p] Y_p,
+// S = sum_p w_c[p] dY_p dY_p^T + R, C = sum_p w_c[p] dX_p dY_p^T -- the centre point's w_c[0], which carries
+// 1 - alpha^2 + beta, included.  One (point, component) evaluation of h per thread.  Out: Sm = S, Ct = C^T [m x n],
+// rv = y - yhat.  Scratch: J (the factor of P), YP (the points through h, then their deviations), rv + m (yhat).
+template <typename T>
+__device__ void ukf_user_moments(const Ctx<T>& c, T* Sm, T* Ct, T* rv) {
+  const Lay& L = c.L;
+  const cdk_desc& d = c.g.k.d;
+  const int n = L.n, m = L.m, ldn = L.ldn, ldm = L.ldm, np = 2 * n + 1;
+  const T* mu = c.p(L.MU);
+  const T* R = c.p(L.R);
+  const T* phi = c.p(L.PHI);
+  const T* yv = c.p(L.YV);
+  T* Lc = c.p(L.J);
+  T* Y = c.p(L.YP);
+  T* yhat = rv + m;
+  chol<T>(c.p(L.P), Lc, n, ldn, T(0));  // ends with a barrier
+  const double lam = d.alpha * d.alpha * (d.n + d.kappa) - d.n;  // ukf_weights (inference_ukf.py:42, :63-89)
+  const T w0m = T(lam / (d.n + lam)), wi = T(1.0 / (2.0 * (d.n + lam)));
+  const T w0c = T(lam / (d.n + lam) + (1.0 - d.alpha * d.alpha + d.beta));
+  const T cs = sqrt(T(d.n + lam));
+  auto xp = [&](int p, int j) -> T {  // component j of sigma point p
+    if (p == 0) return mu[j];
+    const T v = cs * Lc[j * ldn + (p <= n ? p - 1 : p - 1 - n)];
+    return p <= n ? mu[j] + v : mu[j] - v;
+  };
+  FOR_T(e, np * m) {
+    const int p = e / m, a = e - p * m;
+    Y[p * ldm + a] = user_h<T>(phi, n, m, a, [&](int j) { return xp(p, j); });
+  }
+  __syncthreads();
+  FOR_T(a, m) {
+    T s = T(0);
+    for (int p = 0; p < np; ++p) s += (p == 0 ? w0m : wi) * Y[p * ldm + a];
+    yhat[a] = s;
+    rv[a] = yv[a] - s;
+  }
+  __syncthreads();
+  FOR_T(e, np * m) {
+    const int p = e / m, a = e - p * m;
+    Y[p * ldm + a] -= yhat[a];
+  }
+  __syncthreads();
+  FOR_T(e, m * m) {
+    const int a = e / m, b = e - a * m;
+    T s = T(0);
+    for (int p = 0; p < np; ++p) s += (p == 0 ? w0c : wi) * Y[p * ldm + a] * Y[p * ldm + b];
+    Sm[a * ldm + b] = s + R[a * ldm + b];
+  }
+  FOR_T(e, m * n) {
+    const int a = e / n, j = e - a * n;
+    T s = T(0);  // dX_0 = 0
+    for (int p = 1; p < np; ++p) s += wi * (xp(p, j) - mu[j]) * Y[p * ldm + a];
+    Ct[a * ldn + j] = s;
+  }
+}
+
 // Measurement update shared by KF / EKF / UKF.  On entry MU, P hold the prediction; on exit the filtered moments.
 // Returns the log-likelihood increment (same value in every thread).
 template <typename T>
@@ -801,7 +865,8 @@ __device__ T condition_on(const Ctx<T>& c, int algo, int num_iter) {
   const int n = L.n, m = L.m, ldn = L.ldn, ldm = L.ldm;
   T* mu = c.p(L.MU);
   T* P = c.p(L.P);
-  const T* H = c.p(L.H);
+  T* H = c.p(L.H);  // user emission: J = d h / dx at the running mean, re-evaluated in every iteration
+  const T* phi = c.p(L.PHI);
   const T* R = c.p(L.R);
   const T* dv = c.p(L.DV);
   const T* yv = c.p(L.YV);
@@ -815,10 +880,24 @@ __device__ T condition_on(const Ctx<T>& c, int algo, int num_iter) {
   __shared__ T ll_sh;
   // ukf: literal sigma points through chol(P).  The closed-form UKF (linear emission: S = H P H^T + R and the cross term
   // P H^T exactly) takes the H P products of the KF / EKF branch, but -- like the reference's UKF -- never symmetrises.
-  const bool ukf = algo == ALGO_UKF_FILTER && !ukf_closed(d);
+  // A user emission (cdk.h, CDK_EMISSION_USER): the EKF linearises h at the running mean of every iteration (the iterated
+  // update of inference_ekf.py:153-199 with H = jacfwd(h), re-using the running covariance); the UKF takes the literal
+  // sigma-point update (ukf_user_moments) whether its predict runs in closed form or not.
+  const bool ue = algo != ALGO_KF_FILTER && user_emission(d);
+  const bool ukf_user = algo == ALGO_UKF_FILTER && ue;
+  const bool ukf = algo == ALGO_UKF_FILTER && !ukf_closed(d) && !ue;
   const bool no_sym = algo == ALGO_UKF_FILTER;
   for (int it = 0; it < num_iter; ++it) {
-    if (!ukf) {
+    if (ue && !ukf_user) {
+      FOR_T(e, m * n) {
+        const int a = e / n, j = e - a * n;
+        H[a * ldn + j] = user_h_jac<T>(phi, n, m, a, j, mu);
+      }
+      __syncthreads();
+    }
+    if (ukf_user) {
+      ukf_user_moments<T>(c, Sm, HP, rv);
+    } else if (!ukf) {
       mm_dmma<T, false, false>(H, ldn, P, ldn, m, n, n, [&](int a, int j, double v) { HP[a * ldn + j] = (T)v; });
       __syncthreads();
       mm_dmma<T, false, true>(HP, ldn, H, ldn, m, m, n, [&](int a, int b, double v) { Sm[a * ldm + b] = R[a * ldm + b] + (T)v; });
@@ -850,10 +929,17 @@ __device__ T condition_on(const Ctx<T>& c, int algo, int num_iter) {
         HP[a * ldn + j] = c2 * s;  // cross^T
       }
     }
-    FOR_T(a, m) {
-      T s = dv[a];
-      for (int q = 0; q < n; ++q) s += H[a * ldn + q] * mu[q];
-      rv[a] = yv[a] - s;  // yv already has D u subtracted (linear model)
+    if (!ukf_user) {
+      FOR_T(a, m) {
+        T s;
+        if (ue) {
+          s = user_h<T>(phi, n, m, a, [&](int j) { return mu[j]; });
+        } else {
+          s = dv[a];
+          for (int q = 0; q < n; ++q) s += H[a * ldn + q] * mu[q];
+        }
+        rv[a] = yv[a] - s;  // yv already has D u subtracted (linear model)
+      }
     }
     __syncthreads();
     // MVN(.).log_prob(y) factors S un-boosted (TFP); psd_solve(S, .) factors sym(S) + 1e-9 I: two independent m x m
@@ -1216,6 +1302,14 @@ int launch_generic(int algo, const KArgs<T>& a, cudaStream_t s) {
 }
 
 bool has_user_drift() { return CDK_HAS_USER_DRIFT != 0; }
+bool has_user_emission() { return CDK_HAS_USER_EMISSION != 0; }
+int user_emission_params(int n, int m) {
+#if CDK_HAS_USER_EMISSION
+  return cdk_user_emission::num_params(n, m);
+#else
+  return -1;
+#endif
+}
 
 template int launch_generic<double>(int, const KArgs<double>&, cudaStream_t);
 template int launch_generic<float>(int, const KArgs<float>&, cudaStream_t);

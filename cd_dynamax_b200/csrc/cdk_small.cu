@@ -1850,7 +1850,8 @@ int launch_eks_one(const KArgs<T>& a, cudaStream_t s) {
 template <typename T>
 int launch_ekf_small(const KArgs<T>& a, cudaStream_t s) {
   const cdk_desc& d = a.d;
-  if (d.state_order == CDK_ORDER_ZEROTH) return CDK_E_UNSUPPORTED;
+  // the fast path is written for h(x) = H x + d; any other emission runs in the generic kernel
+  if (d.state_order == CDK_ORDER_ZEROTH || d.emission_id != CDK_EMISSION_LINEAR) return CDK_E_UNSUPPORTED;
   if (d.drift_id == CDK_DRIFT_LORENZ63 && d.n == 3) return launch_ny<T, DriftL63>(a, s);
   return CDK_E_UNSUPPORTED;
 }
@@ -1924,7 +1925,7 @@ int launch_eks_small(const KArgs<T>& a, cudaStream_t s) {
     const char* e = getenv("CDK_EKS_FAST");
     return e && e[0] == '0';
   }();
-  if (disabled || d.drift_id != CDK_DRIFT_LORENZ63 || d.n != 3) return CDK_E_UNSUPPORTED;
+  if (disabled || d.drift_id != CDK_DRIFT_LORENZ63 || d.n != 3 || d.emission_id != CDK_EMISSION_LINEAR) return CDK_E_UNSUPPORTED;
   switch (d.solver) {
     case CDK_RK4: return launch_eks_one<T, DriftL63, CDK_RK4>(a, s);
     case CDK_DOPRI5: return launch_eks_one<T, DriftL63, CDK_DOPRI5>(a, s);

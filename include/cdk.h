@@ -65,8 +65,17 @@ enum { CDK_DRIFT_LINEAR = 0, CDK_DRIFT_LORENZ63 = 1, CDK_DRIFT_LORENZ96 = 2, CDK
         * csrc/ with -DCDK_USER_DRIFT_HEADER=<that code> into lib/user/libcdk_user_<hash>.so, which exports this same ABI.
         * theta: any n_theta >= 0 doubles.  The stock libcdk.so rejects this id. */
        CDK_DRIFT_USER = 4 };
-/* emission registry: h(x) = H x + d (LearnableLinear) */
-enum { CDK_EMISSION_LINEAR = 0 };
+/* emission registry.  LINEAR: h(x) = H x + d (LearnableLinear); in[CDK_IN_H] = H [m,n], in[CDK_IN_D] = d [m].
+ * USER: an emission compiled INTO a variant of this library (the reference takes any LearnableFunction.f as emission,
+ *   cdnlgssm_utils.py:13-36).  The caller supplies CUDA device code for n_phi = num_params(n, m), h_a(x; phi) and
+ *   d h_a / d x_j; cd_dynamax_b200.build.build_variant(drift_code, emission_code) compiles csrc/ with
+ *   -DCDK_USER_EMISSION_HEADER=<that code> (a variant may hold a user drift as well).  in[CDK_IN_H] then holds phi
+ *   ([n_phi], or [N, n_phi] with its batched_mask bit: the batched stride is n_phi) and in[CDK_IN_D] is not read (may be
+ *   NULL).  The EKF linearises h at the running mean of every update iteration (H = jac(mu), residual y - h(mu)), the UKF
+ *   pushes its 2n + 1 sigma points through h, the EnKF every member, and cdk_sample_path emits h(x_k) + chol(R) z.
+ *   The stock library and a variant without a user emission reject this id with CDK_E_UNSUPPORTED, and so do every
+ *   gradient entry point and cdk_emission_moments_*. */
+enum { CDK_EMISSION_LINEAR = 0, CDK_EMISSION_USER = 1 };
 /* EKFHyperParams.state_order (inference_ekf.py:40) */
 enum { CDK_ORDER_ZEROTH = 0, CDK_ORDER_FIRST = 1, CDK_ORDER_SECOND = 2 };
 
@@ -82,8 +91,8 @@ enum {
   CDK_IN_BU,      /* kf: dynamics input weights B [n,d_u] or NULL                                   */
   CDK_IN_L,       /* diffusion coefficient L [n,n]                                                  */
   CDK_IN_QC,      /* diffusion covariance Qc [n,n]                                                  */
-  CDK_IN_H,       /* emission weights H   [m,n]                                                     */
-  CDK_IN_D,       /* emission bias d      [m]                                                       */
+  CDK_IN_H,       /* emission weights H   [m,n]   (CDK_EMISSION_USER: emission parameters phi [n_phi]) */
+  CDK_IN_D,       /* emission bias d      [m]     (CDK_EMISSION_USER: not read, may be NULL)         */
   CDK_IN_DU,      /* kf: emission input weights D [m,d_u] or NULL                                   */
   CDK_IN_R,       /* emission covariance R [m,m] ([m] with CDK_FLAG_DIAG_R)                         */
   CDK_IN_FM,      /* smooth: filtered means        [N,K,n]                                          */
@@ -186,7 +195,11 @@ CDK_DECL(cdk_ukf_filter_f64);
 CDK_DECL(cdk_ukf_filter_f32);
 CDK_DECL(cdk_enkf_filter_f64);
 CDK_DECL(cdk_enkf_filter_f32);
-/* Log-likelihood (out[CDK_OUT_LL]) and its gradient with respect to the model parameters (out[CDK_OUT_GRAD],
+/* The gradient entry points below (cdk_ekf_grad_f64, cdk_kf_grad_f64, cdk_ekf_grad_dense_f64, cdk_ukf_grad_dense_f64,
+ * cdk_ukf_grad_sigma_f64) differentiate the linear emission only: the nonlinear ones return CDK_E_UNSUPPORTED for
+ * CDK_EMISSION_USER before any other check.
+ *
+ * Log-likelihood (out[CDK_OUT_LL]) and its gradient with respect to the model parameters (out[CDK_OUT_GRAD],
  * [N, CDK_GRAD_COLS_L63]) of the CD-EKF: what jax.value_and_grad(marginal_log_prob) hands the reference's fit_sgd
  * (src/utils/optimize_utils.py:102, src/ssm_temissions.py:550-568).  Forward-mode derivative of exactly the discrete filter
  * cdk_ekf_filter_f64 runs, one launch per direction.  Columns: theta = sigma, rho, beta (3) | L Qc L^T, packed upper
@@ -275,13 +288,15 @@ CDK_DECL(cdk_ukf_grad_sigma_f64);
 /* Forward sample paths of the model (cdnlgssm_path_sample, cd_nonlinear/models.py:525-656; what
  * SSM.sample_batch(..., transition_type="path") vmaps, src/ssm_temissions.py:187-225): x_0 ~ N(m0, P0), x_k = SDE solve of
  * dx = f(x) dt + L chol(Qc) dW over [t_{k-1}, t_k] (desc.solver = CDK_HEUN, the reference default for SDEs, or CDK_EULER =
- * Euler-Maruyama; diffrax stepping rule with desc.dt0), y_k ~ N(H x_k + d, R).  out[CDK_OUT_FM] = states [N, K, n],
+ * Euler-Maruyama; diffrax stepping rule with desc.dt0), y_k ~ N(H x_k + d, R) (CDK_EMISSION_USER: y_k ~ N(h(x_k), R), the same
+ * deviates).  out[CDK_OUT_FM] = states [N, K, n],
  * out[CDK_OUT_PM] = emissions [N, K, m] (either may be NULL), out[CDK_OUT_STATUS].  Philox4x32-10 stream keyed by
  * desc.rng_seed / rng_offset (the reference's jax.random stream is not reproducible outside JAX).  Model parameters must
  * not be batched (in[CDK_IN_M0] may be). */
 CDK_DECL(cdk_sample_path_f64);
 CDK_DECL(cdk_sample_path_f32);
-/* Emission moments of Gaussian state estimates under the linear emission (emissions_extended_kalman_filter,
+/* Emission moments of Gaussian state estimates under the linear emission (CDK_EMISSION_USER returns CDK_E_UNSUPPORTED;
+ * emissions_extended_kalman_filter,
  * inference_ekf.py:762-855, and its unscented twin): in[CDK_IN_FM] [N, K, n], in[CDK_IN_FP] [N, K, n, n] or NULL (point
  * estimates) -> out[CDK_OUT_PM] = H m + d [N, K, m], out[CDK_OUT_PP] = H P H^T + R [N, K, m, m]. */
 CDK_DECL(cdk_emission_moments_f64);
@@ -344,6 +359,11 @@ int64_t cdk_launch_count(void);
 
 /* 1 when this library is a variant compiled with a user-defined drift (CDK_DRIFT_USER), 0 for the stock build. */
 int cdk_has_user_drift(void);
+/* 1 when this library is a variant compiled with a user-defined emission (CDK_EMISSION_USER), 0 otherwise. */
+int cdk_has_user_emission(void);
+/* Length n_phi of the user emission's parameter vector for state dimension n and emission dimension m (its num_params),
+ * or -1 in a library without a user emission. */
+int cdk_user_emission_params(int n, int m);
 int cdk_version(void);
 const char* cdk_last_error(void);
 
