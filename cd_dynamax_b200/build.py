@@ -117,7 +117,8 @@ def build_variant(drift_code=None, emission_code=None, grad: bool = False, verbo
         template <typename T, class XF> __device__ T h(const T* phi, int n, int m, int a, XF x);   // h_a(x; phi); x(j) = x_j
         template <typename T> __device__ T jac(const T* phi, int n, int m, int a, int j, const T* x); // d h_a / d x_j
 
-    Nothing differentiates the emission: the gradient entry points reject it.  grad=True (the drift's dense EKF gradient)
+    num_params may return 0 (an emission without parameters; phi is then [0] or [N, 0]), as a user drift may take
+    n_theta = 0 parameters (theta [0]).  Nothing differentiates the emission: the gradient entry points reject it.  grad=True (the drift's dense EKF gradient)
     needs a drift.
 
     Returns the path of cd_dynamax_b200/lib/user/libcdk_user_<hash>.so, cached by content hash (variant_key: both codes

@@ -79,6 +79,13 @@ static int validate(const cdk_desc* d, const void* const* in, void* const* out, 
   const bool linear = algo == ALGO_KF_FILTER || algo == ALGO_KF_SMOOTH;
   const bool smooth = algo == ALGO_KF_SMOOTH || algo == ALGO_EKF_SMOOTH;
   const bool user_emission = !linear && d->emission_id == CDK_EMISSION_USER;  // in[CDK_IN_D] is not read
+  // a parameter-free user emission (num_params = 0) or user drift (n_theta = 0) reads nothing from in[CDK_IN_H] /
+  // in[CDK_IN_F]: the caller may pass NULL there (an empty array has no data pointer)
+  const bool no_phi = user_emission && cdk::user_emission_params(d->n, d->m) == 0;
+  const bool no_theta = !linear && d->drift_id == CDK_DRIFT_USER && d->n_theta == 0;
+  auto optional_input = [&](int s) {
+    return (user_emission && s == CDK_IN_D) || (no_phi && s == CDK_IN_H) || (no_theta && s == CDK_IN_F);
+  };
   if (!linear && algo != ALGO_EMISSIONS) {
     if (d->drift_id < CDK_DRIFT_LINEAR || d->drift_id > CDK_DRIFT_USER) return fail(CDK_E_ENUM, "unknown drift_id");
     if (d->drift_id == CDK_DRIFT_USER && !cdk::has_user_drift())
@@ -113,7 +120,7 @@ static int validate(const cdk_desc* d, const void* const* in, void* const* out, 
     static const int req_s[] = {CDK_IN_T, CDK_IN_M0, CDK_IN_F, CDK_IN_L, CDK_IN_QC, CDK_IN_H, CDK_IN_D, CDK_IN_R};
     if (d->N > 0) {
       for (int s : req_s)
-        if (!in[s] && !(user_emission && s == CDK_IN_D)) return fail(CDK_E_NULL, "a required input of the sampler is NULL");
+        if (!in[s] && !optional_input(s)) return fail(CDK_E_NULL, "a required input of the sampler is NULL");
       if (!(d->reserved[2] & CDK_FLAG_FIXED_INIT) && !in[CDK_IN_P0]) return fail(CDK_E_NULL, "sampling x_0 needs P0");
     }
     return CDK_OK;
@@ -131,7 +138,7 @@ static int validate(const cdk_desc* d, const void* const* in, void* const* out, 
       if (d->d_u > 0 && (!in[CDK_IN_U] || !in[CDK_IN_BU] || !in[CDK_IN_DU])) return fail(CDK_E_NULL, "d_u > 0 needs U, BU and DU");
     } else {
       for (int s : req_nl)
-        if (!in[s] && !(ponly && s == CDK_IN_Y) && !(user_emission && s == CDK_IN_D))
+        if (!in[s] && !(ponly && s == CDK_IN_Y) && !optional_input(s))
           return fail(CDK_E_NULL, "a required input of the nonlinear model is NULL");
     }
     if (smooth && (!in[CDK_IN_FM] || !in[CDK_IN_FP])) return fail(CDK_E_NULL, "smoothing needs the filtered moments");

@@ -63,7 +63,8 @@ enum { CDK_DRIFT_LINEAR = 0, CDK_DRIFT_LORENZ63 = 1, CDK_DRIFT_LORENZ96 = 2, CDK
         * cdnlgssm_utils.py:13-36).  The caller supplies CUDA device code for f_i(x; theta) and dJ_ij(x; theta) (and,
         * for EKF state_order 'second', g_k = sum_i d2 f_i / dx_i dx_k); cd_dynamax_b200.build.build_user_drift() compiles
         * csrc/ with -DCDK_USER_DRIFT_HEADER=<that code> into lib/user/libcdk_user_<hash>.so, which exports this same ABI.
-        * theta: any n_theta >= 0 doubles.  The stock libcdk.so rejects this id. */
+        * theta: any n_theta >= 0 doubles; with n_theta = 0, in[CDK_IN_F] is not read (may be NULL).  The stock libcdk.so
+        * rejects this id. */
        CDK_DRIFT_USER = 4 };
 /* emission registry.  LINEAR: h(x) = H x + d (LearnableLinear); in[CDK_IN_H] = H [m,n], in[CDK_IN_D] = d [m].
  * USER: an emission compiled INTO a variant of this library (the reference takes any LearnableFunction.f as emission,
@@ -71,7 +72,8 @@ enum { CDK_DRIFT_LINEAR = 0, CDK_DRIFT_LORENZ63 = 1, CDK_DRIFT_LORENZ96 = 2, CDK
  *   d h_a / d x_j; cd_dynamax_b200.build.build_variant(drift_code, emission_code) compiles csrc/ with
  *   -DCDK_USER_EMISSION_HEADER=<that code> (a variant may hold a user drift as well).  in[CDK_IN_H] then holds phi
  *   ([n_phi], or [N, n_phi] with its batched_mask bit: the batched stride is n_phi) and in[CDK_IN_D] is not read (may be
- *   NULL).  The EKF linearises h at the running mean of every update iteration (H = jac(mu), residual y - h(mu)), the UKF
+ *   NULL).  num_params may be 0 (an emission with no parameters, e.g. a fixed sensor geometry compiled in): in[CDK_IN_H]
+ *   is then not read either and may be NULL.  The EKF linearises h at the running mean of every update iteration (H = jac(mu), residual y - h(mu)), the UKF
  *   pushes its 2n + 1 sigma points through h, the EnKF every member, and cdk_sample_path emits h(x_k) + chol(R) z.
  *   The stock library and a variant without a user emission reject this id with CDK_E_UNSUPPORTED, and so do every
  *   gradient entry point and cdk_emission_moments_*. */

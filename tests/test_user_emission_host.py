@@ -74,3 +74,43 @@ def test_phi_of_the_wrong_length_raises_on_the_host():
     for bad in (np.zeros(4), np.zeros((4, 6)), np.zeros((2, 2, 5))):
         with pytest.raises(ValueError, match="num_params"):
             nonlinear_inputs(_params(bad), np.zeros((1, 3, 2)), np.zeros((1, 3)), 2, 2)
+
+
+@pytest.mark.parametrize("kind", ["range", "wide", "square"])
+def test_test_emissions_jacobian_is_the_derivative_of_h(kind):
+    """The NumPy twins of the GPU matrix's test emissions: the analytic jac against central differences of h."""
+    from tests.test_gpu_user_emission_matrix import _emission
+    n, m = 3, 5
+    rng = np.random.default_rng(1)
+    em = _emission(kind, n, m, rng)
+    x = rng.standard_normal((4, n)) + 0.5
+    eps = 1e-6
+    fd = np.stack([(em.h(x + eps * e) - em.h(x - eps * e)) / (2 * eps) for e in np.eye(n)], axis=-1)
+    J = em.jac(x)
+    assert J.shape == (4, m, n)
+    assert np.max(np.abs(J - fd)) < 1e-8 * max(1.0, np.max(np.abs(fd)))
+
+
+def test_per_trajectory_phi_with_the_wrong_batch_raises_before_any_launch():
+    """phi [N', n_phi] with N' != N (and N' != 1) is refused by the engine's host-side shape check, naming the slot."""
+    import cd_dynamax_b200 as cd
+    y, t = np.zeros((4, 3, 2)), np.tile(np.arange(3.0), (4, 1))[..., None]
+    for bad in (np.zeros((3, 5)), np.zeros((5, 5))):
+        with pytest.raises(ValueError, match="IN_H"):
+            cd.cdnlgssm_filter(_params(bad), y, t, cd.EKFHyperParams())
+    with pytest.raises(ValueError, match="num_params"):
+        cd.cdnlgssm_filter(_params(np.zeros((4, 6))), y, t, cd.EKFHyperParams())
+
+
+def test_parameter_free_emission_phi_classifies():
+    """n_phi = 0: phi [0] is the shared call and [N, 0] a batched one with rows of 0 elements (a NULL device pointer)."""
+    from cd_dynamax_b200 import _engine
+    from cd_dynamax_b200 import _lib as L
+    N, K, n, m = 4, 3, 2, 3
+    fields = dict(emission_id=L.EMISSION_USER, n_phi=0)
+    metas, mask = _engine.classify(N, K, n, m, {L.IN_H: np.zeros(0)}, fields)
+    assert not metas[L.IN_H][1] and metas[L.IN_H][2] == 0 and mask == 0
+    metas, mask = _engine.classify(N, K, n, m, {L.IN_H: np.zeros((N, 0))}, fields)
+    assert metas[L.IN_H][1] and metas[L.IN_H][2] == 0 and mask == 1 << L.IN_H
+    with pytest.raises(ValueError, match="IN_H"):
+        _engine.classify(N, K, n, m, {L.IN_H: np.zeros(1)}, fields)

@@ -189,10 +189,14 @@ def ensemble_kalman_filter(p, em, y, t, dt_final=1e-10, E=64, perturb_measuremen
     return out
 
 
-def sample_paths(p, em, t, seed=0, rng_offset=0, settings=o.SolverSettings(solver="heun"), dtype=np.float64):
-    """States [N,K,n] and emissions [N,K,m] = h(x_k) + chol(R) z on the oracle's stream (x_0 ~ N(m0, P0))."""
+def sample_paths(p, em, t, seed=0, rng_offset=0, settings=o.SolverSettings(solver="heun"), fixed_init=False,
+                 dtype=np.float64):
+    """States [N,K,n] and emissions [N,K,m] = h(x_k) + chol(R) z on the oracle's stream (x_0 ~ N(m0, P0)).
+    fixed_init (a forecast from a point estimate): t is [N,K+1] (t_init first), the path starts AT m0 and the K outputs
+    are the forecast times, as in oracle.cd_oracle.sample_paths."""
     t = np.asarray(t, dtype)
-    N, K = t.shape
+    N = t.shape[0]
+    K = t.shape[1] - 1 if fixed_init else t.shape[1]
     c = lambda x, core: _bN(np.asarray(x, dtype), N, core)
     L, Qc, R = c(p.L, 2), c(p.Qc, 2), c(p.R, 2)
     n, mdim = L.shape[-1], R.shape[-1]
@@ -202,16 +206,20 @@ def sample_paths(p, em, t, seed=0, rng_offset=0, settings=o.SolverSettings(solve
     tdt, dt0, tol = o._stepping(settings, dtype)
     xs, ys = np.zeros((N, K, n), dtype), np.zeros((N, K, mdim), dtype)
 
-    def emit(x, row):
-        z = o.enkf_normals(o.RNG_OBS, traj, row, 0, 1, mdim, seed, rng_offset)[:, 0].astype(dtype)
+    def emit(x, row, step):
+        z = o.enkf_normals(o.RNG_OBS, traj, step, 0, 1, mdim, seed, rng_offset)[:, 0].astype(dtype)
         xs[:, row] = x
         ys[:, row] = em.h(x) + _mv(cholR, z)
 
-    z = o.enkf_normals(o.RNG_INIT, traj, 0, 0, 1, n, seed, rng_offset)[:, 0].astype(dtype)
-    x = c(p.m0, 1) + _mv(o.cholesky(c(p.P0, 2)), z)
-    emit(x, 0)
-    for k in range(1, K):
-        tprev, t1 = t[:, k - 1].astype(tdt), t[:, k].astype(tdt)
+    if fixed_init:
+        x = c(p.m0, 1).copy()
+    else:
+        z = o.enkf_normals(o.RNG_INIT, traj, 0, 0, 1, n, seed, rng_offset)[:, 0].astype(dtype)
+        x = c(p.m0, 1) + _mv(o.cholesky(c(p.P0, 2)), z)
+        emit(x, 0, 0)
+    for k in range(0 if fixed_init else 1, K):
+        tprev = (t[:, k] if fixed_init else t[:, k - 1]).astype(tdt)
+        t1 = (t[:, k + 1] if fixed_init else t[:, k]).astype(tdt)
         tnext = np.minimum(tprev + dt0, t1)
         sub = 0
         nst = np.zeros(N, np.int64)
@@ -232,5 +240,5 @@ def sample_paths(p, em, t, seed=0, rng_offset=0, settings=o.SolverSettings(solve
             tprev = np.where(active, tnext, tprev)
             cand = tprev + dt0
             tnext = np.where(cand > t1 - tol, t1, cand)
-        emit(x, k)
+        emit(x, k, k + 1 if fixed_init else k)
     return xs, ys
