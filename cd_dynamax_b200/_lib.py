@@ -33,6 +33,12 @@ def grad_cols_ekf(n, m, n_theta):
     return n_theta + 2 * n * n + m * n + m * m + n + m
 
 
+def grad_cols_ekf_ue(n, m, n_theta, n_phi):
+    """CDK_GRAD_COLS_EKF_UE(n, m, n_theta, n_phi): columns of out[CDK_OUT_GRAD] of cdk_ekf_grad_dense_f64 with a user
+    emission (phi in place of H | d)."""
+    return n_theta + 2 * n * n + n_phi + m * m + n
+
+
 ENTRY_POINTS = [f"cdk_{a}_{d}_{t}" for a, d in (("kf", "filter"), ("kf", "smooth"), ("ekf", "filter"), ("ekf", "smooth"),
                                                   ("ukf", "filter"), ("enkf", "filter")) for t in ("f64", "f32")]
 ENTRY_POINTS.append("cdk_ekf_grad_f64")

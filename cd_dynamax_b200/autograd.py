@@ -7,7 +7,8 @@ stack (INTEGRATION.md section 2) -- forward = the CUDA filter, backward = the ha
 
 What `fit_sgd` minimises upstream is `-vmap(marginal_log_prob)(...).sum()` (src/ssm_temissions.py:550-568,
 src/utils/optimize_utils.py:102).  Every registry drift, linear emission of any size, fp64 (cdk_ekf_grad_f64 for
-Lorenz-63 with a scalar emission, cdk_ekf_grad_dense_f64 otherwise).  ukf_marginal_log_prob is the same for the
+Lorenz-63 with a scalar emission, cdk_ekf_grad_dense_f64 otherwise); differentiable user drifts and emissions
+(cdk_ekf_grad_dense_f64).  ukf_marginal_log_prob is the same for the
 closed-form CD-UKF (backward = cdk_ukf_grad_dense_f64), ukf_sigma_points_marginal_log_prob for the CD-UKF with literal
 sigma points (backward = cdk_ukf_grad_sigma_f64; registry drifts and differentiable user drifts).
 
@@ -17,7 +18,8 @@ import torch
 
 from .continuous_discrete_linear_gaussian_ssm.inference import cdlgssm_marginal_log_prob_and_grad
 
-from .continuous_discrete_nonlinear_gaussian_ssm._common import reject_user_emission
+from .continuous_discrete_nonlinear_gaussian_ssm._common import (check_user_emission_grad, is_user_emission,
+                                                                 reject_user_emission)
 from .continuous_discrete_nonlinear_gaussian_ssm.inference_ekf import (EKFHyperParams, drift_leaves,
                                                                        ekf_dense_marginal_log_prob_and_grad,
                                                                        ekf_marginal_log_prob_and_grad)
@@ -29,13 +31,17 @@ def _val(x):
 
 
 def _leaves(params):
-    """Leaf name -> value: the drift's own fields (sigma / rho / beta, weights / bias, forcing, a / B / C), then the rest."""
+    """Leaf name -> value: the drift's own fields (sigma / rho / beta, weights / bias, forcing, a / B / C), then the rest
+    (a user emission's parameters are the one leaf "phi")."""
     d, e = params.dynamics, params.emissions
     out = {name: getattr(d.drift, name) for name, _ in drift_leaves(d.drift, 0)}
     out.update(diffusion_coefficient=_val(d.diffusion_coefficient), diffusion_cov=_val(d.diffusion_cov),
-               emission_cov=_val(e.emission_cov), emission_bias=e.emission_function.bias,
-               emission_weights=e.emission_function.weights, initial_mean=_val(params.initial.mean),
-               initial_cov=_val(params.initial.cov))
+               emission_cov=_val(e.emission_cov))
+    if is_user_emission(params):
+        out.update(phi=e.emission_function.phi)
+    else:
+        out.update(emission_bias=e.emission_function.bias, emission_weights=e.emission_function.weights)
+    out.update(initial_mean=_val(params.initial.mean), initial_cov=_val(params.initial.cov))
     return out
 
 
@@ -67,7 +73,6 @@ class _NonlinearLogLik(torch.autograd.Function):
 
 
 def _nonlinear_log_prob(grad_fn, params, emissions, t_emissions, hyperparams):
-    reject_user_emission(params, grad_fn.__name__)
     leaves = _leaves(params)
     names = tuple(leaves)
     tensors = [leaves[n] if isinstance(leaves[n], torch.Tensor) else torch.as_tensor(leaves[n]) for n in names]
@@ -77,10 +82,11 @@ def _nonlinear_log_prob(grad_fn, params, emissions, t_emissions, hyperparams):
 def ekf_marginal_log_prob(params, emissions, t_emissions=None, hyperparams: EKFHyperParams = EKFHyperParams()):
     """Per-trajectory marginal log-likelihood of the CD-EKF as a differentiable torch tensor.  Every leaf of `params`
     that is a torch tensor with requires_grad receives its gradient on `.backward()`: the drift's fields (named as in its
-    registry class) and the diffusion, emission and initial parameters."""
-    reject_user_emission(params, "ekf_marginal_log_prob")
-    H = params.emissions.emission_function.weights
-    scalar_l63 = type(params.dynamics.drift).__name__ == "LearnableLorenz63" and tuple(np.shape(H))[-2] == 1
+    registry class) and the diffusion, emission and initial parameters; for a LearnableUserEmission(...,
+    differentiable=True) the emission's parameters are a torch `phi`."""
+    check_user_emission_grad(params, "ekf_marginal_log_prob")
+    scalar_l63 = (type(params.dynamics.drift).__name__ == "LearnableLorenz63" and not is_user_emission(params)
+                  and tuple(np.shape(params.emissions.emission_function.weights))[-2] == 1)
     fn = ekf_marginal_log_prob_and_grad if scalar_l63 else ekf_dense_marginal_log_prob_and_grad
     return _nonlinear_log_prob(fn, params, emissions, t_emissions, hyperparams)
 
@@ -89,6 +95,7 @@ def ukf_marginal_log_prob(params, emissions, t_emissions=None, hyperparams: UKFH
     """Per-trajectory marginal log-likelihood of the closed-form CD-UKF as a differentiable torch tensor
     (ukf_marginal_log_prob_and_grad).  Every leaf of `params` that is a torch tensor with requires_grad receives its
     gradient on `.backward()`, as in `ekf_marginal_log_prob`."""
+    reject_user_emission(params, "ukf_marginal_log_prob")
     return _nonlinear_log_prob(ukf_marginal_log_prob_and_grad, params, emissions, t_emissions, hyperparams)
 
 
@@ -98,6 +105,7 @@ def ukf_sigma_points_marginal_log_prob(params, emissions, t_emissions=None,
     (ukf_sigma_points_marginal_log_prob_and_grad).  Every leaf of `params` that is a torch tensor with requires_grad
     receives its gradient on `.backward()`, as in `ekf_marginal_log_prob`; for a LearnableUserDrift(...,
     differentiable=True) that includes a torch `theta`."""
+    reject_user_emission(params, "ukf_sigma_points_marginal_log_prob")
     return _nonlinear_log_prob(ukf_sigma_points_marginal_log_prob_and_grad, params, emissions, t_emissions, hyperparams)
 
 

@@ -68,18 +68,20 @@ def build(force=False, verbose=False):
 
 
 USER_SOURCES = ["cdk_api.cu", "cdk_generic.cu", "cdk_enkf.cu", "cdk_aux.cu"]  # the units that see the drift registry
-USER_GRAD_SOURCES = USER_SOURCES + ["cdk_ekfgrad.cu"]  # ... plus the dense EKF gradient (build_user_drift(grad=True))
-USER_KEEP = 8  # variants kept in lib/user, newest first
+USER_GRAD_SOURCES = USER_SOURCES + ["cdk_ekfgrad.cu"]  # ... plus the dense EKF gradient (grad or emission_grad)
+USER_KEEP = 24  # variants kept in lib/user, newest first
 
 
-def variant_key(drift_code=None, emission_code=None, grad=False) -> str:
-    """Content hash naming the variant of build_variant(drift_code, emission_code, grad): the device codes (each marked
-    present or absent), `grad`, the library sources and this file."""
+def variant_key(drift_code=None, emission_code=None, grad=False, emission_grad=False) -> str:
+    """Content hash naming the variant of build_variant(drift_code, emission_code, grad, emission_grad=...): the device
+    codes (each marked present or absent), the two gradient flags, the library sources and this file."""
     import hashlib
     key = hashlib.sha1()
     for part in (drift_code, emission_code):
         key.update(b"-" if part is None else b"%d:" % len(part.encode()) + part.encode())
     key.update(b"grad" if grad else b"filter")
+    if emission_grad:
+        key.update(b"emission_grad")
     for f in sorted(os.listdir(CSRC)) + ["../../include/cdk.h", "../build.py"]:
         key.update(open(os.path.join(CSRC, f), "rb").read())
     return key.hexdigest()[:16]
@@ -108,7 +110,7 @@ def build_user_drift(device_code: str, grad: bool = False, verbose=False) -> str
     return build_variant(device_code, None, grad, verbose)
 
 
-def build_variant(drift_code=None, emission_code=None, grad: bool = False, verbose=False) -> str:
+def build_variant(drift_code=None, emission_code=None, grad: bool = False, verbose=False, emission_grad: bool = False) -> str:
     """Compile a VARIANT of libcdk.so with a user-defined drift (CDK_DRIFT_USER, `drift_code`: see build_user_drift), a
     user-defined emission (CDK_EMISSION_USER, `emission_code`), or both.  `emission_code` must define, inside
     `namespace cdk_user_emission { ... }`, for T = float and double:
@@ -118,19 +120,33 @@ def build_variant(drift_code=None, emission_code=None, grad: bool = False, verbo
         template <typename T> __device__ T jac(const T* phi, int n, int m, int a, int j, const T* x); // d h_a / d x_j
 
     num_params may return 0 (an emission without parameters; phi is then [0] or [N, 0]), as a user drift may take
-    n_theta = 0 parameters (theta [0]).  Nothing differentiates the emission: the gradient entry points reject it.  grad=True (the drift's dense EKF gradient)
-    needs a drift.
+    n_theta = 0 parameters (theta [0]).  grad=True (the drift's dense EKF gradient) needs a drift.
+
+    emission_grad=True also compiles the dense EKF gradient (cdk_ekf_grad_dense_f64) for this emission, the gradient
+    with respect to phi included.  It instantiates h and jac with T = cdk_dual::Dual<W> (csrc/cdk_dual.cuh) and takes
+    d2h/dx dphi, dJ/dx and dJ/dphi from them, so the emission code must then stay within the dual-number contract that
+    build_user_drift states for drifts: arithmetic on T only (+ - * / and unary -, mixed with int / double constants,
+    compound assignment, comparisons, T(c)) and the UNQUALIFIED functions sqrt exp log sin cos tan tanh sinh cosh atan
+    fabs pow(T, double); num_params stays plain int.  examples/range_emission.cuh and examples/linear_emission.cuh do.
+    The cost is (n + n_phi) / W dual evaluations of all m n entries of jac per update VJP: forward mode over phi, so it
+    grows with n_phi.  emission_grad needs an emission.
+
+    The gradient unit (cdk_ekfgrad.cu) is compiled when grad or emission_grad is set, and it sees the drift's code only
+    with grad and the emission's only with emission_grad: code that is not declared dual-safe never reaches it.  The
+    filter units see both codes whatever the flags.
 
     Returns the path of cd_dynamax_b200/lib/user/libcdk_user_<hash>.so, cached by content hash (variant_key: both codes
-    and `grad`; ~1 minute of nvcc the first time; the USER_KEEP newest variants are kept).  The variant exports the same C
-    ABI (include/cdk.h); the units that do not see the registries (cdk_small.cu, cdk_kfwarp.cu, and cdk_ekfgrad.cu unless
-    grad) are linked from the stock build."""
+    and both flags; ~1 minute of nvcc the first time; the USER_KEEP newest variants are kept).  The variant exports the
+    same C ABI (include/cdk.h); the units that do not see the registries (cdk_small.cu, cdk_kfwarp.cu, and cdk_ekfgrad.cu
+    unless grad or emission_grad) are linked from the stock build."""
     if drift_code is None and emission_code is None:
         raise ValueError("build_variant needs a drift code, an emission code or both")
     if grad and drift_code is None:
         raise ValueError("grad=True compiles the gradient of a user drift: it needs drift_code")
+    if emission_grad and emission_code is None:
+        raise ValueError("emission_grad=True compiles the gradient of a user emission: it needs emission_code")
     build()  # the stock objects
-    tag = variant_key(drift_code, emission_code, grad)
+    tag = variant_key(drift_code, emission_code, grad, emission_grad)
     udir = os.path.join(LIBDIR, "user")
     os.makedirs(udir, exist_ok=True)
     lib = os.path.join(udir, f"libcdk_user_{tag}.so")
@@ -138,20 +154,21 @@ def build_variant(drift_code=None, emission_code=None, grad: bool = False, verbo
         return lib
     work = os.path.join(OBJ, f"user_{tag}")
     os.makedirs(work, exist_ok=True)
-    flags = []
-    for code, name, macro in ((drift_code, "cdk_user_drift.cuh", "CDK_USER_DRIFT_HEADER"),
-                              (emission_code, "cdk_user_emission.cuh", "CDK_USER_EMISSION_HEADER")):
+    flags = {}  # header macro -> (its -D flag, whether the gradient unit sees it)
+    for code, name, macro, in_grad in ((drift_code, "cdk_user_drift.cuh", "CDK_USER_DRIFT_HEADER", grad),
+                                       (emission_code, "cdk_user_emission.cuh", "CDK_USER_EMISSION_HEADER", emission_grad)):
         if code is None:
             continue
         header = os.path.join(work, name)
         with open(header, "w") as fh:
             fh.write("// generated by cd_dynamax_b200.build.build_variant\n#pragma once\n" + code + "\n")
-        flags.append(f'-D{macro}="{header}"')
-    units = USER_GRAD_SOURCES if grad else USER_SOURCES
+        flags[macro] = (f'-D{macro}="{header}"', in_grad)
+    units = USER_GRAD_SOURCES if grad or emission_grad else USER_SOURCES
     jobs = []
     for s in units:
         src, obj = os.path.join(CSRC, s), os.path.join(work, s.replace(".cu", ".o"))
-        jobs.append((s, [_nvcc()] + NVCC_FLAGS + flags + ["-c", src, "-o", obj]))
+        unit_flags = [f for f, in_grad in flags.values() if in_grad or s != "cdk_ekfgrad.cu"]
+        jobs.append((s, [_nvcc()] + NVCC_FLAGS + unit_flags + ["-c", src, "-o", obj]))
     with concurrent.futures.ThreadPoolExecutor(max_workers=len(jobs)) as ex:
         futs = {ex.submit(subprocess.run, cmd, capture_output=True, text=True): name for name, cmd in jobs}
         for f in concurrent.futures.as_completed(futs):

@@ -29,8 +29,17 @@ def reject_user_emission(params, what):
     """`what` has no user-emission path: raise before any build or device work."""
     if is_user_emission(params):
         raise NotImplementedError(f"{what} is not available for a LearnableUserEmission (a user-defined emission has no "
-                                  "gradient and no emission-moment helper); it runs through the filters, the EKS and the "
-                                  "path sampler only")
+                                  "UKF gradient and no emission-moment helper); it runs through the filters, the EKS, the "
+                                  "path sampler and, with LearnableUserEmission(..., differentiable=True), the EKF "
+                                  "gradient")
+
+
+def check_user_emission_grad(params, what):
+    """The EKF gradient of a user emission needs differentiable=True: raise before any build or device work."""
+    if is_user_emission(params) and not params.emissions.emission_function.differentiable:
+        raise NotImplementedError(f"{what}: the gradient of a LearnableUserEmission needs LearnableUserEmission(..., "
+                                  "differentiable=True), which declares that its device code stays within the "
+                                  "dual-number contract (cd_dynamax_b200.build.build_variant)")
 
 
 def emission_dim(params):
@@ -58,7 +67,8 @@ def nonlinear_inputs(params, Y, T, n, m):
         user_drift = drift_id == L.DRIFT_USER
         if user_em:
             fields["lib_path"] = _build.build_variant(drift.device_code if user_drift else None, em.device_code,
-                                                      grad=user_drift and bool(drift.differentiable))
+                                                      grad=user_drift and bool(drift.differentiable),
+                                                      emission_grad=bool(em.differentiable))
         else:
             fields["lib_path"] = _build.build_user_drift(drift.device_code, grad=bool(drift.differentiable))
     if user_em:

@@ -102,11 +102,15 @@ class LearnableUserEmission(NamedTuple):
     as CUDA C++ source (see cd_dynamax_b200.build.build_variant for the three functions it must define in
     `namespace cdk_user_emission`) plus its parameter vector `phi` ([n_phi] or [N, n_phi], torch or NumPy); the first use
     compiles a variant of libcdk.so with that code -- and the drift's, when the drift is a LearnableUserDrift -- in the
-    registries (cached by content hash).  The EKF, EKS, UKF, EnKF and the path sampler run it; gradients and the emission
-    moments of cdnlgssm_emissions do not.  `py_h` is an optional NumPy callable h(x, phi) for host-side use (`.f`)."""
+    registries (cached by content hash).  The EKF, EKS, UKF, EnKF and the path sampler run it; the emission moments of
+    cdnlgssm_emissions and the UKF gradients do not.  `py_h` is an optional NumPy callable h(x, phi) for host-side use
+    (`.f`).  `differentiable=True` declares that the code stays within the dual-number contract (build_variant) and
+    compiles the EKF gradient for it: ekf_marginal_log_prob_and_grad, ekf_dense_marginal_log_prob_and_grad and
+    autograd.ekf_marginal_log_prob then differentiate every parameter, phi included (grads["phi"])."""
     device_code: str
     phi: Any
     py_h: Any = None
+    differentiable: bool = False
 
     def f(self, x, u=None, t=None):
         if self.py_h is None:

@@ -9,7 +9,7 @@ from .. import _engine as E
 from .. import _lib as L
 from ..continuous_discrete_linear_gaussian_ssm.inference import _sq
 from ..types import PosteriorGSSMFiltered, PosteriorGSSMSmoothed
-from ._common import DEFAULT_FIELDS, reject_user_emission, run_filter
+from ._common import DEFAULT_FIELDS, check_user_emission_grad, is_user_emission, run_filter
 
 
 class EKFHyperParams(NamedTuple):
@@ -92,7 +92,9 @@ def ekf_marginal_log_prob_and_grad(params, emissions, t_emissions=None, hyperpar
     its own kernels (cdk_ekf_grad_f64, below): a scalar emission only, anything else raises NotImplementedError; call
     `ekf_dense_marginal_log_prob_and_grad` for Lorenz-63 with a multi-component emission.  A LearnableUserDrift with
     differentiable=True runs through the dense function too and gets its gradient under "theta" ([n_theta] or
-    [N, n_theta]); with differentiable=False it raises NotImplementedError before any build or device work.
+    [N, n_theta]); with differentiable=False it raises NotImplementedError before any build or device work.  So does a
+    LearnableUserEmission: with differentiable=True it runs through the dense function (whatever the drift, Lorenz-63
+    included) and its parameters' gradient is "phi", in place of "emission_weights" / "emission_bias".
 
     This is what `jax.value_and_grad(lambda p: model.marginal_log_prob(p, ...))` yields upstream
     (src/utils/optimize_utils.py:102, src/ssm_temissions.py:550-568) -- here as the derivative of exactly the discrete
@@ -101,13 +103,12 @@ def ekf_marginal_log_prob_and_grad(params, emissions, t_emissions=None, hyperpar
     + one backward launch for all 23 columns, ~4 filter passes), forward mode otherwise (one launch per column), so that
     a `jax.custom_vjp` around the filter can be fed (INTEGRATION.md).  Symmetric matrices (diffusion_cov, initial_cov) are differentiated
     along symmetric directions: the result is the symmetric part (G + G^T)/2 of the entry-wise gradient G, which is what
-    any PSD parameterisation consumes; diffusion_coefficient's gradient is exact.  Both paths: num_iter = 1, fp64.
-    A LearnableUserEmission raises NotImplementedError: a user-defined emission has no gradient."""
-    reject_user_emission(params, "ekf_marginal_log_prob_and_grad")
+    any PSD parameterisation consumes; diffusion_coefficient's gradient is exact.  Both paths: num_iter = 1, fp64."""
+    check_user_emission_grad(params, "ekf_marginal_log_prob_and_grad")
     import torch
     from ._common import nonlinear_inputs, _val
     from ..continuous_discrete_linear_gaussian_ssm.inference import _shape, prepare_data
-    if type(params.dynamics.drift).__name__ != "LearnableLorenz63":
+    if type(params.dynamics.drift).__name__ != "LearnableLorenz63" or is_user_emission(params):
         return ekf_dense_marginal_log_prob_and_grad(params, emissions, t_emissions, hyperparams, inputs, wrt)
     wrt = _parse_wrt(wrt)
     groups = 0
@@ -205,11 +206,16 @@ def unflatten_theta(G_theta, drift, n):
     return out
 
 
-def _parse_wrt(wrt):
-    wrt = tuple(_GRAD_GROUPS) if wrt == "all" else ((wrt,) if isinstance(wrt, str) else tuple(wrt))
-    unknown = [w for w in wrt if w not in _GRAD_GROUPS]
+def _parse_wrt(wrt, user_emission=False):
+    """`wrt` -> tuple of group names.  With a user emission its parameters are the group "phi", which takes the place of
+    "emission_bias" and "emission_weights"."""
+    groups = tuple(_GRAD_GROUPS)
+    if user_emission:
+        groups = tuple("phi" if g == "emission_bias" else g for g in groups if g != "emission_weights")
+    wrt = groups if wrt == "all" else ((wrt,) if isinstance(wrt, str) else tuple(wrt))
+    unknown = [w for w in wrt if w not in groups]
     if unknown:
-        raise ValueError(f"unknown gradient groups {unknown}; choose from {sorted(_GRAD_GROUPS)}")
+        raise ValueError(f"unknown gradient groups {unknown} for this model; choose from {sorted(groups)}")
     return wrt
 
 
@@ -225,15 +231,19 @@ def ekf_dense_marginal_log_prob_and_grad(params, emissions, t_emissions=None,
     memory runs in several launches, with the same result bit for bit.  fp64, state_order first / second, num_iter = 1.
     A LearnableUserDrift with differentiable=True gets its gradient under "theta": the variant library built with
     build_user_drift(code, grad=True) takes the drift's derivatives from dual-number evaluations of its own device code.
-    A LearnableUserDrift with differentiable=False, the zeroth order and fp32 raise NotImplementedError, mis-shaped
-    parameters ValueError (before any device work).  A LearnableUserEmission raises NotImplementedError."""
-    reject_user_emission(params, "ekf_dense_marginal_log_prob_and_grad")
+    A LearnableUserEmission with differentiable=True gets its parameters' gradient under "phi" ([n_phi] or [N, n_phi]),
+    in place of "emission_weights" / "emission_bias" (asking for those, or for "phi" with a linear emission, raises
+    ValueError): its variant library (build_variant(..., emission_grad=True)) takes the emission's derivatives from
+    dual-number evaluations of its own device code.
+    A LearnableUserDrift or LearnableUserEmission with differentiable=False, the zeroth order and fp32 raise
+    NotImplementedError, mis-shaped parameters ValueError (before any device work)."""
+    check_user_emission_grad(params, "ekf_dense_marginal_log_prob_and_grad")
     drift = params.dynamics.drift
     if type(drift).__name__ == "LearnableUserDrift" and not drift.differentiable:
         raise NotImplementedError("the gradient of a user-defined drift needs LearnableUserDrift(..., differentiable=True), "
                                   "which declares that its device code stays within the dual-number contract "
                                   "(cd_dynamax_b200.build.build_user_drift)")
-    wrt = _parse_wrt(wrt)
+    wrt = _parse_wrt(wrt, is_user_emission(params))
     if E.pick_dtype(emissions) != "f64":
         raise NotImplementedError("gradients are fp64 only")
     if hyperparams.state_order == "zeroth":
@@ -258,7 +268,8 @@ def dense_marginal_log_prob_and_grad(entry, params, emissions, t_emissions, diff
     fields = dict(E.parse_settings(diffeqsolve_settings), **drift_fields, **filter_fields)
     n_theta = int(fields["n_theta"])
     E.classify(N, K, n, m, ins, fields)  # reject mis-shaped parameters before the library is loaded
-    cols = L.grad_cols_ekf(n, m, n_theta)
+    n_phi = fields.get("n_phi")  # a user emission: phi in place of H | d
+    cols = L.grad_cols_ekf(n, m, n_theta) if n_phi is None else L.grad_cols_ekf_ue(n, m, n_theta, n_phi)
     d = L.new_desc()
     d.N, d.K, d.n, d.m, d.solver = 1, K, n, m, int(fields["solver"])
     chunk = _grad_chunk(N, int(L.lib().cdk_scratch_bytes(ctypes.byref(d), entry.encode())))
@@ -267,7 +278,8 @@ def dense_marginal_log_prob_and_grad(entry, params, emissions, t_emissions, diff
         hi = min(N, lo + chunk)
         dev_ins = {}
         try:
-            out = E.run(entry, "f64", hi - lo, K, n, m, _rows(ins, lo, hi, N, theta_core_ndim=1),
+            out = E.run(entry, "f64", hi - lo, K, n, m, _rows(ins, lo, hi, N, theta_core_ndim=1,
+                                                                      core_ndim_override=None if n_phi is None else {L.IN_H: 1}),
                         (L.OUT_LL, L.OUT_GRAD), fields, host_out=(kind != "cuda"), dev_inputs=dev_ins,
                         out_shapes={L.OUT_GRAD: (hi - lo, cols)})
         except L.CdkError as e:
@@ -281,7 +293,8 @@ def dense_marginal_log_prob_and_grad(entry, params, emissions, t_emissions, diff
     g = lambda t: E.from_dev(_sq(t, batched), kind)
     o = n_theta
     blocks = {}
-    for name, shp in (("Sigma", (n, n)), ("H", (m, n)), ("d", (m,)), ("R", (m, m)), ("m0", (n,)), ("P0", (n, n))):
+    emission_blocks = (("H", (m, n)), ("d", (m,))) if n_phi is None else (("phi", (n_phi,)),)
+    for name, shp in (("Sigma", (n, n)),) + emission_blocks + (("R", (m, m)), ("m0", (n,)), ("P0", (n, n))):
         size = int(np.prod(shp))
         blocks[name] = G[:, o:o + size].reshape((N,) + shp)
         o += size
@@ -289,8 +302,8 @@ def dense_marginal_log_prob_and_grad(entry, params, emissions, t_emissions, diff
     if "drift" in wrt:
         grads.update({k: g(v) for k, v in unflatten_theta(G[:, :n_theta], params.dynamics.drift, n).items()})
     for key, val in (("diffusion_coefficient", gL), ("diffusion_cov", gQc), ("emission_cov", blocks["R"]),
-                     ("emission_bias", blocks["d"]), ("emission_weights", blocks["H"]), ("initial_mean", blocks["m0"]),
-                     ("initial_cov", blocks["P0"])):
+                     ("emission_bias", blocks.get("d")), ("emission_weights", blocks.get("H")), ("phi", blocks.get("phi")),
+                     ("initial_mean", blocks["m0"]), ("initial_cov", blocks["P0"])):
         if key in wrt:
             grads[key] = g(val)
     return g(ll), grads

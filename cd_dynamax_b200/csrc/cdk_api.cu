@@ -358,8 +358,9 @@ CDK_DEF(cdk_sample_path_f32, float, ALGO_SAMPLE)
 CDK_DEF(cdk_emission_moments_f64, double, ALGO_EMISSIONS)
 CDK_DEF(cdk_emission_moments_f32, float, ALGO_EMISSIONS)
 
-// Every gradient entry point reads in[CDK_IN_H] as the m x n matrix of a linear emission: a user emission is refused
-// before any other check or launch.
+// The gradient entry points other than cdk_ekf_grad_dense_f64 read in[CDK_IN_H] as the m x n matrix of a linear
+// emission: a user emission is refused before any other check or launch.  cdk_ekf_grad_dense_f64 refuses it only when
+// its gradient unit was compiled without the emission.
 static bool user_emission_grad(const cdk_desc* d) { return d && d->emission_id == CDK_EMISSION_USER; }
 static const char* const kUserEmissionGrad = "a user-defined emission (CDK_EMISSION_USER) has no gradient";
 
@@ -405,7 +406,11 @@ static int dense_grad(int algo, const cdk_desc* d, const void* const* in, void* 
     return fail(code, msg);
   };
   if (!cdk::ekf_grad_dense_fits(*d, sigma)) {
-    if (d->drift_id == CDK_DRIFT_USER)
+    if (d->emission_id == CDK_EMISSION_USER)
+      snprintf(msg, sizeof(msg), "%s: n = %d, m = %d, n_phi = %d, n_theta = %d: the backward working set with the user "
+               "emission's phi and dual copies of [x | phi] exceeds the 227 KB of one CTA (see cdk.h)", me, d->n, d->m,
+               cdk::user_emission_params(d->n, d->m), d->n_theta);
+    else if (d->drift_id == CDK_DRIFT_USER)
       snprintf(msg, sizeof(msg), "%s: n = %d, m = %d, n_theta = %d: the backward working set with the user drift's dual "
                "copy of [x | theta] exceeds the 227 KB of one CTA (see cdk.h)", me, d->n, d->m, d->n_theta);
     else
@@ -447,7 +452,10 @@ int cdk_ekf_grad_dense_f64(const cdk_desc* d, const void* const* in, void* const
     snprintf(msg, sizeof(msg), "%s: %s", me, why);
     return fail(code, msg);
   };
-  if (user_emission_grad(d)) return reject(CDK_E_UNSUPPORTED, kUserEmissionGrad);
+  if (user_emission_grad(d) && !cdk::ekf_grad_has_user_emission())
+    return reject(CDK_E_UNSUPPORTED, "a user-defined emission is differentiated only by a variant library built with "
+                                     "its gradient unit: build_variant(..., emission_grad=True), i.e. "
+                                     "LearnableUserEmission(..., differentiable=True)");
   if (d && (d->reserved[2] & CDK_FLAG_PREDICT_ONLY)) return reject(CDK_E_UNSUPPORTED, "CDK_FLAG_PREDICT_ONLY has no log-likelihood to differentiate");
   if (d && (d->reserved[2] & CDK_FLAG_DIAG_R)) return reject(CDK_E_UNSUPPORTED, "CDK_FLAG_DIAG_R is not supported");
   if (d && d->drift_id == CDK_DRIFT_USER && !cdk::ekf_grad_has_user_drift())

@@ -209,6 +209,8 @@ inline bool fill_rt_tab(int solver, RtTab& t) {
 bool has_user_drift();  // cdk_generic.cu: was this library compiled with CDK_USER_DRIFT_HEADER?
 // cdk_ekfgrad.cu: was its dense gradient compiled with CDK_USER_DRIFT_HEADER (build_user_drift(code, grad=True))?
 bool ekf_grad_has_user_drift();
+// cdk_ekfgrad.cu: ... with CDK_USER_EMISSION_HEADER (build_variant(..., emission_grad=True))?
+bool ekf_grad_has_user_emission();
 bool has_user_emission();             // cdk_generic.cu: ... with CDK_USER_EMISSION_HEADER?
 int user_emission_params(int n, int m);  // cdk_generic.cu: its num_params(n, m), or -1 without a user emission
 

@@ -19,7 +19,10 @@
 // with the registry contractions of cdk_dense.cuh.  The gap after the last observation does not affect the
 // log-likelihood and is not differentiated.  A user drift (CDK_DRIFT_USER, in a variant built with
 // build_user_drift(code, grad=True)) replaces the registry contractions by dual-number evaluations of its own code
-// (eg_user_vjp, cdk_dual.cuh, DESIGN 4.2f); all of that is compiled only under CDK_HAS_USER_DRIFT.
+// (eg_user_vjp, cdk_dual.cuh, DESIGN 4.2f); all of that is compiled only under CDK_HAS_USER_DRIFT.  A user emission
+// (CDK_EMISSION_USER, in a variant built with build_variant(..., emission_grad=True)) re-linearises h at every step's
+// predicted mean and contracts the second derivatives of its own h / jac, again from dual numbers (eg_emission_vjp,
+// DESIGN 4.2h); all of that is compiled only under CDK_HAS_USER_EMISSION.
 //
 // UKF mode (EgArgs::ukf).  The closed-form unscented predict (cdk_generic.cu, ODE_UKFC) replaces the bracketed EKF term
 // by the exact half-trace 0.5 tr(Hess f . sym P) (drift_half_trhp, for every drift whatever state_order says), whose VJP
@@ -31,7 +34,7 @@
 // is carried unchanged across a gap by the symmetric right-hand side, here as in the filter.  The torch reference
 // (oracle/cd_torch_ukf.py) differentiates the unsymmetrised update literally and pins the gradient.
 #include "cdk_dense.cuh"
-#if CDK_HAS_USER_DRIFT
+#if CDK_HAS_USER_DRIFT || CDK_HAS_USER_EMISSION
 #include "cdk_dual.cuh"
 #endif
 
@@ -51,6 +54,12 @@ __host__ __device__ inline int eg_threads(int n, int m) {
 constexpr int EG_DW = 8;
 using EgDual = cdk_dual::Dual<EG_DW>;
 #endif
+#if CDK_HAS_USER_EMISSION
+// Directions seeded per dual evaluation of the user's emission: 4 rather than 8, so that the dual copy of [x | phi] of
+// the range emission to 20 beacons at n = 40 fits in the moment buffers it aliases (DESIGN 4.2h).
+constexpr int EG_EW = 4;
+using EgEDual = cdk_dual::Dual<EG_EW>;
+#endif
 
 // Shared-memory layout (doubles), computed on the host.  A moment state [mu | P] has st = mpoff + n * ldn entries, the
 // layout of generic_filter_kernel.  With m <= n the update's [m x n] buffers alias ODE buffers that are idle then.
@@ -60,6 +69,9 @@ struct EgLay {
   int G, KT, U, GB, SM, L0, LB, SI, SB, RV, ZV, RBV, YV, CLK, total;
 #if CDK_HAS_USER_DRIFT
   int DU, PART, WQ, GV;
+#endif
+#if CDK_HAS_USER_EMISSION
+  int nph, PHI, PHB, ED;
 #endif
   EgLay() = default;
   __host__ __device__ EgLay(const cdk_desc& d, int stages) {
@@ -88,6 +100,20 @@ struct EgLay {
       PART = take(eg_threads(n, m) * EG_DW);
       WQ = take(n);
       GV = take(n);
+    }
+#endif
+#if CDK_HAS_USER_EMISSION
+    // user emission: phi and its cotangent, and the emission's dual scratch ED = [per-thread partial sums | dual x |
+    // dual phi].  ED is needed only after the update VJP, when the four moment buffers YC..ACC are idle until the next
+    // gap reloads them: it aliases them when it fits there, else it is appended.  Aliased, the dual x lies behind the
+    // partial sums (threads * EG_EW >= 128 >= n doubles), so copying mu out of YC into it overwrites nothing unread.
+    nph = PHI = PHB = ED = 0;
+    if (d.emission_id == CDK_EMISSION_USER) {
+      nph = cdk_user_emission::num_params(n, m);
+      PHI = take(nph);
+      PHB = take(nph);
+      const int need = eg_threads(n, m) * EG_EW + (n + nph) * (EG_EW + 1);
+      ED = need <= YB - YC ? YC : take(need);
     }
 #endif
     total = o;
@@ -168,16 +194,50 @@ __device__ void eg_rhs(const Eg& c, const double* y, double* k, double dt) {
   __syncthreads();
 }
 
+#if CDK_HAS_USER_DRIFT || CDK_HAS_USER_EMISSION
+// The chunk loop of the dual-number contractions: the nv directions of the dual copies (dual(v), v < nv; the first nx
+// of them the state's, then the parameters') are seeded W at a time; for each chunk the threads share out the E
+// evaluations, eval(e, c0, fth, acc) adding evaluation e's weighted tangents of the chunk starting at direction c0 to the
+// thread's acc[W] in registers (fth: the chunk holds parameter directions), and one thread per direction adds the
+// per-thread partial sums (part, blockDim.x * W doubles) in thread order and hands the sum to sink(v, s): the result is
+// the same bits from run to run.  The dual copies hold their values on entry.  Ends with a barrier.
+template <int W, class DA, class EV, class SK>
+__device__ __forceinline__ void eg_dual_chunks(DA dual, int nx, int nv, int E, double* part, EV eval, SK sink) {
+  for (int c0 = 0; c0 < nv; c0 += W) {
+    FOR_T(e, nv * W) {
+      const int v = e / W, w = e - v * W;
+      dual(v).d[w] = c0 + w == v ? 1.0 : 0.0;
+    }
+    __syncthreads();
+    const bool fth = c0 + W > nx;
+    double acc[W];
+#pragma unroll
+    for (int w = 0; w < W; ++w) acc[w] = 0.0;
+    for (int e = threadIdx.x; e < E; e += blockDim.x) eval(e, c0, fth, acc);
+#pragma unroll
+    for (int w = 0; w < W; ++w) part[threadIdx.x * W + w] = acc[w];
+    __syncthreads();
+    FOR_T(w, W) {
+      const int v = c0 + w;
+      if (v < nv) {
+        double s = 0.0;
+        for (int t = 0; t < (int)blockDim.x; ++t) s += part[t * W + w];
+        sink(v, s);
+      }
+    }
+  }
+  __syncthreads();
+}
+#endif
+
 #if CDK_HAS_USER_DRIFT
 // The mean and parameter cotangents of eg_rhs_vjp for the user drift, from dual evaluations of its own f / jac / graddiv
 // at the stage input y (J, Jb and outP = J^T As are in place).  With w_q = 0.5 sum_i P_qi a_i ('second' order only):
 //   m_bar_l      = (J^T a)_l + sum_ik Jb_ik dJ_ik/dx_l + sum_q w_q dg_q/dx_l
 //   theta_bar_e += sum_i a_i df_i/dtheta_e + sum_ik Jb_ik dJ_ik/dtheta_e + sum_q w_q dg_q/dtheta_e
 //   P_bar       += 0.5 g(x) a^T
-// The n + n_theta directions (x, then theta) are seeded EG_DW at a time into the CTA's one dual copy of [x | theta];
-// for each chunk the threads share out the evaluations (jac (i, k), f i, graddiv q), each sums its weighted tangents in
-// registers, and one thread per direction adds the per-thread partial sums in thread order: the result is the same bits
-// from run to run.  Ends with a barrier.
+// The n + n_theta directions (x, then theta) are seeded EG_DW at a time into the CTA's one dual copy of [x | theta]
+// (eg_dual_chunks); the threads share out the evaluations jac (i, k), f i and graddiv q.  Ends with a barrier.
 __device__ void eg_user_vjp(const Eg& c, const double* y, const double* ab, const double* Jb, double* out, double* outP,
                             bool second) {
   const EgLay& L = c.L;
@@ -211,52 +271,34 @@ __device__ void eg_user_vjp(const Eg& c, const double* y, const double* ab, cons
     }
   }
   const int nj = n * n, E = nj + n + (second ? n : 0);
-  for (int c0 = 0; c0 < nv; c0 += EG_DW) {
-    FOR_T(e, nv * EG_DW) {
-      const int v = e / EG_DW, w = e - v * EG_DW;
-      xd[v].d[w] = c0 + w == v ? 1.0 : 0.0;
-    }
-    __syncthreads();
-    const bool fth = c0 + EG_DW > n;  // the chunk holds parameter directions: f's tangents enter (its x-tangents are J)
-    double acc[EG_DW];
+  eg_dual_chunks<EG_DW>(
+      [&](int v) -> EgDual& { return xd[v]; }, n, nv, E, part,
+      [&](int e, int c0, bool fth, double(&acc)[EG_DW]) {
+        if (e < nj) {
+          const int i = e / n, k = e - i * n;
+          const EgDual v = cdk_user::jac<EgDual>(td, n, i, k, xd);
+          const double wt = Jb[i * ld + k];
 #pragma unroll
-    for (int w = 0; w < EG_DW; ++w) acc[w] = 0.0;
-    for (int e = threadIdx.x; e < E; e += blockDim.x) {
-      if (e < nj) {
-        const int i = e / n, k = e - i * n;
-        const EgDual v = cdk_user::jac<EgDual>(td, n, i, k, xd);
-        const double wt = Jb[i * ld + k];
+          for (int w = 0; w < EG_DW; ++w) acc[w] += wt * v.d[w];
+        } else if (e < nj + n) {
+          if (!fth) return;  // no parameter direction in the chunk: f's x-tangents are J
+          const int i = e - nj;
+          const EgDual v = cdk_user::f<EgDual>(td, n, i, [&](int j) { return xd[j]; });
+          const double wt = ab[i];
 #pragma unroll
-        for (int w = 0; w < EG_DW; ++w) acc[w] += wt * v.d[w];
-      } else if (e < nj + n) {
-        if (!fth) continue;
-        const int i = e - nj;
-        const EgDual v = cdk_user::f<EgDual>(td, n, i, [&](int j) { return xd[j]; });
-        const double wt = ab[i];
+          for (int w = 0; w < EG_DW; ++w)
+            if (c0 + w >= n) acc[w] += wt * v.d[w];
+        } else {
+          const int q = e - nj - n;
+          const EgDual v = cdk_user::graddiv<EgDual>(td, n, q, xd);
+          const double wt = wq[q];
 #pragma unroll
-        for (int w = 0; w < EG_DW; ++w)
-          if (c0 + w >= n) acc[w] += wt * v.d[w];
-      } else {
-        const int q = e - nj - n;
-        const EgDual v = cdk_user::graddiv<EgDual>(td, n, q, xd);
-        const double wt = wq[q];
-#pragma unroll
-        for (int w = 0; w < EG_DW; ++w) acc[w] += wt * v.d[w];
-      }
-    }
-#pragma unroll
-    for (int w = 0; w < EG_DW; ++w) part[threadIdx.x * EG_DW + w] = acc[w];
-    __syncthreads();
-    FOR_T(w, EG_DW) {
-      const int v = c0 + w;
-      if (v < nv) {
-        double s = 0.0;
-        for (int t = 0; t < (int)blockDim.x; ++t) s += part[t * EG_DW + w];
+          for (int w = 0; w < EG_DW; ++w) acc[w] += wt * v.d[w];
+        }
+      },
+      [&](int v, double s) {
         if (v < n) out[v] += s; else thb[v - n] += s;
-      }
-    }
-  }
-  __syncthreads();
+      });
 }
 #endif
 
@@ -320,47 +362,26 @@ __device__ void eg_rhs_vjp(const Eg& c, const double* y, const double* kb, doubl
 #if CDK_HAS_USER_DRIFT
 // theta_bar_e += sum_p sum_j Fb[p][j] df_j/dtheta_e (X_p) over the np points X (rows of ldn; Fb likewise) for the user
 // drift: dual evaluations of its f with only theta seeded, EG_DW directions at a time, into the CTA's one dual copy of
-// theta; x enters as plain constants.  The per-thread partial sums are added in thread order, as in eg_user_vjp.
-// Ends with a barrier.
+// theta (eg_dual_chunks); x enters as plain constants.  Ends with a barrier.
 __device__ void eg_user_theta(const Eg& c, const double* X, const double* Fb, int np) {
   const EgLay& L = c.L;
   const int n = L.n, ld = L.ldn, nth = L.nth, E = np * n;
   const double* th = c.p(L.TH);
-  double* part = c.p(L.PART);
   double* thb = c.p(L.THB);
   EgDual* td = reinterpret_cast<EgDual*>(c.p(L.DU)) + n;
   FOR_T(v, nth) td[v] = EgDual(th[v]);
   __syncthreads();
-  for (int c0 = 0; c0 < nth; c0 += EG_DW) {
-    FOR_T(e, nth * EG_DW) {
-      const int v = e / EG_DW, w = e - v * EG_DW;
-      td[v].d[w] = c0 + w == v ? 1.0 : 0.0;
-    }
-    __syncthreads();
-    double acc[EG_DW];
+  eg_dual_chunks<EG_DW>(
+      [&](int v) -> EgDual& { return td[v]; }, 0, nth, E, c.p(L.PART),
+      [&](int e, int, bool, double(&acc)[EG_DW]) {
+        const int p = e / n, j = e - p * n;
+        const double* x = X + p * ld;
+        const EgDual v = cdk_user::f<EgDual>(td, n, j, [&](int q) { return EgDual(x[q]); });
+        const double wt = Fb[p * ld + j];
 #pragma unroll
-    for (int w = 0; w < EG_DW; ++w) acc[w] = 0.0;
-    for (int e = threadIdx.x; e < E; e += blockDim.x) {
-      const int p = e / n, j = e - p * n;
-      const double* x = X + p * ld;
-      const EgDual v = cdk_user::f<EgDual>(td, n, j, [&](int q) { return EgDual(x[q]); });
-      const double wt = Fb[p * ld + j];
-#pragma unroll
-      for (int w = 0; w < EG_DW; ++w) acc[w] += wt * v.d[w];
-    }
-#pragma unroll
-    for (int w = 0; w < EG_DW; ++w) part[threadIdx.x * EG_DW + w] = acc[w];
-    __syncthreads();
-    FOR_T(w, EG_DW) {
-      const int v = c0 + w;
-      if (v < nth) {
-        double s = 0.0;
-        for (int t = 0; t < (int)blockDim.x; ++t) s += part[t * EG_DW + w];
-        thb[v] += s;
-      }
-    }
-  }
-  __syncthreads();
+        for (int w = 0; w < EG_DW; ++w) acc[w] += wt * v.d[w];
+      },
+      [&](int v, double s) { thb[v] += s; });
 }
 #endif
 
@@ -556,9 +577,59 @@ __device__ void eg_step_vjp(const Eg& c, double dt, const double* __restrict__ s
   __syncthreads();
 }
 
+#if CDK_HAS_USER_EMISSION
+// The user emission's part of the update VJP at the predicted mean mu (YC), once the linear update VJP has run with
+// H = J(mu) and r = y - h(mu): HB holds this step's cotangent Hb of J(mu), RBV the residual's r_bar.  Then
+//   mu_bar_l  += sum_aj Hb_aj dJ_aj/dx_l                      (-sum_a r_bar_a J_al is the linear VJP's -H^T r_bar)
+//   phi_bar_e += sum_aj Hb_aj dJ_aj/dphi_e - sum_a r_bar_a dh_a/dphi_e
+// from dual evaluations of the user's jac (a, j) and h (a), the n + n_phi directions (x, then phi) seeded EG_EW at a time
+// (eg_dual_chunks); h enters only chunks that hold phi directions, its x-tangents being J.  Ends with a barrier.
+__device__ void eg_emission_vjp(const Eg& c) {
+  const EgLay& L = c.L;
+  const int n = L.n, m = L.m, ld = L.ldn, nph = L.nph, nj = m * n;
+  const double* mu = c.p(L.YC);
+  const double* phi = c.p(L.PHI);
+  const double* Hb = c.p(L.HB);
+  const double* rb = c.p(L.RBV);
+  double* mub = c.p(L.YB);
+  double* phb = c.p(L.PHB);
+  double* part = c.p(L.ED);
+  EgEDual* xd = reinterpret_cast<EgEDual*>(part + eg_threads(n, m) * EG_EW);
+  EgEDual* pd = xd + n;
+  FOR_T(v, n) xd[v] = EgEDual(mu[v]);  // before pd, which may overwrite YC
+  __syncthreads();
+  FOR_T(v, nph) pd[v] = EgEDual(phi[v]);
+  __syncthreads();
+  eg_dual_chunks<EG_EW>(
+      [&](int v) -> EgEDual& { return v < n ? xd[v] : pd[v - n]; }, n, n + nph, nj + m, part,
+      [&](int e, int c0, bool fth, double(&acc)[EG_EW]) {
+        if (e < nj) {
+          const int a = e / n, j = e - a * n;
+          const EgEDual v = cdk_user_emission::jac<EgEDual>(pd, n, m, a, j, xd);
+          const double wt = Hb[a * ld + j];
+#pragma unroll
+          for (int w = 0; w < EG_EW; ++w) acc[w] += wt * v.d[w];
+        } else {
+          if (!fth) return;  // no parameter direction in the chunk
+          const int a = e - nj;
+          const EgEDual v = cdk_user_emission::h<EgEDual>(pd, n, m, a, [&](int q) { return xd[q]; });
+          const double wt = -rb[a];
+#pragma unroll
+          for (int w = 0; w < EG_EW; ++w)
+            if (c0 + w >= n) acc[w] += wt * v.d[w];
+        }
+      },
+      [&](int v, double s) {
+        if (v < n) mub[v] += s; else phb[v - n] += s;
+      });
+}
+#endif
+
 // VJP of the measurement update (condition_on, num_iter = 1, then the symmetrisation) at the predicted moments in YC for
 // the emission in YV: YB holds the cotangent of the filtered moments on entry and of the predicted ones on exit, plus
-// the log-density's own derivative.  Accumulates H_bar, d_bar, R_bar.
+// the log-density's own derivative.  Accumulates H_bar, d_bar, R_bar.  A user emission (ue) runs the same VJP with
+// H = J(mu) and r = y - h(mu), recomputed by the filter's code; its H_bar is this step's alone (J moves with mu), the
+// terms of H mu + d are dropped, and eg_emission_vjp contracts H_bar and r_bar with the emission's derivatives.
 __device__ void eg_update_vjp(const Eg& c) {
   const EgLay& L = c.L;
   const int n = L.n, m = L.m, ldn = L.ldn, ldm = L.ldm;
@@ -583,6 +654,20 @@ __device__ void eg_update_vjp(const Eg& c) {
   double* zv = c.p(L.ZV);
   double* rb = c.p(L.RBV);
   double* W1 = c.p(L.W1);
+  const bool ue = user_emission(c.g.k.d);
+#if CDK_HAS_USER_EMISSION
+  if (ue) {  // H = J(mu) as condition_on computes it; this step's H_bar starts from zero
+    double* Hw = c.p(L.H);
+    double* HBw = c.p(L.HB);
+    const double* phi = c.p(L.PHI);
+    FOR_T(e, m * n) {
+      const int a = e / n, j = e - a * n;
+      Hw[a * ldn + j] = user_h_jac<double>(phi, n, m, a, j, mu);
+      HBw[a * ldn + j] = 0.0;
+    }
+    __syncthreads();
+  }
+#endif
   FOR_T(e, n * n) {  // the filter symmetrises P_f
     const int i = e / n, j = e - i * n;
     if (i < j) {
@@ -593,8 +678,16 @@ __device__ void eg_update_vjp(const Eg& c) {
   }
   mm_dmma<double, false, false>(H, ldn, P, ldn, m, n, n, [&](int a, int j, double v) { G[a * ldn + j] = v; });
   FOR_T(a, m) {
-    double s = dv[a];
-    for (int q = 0; q < n; ++q) s += H[a * ldn + q] * mu[q];
+    double s;
+#if CDK_HAS_USER_EMISSION
+    if (ue) {
+      s = user_h<double>(c.p(L.PHI), n, m, a, [&](int j) { return mu[j]; });
+    } else
+#endif
+    {
+      s = dv[a];
+      for (int q = 0; q < n; ++q) s += H[a * ldn + q] * mu[q];
+    }
     rv[a] = yv[a] - s;
   }
   __syncthreads();
@@ -642,11 +735,11 @@ __device__ void eg_update_vjp(const Eg& c) {
   mm_dmma<double, false, false>(Sb, ldm, G, ldn, m, n, m, [&](int a, int j, double v) { HBg[a * ldn + j] += 2.0 * v; });
   __syncthreads();
   mm_dmma<double, false, false>(Gb, ldn, P, ldn, m, n, n, [&](int a, int j, double v) {
-    HBg[a * ldn + j] += v - rb[a] * mu[j];
+    HBg[a * ldn + j] += ue ? v : v - rb[a] * mu[j];
   });
   mm_dmma<double, false, false>(Sb, ldm, H, ldn, m, n, m, [&](int a, int j, double v) { U[a * ldn + j] = v + Gb[a * ldn + j]; });
   double* DBg = c.p(L.DB);
-  FOR_T(a, m) DBg[a] -= rb[a];
+  if (!ue) FOR_T(a, m) DBg[a] -= rb[a];
   FOR_T(l, n) {  // mu_bar = mu_f_bar - H^T r_bar
     double s = 0.0;
     for (int a = 0; a < m; ++a) s += H[a * ldn + l] * rb[a];
@@ -660,6 +753,9 @@ __device__ void eg_update_vjp(const Eg& c) {
     Pb[i * ldn + j] += 0.5 * (W1[i * ldn + j] + W1[j * ldn + i]);
   }
   __syncthreads();
+#if CDK_HAS_USER_EMISSION
+  if (ue) eg_emission_vjp(c);
+#endif
 }
 
 __device__ void eg_load(double* dst, const double* __restrict__ src, int st) {
@@ -688,8 +784,16 @@ __device__ __forceinline__ void eg_body(const EgArgs& g, double* smem) {
   auto src = [&](int slot) { return a.in[slot] + traj * a.in_stride[slot]; };
   {  // model: theta, H, R, d and L Qc L^T (J, W1, W2 as scratch)
     FOR_T(i, L.nth) c.p(L.TH)[i] = src(CDK_IN_F)[i];
+#if CDK_HAS_USER_EMISSION
+    if (user_emission(d)) {  // phi from the H slot (n_phi per trajectory); d is not read
+      FOR_T(i, L.nph) c.p(L.PHI)[i] = src(CDK_IN_H)[i];
+    } else
+#endif
     FOR_T(e, m * n) c.p(L.H)[(e / n) * ldn + e % n] = src(CDK_IN_H)[e];
     FOR_T(e, m * m) c.p(L.R)[(e / m) * ldm + e % m] = src(CDK_IN_R)[e];
+#if CDK_HAS_USER_EMISSION
+    if (!user_emission(d))
+#endif
     FOR_T(i, m) c.p(L.DV)[i] = src(CDK_IN_D)[i];
     double* Lm = c.p(L.J);
     double* Qc = c.p(L.W1);
@@ -800,7 +904,7 @@ __device__ __forceinline__ void eg_body(const EgArgs& g, double* smem) {
     __syncthreads();
     eg_update_vjp(c);
   }
-  // ---- gradient row: theta | Sigma (sym) | H | d | R (sym) | m0 | P0 (sym) ----
+  // ---- gradient row: theta | Sigma (sym) | H | d | R (sym) | m0 | P0 (sym); a user emission: phi in place of H | d ----
   const double* sigb = c.p(L.SIGB);
   const double* HB = c.p(L.HB);
   const double* RB = c.p(L.RB);
@@ -811,6 +915,9 @@ __device__ __forceinline__ void eg_body(const EgArgs& g, double* smem) {
   double* gH = gS + n * n;
   double* gd = gH + m * n;
   double* gR = gd + m;
+#if CDK_HAS_USER_EMISSION
+  if (user_emission(d)) gR = gH + L.nph;
+#endif
   double* gm0 = gR + m * m;
   double* gP0 = gm0 + n;
   FOR_T(e, n * n) {
@@ -818,8 +925,15 @@ __device__ __forceinline__ void eg_body(const EgArgs& g, double* smem) {
     gS[e] = 0.5 * (sigb[i * ldn + j] + sigb[j * ldn + i]);
     gP0[e] = 0.5 * (yb[L.mpoff + i * ldn + j] + yb[L.mpoff + j * ldn + i]);
   }
-  FOR_T(e, m * n) gH[e] = HB[(e / n) * ldn + e % n];
-  FOR_T(i, m) gd[i] = c.p(L.DB)[i];
+#if CDK_HAS_USER_EMISSION
+  if (user_emission(d)) {
+    FOR_T(e, L.nph) gH[e] = c.p(L.PHB)[e];
+  } else
+#endif
+  {
+    FOR_T(e, m * n) gH[e] = HB[(e / n) * ldn + e % n];
+    FOR_T(i, m) gd[i] = c.p(L.DB)[i];
+  }
   FOR_T(e, m * m) {
     const int i = e / m, j = e - i * m;
     gR[e] = 0.5 * (RB[i * ldm + j] + RB[j * ldm + i]);
@@ -860,6 +974,7 @@ bool ekf_grad_dense_fits(const cdk_desc& d, bool sigma) {
 }
 
 bool ekf_grad_has_user_drift() { return CDK_HAS_USER_DRIFT != 0; }
+bool ekf_grad_has_user_emission() { return CDK_HAS_USER_EMISSION != 0; }
 
 long long ekf_grad_dense_scratch_doubles(const cdk_desc& d) {
   EgLay lay;
@@ -882,6 +997,9 @@ int launch_ekf_grad_dense(const KArgs<double>& a, const int* status, double* gra
   g.status = status;
   g.grad = grad;
   g.cols = CDK_GRAD_COLS_EKF(a.d.n, a.d.m, a.d.n_theta);
+#if CDK_HAS_USER_EMISSION
+  if (user_emission(a.d)) g.cols = CDK_GRAD_COLS_EKF_UE(a.d.n, a.d.m, a.d.n_theta, g.lay.nph);
+#endif
   g.ukf = ukf || sigma ? 1 : 0;
   const int threads = eg_threads(a.d.n, a.d.m);
   const size_t smem = (size_t)eg_smem_doubles(g.lay, sigma) * sizeof(double);

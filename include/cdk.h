@@ -198,8 +198,9 @@ CDK_DECL(cdk_ukf_filter_f32);
 CDK_DECL(cdk_enkf_filter_f64);
 CDK_DECL(cdk_enkf_filter_f32);
 /* The gradient entry points below (cdk_ekf_grad_f64, cdk_kf_grad_f64, cdk_ekf_grad_dense_f64, cdk_ukf_grad_dense_f64,
- * cdk_ukf_grad_sigma_f64) differentiate the linear emission only: the nonlinear ones return CDK_E_UNSUPPORTED for
- * CDK_EMISSION_USER before any other check.
+ * cdk_ukf_grad_sigma_f64) differentiate the linear emission.  cdk_ekf_grad_dense_f64 also differentiates CDK_EMISSION_USER
+ * in a variant whose gradient unit was compiled with the emission (build_variant(..., emission_grad=True)); everywhere
+ * else the nonlinear entry points return CDK_E_UNSUPPORTED for CDK_EMISSION_USER before any other check.
  *
  * Log-likelihood (out[CDK_OUT_LL]) and its gradient with respect to the model parameters (out[CDK_OUT_GRAD],
  * [N, CDK_GRAD_COLS_L63]) of the CD-EKF: what jax.value_and_grad(marginal_log_prob) hands the reference's fit_sgd
@@ -251,6 +252,16 @@ CDK_DECL(cdk_kf_grad_f64);
  * fits with every solver) -- all host-side checks, before any CUDA call.
  * CDK_GRAD_COLS_EKF is shared with cdk_ukf_grad_dense_f64, whose rows have the same layout. */
 #define CDK_GRAD_COLS_EKF(n, m, n_theta) ((n_theta) + 2 * (n) * (n) + (m) * (n) + (m) * (m) + (n) + (m))
+/* CDK_EMISSION_USER in a variant built with build_variant(..., emission_grad=True) (LearnableUserEmission(...,
+ * differentiable=True)): the emission is re-linearised at every step's predicted mean, as the filter does, and the
+ * second derivatives of the user's h / jac come from dual-number evaluations of its own code (DESIGN 4.2h).  The row is
+ * theta | Sigma | phi (n_phi) | R | m0 | P0: phi takes the place of H | d (for the linear emission written as user
+ * code, phi = [H | d] and the row has the stock layout).  The shared memory adds phi, its cotangent and the dual copies
+ * of [x | phi] (aliasing the moment buffers when they fit there); an n_phi that does not fit returns CDK_E_SIZE naming
+ * n_phi (registry drifts; n = 40, m = 20: n_phi <= 1,099; n = 2, m = 1: n_phi <= 4,070).  A drift may be a registry drift or a
+ * differentiable CDK_DRIFT_USER.  The stock library and a variant whose gradient unit lacks the emission reject
+ * CDK_EMISSION_USER with CDK_E_UNSUPPORTED before any other check. */
+#define CDK_GRAD_COLS_EKF_UE(n, m, n_theta, n_phi) ((n_theta) + 2 * (n) * (n) + (n_phi) + (m) * (m) + (n))
 CDK_DECL(cdk_ekf_grad_dense_f64);
 /* Log-likelihood (out[CDK_OUT_LL]), status (out[CDK_OUT_STATUS]) and reverse-mode gradient (out[CDK_OUT_GRAD],
  * [N, CDK_GRAD_COLS_EKF(n, m, n_theta)], the row layout of cdk_ekf_grad_dense_f64) of the CD-UKF for every registry
